@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the FMT motion-latent sampling path (BASELINE.json metric: motion-latent frames/s, FMT, nfe=10).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--frames T]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--frames T] [--dump-outputs DIR]
 
 One "step" = one sampler call (= ``_perform_ode_sampling_loop``) over one batch of synthetic clips:
 ``ceil(T/50)`` windows x ``nfe-1`` Euler steps x 3-way CFG.  Default workload = BASELINE.json configs[1]:
@@ -18,6 +18,10 @@ frames in total, 256/N clips per GPU (strong scaling of a fixed job, tensor-pipe
 
 The product arm imports nothing from ``oracle/``: the seeded synthetic weights and inputs come from the package's ``synth``
 module; ``oracle/`` is executed by the baseline legs alone (``cpu_baseline``, ``gpu_eager_baseline``, ``--impl reference``).
+
+``--dump-outputs DIR`` writes the motion latents the timed path returned in its last timed step to ``DIR/r_d.npy`` (float32,
+(clips, frames, dim_w); with N GPUs the gathered latents of all ranks; ``--impl reference``: the first window's frames).  Weights,
+inputs and noise are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -34,6 +38,20 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 NFE, A_CFG, E_CFG, R_CFG = 10, 2.0, 1.0, 1.0
+DUMP_BYTES = 60_000_000          # --dump-outputs stays below 64 MB including the .npy header
+
+
+def dump_outputs(out_dir, r_d):
+    """Writes ``r_d`` as ``out_dir/r_d.npy`` (float32).  Latents larger than DUMP_BYTES are cut to a fixed sample of their
+    frame rows (seed 0, kept in row order), shape (rows, dim_w), so that runs with the same arguments stay comparable."""
+    import numpy as np
+    r_d = r_d.detach().float().cpu()
+    rows = r_d.reshape(-1, r_d.shape[-1])
+    keep = DUMP_BYTES // (4 * rows.shape[1])
+    if rows.shape[0] > keep:
+        r_d = rows[torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "r_d.npy"), r_d.contiguous().numpy())
 
 
 def peaks():
@@ -221,8 +239,9 @@ def measure_handoff(pkg, model, dims, B, T, dev, iters=10):
     return out
 
 
-def measure_product(pkg, be, model, dims, B, T, rank, world, dev, dist, steps, warmup, e2e_iters):
-    """Times the product path on this rank's B clips x T frames: resident (CUDA events) and end to end (node, CPU tensors)."""
+def measure_product(pkg, be, model, dims, B, T, rank, world, dev, dist, steps, warmup, e2e_iters, keep_output=False):
+    """Times the product path on this rank's B clips x T frames: resident (CUDA events) and end to end (node, CPU tensors).
+    With ``keep_output`` the result's ``output`` holds the latents of the last timed resident step (gathered over ranks), on the CPU."""
     L = dims.frames_per_clip
     n_win = math.ceil(T / L)
     be.configure(B, 3, False, NFE, "euler", "bf16")
@@ -281,6 +300,7 @@ def measure_product(pkg, be, model, dims, B, T, rank, world, dev, dist, steps, w
     be.launch_count(reset=True)
     t_res = timed(step_resident, steps)
     launches = be.launch_count(reset=True)
+    output = (gathered if world > 1 else out_d).cpu() if keep_output else None
     for _ in range(min(3, warmup)):
         step_e2e()
     t_e2e = timed(step_e2e, e2e_iters, wall=True)        # host-visible latency: the call returns a CPU tensor
@@ -289,7 +309,7 @@ def measure_product(pkg, be, model, dims, B, T, rank, world, dev, dist, steps, w
     d2h = B * T * dims.dim_w * 4
     del flush, gathered, out_d, noise_d
     return dict(t_step=t_res / steps, t_e2e=t_e2e / e2e_iters, launches=int(launches), clocks=clk, h2d=h2d, d2h=d2h, n_win=n_win,
-                window_kernel=be.window_kernel_status())
+                window_kernel=be.window_kernel_status(), output=output)
 
 
 def roofline_record(dims, B, T, t_step, n_win, pk):
@@ -329,7 +349,10 @@ def main():
     ap.add_argument("--large-clips", type=int, default=256, help="total clips of the large_batch record (configs[3]); 0 = skip it")
     ap.add_argument("--large-frames", type=int, default=200)
     ap.add_argument("--force-port", action="store_true", help="reference arm: time the oracle port even when the reference copy exists")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the latents of the last timed step to DIR/r_d.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -364,8 +387,12 @@ def main():
             run(r_s, wa[:, :frames], we, frames, 15)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            run(r_s, wa[:, :frames], we, frames, 15)
+            r_d = run(r_s, wa[:, :frames], we, frames, 15)
         el = time.perf_counter() - t0
+        if args.dump_outputs:
+            # whether a step covers the whole clip or its first window depends on this host's speed: dump the first window,
+            # which both compute alike, so that the file's shape follows from the arguments
+            dump_outputs(args.dump_outputs, r_d[:, :L])
         v = args.steps * B * frames / el
         print(json.dumps(dict(impl="reference", metric="motion-latent frames/s (FMT, nfe=10)", value=v, unit="frames/s", n_gpus=args.gpus,
                               steps=args.steps, warmup=args.warmup, ms_per_step=1e3 * el / args.steps, higher_is_better=True, scaling="weak",
@@ -390,7 +417,8 @@ def main():
     be = pkg.backend_for(model, dev)
     pk = peaks()
 
-    m = measure_product(pkg, be, model, dims, B, T, rank, world, dev, dist, args.steps, max(3, args.warmup), max(10, args.steps // 4))
+    m = measure_product(pkg, be, model, dims, B, T, rank, world, dev, dist, args.steps, max(3, args.warmup), max(10, args.steps // 4),
+                        keep_output=bool(args.dump_outputs) and rank == 0)
     graph_nodes = be.graph_kernel_nodes()
 
     # ---- configs[3]: a fixed job of 256 clips x 200 frames split over the GPUs (strong scaling; tensor-pipe regime)
@@ -433,6 +461,8 @@ def main():
         res["cpu_baseline"] = time_cpu_baseline(W, dims, B, T, budget_s=25.0)
         if B <= 32:
             res["gpu_eager_baseline"] = time_gpu_eager_baseline(W, dims, B, T, dev)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, m["output"])
     print(json.dumps(res))
     if world > 1:
         dist.destroy_process_group()

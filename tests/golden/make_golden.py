@@ -1,6 +1,6 @@
 """Generate the committed golden fixtures by running the REAL reference in this container.
 
-    python tests/golden/make_golden.py            # writes tests/golden/*.npz + manifest.json
+    python tests/golden/make_golden.py            # writes tests/golden/*.npz + manifest.json + node_surface.json
 
 The reference (``/root/reference/src/nodes``) is imported in place through ``refshim.py`` and
 fed the seeded synthetic weights / inputs from ``oracle/synth.py``; its node entry points are
@@ -58,6 +58,26 @@ CASES = {
     "proj_stacked": dict(entry="proj", dims="full", B=2, T=37, in_dim=9216, seed=60),
     "proj_last": dict(entry="proj", dims="full", B=1, T=100, in_dim=768, seed=61),
 }
+
+
+# node_surface.json: what a saved ComfyUI workflow depends on in the three sampler nodes (class name -> reference module)
+NODE_SURFACE = {"FloatSampleMotionSequenceRD_VA": "nodes_vadv", "FloatSampleMotionSequenceRD": "nodes_adv", "FloatProcess": "nodes"}
+SURFACE_FIELDS = ("default", "min", "max", "step", "forceInput")
+
+
+def node_surface(cls) -> dict:
+    """UNIQUE_NAME, FUNCTION, RETURN_TYPES and, in order, [name, type or enum, {default/min/max/step/forceInput}] of every
+    INPUT_TYPES()["required"] entry, as plain JSON values."""
+    req = cls.INPUT_TYPES()["required"]
+    rows = [[k, v[0], {f: v[1][f] for f in SURFACE_FIELDS if len(v) > 1 and f in v[1]}] for k, v in req.items()]
+    return json.loads(json.dumps(dict(UNIQUE_NAME=cls.UNIQUE_NAME, FUNCTION=cls.FUNCTION, RETURN_TYPES=list(cls.RETURN_TYPES), required=rows)))
+
+
+def write_node_surface():
+    refshim.load_reference()
+    surface = {name: node_surface(getattr(importlib.import_module("refnodes." + mod), name)) for name, mod in NODE_SURFACE.items()}
+    surface["_meta"] = dict(source="the reference's node classes, imported in place via tests/golden/refshim.py")
+    json.dump(surface, open(os.path.join(HERE, "node_surface.json"), "w"), indent=1)
 
 
 def dims_of(rec):
@@ -176,6 +196,8 @@ def main():
                              inputs="oracle.synth.synth_inputs(dims, B, T_wa or T, seed=100 + seed % 1000, ...)",
                              reference="/root/reference v1.1.2, imported in place via tests/golden/refshim.py")
     json.dump(manifest, open(manifest_path, "w"), indent=1, sort_keys=True)
+    if not only or "node_surface" in only:
+        write_node_surface()
 
 
 if __name__ == "__main__":

@@ -174,24 +174,18 @@ def test_node_surface_matches_reference(pkg):
     assert list(ap.INPUT_TYPES()["optional"]) == ["keep_on_device"] and ap.INPUT_TYPES()["optional"]["keep_on_device"][1]["default"] is False
 
 
-@pytest.mark.refimpl
 def test_required_inputs_equal_the_reference_classes(pkg):
-    """INPUT_TYPES()["required"] of the three sampler nodes, compared entry by entry with the reference's own classes."""
-    import importlib
-    from oracle import refshim
-    refshim.load_reference()
-    pairs = [(pkg.FloatSampleMotionSequenceRD_VA, importlib.import_module("refnodes.nodes_vadv").FloatSampleMotionSequenceRD_VA),
-             (pkg.FloatSampleMotionSequenceRD, importlib.import_module("refnodes.nodes_adv").FloatSampleMotionSequenceRD),
-             (pkg.FloatProcess, importlib.import_module("refnodes.nodes").FloatProcess)]
-    for ours, ref in pairs:
-        a, b = ours.INPUT_TYPES()["required"], ref.INPUT_TYPES()["required"]
-        assert list(a) == list(b), ours.__name__
-        for k in a:
-            assert a[k][0] == b[k][0], (ours.__name__, k)                              # type / enum
-            da, db = (a[k][1] if len(a[k]) > 1 else {}), (b[k][1] if len(b[k]) > 1 else {})
-            for f in ("default", "min", "max", "step", "forceInput"):
-                assert da.get(f) == db.get(f), (ours.__name__, k, f)
-        assert ours.RETURN_TYPES == ref.RETURN_TYPES and ours.FUNCTION == ref.FUNCTION and ours.UNIQUE_NAME == ref.UNIQUE_NAME
+    """INPUT_TYPES()["required"] of the three sampler nodes, compared entry by entry with the reference's own classes as stored in
+    tests/golden/node_surface.json (type / enum, default, min, max, step, forceInput; RETURN_TYPES, FUNCTION, UNIQUE_NAME)."""
+    import json
+    from golden.make_golden import NODE_SURFACE, node_surface
+    want = json.load(open(os.path.join(cases.GOLDEN_DIR, "node_surface.json")))
+    for name in NODE_SURFACE:
+        ours, ref = node_surface(getattr(pkg, name)), want[name]
+        assert [r[0] for r in ours["required"]] == [r[0] for r in ref["required"]], name
+        for a, b in zip(ours["required"], ref["required"]):
+            assert a == b, (name, a, b)
+        assert (ours["RETURN_TYPES"], ours["FUNCTION"], ours["UNIQUE_NAME"]) == (ref["RETURN_TYPES"], ref["FUNCTION"], ref["UNIQUE_NAME"]), name
 
 
 def test_precision_mode_resolution(pkg, monkeypatch):
