@@ -7,9 +7,11 @@ from .build import LIB_PATH
 FMT_W_NUM_GLOBAL = 13
 FMT_W_PER_BLOCK = 10
 FMT_LOC_DEVICE, FMT_LOC_HOST = 0, 1
-FMT_MODE_BF16, FMT_MODE_FP32_VALIDATE = 0, 1
+FMT_MODE_BF16, FMT_MODE_FP32_VALIDATE, FMT_MODE_BF16X3 = 0, 1, 2
+# precision-mode names of sampler.PRECISION_MODES -> FmtPlan.mode / fmt_proj_apply's mode
+MODE_IDS = {"bf16": FMT_MODE_BF16, "fp32": FMT_MODE_FP32_VALIDATE, "bf16x3": FMT_MODE_BF16X3}
 FMT_MAX_STAGES = 4
-FMT_ABI_VERSION = 1
+FMT_ABI_VERSION = 2
 
 # state-dict key order expected by fmt_create (include/fmt_b200.h enums)
 GLOBAL_KEYS = [
@@ -74,6 +76,9 @@ _SIGNATURES = {
     "fmt_proj_launch_count": (C.c_int64, [C.c_void_p, C.c_int32]),
     "fmt_debug_gemm_bf16": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "fmt_debug_gemm_bench": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "fmt_debug_gemm_bf16x3": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "fmt_debug_gemm_bench_bf16x3": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                                C.c_void_p]),
     "fmt_debug_gemm_fp32": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
 }
 

@@ -16,7 +16,7 @@ from . import _cabi
 from ._cabi import FmtError, check
 
 logger = logging.getLogger("FLOAT_Optimized.b200_fmt")
-_MODES = {"bf16": _cabi.FMT_MODE_BF16, "fp32": _cabi.FMT_MODE_FP32_VALIDATE}
+_MODES = _cabi.MODE_IDS      # "bf16x3" needs in_dim % 64 == 0 (9216 and 768 are)
 
 
 class AudioProjectionBackend:

@@ -1,8 +1,8 @@
 // libfmt_b200.so - host side of the C ABI declared in include/fmt_b200.h.
 //
-// Owns: the packed weights (bf16 for the tcgen05 path + fp32 for the validation mode), the workspace, the per-plan
-// CUDA graph of one sampling window, and the window loop of _perform_ode_sampling_loop (nodes_adv.py:545-694),
-// which runs entirely on the device: windows are chained through prev_x / prev_wa / prev_we without host syncs.
+// Owns: the packed weights (bf16 for the tcgen05 path, fp32 for the validation mode, bf16x3 pairs once a plan selects that
+// mode), the workspace, the per-plan CUDA graph of one sampling window, and the window loop of _perform_ode_sampling_loop
+// (nodes_adv.py:545-694), which runs entirely on the device: windows are chained through prev_x / prev_wa / prev_we without host syncs.
 #include "../../include/fmt_b200.h"
 #include "kernels.cuh"
 #include "window.cuh"
@@ -55,6 +55,7 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
 struct Linear {
   bf16* w16 = nullptr;    // (N, K) bf16, K possibly padded
   float* w32 = nullptr;   // (N, K) fp32 (validation mode)
+  bf16* w3 = nullptr;     // (N, 2K) bf16x3 pairs (gemm.cuh), packed from w32 the first time a plan or projection selects FMT_MODE_BF16X3
   float* b = nullptr;     // (N)
   int N = 0, K = 0;
 };
@@ -195,33 +196,37 @@ static int make_tmap_ex(FmtHandle* h, CUtensorMap* m, const void* ptr, CUtensorM
   return 0;
 }
 
-template <int BN>
+// SPLIT (FMT_MODE_BF16X3): A and W are pair matrices (gemm.cuh), lda / ldw / K count logical columns; the tensor maps cover the
+// 2K bf16 columns of their rows.  Gate tables are fp32 in that mode.
+template <int BN, bool SPLIT>
 static int launch_tc(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ldw, const EpiParams& ep, int K, cudaStream_t st) {
-  using C = TcCfg<BN>;
+  using C = TcCfg<BN, SPLIT>;
+  const auto kern = gemm_tc_kernel<BN, typename std::conditional<SPLIT, float, bf16>::type, SPLIT>;
   static bool attr_set[64] = {};
   if (!attr_set[h->device & 63]) {   // per device: the attribute lives in the device's module image
-    CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<BN, bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
+    CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
     attr_set[h->device & 63] = true;
   }
   CUtensorMap ta, tb;
-  FMT_OK(make_tmap(h, &ta, A, ep.M, K, lda, C::BM));
-  FMT_OK(make_tmap(h, &tb, W, ep.N, K, ldw, BN));
+  FMT_OK(make_tmap(h, &ta, A, ep.M, K * C::HALVES, lda * C::HALVES, C::BM));
+  FMT_OK(make_tmap(h, &tb, W, ep.N, K * C::HALVES, ldw * C::HALVES, BN));
   const int tiles = ((ep.M + C::BM - 1) / C::BM) * ((ep.N + BN - 1) / BN);
   const int grid = tiles < h->num_sms ? tiles : h->num_sms;
-  return launch(h, gemm_tc_kernel<BN, bf16>, dim3(grid), dim3(C::THREADS), C::SMEM_BYTES, st, 1, ta, tb, ep, K);
+  return launch(h, kern, dim3(grid), dim3(C::THREADS), C::SMEM_BYTES, st, 1, ta, tb, ep, K);
 }
 
-template <int BN>
+template <int BN, bool SPLIT>
 static int launch_tc2(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ldw, const EpiParams& ep, int K, cudaStream_t st, int ksplit = 1) {
-  using C = Tc2Cfg<BN>;
+  using C = Tc2Cfg<BN, SPLIT>;
+  const auto kern = gemm_tc2_kernel<BN, typename std::conditional<SPLIT, float, bf16>::type, SPLIT>;
   static bool attr_set[64] = {};
   if (!attr_set[h->device & 63]) {
-    CUDA_OK(cudaFuncSetAttribute(gemm_tc2_kernel<BN, bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
+    CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
     attr_set[h->device & 63] = true;
   }
   CUtensorMap ta, tb;
-  FMT_OK(make_tmap(h, &ta, A, ep.M, K, lda, C::BMH));
-  FMT_OK(make_tmap(h, &tb, W, ep.N, K, ldw, BN / 2));
+  FMT_OK(make_tmap(h, &ta, A, ep.M, K * C::HALVES, lda * C::HALVES, C::BMH));
+  FMT_OK(make_tmap(h, &tb, W, ep.N, K * C::HALVES, ldw * C::HALVES, BN / 2));
   const int tiles = ((ep.M + C::BM - 1) / C::BM) * ((ep.N + BN - 1) / BN) * ((ksplit > 1 && ep.kind == EPI_GATE_RES) ? ksplit : 1);
   const int max_pairs = h->num_sms / 2;
   const int pairs = tiles < max_pairs ? tiles : max_pairs;
@@ -229,7 +234,7 @@ static int launch_tc2(FmtHandle* h, const bf16* A, int lda, const bf16* W, int l
   ep2.raster_gm = h->raster_gm;
   ep2.ksplit = (ksplit > 1 && ep.kind == EPI_GATE_RES) ? ksplit : 1;
   // the kernel carries __cluster_dims__(2,1,1); launch() only adds the PDL attribute
-  return launch(h, gemm_tc2_kernel<BN, bf16>, dim3(2 * pairs), dim3(C::THREADS), C::SMEM_BYTES, st, 1, ta, tb, ep2, K);
+  return launch(h, kern, dim3(2 * pairs), dim3(C::THREADS), C::SMEM_BYTES, st, 1, ta, tb, ep2, K);
 }
 
 static int pick_bn(const FmtHandle* h, int M, int N) {
@@ -239,11 +244,14 @@ static int pick_bn(const FmtHandle* h, int M, int N) {
   return 64;
 }
 
+// SPLIT: the bf16x3 GEMM on pair operands (FMT_MODE_BF16X3): K % 64 == 0, never K-sliced (its results stay bitwise reproducible)
+template <bool SPLIT = false>
 static int gemm_bf16(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ldw, const EpiParams& ep, int K, cudaStream_t st, int force_bn = 0) {
   REQUIRE(ep.N % 32 == 0 && K % 8 == 0 && lda % 8 == 0 && ldw % 8 == 0, "gemm_bf16: N %% 32, K/lda/ldw %% 8 required (N=%d K=%d)", ep.N, K);
+  REQUIRE(!SPLIT || (K % 64 == 0 && lda % 64 == 0 && ldw % 64 == 0), "gemm_bf16x3: K, lda, ldw %% 64 required (K=%d)", K);
   // CTA-pair kernel (force_bn 512 / 1024 = pair tiles 256x256 / 256x128): the default once there are enough 256-row tiles
-  if (force_bn == 512) return launch_tc2<256>(h, A, lda, W, ldw, ep, K, st);
-  if (force_bn == 1024) return launch_tc2<128>(h, A, lda, W, ldw, ep, K, st);
+  if (force_bn == 512) return launch_tc2<256, SPLIT>(h, A, lda, W, ldw, ep, K, st);
+  if (force_bn == 1024) return launch_tc2<128, SPLIT>(h, A, lda, W, ldw, ep, K, st);
   if (force_bn == 0 && h->use_pair && ep.M >= 512 && ep.N % 256 == 0 && K % 64 == 0) {
     // Wave model calibrated on B200 (tools/gemm_bench.py): time ~ waves x per-wave cost.  A pair tile (256x256 on two SMs)
     // and a single-CTA 128x256 tile cost the same per wave at 32 clips, but at >= 128 clips the pair kernel is 20 % cheaper
@@ -254,20 +262,24 @@ static int gemm_bf16(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ld
     const double c_pair = waves(mt256 * (ep.N / 256), pairs);
     const double c_256 = waves(mt128 * (ep.N / 256), sms) * (ep.M >= 16384 ? 1.2 : 1.02);
     const double c_128 = waves(mt128 * (ep.N / 128), sms) * 0.56;
+    // bf16x3: the same model (its operand bytes and MMAs both grow ~2-3x on every tile shape); a single-CTA 128 x 256 tile would
+    // keep only 2 of its 96 KB stages, so the pair tile or 128 x 128 it is
+    if (SPLIT) return c_pair <= c_128 ? launch_tc2<256, true>(h, A, lda, W, ldw, ep, K, st) : launch_tc<128, true>(h, A, lda, W, ldw, ep, K, st);
     if (ep.kind == EPI_GATE_RES && h->use_splitk && K >= 1024 && c_pair >= 2.0) {   // single-wave problems stay bitwise deterministic
       // x += gate * (.) is additive, so a tile may be cut into 2 K slices whose partial sums meet in x (fp32 RED):
       // N = 1024 at 32 clips = 92 pair tiles on 74 pairs (2 waves) -> 184 half-K units (2.5 half-waves)
       const double c_split = 0.5 * waves(2 * mt256 * (ep.N / 256), pairs) + 0.08;
-      if (c_split < c_pair && c_split < c_256 && c_split < c_128) return launch_tc2<256>(h, A, lda, W, ldw, ep, K, st, 2);
+      if (c_split < c_pair && c_split < c_256 && c_split < c_128) return launch_tc2<256, false>(h, A, lda, W, ldw, ep, K, st, 2);
     }
-    if (c_pair <= c_256 && c_pair <= c_128) return launch_tc2<256>(h, A, lda, W, ldw, ep, K, st);
-    return c_128 < c_256 ? launch_tc<128>(h, A, lda, W, ldw, ep, K, st) : launch_tc<256>(h, A, lda, W, ldw, ep, K, st);
+    if (c_pair <= c_256 && c_pair <= c_128) return launch_tc2<256, false>(h, A, lda, W, ldw, ep, K, st);
+    return c_128 < c_256 ? launch_tc<128, false>(h, A, lda, W, ldw, ep, K, st) : launch_tc<256, false>(h, A, lda, W, ldw, ep, K, st);
   }
-  const int bn = force_bn > 0 ? force_bn : pick_bn(h, ep.M, ep.N);
+  int bn = force_bn > 0 ? force_bn : pick_bn(h, ep.M, ep.N);
+  if (SPLIT && force_bn == 0 && bn == 256) bn = 128;      // 2 stages of 96 KB: explicit block_n only
   switch (bn) {
-    case 256: return launch_tc<256>(h, A, lda, W, ldw, ep, K, st);
-    case 128: return launch_tc<128>(h, A, lda, W, ldw, ep, K, st);
-    case 64: return launch_tc<64>(h, A, lda, W, ldw, ep, K, st);
+    case 256: return launch_tc<256, SPLIT>(h, A, lda, W, ldw, ep, K, st);
+    case 128: return launch_tc<128, SPLIT>(h, A, lda, W, ldw, ep, K, st);
+    case 64: return launch_tc<64, SPLIT>(h, A, lda, W, ldw, ep, K, st);
   }
   return set_err(-1, "gemm_bf16: block_n must be 64, 128 or 256 (got %d)", bn);
 }
@@ -278,15 +290,24 @@ static int gemm_f32(FmtHandle* h, const float* A, int lda, const float* W, int l
   return launch(h, gemm_simt_kernel, grid, dim3(256), 0, st, 1, A, lda, W, ldw, ep, K);
 }
 
+// T = GEMM operand (activation) type of a mode; Tab = type of its AdaLN tables and of QKV
 template <typename T> struct ModeOps;
 template <> struct ModeOps<bf16> {
+  using Tab = bf16;
   static int gemm(FmtHandle* h, const void* A, int lda, const Linear& L, const EpiParams& ep, cudaStream_t st) {
     return gemm_bf16(h, static_cast<const bf16*>(A), lda, L.w16, L.K, ep, L.K, st);
   }
 };
 template <> struct ModeOps<float> {
+  using Tab = float;
   static int gemm(FmtHandle* h, const void* A, int lda, const Linear& L, const EpiParams& ep, cudaStream_t st) {
     return gemm_f32(h, static_cast<const float*>(A), lda, L.w32, L.K, ep, L.K, st);
+  }
+};
+template <> struct ModeOps<bf16x3_t> {
+  using Tab = float;                                   // only GEMM operands are pairs: tables and QKV stay fp32, as in the fp32 mode
+  static int gemm(FmtHandle* h, const void* A, int lda, const Linear& L, const EpiParams& ep, cudaStream_t st) {
+    return gemm_bf16<true>(h, static_cast<const bf16*>(A), lda, L.w3, L.K, ep, L.K, st);
   }
 };
 
@@ -315,13 +336,14 @@ static int enqueue_tables(FmtHandle* h, int e0, int n, cudaStream_t st) {
   const size_t total = static_cast<size_t>(n) * h->U * s.H;
   FMT_OK(launch(h, silu_cond_kernel<T>, dim3(static_cast<unsigned>((total / 4 + 255) / 256)), dim3(256), 0, st, 1,
                 static_cast<const float*>(h->cemb.p), static_cast<const float*>(h->temb.p), e0, h->U, s.H, static_cast<T*>(h->silu.p), total));
-  EpiParams ep = epi(EPI_STORE, n * h->U, h->NT, h->ada.b, h->table.p, h->NT, 0);
+  EpiParams ep = epi(EPI_STORE, n * h->U, h->NT, h->ada.b, h->table.p, h->NT, sizeof(typename ModeOps<T>::Tab) == 4);
   FMT_OK(ModeOps<T>::gemm(h, h->silu.p, s.H, h->ada, ep, st));
   return 0;
 }
 
 template <typename T>
-static int launch_lnmod(FmtHandle* h, const T* table_e, long long shift_off, long long scale_off, cudaStream_t st) {
+static int launch_lnmod(FmtHandle* h, const typename ModeOps<T>::Tab* table_e, long long shift_off, long long scale_off, cudaStream_t st) {
+  using TT = typename ModeOps<T>::Tab;
   const ModelShape& s = h->shape;
   const int warps = 4;
   const dim3 grid((h->R + warps - 1) / warps), block(warps * 32);
@@ -330,10 +352,10 @@ static int launch_lnmod(FmtHandle* h, const T* table_e, long long shift_off, lon
   const int* urow = h->dedup ? static_cast<const int*>(h->urow_buf.p) : nullptr;
   const long long ldt = h->NT;
   switch (s.H / 128) {
-    case 1: return launch(h, lnmod_kernel<T, T, 1>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
-    case 2: return launch(h, lnmod_kernel<T, T, 2>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
-    case 4: return launch(h, lnmod_kernel<T, T, 4>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
-    case 8: return launch(h, lnmod_kernel<T, T, 8>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
+    case 1: return launch(h, lnmod_kernel<T, TT, 1>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
+    case 2: return launch(h, lnmod_kernel<T, TT, 2>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
+    case 4: return launch(h, lnmod_kernel<T, TT, 4>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
+    case 8: return launch(h, lnmod_kernel<T, TT, 8>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
   }
   return set_err(-1, "dim_h %d unsupported by the LayerNorm kernel (128, 256, 512, 1024)", s.H);
 }
@@ -345,7 +367,8 @@ static int launch_attn(FmtHandle* h, cudaStream_t st) {
   const int n_seq = s.nb * s.B, total_warps = n_seq * heads * s.N, warps = 4;
   const float scale = 1.0f / sqrtf(static_cast<float>(hd));
   const dim3 grid((total_warps + warps - 1) / warps), block(warps * 32);
-  const T* qkv = static_cast<const T*>(h->QKV.p);
+  using Q = typename ModeOps<T>::Tab;
+  const Q* qkv = static_cast<const Q*>(h->QKV.p);
   T* out = static_cast<T*>(h->A2.p);
   const int win = h->d.attention_window;
   if constexpr (sizeof(T) == 2) {
@@ -360,9 +383,9 @@ static int launch_attn(FmtHandle* h, cudaStream_t st) {
     }
   }
   switch (hd) {
-    case 32: return launch(h, band_attention_kernel<T, 1>, grid, block, 0, st, 1, qkv, n_seq, s.N, heads, win, scale, out);
-    case 64: return launch(h, band_attention_kernel<T, 2>, grid, block, 0, st, 1, qkv, n_seq, s.N, heads, win, scale, out);
-    case 128: return launch(h, band_attention_kernel<T, 4>, grid, block, 0, st, 1, qkv, n_seq, s.N, heads, win, scale, out);
+    case 32: return launch(h, band_attention_kernel<Q, 1, T>, grid, block, 0, st, 1, qkv, n_seq, s.N, heads, win, scale, out);
+    case 64: return launch(h, band_attention_kernel<Q, 2, T>, grid, block, 0, st, 1, qkv, n_seq, s.N, heads, win, scale, out);
+    case 128: return launch(h, band_attention_kernel<Q, 4, T>, grid, block, 0, st, 1, qkv, n_seq, s.N, heads, win, scale, out);
   }
   return set_err(-1, "head_dim %d unsupported (32, 64, 128)", hd);
 }
@@ -374,7 +397,9 @@ static int enqueue_forward(FmtHandle* h, int table_slot, cudaStream_t st) {
   const ModelShape& s = h->shape;
   const FmtDims& d = h->d;
   const int R = h->R, H = s.H;
-  const T* table_e = static_cast<const T*>(h->table.p) + static_cast<size_t>(table_slot) * h->U * h->NT;
+  using TT = typename ModeOps<T>::Tab;
+  const TT* table_e = static_cast<const TT*>(h->table.p) + static_cast<size_t>(table_slot) * h->U * h->NT;
+  const int qkv_f32 = sizeof(TT) == 4;
   {
     EpiParams ep = epi(EPI_POS, R, H, h->x_emb.b, h->X.p, H, 1);
     ep.pos = h->pos; ep.frames = s.N;
@@ -383,7 +408,7 @@ static int enqueue_forward(FmtHandle* h, int table_slot, cudaStream_t st) {
   for (int i = 0; i < d.depth; ++i) {
     const long long base = static_cast<long long>(i) * 6 * H;
     FMT_OK(launch_lnmod<T>(h, table_e, base + 0, base + H, st));
-    FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->qkv[i], epi(EPI_STORE, R, 3 * H, h->qkv[i].b, h->QKV.p, 3 * H, 0), st));
+    FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->qkv[i], epi(EPI_STORE, R, 3 * H, h->qkv[i].b, h->QKV.p, 3 * H, qkv_f32), st));
     FMT_OK(launch_attn<T>(h, st));
     {
       EpiParams ep = epi(EPI_GATE_RES, R, H, h->proj[i].b, h->X.p, H, 1);
@@ -828,7 +853,11 @@ static int enqueue_window(FmtHandle* h, cudaStream_t st) {
 }
 
 static int enqueue_window_mode(FmtHandle* h, cudaStream_t st) {
-  return h->plan.mode == FMT_MODE_BF16 ? enqueue_window<bf16>(h, st) : enqueue_window<float>(h, st);
+  switch (h->plan.mode) {
+    case FMT_MODE_BF16: return enqueue_window<bf16>(h, st);
+    case FMT_MODE_BF16X3: return enqueue_window<bf16x3_t>(h, st);
+  }
+  return enqueue_window<float>(h, st);
 }
 
 // ------------------------------------------------------------------------------------------------ create / destroy
@@ -838,6 +867,26 @@ static int upload(FmtHandle* h, const void* src, size_t n_floats, int location, 
   h->owned.push_back(p);
   CUDA_OK(cudaMemcpy(p, src, n_floats * sizeof(float), location == FMT_LOC_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice));
   *out = p;
+  return 0;
+}
+
+// FMT_MODE_BF16X3 operand of a Linear: (N, 2K) pairs from its fp32 (padded) weight, once per Linear
+static int pack_split(FmtHandle* h, Linear& L, cudaStream_t st) {
+  if (L.w3) return 0;
+  REQUIRE(L.K % 64 == 0, "bf16x3 mode: K = %d is not a multiple of 64", L.K);
+  const size_t n = static_cast<size_t>(L.N) * L.K;
+  CUDA_OK(cudaMalloc(&L.w3, n * sizeof(bf16x3_t)));
+  h->owned.push_back(L.w3);
+  f32_to_split_kernel<<<static_cast<unsigned>(std::min<size_t>((n / 4 + 255) / 256, static_cast<size_t>(h->num_sms) * 16)), 256, 0, st>>>(
+      L.w32, reinterpret_cast<bf16x3_t*>(L.w3), n / 4);
+  LAUNCH_CHECK();
+  return 0;
+}
+
+static int pack_split_all(FmtHandle* h, cudaStream_t st) {
+  for (Linear* L : {&h->x_emb, &h->c_emb, &h->ada, &h->dec}) FMT_OK(pack_split(h, *L, st));
+  for (int i = 0; i < h->d.depth; ++i)
+    for (Linear* L : {&h->qkv[i], &h->proj[i], &h->fc1[i], &h->fc2[i]}) FMT_OK(pack_split(h, *L, st));
   return 0;
 }
 
@@ -1100,10 +1149,14 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
   CUDA_OK(cudaSetDevice(h->device));
   REQUIRE(p->batch >= 1, "fmt_configure: batch must be >= 1");
   REQUIRE(p->n_branches == 1 || p->n_branches == 3 || p->n_branches == 4, "fmt_configure: n_branches must be 1, 3 or 4");
-  REQUIRE(p->mode == FMT_MODE_BF16 || p->mode == FMT_MODE_FP32_VALIDATE, "fmt_configure: unknown mode %d", p->mode);
+  REQUIRE(p->mode == FMT_MODE_BF16 || p->mode == FMT_MODE_FP32_VALIDATE || p->mode == FMT_MODE_BF16X3, "fmt_configure: unknown mode %d", p->mode);
   REQUIRE(p->n_steps >= 0 && p->n_stages >= 1 && p->n_stages <= FMT_MAX_STAGES, "fmt_configure: bad n_steps/n_stages");
   REQUIRE(p->rk_a && p->rk_b && (p->n_steps == 0 || (p->t_eval && p->dt)), "fmt_configure: null schedule arrays");
   if (same_plan(h, p)) return 0;
+  if (p->mode == FMT_MODE_BF16X3) {
+    FMT_OK(pack_split_all(h, st));
+    CUDA_OK(cudaStreamSynchronize(st));
+  }
 
   const FmtDims& d = h->d;
   const int ne = p->n_steps * p->n_stages;
@@ -1146,7 +1199,7 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
       }
     }
   }
-  const size_t ts = p->mode == FMT_MODE_BF16 ? 2 : 4;
+  const size_t ts = p->mode == FMT_MODE_BF16 ? 2 : 4;   // bf16x3: 4-byte pairs, fp32 tables and QKV
   h->tsize = ts;
   const size_t R = h->R, U = h->U, H = s.H;
   // table chunking: the AdaLN tables of as many evaluations as fit in half of the memory that is free right now (what this handle
@@ -1313,6 +1366,22 @@ int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
   return 0;
 }
 
+}  // extern "C"
+
+template <typename T>
+static int enqueue_velocity(FmtHandle* h, const FmtEval* ev, cudaStream_t st) {
+  const ModelShape& s = h->shape;
+  FMT_OK(enqueue_prepare<T>(h, st));
+  FMT_OK(enqueue_tables<T>(h, ev->eval_index, 1, st));
+  FMT_OK(launch(h, pack_x_kernel<T>, dim3(s.B * s.N), dim3(128), 0, st, 1, static_cast<const WindowArgs*>(h->wargs.p), s, ev->x,
+                static_cast<const float*>(h->prevx.p), static_cast<T*>(h->ax.p)));
+  FMT_OK(enqueue_forward<T>(h, 0, st));
+  FMT_OK(launch_combine<T>(h, 0, ev->v_out, nullptr, st));
+  return 0;
+}
+
+extern "C" {
+
 int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream) {
   REQUIRE(h && ev, "fmt_velocity: null argument");
   REQUIRE(h->configured, "fmt_velocity: call fmt_configure first");
@@ -1328,22 +1397,11 @@ int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream) {
   a.T_wa = s.L; a.T_we = s.we_dynamic ? s.L : 1; a.T_out = s.L; a.win_start = 0; a.first_window = 0; a.use_ext = 1;
   a.a_scale = ev->a_cfg_scale; a.r_scale = ev->r_cfg_scale; a.e_scale = ev->e_cfg_scale;
   FMT_OK(set_wargs(h, a, st));
-  if (h->plan.mode == FMT_MODE_BF16) {
-    FMT_OK(enqueue_prepare<bf16>(h, st));
-    FMT_OK(enqueue_tables<bf16>(h, ev->eval_index, 1, st));
-    FMT_OK(launch(h, pack_x_kernel<bf16>, dim3(s.B * s.N), dim3(128), 0, st, 1, static_cast<const WindowArgs*>(h->wargs.p), s, ev->x,
-                  static_cast<const float*>(h->prevx.p), static_cast<bf16*>(h->ax.p)));
-    FMT_OK(enqueue_forward<bf16>(h, 0, st));
-    FMT_OK(launch_combine<bf16>(h, 0, ev->v_out, nullptr, st));
-  } else {
-    FMT_OK(enqueue_prepare<float>(h, st));
-    FMT_OK(enqueue_tables<float>(h, ev->eval_index, 1, st));
-    FMT_OK(launch(h, pack_x_kernel<float>, dim3(s.B * s.N), dim3(128), 0, st, 1, static_cast<const WindowArgs*>(h->wargs.p), s, ev->x,
-                  static_cast<const float*>(h->prevx.p), static_cast<float*>(h->ax.p)));
-    FMT_OK(enqueue_forward<float>(h, 0, st));
-    FMT_OK(launch_combine<float>(h, 0, ev->v_out, nullptr, st));
+  switch (h->plan.mode) {
+    case FMT_MODE_BF16: return enqueue_velocity<bf16>(h, ev, st);
+    case FMT_MODE_BF16X3: return enqueue_velocity<bf16x3_t>(h, ev, st);
   }
-  return 0;
+  return enqueue_velocity<float>(h, ev, st);
 }
 
 // ------------------------------------------------------------------------------------------------ diagnostics
@@ -1392,11 +1450,11 @@ int32_t fmt_proj_destroy(FmtProj* p) {
 }
 
 // x: (rows, in_dim) fp32, out: (rows, out_dim) fp32, both at `location`.  FMT_MODE_BF16: bf16 tcgen05 GEMM with fp32 accumulation,
-// LayerNorm / SiLU in fp32; FMT_MODE_FP32_VALIDATE: fp32 SIMT GEMM.
+// LayerNorm / SiLU in fp32; FMT_MODE_BF16X3: the split bf16x3 GEMM (in_dim % 64); FMT_MODE_FP32_VALIDATE: fp32 SIMT GEMM.
 int32_t fmt_proj_apply(FmtProj* p, const float* x, int64_t rows, float* out, int32_t mode, int32_t location, void* stream) {
   REQUIRE(p && x && out, "fmt_proj_apply: null argument");
   REQUIRE(rows > 0 && rows < (1ll << 31), "fmt_proj_apply: rows = %lld out of range", static_cast<long long>(rows));
-  REQUIRE(mode == FMT_MODE_BF16 || mode == FMT_MODE_FP32_VALIDATE, "fmt_proj_apply: unknown mode %d", mode);
+  REQUIRE(mode == FMT_MODE_BF16 || mode == FMT_MODE_FP32_VALIDATE || mode == FMT_MODE_BF16X3, "fmt_proj_apply: unknown mode %d", mode);
   FmtHandle* h = &p->h;
   CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1417,6 +1475,15 @@ int32_t fmt_proj_apply(FmtProj* p, const float* x, int64_t rows, float* out, int
     f32_to_bf16_kernel<<<blocks, 256, 0, st>>>(xd, static_cast<bf16*>(p->x16.p), n8);
     LAUNCH_CHECK(); count_launch(h);
     FMT_OK(gemm_bf16(h, static_cast<const bf16*>(p->x16.p), K, p->lin.w16, K, ep, K, st));
+  } else if (mode == FMT_MODE_BF16X3) {
+    REQUIRE(K % 64 == 0, "fmt_proj_apply: bf16x3 mode needs in_dim %% 64 == 0 (got %d)", K);
+    FMT_OK(pack_split(h, p->lin, st));
+    FMT_OK(dev_alloc(h, p->x16, nx * sizeof(bf16x3_t)));       // x16 holds the GEMM operand of whichever mode ran last
+    const size_t n4 = nx / 4;
+    const unsigned blocks = static_cast<unsigned>(std::min<size_t>((n4 + 255) / 256, static_cast<size_t>(h->num_sms) * 16));
+    f32_to_split_kernel<<<blocks, 256, 0, st>>>(xd, static_cast<bf16x3_t*>(p->x16.p), n4);
+    LAUNCH_CHECK(); count_launch(h);
+    FMT_OK(gemm_bf16<true>(h, static_cast<const bf16*>(p->x16.p), K, p->lin.w3, K, ep, K, st));
   } else {
     FMT_OK(gemm_f32(h, xd, K, p->lin.w32, K, ep, K, st));
   }
@@ -1464,6 +1531,39 @@ int32_t fmt_debug_gemm_bench(const void* A, const void* W, const float* bias, fl
   EpiParams ep = epi(EPI_STORE, M, N, bias, out, N, 0);     // bf16 output, like the qkv / fc1 GEMMs of the step
   for (int i = 0; i < iters; ++i)
     FMT_OK(gemm_bf16(&h, static_cast<const bf16*>(A), K, static_cast<const bf16*>(W), K, ep, K, static_cast<cudaStream_t>(stream), block_n));
+  return 0;
+}
+
+int32_t fmt_debug_gemm_bf16x3(const float* A, const float* W, const float* bias, float* out, int32_t M, int32_t N, int32_t K, int32_t block_n,
+                              void* stream) {
+  REQUIRE(A && W && out && M > 0 && N > 0 && K > 0 && K % 64 == 0, "fmt_debug_gemm_bf16x3: K %% 64 == 0 and non-null operands required (K=%d)", K);
+  FmtHandle h;
+  FMT_OK(debug_handle(h));
+  h.use_pdl = false;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t na = static_cast<size_t>(M) * K, nw = static_cast<size_t>(N) * K;
+  void *a3 = nullptr, *w3 = nullptr;
+  CUDA_OK(cudaMallocAsync(&a3, na * sizeof(bf16x3_t), st));
+  CUDA_OK(cudaMallocAsync(&w3, nw * sizeof(bf16x3_t), st));
+  f32_to_split_kernel<<<static_cast<unsigned>(std::min<size_t>((na / 4 + 255) / 256, 2368)), 256, 0, st>>>(A, static_cast<bf16x3_t*>(a3), na / 4);
+  f32_to_split_kernel<<<static_cast<unsigned>(std::min<size_t>((nw / 4 + 255) / 256, 2368)), 256, 0, st>>>(W, static_cast<bf16x3_t*>(w3), nw / 4);
+  LAUNCH_CHECK();
+  const int rc = gemm_bf16<true>(&h, static_cast<const bf16*>(a3), K, static_cast<const bf16*>(w3), K, epi(EPI_STORE, M, N, bias, out, N, 1), K, st, block_n);
+  (void)cudaFreeAsync(a3, st);
+  (void)cudaFreeAsync(w3, st);
+  return rc;
+}
+
+// `iters` back-to-back launches of one bf16x3 GEMM variant on operands already in the pair layout, fp32 output
+int32_t fmt_debug_gemm_bench_bf16x3(const void* A, const void* W, const float* bias, float* out, int32_t M, int32_t N, int32_t K, int32_t block_n,
+                                    int32_t iters, void* stream) {
+  static FmtHandle* hp = nullptr;
+  if (!hp) { hp = new FmtHandle(); FMT_OK(debug_handle(*hp)); }
+  FmtHandle& h = *hp;
+  h.use_pdl = false;
+  EpiParams ep = epi(EPI_STORE, M, N, bias, out, N, 1);
+  for (int i = 0; i < iters; ++i)
+    FMT_OK(gemm_bf16<true>(&h, static_cast<const bf16*>(A), K, static_cast<const bf16*>(W), K, ep, K, static_cast<cudaStream_t>(stream), block_n));
   return 0;
 }
 

@@ -3,10 +3,14 @@
 //                        TMEM, operands staged by TMA (128B swizzle) through an mbarrier ring; persistent over
 //                        output tiles with a double-buffered accumulator so the epilogue of tile i overlaps the
 //                        MMAs of tile i+1.  Warp roles: 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocator, 4..11 = epilogue.
+//                        SPLIT = true (FMT_MODE_BF16X3): bf16 hi / lo operand pairs (bf16x3_t below), three MMAs per K step
+//                        (Ah.Wh + Ah.Wl + Al.Wh) into the same accumulator; fp32-class products on the tensor pipe.
+//   * gemm_tc2_kernel  - the same on CTA pairs (cta_group::2), same SPLIT variant.
 //   * gemm_simt_kernel - fp32 operands, plain FFMA tiles; FMT_MODE_FP32_VALIDATE only (the 1e-4 parity mode).
 // Both share epi_apply(), which carries the fused epilogues of the reference's block
 // (FMT.py:171-176): bias, GELU(tanh), +pos_embed, and x += gate * (.).
 #pragma once
+#include <type_traits>
 #include "ptx.cuh"
 
 namespace fmt {
@@ -80,6 +84,29 @@ __device__ __forceinline__ void store_row32(__nv_bfloat16* p, const float (&v)[3
                  pack_bf16x2(v[16 * i + 12], v[16 * i + 13]), pack_bf16x2(v[16 * i + 14], v[16 * i + 15]));
 }
 
+// bf16x3 operands (FMT_MODE_BF16X3): x = hi + lo with hi = bf16(x) and lo = bf16(x - hi); the split GEMM sums Ah.Wh + Ah.Wl + Al.Wh
+// (Al.Wl, ~2^-16 relative, is dropped).  A pair matrix has rows of 2K bf16 values in which every 64-column K block of hi is followed by
+// the same block of lo: [hi 0:64 | lo 0:64 | hi 64:128 | lo 64:128 | ...], so one tensor map per operand serves both halves (box
+// columns 128 kb and 128 kb + 64).  bf16x3_t stands for one element of such a row and is 4 bytes, so a pair row takes the bytes of
+// an fp32 row of the same K and kernels index a pair matrix like any other (p = base + row * ld + c).  Buffers are 256-byte aligned
+// and ld is a multiple of 64, so the byte offset of p names the element's 64-column block (offset / 256) and its column c % 64
+// in the block (offset % 256 / 4): split_hi(p) is where its hi part really is, its lo part sits 64 values (128 bytes) further.
+struct bf16x3_t { uint32_t bits; };
+__device__ __forceinline__ __nv_bfloat16* split_hi(bf16x3_t* p) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(p);
+  return reinterpret_cast<__nv_bfloat16*>((a & ~static_cast<uintptr_t>(255)) + ((a & 255) >> 1));
+}
+__device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bfloat16& lo) {
+  hi = __float2bfloat16_rn(x);
+  lo = __float2bfloat16_rn(x - __bfloat162float(hi));
+}
+__device__ __forceinline__ void split_bf16x2(float a, float b, uint32_t& hi, uint32_t& lo) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+  const __nv_bfloat162 l = __floats2bfloat162_rn(a - __low2float(h), b - __high2float(h));
+  hi = *reinterpret_cast<const uint32_t*>(&h);
+  lo = *reinterpret_cast<const uint32_t*>(&l);
+}
+
 template <typename T, int NC> struct VecIO;
 template <int NC> struct VecIO<float, NC> {
   static_assert(NC % 4 == 0, "");
@@ -113,6 +140,30 @@ template <int NC> struct VecIO<__nv_bfloat16, NC> {
       t.x = *reinterpret_cast<uint32_t*>(&a);
       t.y = *reinterpret_cast<uint32_t*>(&b);
       reinterpret_cast<uint2*>(p)[i] = t;
+    }
+  }
+};
+
+// NC consecutive elements starting at a multiple of NC (NC divides 64: one K block): NC hi values, then NC lo values 128 bytes further
+template <int NC> struct VecIO<bf16x3_t, NC> {
+  static_assert(NC % 4 == 0 && 64 % NC == 0, "");
+  static __device__ __forceinline__ void store(bf16x3_t* p, const float (&v)[NC]) {
+    uint32_t hi[NC / 2], lo[NC / 2];
+#pragma unroll
+    for (int i = 0; i < NC / 2; ++i) split_bf16x2(v[2 * i], v[2 * i + 1], hi[i], lo[i]);
+    __nv_bfloat16* hp = split_hi(p);
+    if constexpr (NC % 16 == 0) {
+#pragma unroll
+      for (int i = 0; i < NC / 16; ++i) {
+        st_global_v8(hp + 16 * i, hi[8 * i], hi[8 * i + 1], hi[8 * i + 2], hi[8 * i + 3], hi[8 * i + 4], hi[8 * i + 5], hi[8 * i + 6], hi[8 * i + 7]);
+        st_global_v8(hp + 64 + 16 * i, lo[8 * i], lo[8 * i + 1], lo[8 * i + 2], lo[8 * i + 3], lo[8 * i + 4], lo[8 * i + 5], lo[8 * i + 6], lo[8 * i + 7]);
+      }
+    } else {
+#pragma unroll
+      for (int i = 0; i < NC / 4; ++i) {
+        reinterpret_cast<uint2*>(hp)[i] = make_uint2(hi[2 * i], hi[2 * i + 1]);
+        reinterpret_cast<uint2*>(hp + 64)[i] = make_uint2(lo[2 * i], lo[2 * i + 1]);
+      }
     }
   }
 };
@@ -160,12 +211,13 @@ __device__ __forceinline__ void epi_apply(const EpiParams& p, int m, int n0, flo
 // ------------------------------------------------------------------------------------------------
 // tcgen05 / TMA GEMM
 // ------------------------------------------------------------------------------------------------
-template <int BN> struct TcCfg {
+template <int BN, bool SPLIT = false> struct TcCfg {
   static constexpr int BM = 128, BK = 64, UMMA_K = 16;
   static constexpr int A_BYTES = BM * BK * 2;
   static constexpr int B_BYTES = BN * BK * 2;
-  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int STAGES = (BN == 256) ? 4 : (BN == 128 ? 6 : 8);
+  static constexpr int HALVES = SPLIT ? 2 : 1;           // SPLIT: a stage holds [Ah | Wh | Al | Wl] of one K block
+  static constexpr int STAGE_BYTES = HALVES * (A_BYTES + B_BYTES);
+  static constexpr int STAGES = SPLIT ? ((BN == 256) ? 2 : (BN == 128 ? 3 : 4)) : ((BN == 256) ? 4 : (BN == 128 ? 6 : 8));
   static constexpr int ACC_STAGES = 2;
   static constexpr int TMEM_COLS = ACC_STAGES * BN;     // 128 / 256 / 512: powers of two >= 32
   static constexpr int BAR_BYTES = 256;
@@ -175,10 +227,12 @@ template <int BN> struct TcCfg {
   static_assert(BN == 64 || BN == 128 || BN == 256, "BN");
 };
 
-template <int BN, typename TT>
-__global__ void __launch_bounds__(TcCfg<BN>::THREADS, 1)
+// SPLIT: tmA / tmB describe pair matrices (2K bf16 columns), K is the logical depth; activation outputs are bf16x3_t pairs.
+template <int BN, typename TT, bool SPLIT>
+__global__ void __launch_bounds__(TcCfg<BN, SPLIT>::THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const EpiParams ep, const int K) {
-  using C = TcCfg<BN>;
+  using C = TcCfg<BN, SPLIT>;
+  using AT = typename std::conditional<SPLIT, bf16x3_t, __nv_bfloat16>::type;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + C::STAGES * C::STAGE_BYTES);
@@ -227,8 +281,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           mbar_wait(&empty_bar[stage], phase ^ 1);
           uint8_t* sa = smem + stage * C::STAGE_BYTES;
           mbar_expect_tx(&full_bar[stage], C::STAGE_BYTES);
-          tma_load_2d(&tmA, &full_bar[stage], sa, kb * C::BK, m0, kEvictNormal);
-          tma_load_2d(&tmB, &full_bar[stage], sa + C::A_BYTES, kb * C::BK, n0, kEvictNormal);
+          tma_load_2d(&tmA, &full_bar[stage], sa, kb * C::BK * C::HALVES, m0, kEvictNormal);
+          tma_load_2d(&tmB, &full_bar[stage], sa + C::A_BYTES, kb * C::BK * C::HALVES, n0, kEvictNormal);
+          if constexpr (SPLIT) {
+            tma_load_2d(&tmA, &full_bar[stage], sa + C::A_BYTES + C::B_BYTES, kb * C::BK * 2 + C::BK, m0, kEvictNormal);
+            tma_load_2d(&tmB, &full_bar[stage], sa + 2 * C::A_BYTES + C::B_BYTES, kb * C::BK * 2 + C::BK, n0, kEvictNormal);
+          }
           if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
         }
       }
@@ -254,6 +312,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           for (int k = 0; k < C::BK / C::UMMA_K; ++k) {
             // advance along K inside the 128B swizzle atom: +32 bytes (>>4 = 2) per UMMA_K
             umma_bf16(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0);
+          }
+          if constexpr (SPLIT) {                           // the lo products of the same K block: Ah.Wl + Al.Wh
+            const uint64_t dal = make_sw128_kmajor_desc(sa + C::A_BYTES + C::B_BYTES), dbl = make_sw128_kmajor_desc(sa + 2 * C::A_BYTES + C::B_BYTES);
+#pragma unroll
+            for (int k = 0; k < C::BK / C::UMMA_K; ++k) {
+              umma_bf16(d_tmem, da + 2 * k, dbl + 2 * k, idesc, 1u);
+              umma_bf16(d_tmem, dal + 2 * k, db + 2 * k, idesc, 1u);
+            }
           }
           umma_commit(&empty_bar[stage]);                  // frees the smem slot when these MMAs retire
           if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
@@ -341,7 +407,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           tmem_ld32(t_addr + c * 32, v);
           tmem_ld_wait();
           const int n = n0 + c * 32;
-          if (m < ep.M && n < ep.N) epi_apply<__nv_bfloat16, TT, 32>(ep, m, n, v);
+          if (m < ep.M && n < ep.N) epi_apply<AT, TT, 32>(ep, m, n, v);
         }
       }
       tc_fence_before();
@@ -375,12 +441,13 @@ __device__ __forceinline__ void raster_tile(int t, int m_tiles, int n_tiles, int
   nt = r / m_in_group;
 }
 
-template <int BN> struct Tc2Cfg {
+template <int BN, bool SPLIT = false> struct Tc2Cfg {
   static constexpr int BM = 256, BMH = 128, BK = 64, UMMA_K = 16;
   static constexpr int A_BYTES = BMH * BK * 2;
   static constexpr int B_BYTES = (BN / 2) * BK * 2;
-  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int STAGES = (BN == 256) ? 6 : 8;
+  static constexpr int HALVES = SPLIT ? 2 : 1;           // SPLIT: a stage holds [Ah | Wh | Al | Wl] of one K block
+  static constexpr int STAGE_BYTES = HALVES * (A_BYTES + B_BYTES);
+  static constexpr int STAGES = SPLIT ? ((BN == 256) ? 3 : 4) : ((BN == 256) ? 6 : 8);
   static constexpr int ACC_STAGES = 2;
   static constexpr int TMEM_COLS = ACC_STAGES * BN;
   static constexpr int BAR_BYTES = 256 + BN * 4;        // barriers + tmem slot, then the tile's bias (BN floats)
@@ -390,10 +457,10 @@ template <int BN> struct Tc2Cfg {
   static_assert(BN == 128 || BN == 256, "BN");
 };
 
-template <int BN, typename TT>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Tc2Cfg<BN>::THREADS, 1)
+template <int BN, typename TT, bool SPLIT>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Tc2Cfg<BN, SPLIT>::THREADS, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const EpiParams ep, const int K) {
-  using C = Tc2Cfg<BN>;
+  using C = Tc2Cfg<BN, SPLIT>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + C::STAGES * C::STAGE_BYTES);
@@ -449,8 +516,12 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           uint8_t* sa = smem + stage * C::STAGE_BYTES;
           const uint32_t leader_full = mapa_u32(smem_u32(&full_bar[stage]), 0);
           if (rank == 0) mbar_expect_tx(&full_bar[stage], 2 * C::STAGE_BYTES);
-          tma_load_2d_cg2(&tmA, leader_full, sa, kb * C::BK, m0, kEvictNormal);
-          tma_load_2d_cg2(&tmB, leader_full, sa + C::A_BYTES, kb * C::BK, n0, kEvictNormal);
+          tma_load_2d_cg2(&tmA, leader_full, sa, kb * C::BK * C::HALVES, m0, kEvictNormal);
+          tma_load_2d_cg2(&tmB, leader_full, sa + C::A_BYTES, kb * C::BK * C::HALVES, n0, kEvictNormal);
+          if constexpr (SPLIT) {
+            tma_load_2d_cg2(&tmA, leader_full, sa + C::A_BYTES + C::B_BYTES, kb * C::BK * 2 + C::BK, m0, kEvictNormal);
+            tma_load_2d_cg2(&tmB, leader_full, sa + 2 * C::A_BYTES + C::B_BYTES, kb * C::BK * 2 + C::BK, n0, kEvictNormal);
+          }
           if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
         }
       }
@@ -475,6 +546,14 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           const uint64_t db = make_sw128_kmajor_desc(sa + C::A_BYTES);
 #pragma unroll
           for (int k = 0; k < C::BK / C::UMMA_K; ++k) umma_bf16_cg2(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb > kb_lo || k > 0) ? 1u : 0u);
+          if constexpr (SPLIT) {                           // the lo products of the same K block: Ah.Wl + Al.Wh
+            const uint64_t dal = make_sw128_kmajor_desc(sa + C::A_BYTES + C::B_BYTES), dbl = make_sw128_kmajor_desc(sa + 2 * C::A_BYTES + C::B_BYTES);
+#pragma unroll
+            for (int k = 0; k < C::BK / C::UMMA_K; ++k) {
+              umma_bf16_cg2(d_tmem, da + 2 * k, dbl + 2 * k, idesc, 1u);
+              umma_bf16_cg2(d_tmem, dal + 2 * k, db + 2 * k, idesc, 1u);
+            }
+          }
           umma_commit_cg2(&empty_bar[stage], 0b11);        // frees the slot in BOTH CTAs when these MMAs retire
           if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
         }
@@ -596,7 +675,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           for (int i = 0; i < 32; ++i) v[i] += bias_s[c * 32 + i];
           if (ep.kind == EPI_GELU) {
 #pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] = gelu_tanh_approx(v[i]);   // tanh.approx: 2^-11, below the bf16 rounding of the output
+            for (int i = 0; i < 32; ++i) v[i] = SPLIT ? gelu_tanh(v[i]) : gelu_tanh_approx(v[i]);   // tanh.approx: 2^-11, below the bf16 rounding of the output (not of a pair)
           } else if (ep.kind == EPI_POS) {
 #pragma unroll
             for (int i = 0; i < 8; ++i) { v[4 * i] += pq[i].x; v[4 * i + 1] += pq[i].y; v[4 * i + 2] += pq[i].z; v[4 * i + 3] += pq[i].w; }
@@ -604,6 +683,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           }
           if (row_ok && n0 + c * 32 < ep.N) {
             if (ep.out_f32) store_row32(reinterpret_cast<float*>(ep.out) + static_cast<size_t>(m) * ep.ldo + n0 + c * 32, v);
+            else if constexpr (SPLIT) VecIO<bf16x3_t, 32>::store(reinterpret_cast<bf16x3_t*>(ep.out) + static_cast<size_t>(m) * ep.ldo + n0 + c * 32, v);
             else store_row32(reinterpret_cast<__nv_bfloat16*>(ep.out) + static_cast<size_t>(m) * ep.ldo + n0 + c * 32, v);
           }
         }

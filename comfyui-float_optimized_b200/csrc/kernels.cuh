@@ -1,7 +1,7 @@
 // Non-GEMM kernels of the FMT sampling step.  All are bandwidth-trivial next to the weight stream; they exist to
 // keep the data in the layout / precision the GEMMs want and to fuse what the reference does in separate torch ops.
-//   AT = activation (GEMM operand) type: __nv_bfloat16 (FMT_MODE_BF16) or float (FMT_MODE_FP32_VALIDATE)
-//   TT = AdaLN table type:               __nv_bfloat16                 or float
+//   AT = activation (GEMM operand) type: __nv_bfloat16 (FMT_MODE_BF16), bf16x3_t (FMT_MODE_BF16X3, gemm.cuh) or float (FMT_MODE_FP32_VALIDATE)
+//   TT = AdaLN table type:               __nv_bfloat16                 float                                   or float
 // Row layout of every activation matrix: m = branch * (B*N) + b * N + f, N = P + L frames (context first) - the
 // same order the reference's batch-concatenated CFG forward uses (FMT.py:360-372).
 #pragma once
@@ -37,6 +37,12 @@ __global__ void set_window_args_kernel(WindowArgs* dst, WindowArgs v) { *dst = v
 template <typename T> __device__ __forceinline__ T from_f32(float v);
 template <> __device__ __forceinline__ float from_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+// *p = v in the activation type; a bf16x3_t element writes its hi and lo parts where the pair layout puts them
+template <typename T> __device__ __forceinline__ void store_act(T* p, float v) { *p = from_f32<T>(v); }
+template <> __device__ __forceinline__ void store_act<bf16x3_t>(bf16x3_t* p, float v) {
+  __nv_bfloat16* hp = split_hi(p);
+  split_bf16(v, hp[0], hp[64]);
+}
 
 // ---------------------------------------------------------------------------------------------------------------
 // Condition rows  [wr | wa | we | 0-pad]  for every (branch, clip, frame)   (FMT.py:312-333, nodes_adv.py:609-627,663-686)
@@ -81,7 +87,7 @@ __global__ void cond_gather_kernel(const WindowArgs* __restrict__ wargs, ModelSh
         }
       }
     }
-    out[j] = from_f32<AT>(v);
+    store_act(out + j, v);
   }
 }
 
@@ -211,9 +217,10 @@ template <> struct RowVec<__nv_bfloat16, 1> { static __device__ __forceinline__ 
 template <> struct RowVec<__nv_bfloat16, 2> { static __device__ __forceinline__ void load(const __nv_bfloat16* p, float (&v)[2]) { __nv_bfloat162 t = *reinterpret_cast<const __nv_bfloat162*>(p); v[0] = __low2float(t); v[1] = __high2float(t); } };
 template <> struct RowVec<__nv_bfloat16, 4> { static __device__ __forceinline__ void load(const __nv_bfloat16* p, float (&v)[4]) { VecIO<__nv_bfloat16, 4>::load(p, v); } };
 
-template <typename AT, int VPL /* head_dim / 32 */>
+// OT: output type (bf16x3 mode reads fp32 q / k / v and writes the proj GEMM's pair operand)
+template <typename AT, int VPL /* head_dim / 32 */, typename OT>
 __global__ void band_attention_kernel(const AT* __restrict__ qkv, int n_seq, int N, int heads, int window, float scale,
-                                      AT* __restrict__ out) {
+                                      OT* __restrict__ out) {
   pdl_launch_dependents();
   pdl_wait_prior_grid();
   const int gw = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -265,11 +272,11 @@ __global__ void band_attention_kernel(const AT* __restrict__ qkv, int n_seq, int
   float o[VPL];
 #pragma unroll
   for (int k = 0; k < VPL; ++k) o[k] = acc[k] * inv;
-  AT* op = out + (static_cast<size_t>(sq) * N + i) * Hd + h * hd + lane * VPL;
-  if constexpr (VPL == 4) VecIO<AT, 4>::store(op, reinterpret_cast<float(&)[4]>(o));
+  OT* op = out + (static_cast<size_t>(sq) * N + i) * Hd + h * hd + lane * VPL;
+  if constexpr (VPL == 4) VecIO<OT, 4>::store(op, reinterpret_cast<float(&)[4]>(o));
   else {
 #pragma unroll
-    for (int k = 0; k < VPL; ++k) op[k] = from_f32<AT>(o[k]);
+    for (int k = 0; k < VPL; ++k) store_act(op + k, o[k]);
   }
 }
 
@@ -444,8 +451,17 @@ __device__ __forceinline__ float cfg_combine(const float* __restrict__ V, size_t
 // branches, FMT.py:363): ax[(br, b, P + f), :] = bf16(y[b, f, :]).  Context rows are written once per window.
 template <typename AT>
 __device__ __forceinline__ void store_ax(const ModelShape& s, AT* __restrict__ ax, int b, int f_full, int j, float v) {
-  const AT t = from_f32<AT>(v);
-  for (int br = 0; br < s.nb; ++br) ax[((static_cast<size_t>(br) * s.B + b) * s.N + f_full) * s.W + j] = t;
+  if constexpr (std::is_same<AT, bf16x3_t>::value) {
+    __nv_bfloat16 hi, lo;
+    split_bf16(v, hi, lo);
+    for (int br = 0; br < s.nb; ++br) {
+      __nv_bfloat16* hp = split_hi(ax + ((static_cast<size_t>(br) * s.B + b) * s.N + f_full) * s.W + j);
+      hp[0] = hi; hp[64] = lo;
+    }
+  } else {
+    const AT t = from_f32<AT>(v);
+    for (int br = 0; br < s.nb; ++br) ax[((static_cast<size_t>(br) * s.B + b) * s.N + f_full) * s.W + j] = t;
+  }
 }
 
 // mode 0: v_full[b, f, :] = combined, all N frames (fmt_velocity)
@@ -549,6 +565,17 @@ __global__ void f32_to_bf16_kernel(const float* __restrict__ src, __nv_bfloat16*
     uint4 t;
     t.x = pack_bf16x2(a.x, a.y); t.y = pack_bf16x2(a.z, a.w); t.z = pack_bf16x2(b.x, b.y); t.w = pack_bf16x2(b.z, b.w);
     reinterpret_cast<uint4*>(dst)[i] = t;
+  }
+}
+
+// fp32 -> bf16x3 pairs, 4 elements per thread: the weights (once per handle, from Linear::w32) and the audio-projection input.
+// Rows must hold a multiple of 64 elements (n4 = elements / 4).
+__global__ void f32_to_split_kernel(const float* __restrict__ src, bf16x3_t* __restrict__ dst, size_t n4) {
+  const size_t stride = static_cast<size_t>(gridDim.x) * blockDim.x;
+  for (size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n4; i += stride) {
+    const float4 a = __ldcs(reinterpret_cast<const float4*>(src) + i);
+    const float v[4] = {a.x, a.y, a.z, a.w};
+    VecIO<bf16x3_t, 4>::store(dst + 4 * i, v);
   }
 }
 

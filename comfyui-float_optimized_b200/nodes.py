@@ -30,10 +30,14 @@ def _progress_bar(total):
 
 # Optional widget both sampler nodes add to the reference's inputs (everything else is identical).  "default" = the FMT_MODE
 # environment variable, else bf16.  The reference computes in fp32: "fp32" reproduces it to 1e-4 relative (and passes the
-# PSNR >= 40 dB decoded-frame gate); "bf16" is ~10x faster and within 2e-2 max-abs of the reference latents, which a
-# RANDOM-INIT decoder turns into 20-35 dB (profiles/r02_psnr.json) - see README.md "Precision".
-PRECISION_WIDGET = (("default",) + PRECISION_MODES, {"default": "default", "tooltip": "GEMM operand precision: bf16 (fast, tcgen05) or fp32 "
-                                                     "(validation mode, matches the reference to 1e-4). default = $FMT_MODE or bf16."})
+# PSNR >= 40 dB decoded-frame gate); "bf16" is the fastest and within 2e-2 max-abs of the reference latents, which a
+# RANDOM-INIT decoder turns into 20-35 dB (profiles/r02_psnr.json); "bf16x3" meets the fp32 mode's gates on the tensor pipe
+# (split bf16 operands) - see README.md "Precision".
+PRECISION_WIDGET = (("default",) + PRECISION_MODES, {"default": "default", "tooltip": "GEMM operand precision: bf16 (fastest, tcgen05); "
+                                                     "fp32 (validation mode, matches the reference to 1e-4, slowest); bf16x3 (matches the "
+                                                     "reference like fp32 at tensor-core speed: every GEMM operand is split into two bf16 and "
+                                                     "costs three MMAs, so its GEMMs take ~3x their bf16 time, and the first use packs 627 MB more "
+                                                     "weights). default = $FMT_MODE or bf16."})
 
 
 # Second optional widget (SURVEY.md 8f rank 2, second half): the reference moves every tensor back to the CPU between nodes

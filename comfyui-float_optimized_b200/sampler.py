@@ -104,13 +104,15 @@ def _build_schedule(nfe: int, method: str):
     return dict(n_steps=max(0, int(nfe) - 1), n_stages=stages, t_eval=t_eval, dt=[float(x) for x in dt], a=a_flat, b=tab["b"])
 
 
-PRECISION_MODES = ("bf16", "fp32")
+PRECISION_MODES = ("bf16", "fp32", "bf16x3")
 
 
 def resolve_mode(mode: Optional[str] = None) -> str:
     """Operand precision of the GEMMs: "bf16" (tcgen05, fp32 accumulate / residual / softmax / ODE state; latents within 2e-2
-    max-abs of the reference) or "fp32" (validation mode, fp32 FFMA GEMMs; within 1e-4 relative, ~10x slower).  An explicit
-    argument wins, then the environment variable FMT_MODE, then "bf16".  The reference itself computes in fp32."""
+    max-abs of the reference), "fp32" (validation mode, fp32 FFMA GEMMs; within 1e-4 relative, the slowest) or "bf16x3" (tcgen05
+    on operands split into two bf16 each, x = hi + lo, three MMAs per product; within 1e-4 relative like "fp32", faster than it,
+    and the weights are packed once more, 627 MB for the FMT).  An explicit argument wins, then the environment variable
+    FMT_MODE, then "bf16".  The reference itself computes in fp32."""
     m = mode if mode not in (None, "", "default") else os.environ.get("FMT_MODE", "bf16")
     m = str(m).lower()
     if m not in PRECISION_MODES:
@@ -180,7 +182,7 @@ class FmtBackend:
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     def configure(self, batch: int, n_branches: int, we_dynamic: bool, nfe: int, method: str = "euler", mode: str = "bf16"):
-        mode_id = {"bf16": _cabi.FMT_MODE_BF16, "fp32": _cabi.FMT_MODE_FP32_VALIDATE}[resolve_mode(mode)]
+        mode_id = _cabi.MODE_IDS[resolve_mode(mode)]
         key = (batch, n_branches, bool(we_dynamic), int(nfe), method, mode_id)
         if key == self._plan_key:
             return

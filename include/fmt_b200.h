@@ -29,7 +29,7 @@ extern "C" {
 #endif
 
 #define FMT_API __attribute__((visibility("default")))
-#define FMT_ABI_VERSION 1
+#define FMT_ABI_VERSION 2
 
 typedef struct FmtHandle FmtHandle;
 
@@ -81,7 +81,12 @@ enum {
 
 enum { FMT_LOC_DEVICE = 0, FMT_LOC_HOST = 1 };
 enum { FMT_MODE_BF16 = 0,       /* bf16 tcgen05/TMA GEMMs, fp32 accumulate / residual / LN / softmax / ODE state */
-       FMT_MODE_FP32_VALIDATE = 1 /* same kernels' epilogues + fp32 SIMT GEMMs: the 1e-4 parity mode          */ };
+       FMT_MODE_FP32_VALIDATE = 1, /* same kernels' epilogues + fp32 SIMT GEMMs: the 1e-4 parity mode         */
+       FMT_MODE_BF16X3 = 2         /* tcgen05 GEMMs on split operands x = hi + lo (two bf16 each), Ah.Wh + Ah.Wl + Al.Wh in fp32:
+                                      fp32-class accuracy (the 1e-4 gates) on the tensor pipe; AdaLN tables, QKV and every
+                                      non-GEMM step in fp32.  The first plan in this mode packs the weights once more
+                                      (4 bytes per weight: 627 MB for the FMT).  Plans of <= 256 token rows run one kernel per
+                                      op (the persistent window kernels are bf16-only).                                    */ };
 
 #define FMT_MAX_STAGES 4
 
@@ -135,7 +140,7 @@ typedef struct FmtEval {
 FMT_API int32_t fmt_abi_version(void);
 FMT_API const char* fmt_last_error(void);
 
-/* Packs the reference's fp32 weights into resident bf16 (and keeps fp32 for the validation mode).
+/* Packs the reference's fp32 weights into resident bf16 (and keeps fp32 for the validation mode and the bf16x3 packing).
  * weight_ptrs: FMT_W_NUM_GLOBAL + depth*FMT_W_PER_BLOCK pointers, all at `location`. */
 FMT_API int32_t fmt_create(const FmtDims* dims, const void* const* weight_ptrs, int32_t n_ptrs, int32_t location,
                            int32_t device, FmtHandle** out);
@@ -190,6 +195,15 @@ FMT_API int32_t fmt_debug_gemm_bf16(const void* A, const void* W, const float* b
 /* `iters` back-to-back launches of one GEMM variant (bf16 output); block_n as above, 512 / 1024 = CTA-pair kernel. */
 FMT_API int32_t fmt_debug_gemm_bench(const void* A, const void* W, const float* bias, float* out, int32_t M, int32_t N,
                                      int32_t K, int32_t block_n, int32_t iters, void* stream);
+/* out[M,N] (fp32) = A[M,K] (fp32) @ W[N,K]^T (fp32) + bias[N] through the bf16x3 GEMM of FMT_MODE_BF16X3: the operands are split
+ * into hi / lo bf16 pairs on the device (K % 64 == 0).  block_n as in fmt_debug_gemm_bf16: 64 / 128 / 256 single-CTA kernel,
+ * 512 / 1024 CTA-pair kernel, 0 = the choice the sampler makes. */
+FMT_API int32_t fmt_debug_gemm_bf16x3(const float* A, const float* W, const float* bias, float* out, int32_t M, int32_t N,
+                                      int32_t K, int32_t block_n, void* stream);
+/* `iters` back-to-back launches of one bf16x3 GEMM variant, fp32 output.  A (M, 2K) and W (N, 2K) are bf16 bits already in the pair
+ * layout: every 64-column K block of hi = bf16(x) followed by the same block of lo = bf16(x - hi). */
+FMT_API int32_t fmt_debug_gemm_bench_bf16x3(const void* A, const void* W, const float* bias, float* out, int32_t M, int32_t N,
+                                            int32_t K, int32_t block_n, int32_t iters, void* stream);
 /* Same through the fp32 SIMT GEMM used by FMT_MODE_FP32_VALIDATE (A, W fp32). */
 FMT_API int32_t fmt_debug_gemm_fp32(const float* A, const float* W, const float* bias, float* out, int32_t M, int32_t N,
                                     int32_t K, void* stream);
