@@ -49,6 +49,14 @@ class FmtClip(C.Structure):
                 ("progress", PROGRESS_FN), ("progress_user", C.c_void_p)]
 
 
+class FmtClipSet(C.Structure):
+    _fields_ = [("n_clips", C.c_int32), ("r_s", C.POINTER(C.c_void_p)), ("wa", C.POINTER(C.c_void_p)), ("we", C.POINTER(C.c_void_p)),
+                ("noise", C.POINTER(C.c_void_p)), ("r_d", C.POINTER(C.c_void_p)), ("T_wa", C.POINTER(C.c_int32)),
+                ("T_we", C.POINTER(C.c_int32)), ("audio_num_frames", C.POINTER(C.c_int32)),
+                ("a_cfg_scale", C.c_float), ("r_cfg_scale", C.c_float), ("e_cfg_scale", C.c_float),
+                ("progress", PROGRESS_FN), ("progress_user", C.c_void_p)]
+
+
 class FmtEval(C.Structure):
     _fields_ = [("x", C.c_void_p), ("prev_x", C.c_void_p), ("wa", C.c_void_p), ("prev_wa", C.c_void_p), ("we", C.c_void_p),
                 ("prev_we", C.c_void_p), ("r_s", C.c_void_p), ("v_out", C.c_void_p), ("eval_index", C.c_int32),
@@ -63,6 +71,9 @@ _SIGNATURES = {
     "fmt_configure": (C.c_int32, [C.c_void_p, C.POINTER(FmtPlan), C.c_void_p]),
     "fmt_workspace_bytes": (C.c_int64, [C.c_void_p]),
     "fmt_sample_clip": (C.c_int32, [C.c_void_p, C.POINTER(FmtClip), C.c_void_p]),
+    "fmt_sample_clips": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.c_void_p]),
+    "fmt_clip_schedule": (C.c_int32, [C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                      C.POINTER(C.c_int32)]),
     "fmt_velocity": (C.c_int32, [C.c_void_p, C.POINTER(FmtEval), C.c_void_p]),
     "fmt_launch_count": (C.c_int64, [C.c_void_p, C.c_int32]),
     "fmt_graph_kernel_nodes": (C.c_int32, [C.c_void_p]),

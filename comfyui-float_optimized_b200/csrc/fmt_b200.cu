@@ -9,7 +9,9 @@
 #include "flow.cuh"
 
 #include <algorithm>
+#include <functional>
 #include <map>
+#include <queue>
 #include <tuple>
 #include <cstdlib>
 
@@ -91,6 +93,12 @@ struct FmtHandle {
   bool dedup = false;                            // U < R: the AdaLN tables hold one row per DISTINCT condition row (FMT_DEDUP=0 switches it off)
   int use_dedup = 1;
   DevBuf st_rs, st_wa, st_we, st_noise, st_rd;   // staging for host-located clips
+  // fmt_sample_clips: the slot records of every window of a call ([window][slot]), uploaded with one copy from a pinned staging
+  // buffer; slot_ev marks the end of that copy, so the next call waits for it before it refills the staging buffer
+  DevBuf slot_buf, slot_zero;                    // slot_zero: the inputs of an idle slot
+  SlotArgs* slot_host = nullptr;
+  size_t slot_host_n = 0;
+  cudaEvent_t slot_ev = nullptr;
   bool use_splitk = false;                       // 2-way K slicing of gate+residual GEMMs with a ragged last wave (FMT_SPLITK=1; measured 3 % slower at 32 clips)
   int raster_gm = 8;                             // FMT_RASTER_GM
   bool use_pair = true;                          // CTA-pair (cta_group::2) GEMM for M >= 512 (FMT_PAIR=0 disables)
@@ -1051,10 +1059,13 @@ int32_t fmt_destroy(FmtHandle* h) {
   DevBuf* bufs[] = {&h->cond, &h->cemb, &h->temb, &h->tfreq, &h->th, &h->silu, &h->table, &h->xstate, &h->ystage, &h->kbuf, &h->prevx, &h->ax,
                     &h->X, &h->A1, &h->QKV, &h->A2, &h->Hm, &h->V, &h->ddt, &h->dteval, &h->wargs, &h->st_rs, &h->st_wa, &h->st_we, &h->st_noise, &h->st_rd,
                     &h->win_params, &h->win_tmaps, &h->win_acc, &h->win_bar, &h->win_trace, &h->win_act,
-                    &h->flow_gemms, &h->flow_tmaps, &h->flow_acc, &h->flow_act, &h->flow_flags, &h->flow_trace, &h->urow_buf, &h->uidx_buf};
+                    &h->flow_gemms, &h->flow_tmaps, &h->flow_acc, &h->flow_act, &h->flow_flags, &h->flow_trace, &h->urow_buf, &h->uidx_buf,
+                    &h->slot_buf, &h->slot_zero};
   for (DevBuf* b : bufs)
     if (b->p) cudaFree(b->p);
   if (h->win_err_host) cudaFreeHost(h->win_err_host);
+  if (h->slot_host) cudaFreeHost(h->slot_host);
+  if (h->slot_ev) cudaEventDestroy(h->slot_ev);
   delete h;
   return 0;
 }
@@ -1127,6 +1138,52 @@ int32_t fmt_debug_condition_rows(int32_t n_branches, int32_t batch, int32_t n_fr
   distinct_condition_rows(s, urow, uidx);
   if (urow_out != nullptr) std::copy(urow.begin(), urow.end(), urow_out);
   return static_cast<int32_t>(uidx.size());
+}
+
+// Slot schedule of fmt_sample_clips.  List scheduling in order of window count, descending (ties in input order): each clip goes to
+// the slot that is free first (ties: the lowest slot) and starts at its own window 0 in the window that slot becomes free.
+static const int kMaxSlots = 256;
+static int list_schedule(const std::vector<int>& order, const int32_t* n_win, int n_slots, int32_t* slot, int32_t* start) {
+  typedef std::pair<int, int> FreeAt;            // (first free window, slot)
+  std::priority_queue<FreeAt, std::vector<FreeAt>, std::greater<FreeAt>> q;
+  for (int k = 0; k < n_slots; ++k) q.push(FreeAt(0, k));
+  int makespan = 0;
+  for (int i : order) {
+    const FreeAt f = q.top();
+    q.pop();
+    if (slot) slot[i] = f.second;
+    if (start) start[i] = f.first;
+    q.push(FreeAt(f.first + n_win[i], f.second));
+    makespan = std::max(makespan, f.first + n_win[i]);
+  }
+  return makespan;
+}
+
+// n_slots = 0: the smallest slot count whose schedule ends with the longest clip (which bounds the call anyway), at most kMaxSlots
+static int clip_schedule(int n, const int32_t* n_win, int n_slots, int32_t* slot, int32_t* start, int* makespan) {
+  std::vector<int> order(n);
+  long long total = 0;
+  int longest = 0;
+  for (int i = 0; i < n; ++i) { order[i] = i; total += n_win[i]; longest = std::max(longest, static_cast<int>(n_win[i])); }
+  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return n_win[a] > n_win[b]; });
+  int S = n_slots;
+  if (S == 0) {
+    S = kMaxSlots;
+    for (long long k = (total + longest - 1) / longest; k < kMaxSlots; ++k)      // fewer slots than total / longest cannot finish in time
+      if (list_schedule(order, n_win, static_cast<int>(k), nullptr, nullptr) == longest) { S = static_cast<int>(k); break; }
+  }
+  *makespan = list_schedule(order, n_win, S, slot, start);
+  return S;
+}
+
+int32_t fmt_clip_schedule(int32_t n_clips, const int32_t* n_windows, int32_t n_slots, int32_t* slot_out, int32_t* start_out, int32_t* makespan_out) {
+  if (n_clips < 1 || n_windows == nullptr || n_slots < 0 || n_slots > kMaxSlots) return -1;
+  for (int i = 0; i < n_clips; ++i)
+    if (n_windows[i] < 1) return -1;
+  int makespan = 0;
+  const int S = clip_schedule(n_clips, n_windows, n_slots, slot_out, start_out, &makespan);
+  if (makespan_out != nullptr) *makespan_out = makespan;
+  return S;
 }
 
 static bool same_plan(const FmtHandle* h, const FmtPlan* p) {
@@ -1362,6 +1419,77 @@ int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
     CUDA_OK(cudaStreamSynchronize(st));
     // the persistent kernels report a tripped bounded spin through a mapped status word (the launch fails as well)
     if (h->window_active && h->win_err_host && *h->win_err_host != 0) return set_err(-6, "window kernel reported status 0x%08x", *h->win_err_host);
+  }
+  return 0;
+}
+
+// Many clips on plan.batch slots: window w of the call runs, in slot k, whichever clip the schedule put there (at that clip's own
+// window), through the same captured window graph; only cond_gather / init_window / finalize_window read the per-slot records.
+int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) {
+  REQUIRE(h && cs, "fmt_sample_clips: null argument");
+  REQUIRE(h->configured, "fmt_sample_clips: call fmt_configure first");
+  const int n = cs->n_clips;
+  REQUIRE(n >= 1, "fmt_sample_clips: no clips");
+  REQUIRE(cs->r_s && cs->wa && cs->we && cs->noise && cs->r_d && cs->T_wa && cs->T_we && cs->audio_num_frames, "fmt_sample_clips: null array");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CUDA_OK(cudaSetDevice(h->device));
+  const ModelShape& s = h->shape;
+  std::vector<int32_t> n_win(n), slot(n), start(n);
+  for (int i = 0; i < n; ++i) {   // fmt_sample_clip's checks, per clip
+    REQUIRE(cs->r_s[i] && cs->wa[i] && cs->we[i] && cs->noise[i] && cs->r_d[i], "fmt_sample_clips: clip %d: null tensor pointer", i);
+    const int T = cs->audio_num_frames[i], T_wa = cs->T_wa[i], T_we = cs->T_we[i];
+    REQUIRE(T >= 1 && T_wa >= 1 && T_we >= 1, "fmt_sample_clips: clip %d is empty", i);
+    REQUIRE(s.we_dynamic ? T_we > 1 : T_we == 1, "fmt_sample_clips: clip %d: T_we=%d does not match plan.we_dynamic=%d", i, T_we, s.we_dynamic);
+    n_win[i] = (T + s.L - 1) / s.L;
+    REQUIRE((n_win[i] - 1) * s.L < T_wa, "fmt_sample_clips: clip %d: wa has %d frames but window %d starts at frame %d", i, T_wa, n_win[i] - 1,
+            (n_win[i] - 1) * s.L);
+    REQUIRE(!s.we_dynamic || (n_win[i] - 1) * s.L < T_we, "fmt_sample_clips: clip %d: dynamic we has %d frames but the last window starts at %d",
+            i, T_we, (n_win[i] - 1) * s.L);
+  }
+  int makespan = 0;
+  const int S = clip_schedule(n, n_win.data(), 0, slot.data(), start.data(), &makespan);
+  REQUIRE(s.B == S, "fmt_sample_clips: the plan has batch %d, but these %d clips are scheduled on %d slots (fmt_clip_schedule)", s.B, n, S);
+
+  // idle slots read zeros: (L, W) noise, and r_s / wa / we rows no wider than that
+  const size_t n_zero = std::max<size_t>(static_cast<size_t>(s.L) * s.W, static_cast<size_t>(std::max(s.A, s.E)));
+  FMT_OK(dev_alloc(h, h->slot_zero, n_zero * sizeof(float)));
+  CUDA_OK(cudaMemsetAsync(h->slot_zero.p, 0, n_zero * sizeof(float), st));
+  const float* zero = static_cast<const float*>(h->slot_zero.p);
+  const size_t n_rec = static_cast<size_t>(makespan) * S;
+  if (h->slot_ev) CUDA_OK(cudaEventSynchronize(h->slot_ev));   // the previous call's upload has read the staging buffer
+  if (h->slot_host_n < n_rec) {
+    if (h->slot_host) { CUDA_OK(cudaFreeHost(h->slot_host)); h->slot_host = nullptr; h->slot_host_n = 0; }
+    CUDA_OK(cudaHostAlloc(reinterpret_cast<void**>(&h->slot_host), n_rec * sizeof(SlotArgs), cudaHostAllocDefault));
+    h->slot_host_n = n_rec;
+  }
+  SlotArgs* rec = h->slot_host;
+  for (size_t r = 0; r < n_rec; ++r) {
+    SlotArgs& z = rec[r];
+    z.r_s = zero; z.wa = zero; z.we = zero; z.x0 = zero; z.r_d = nullptr;
+    z.T_wa = 1; z.T_we = 1; z.T_out = 0; z.win_start = 0; z.first_window = 1;
+  }
+  for (int i = 0; i < n; ++i) {
+    for (int w = 0; w < n_win[i]; ++w) {
+      SlotArgs& z = rec[static_cast<size_t>(start[i] + w) * S + slot[i]];
+      z.r_s = cs->r_s[i]; z.wa = cs->wa[i]; z.we = cs->we[i]; z.r_d = cs->r_d[i];
+      z.x0 = cs->noise[i] + static_cast<size_t>(w) * s.L * s.W;
+      z.T_wa = cs->T_wa[i]; z.T_we = cs->T_we[i]; z.T_out = cs->audio_num_frames[i];
+      z.win_start = w * s.L; z.first_window = (w == 0);
+    }
+  }
+  FMT_OK(dev_alloc(h, h->slot_buf, n_rec * sizeof(SlotArgs)));
+  CUDA_OK(cudaMemcpyAsync(h->slot_buf.p, rec, n_rec * sizeof(SlotArgs), cudaMemcpyHostToDevice, st));
+  if (!h->slot_ev) CUDA_OK(cudaEventCreateWithFlags(&h->slot_ev, cudaEventDisableTiming));
+  CUDA_OK(cudaEventRecord(h->slot_ev, st));
+  const SlotArgs* base = static_cast<const SlotArgs*>(h->slot_buf.p);
+  for (int w = 0; w < makespan; ++w) {
+    WindowArgs a{};
+    a.slots = base + static_cast<size_t>(w) * S;
+    a.a_scale = cs->a_cfg_scale; a.r_scale = cs->r_cfg_scale; a.e_scale = cs->e_cfg_scale;
+    FMT_OK(set_wargs(h, a, st));
+    CUDA_OK(cudaGraphLaunch(h->graph_exec, st));
+    h->launches += h->capture_launches;
+    if (cs->progress) cs->progress(w, makespan, cs->progress_user);
   }
   return 0;
 }

@@ -9,6 +9,19 @@
 
 namespace fmt {
 
+// What one batch slot computes in one window of fmt_sample_clips: a window of its own clip (tensors of that clip alone, batch 1).
+// An idle slot points at zeros, has r_d == nullptr and first_window == 1: it is computed and its output is dropped.
+struct SlotArgs {
+  const float* r_s;        // (W)
+  const float* wa;         // (T_wa, A)
+  const float* we;         // (T_we, E)
+  const float* x0;         // (L, W) noise of this window of the clip
+  float* r_d;              // (T_out, W), or nullptr for an idle slot
+  int T_wa, T_we, T_out;
+  int win_start;           // first frame of this window in the clip
+  int first_window;        // 1: the clip starts in this window: zero context, whatever the slot ran before
+};
+
 // Per-window arguments, written to device memory by set_window_args so that the captured graph never changes.
 struct WindowArgs {
   const float* r_s;        // (B, W)
@@ -24,6 +37,7 @@ struct WindowArgs {
   int first_window;        // 1: context is all-zero (nodes_adv.py:591-593)
   int use_ext;             // 1: prev_* come from the *_ext pointers
   float a_scale, r_scale, e_scale;
+  const SlotArgs* slots;   // (B) per-slot clip arguments (fmt_sample_clips): replace r_s .. first_window above; nullptr elsewhere
 };
 
 struct ModelShape {
@@ -59,31 +73,39 @@ __global__ void cond_gather_kernel(const WindowArgs* __restrict__ wargs, ModelSh
   const int br = row / (s.B * s.N), b = (row / s.N) % s.B, f = row % s.N;
   const bool za = (s.null_a >> br) & 1, zr = (s.null_r >> br) & 1, ze = (s.null_e >> br) & 1;
   const bool ctx = f < s.P;
+  // the clip this row belongs to: clip b of the batch, or the clip that slot b runs (fmt_sample_clips; its tensors have batch 1)
+  const float *r_s = a.r_s, *wa = a.wa, *we = a.we;
+  int cb = b, T_wa = a.T_wa, T_we = a.T_we, win_start = a.win_start, first_window = a.first_window;
+  if (a.slots != nullptr) {
+    const SlotArgs& sl = a.slots[b];
+    r_s = sl.r_s; wa = sl.wa; we = sl.we; cb = 0;
+    T_wa = sl.T_wa; T_we = sl.T_we; win_start = sl.win_start; first_window = sl.first_window;
+  }
   // frame of the clip this row looks at; replicate padding == clamp to the last available frame
-  const int g = a.win_start + f - s.P;
+  const int g = win_start + f - s.P;
   AT* out = cond + static_cast<size_t>(blockIdx.x) * s.Kc;
   for (int j = threadIdx.x; j < s.Kc; j += blockDim.x) {
     float v = 0.f;
     if (j < s.W) {
-      v = zr ? 0.f : a.r_s[static_cast<size_t>(b) * s.W + j];
+      v = zr ? 0.f : r_s[static_cast<size_t>(cb) * s.W + j];
     } else if (j < s.W + s.A) {
       const int k = j - s.W;
       if (ctx) {   // prev_wa is replicated un-nulled in every branch (FMT.py:366,388)
         if (a.use_ext) v = a.prev_wa_ext[(static_cast<size_t>(b) * s.P + f) * s.A + k];
-        else if (!a.first_window) v = a.wa[(static_cast<size_t>(b) * a.T_wa + min(g, a.T_wa - 1)) * s.A + k];
+        else if (!first_window) v = wa[(static_cast<size_t>(cb) * T_wa + min(g, T_wa - 1)) * s.A + k];
       } else if (!za) {
-        v = a.wa[(static_cast<size_t>(b) * a.T_wa + min(g, a.T_wa - 1)) * s.A + k];
+        v = wa[(static_cast<size_t>(cb) * T_wa + min(g, T_wa - 1)) * s.A + k];
       }
     } else if (j < s.W + s.A + s.E) {
       const int k = j - s.W - s.A;
       if (!ze) {
         if (!s.we_dynamic) {
-          v = a.we[static_cast<size_t>(b) * s.E + k];     // static emotion covers the context frames too (FMT.py:325-326)
+          v = we[static_cast<size_t>(cb) * s.E + k];     // static emotion covers the context frames too (FMT.py:325-326)
         } else if (ctx) {
           if (a.use_ext) v = a.prev_we_ext[(static_cast<size_t>(b) * s.P + f) * s.E + k];
-          else if (!a.first_window) v = a.we[(static_cast<size_t>(b) * a.T_we + min(g, a.T_we - 1)) * s.E + k];
+          else if (!first_window) v = we[(static_cast<size_t>(cb) * T_we + min(g, T_we - 1)) * s.E + k];
         } else {
-          v = a.we[(static_cast<size_t>(b) * a.T_we + min(g, a.T_we - 1)) * s.E + k];
+          v = we[(static_cast<size_t>(cb) * T_we + min(g, T_we - 1)) * s.E + k];
         }
       }
     }
@@ -521,14 +543,18 @@ __global__ void init_window_kernel(const WindowArgs* __restrict__ wargs, ModelSh
   const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<size_t>(s.B) * s.N * s.W) return;
   const int j = static_cast<int>(i % s.W), f = static_cast<int>((i / s.W) % s.N), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.N));
+  // per slot (fmt_sample_clips): the slot's own noise (L, W) and context reset
+  const float* x0 = a.x0;
+  int cb = b, first_window = a.first_window;
+  if (a.slots != nullptr) { x0 = a.slots[b].x0; first_window = a.slots[b].first_window; cb = 0; }
   float v;
   if (f < s.P) {
     const size_t o = (static_cast<size_t>(b) * s.P + f) * s.W + j;
-    if (a.first_window) { v = 0.f; prev_x_state[o] = 0.f; }
+    if (first_window) { v = 0.f; prev_x_state[o] = 0.f; }
     else v = prev_x_state[o];
   } else {
     const size_t o = (static_cast<size_t>(b) * s.L + (f - s.P)) * s.W + j;
-    v = a.x0[o];
+    v = x0[(static_cast<size_t>(cb) * s.L + (f - s.P)) * s.W + j];
     x_state[o] = v;
   }
   store_ax<AT>(s, ax, b, f, j, v);
@@ -543,8 +569,12 @@ __global__ void finalize_window_kernel(const WindowArgs* __restrict__ wargs, Mod
   if (i >= static_cast<size_t>(s.B) * s.L * s.W) return;
   const int j = static_cast<int>(i % s.W), f = static_cast<int>((i / s.W) % s.L), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.L));
   const float v = x_state[i];
-  const int g = a.win_start + f;
-  if (a.r_d != nullptr && g < a.T_out) a.r_d[(static_cast<size_t>(b) * a.T_out + g) * s.W + j] = v;
+  // per slot (fmt_sample_clips): frames below the slot's own clip length, into that clip's output; idle slots write nothing
+  float* r_d = a.r_d;
+  int cb = b, T_out = a.T_out, win_start = a.win_start;
+  if (a.slots != nullptr) { const SlotArgs& sl = a.slots[b]; r_d = sl.r_d; T_out = sl.T_out; win_start = sl.win_start; cb = 0; }
+  const int g = win_start + f;
+  if (r_d != nullptr && g < T_out) r_d[(static_cast<size_t>(cb) * T_out + g) * s.W + j] = v;
   if (f >= s.L - s.P) prev_x_state[(static_cast<size_t>(b) * s.P + (f - (s.L - s.P))) * s.W + j] = v;
 }
 

@@ -13,7 +13,7 @@ import math
 import os
 import weakref
 from dataclasses import dataclass
-from typing import Callable, Dict, Optional
+from typing import Callable, Dict, List, Mapping, Optional, Sequence
 
 import torch
 
@@ -270,6 +270,61 @@ class FmtBackend:
             _cabi.check(self.lib.fmt_sample_clip(self._handle, C.byref(clip), self._stream()), "fmt_sample_clip")
         return out
 
+    def sample_clips(self, r_s, wa, we, audio_num_frames, noise, a_cfg_scale, r_cfg_scale, e_cfg_scale,
+                     progress: Optional[Callable[[int, int], None]] = None, out: Optional[Sequence[torch.Tensor]] = None) -> List[torch.Tensor]:
+        """Many clips of different lengths in one call on the plan's batch of slots (:func:`clip_schedule`).  Per clip i: r_s[i]
+        (1, dim_w), wa[i] (1, T_wa, dim_a), we[i] (1, 1 or T_we, dim_e), noise[i] (n_win_i, L, dim_w) or (n_win_i, 1, L, dim_w), all on
+        ``self.device`` (fp32, contiguous).  Returns one (1, audio_num_frames[i], dim_w) tensor per clip (``out[i]`` if given: any
+        contiguous fp32 tensor of that many elements); asynchronous."""
+        d = self.dims
+        if self._plan_key is None:
+            raise FmtError("sample_clips: configure() has not been called")
+        n = len(wa)
+        if n < 1 or not all(len(x) == n for x in (r_s, we, audio_num_frames, noise)) or (out is not None and len(out) != n):
+            raise ValueError("sample_clips: r_s, wa, we, audio_num_frames, noise (and out) need one entry per clip")
+        L = d.frames_per_clip
+        dynamic = self._plan_key[2]
+        outs = []
+        for i in range(n):
+            for name, t in (("r_s", r_s[i]), ("wa", wa[i]), ("we", we[i]), ("noise", noise[i])):
+                if not torch.is_tensor(t):
+                    raise TypeError(f"clip {i}: {name} must be a torch.Tensor")
+                if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device:
+                    raise ValueError(f"clip {i}: {name} must be a contiguous float32 tensor on {self.device}")
+            T = int(audio_num_frames[i])
+            n_win = -(-T // L)
+            if T < 1:
+                raise ValueError(f"clip {i}: audio_num_frames must be >= 1 (got {T})")
+            if wa[i].dim() != 3 or wa[i].shape[0] != 1 or wa[i].shape[2] != d.dim_a or (n_win - 1) * L >= wa[i].shape[1]:
+                raise ValueError(f"clip {i}: wa shape {tuple(wa[i].shape)} != (1, T > {(n_win - 1) * L}, dim_a={d.dim_a})")
+            if r_s[i].shape[0] != 1 or r_s[i].numel() != d.dim_w:
+                raise ValueError(f"clip {i}: r_s shape {tuple(r_s[i].shape)} != (1, dim_w={d.dim_w})")
+            if we[i].dim() != 3 or we[i].shape[0] != 1 or we[i].shape[2] != d.dim_e or dynamic != (we[i].shape[1] > 1):
+                raise ValueError(f"clip {i}: we shape {tuple(we[i].shape)} does not match (1, {'T' if dynamic else 1}, dim_e={d.dim_e})")
+            if tuple(noise[i].shape) not in ((n_win, L, d.dim_w), (n_win, 1, L, d.dim_w)):
+                raise ValueError(f"clip {i}: noise shape {tuple(noise[i].shape)} != {(n_win, L, d.dim_w)}")
+            if out is None:
+                outs.append(torch.empty(1, T, d.dim_w, device=self.device, dtype=torch.float32))
+            else:
+                o = out[i]
+                if o.numel() != T * d.dim_w or o.dtype != torch.float32 or not o.is_contiguous() or o.device != self.device:
+                    raise ValueError(f"clip {i}: out must be a contiguous float32 tensor of {T} x {d.dim_w} elements on {self.device}")
+                outs.append(o)
+
+        def ptrs(ts):
+            return (C.c_void_p * n)(*[t.data_ptr() for t in ts])
+
+        def ints(vals):
+            return (C.c_int32 * n)(*[int(v) for v in vals])
+
+        cb = _cabi.PROGRESS_FN(lambda w, m, _u: progress(w, m)) if progress is not None else _cabi.PROGRESS_FN(0)
+        cs = _cabi.FmtClipSet(n, ptrs(r_s), ptrs(wa), ptrs(we), ptrs(noise), ptrs(outs), ints(t.shape[1] for t in wa),
+                              ints(t.shape[1] for t in we), ints(audio_num_frames), float(a_cfg_scale), float(r_cfg_scale),
+                              float(e_cfg_scale), cb, None)
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.fmt_sample_clips(self._handle, C.byref(cs), self._stream()), "fmt_sample_clips")
+        return outs
+
     def velocity(self, eval_index: int, x, wa, r_s, we, prev_x, prev_wa, prev_we, a_cfg_scale, r_cfg_scale, e_cfg_scale) -> torch.Tensor:
         """One ``forward_with_cfv`` (FMT.py:342-401) at plan time ``t_eval[eval_index]``; returns (B, P+L, dim_w)."""
         d = self.dims
@@ -312,6 +367,11 @@ def _weights_fingerprint(sd) -> tuple:
     return tuple((k, v.data_ptr(), getattr(v, "_version", 0), tuple(v.shape)) for k, v in sd.items() if torch.is_tensor(v))
 
 
+def _model_dims(fmt_model, sd) -> Dims:
+    src = getattr(fmt_model, "final_construction_options", None) or getattr(fmt_model, "opt", None) or {}
+    return Dims.from_options(src, sd)
+
+
 def backend_for(fmt_model, device, dims: Optional[Dims] = None) -> FmtBackend:
     """``fmt_model``: anything with ``state_dict()`` (the reference ``FlowMatchingTransformer`` or :class:`FmtModel`)."""
     device = torch.device(device)
@@ -327,8 +387,7 @@ def backend_for(fmt_model, device, dims: Optional[Dims] = None) -> FmtBackend:
     if hit is not None and hit[0] == fp:
         return hit[1]
     if dims is None:
-        src = getattr(fmt_model, "final_construction_options", None) or getattr(fmt_model, "opt", None) or {}
-        dims = Dims.from_options(src, sd)
+        dims = _model_dims(fmt_model, sd)
     if hit is not None:
         hit[1].close()
     be = FmtBackend(sd, dims, device)
@@ -389,6 +448,109 @@ def perform_ode_sampling_loop(fmt_model, r_s_latent_dev, wa_latent_dev, we_laten
         raise ValueError(f"noise shape {tuple(noise.shape)} != {(n_win, B, d.frames_per_clip, d.dim_w)}")
     progress = (lambda w, n: progress_bar.update(1)) if progress_bar is not None else None
     return be.sample_clip(r_s, wa, we, int(audio_num_frames), noise, a_cfg_scale, r_cfg_scale, e_cfg_scale, progress)
+
+
+# ----------------------------------------------------------------------------------------------------
+# many clips of different lengths in one call: B slots, refilled as clips finish
+# ----------------------------------------------------------------------------------------------------
+@dataclass(frozen=True)
+class ClipSchedule:
+    slots: int             # S: the plan's batch
+    slot: tuple            # slot of every clip, in input order
+    start: tuple           # window of the call in which every clip starts (its own window 0)
+    makespan: int          # windows the call runs
+
+
+def clip_schedule(n_windows: Sequence[int], n_slots: int = 0) -> ClipSchedule:
+    """Slot schedule of :func:`sample_clips` for clips of ``n_windows[i]`` windows, computed by the library
+    (``fmt_clip_schedule``, host-only).  ``n_slots = 0``: the fewest slots (<= 256) that still finish with the longest clip."""
+    lib = _cabi.load_library()
+    n = len(n_windows)
+    nw = (C.c_int32 * max(1, n))(*[int(x) for x in n_windows])
+    slot, start, makespan = (C.c_int32 * max(1, n))(), (C.c_int32 * max(1, n))(), C.c_int32()
+    S = lib.fmt_clip_schedule(n, nw, int(n_slots), slot, start, C.byref(makespan))
+    if S < 0:
+        raise ValueError(f"fmt_clip_schedule: bad arguments (n_clips={n}, n_slots={n_slots}, every clip needs >= 1 window)")
+    return ClipSchedule(S, tuple(slot[:n]), tuple(start[:n]), makespan.value)
+
+
+def clip_noise(seed: int, dims: Dims, n_windows: int, device) -> torch.Tensor:
+    """(n_windows, 1, L, dim_w): the x0 of every window of one clip drawn from its own seed - what the VA node draws for a batch of
+    one clip with ``fix_noise_seed`` (a ``torch.Generator`` on the target device, nodes_vadv.py:673-689)."""
+    return draw_window_noise(1, dims, n_windows, device, torch.Generator(torch.device(device)).manual_seed(int(seed)))
+
+
+def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str = "euler", a_cfg_scale: float = 2.0,
+                 r_cfg_scale: float = 1.0, e_cfg_scale: float = 1.0, include_r_cfg: bool = False, mode: Optional[str] = None,
+                 device=None, progress: Optional[Callable[[int, int], None]] = None) -> List[torch.Tensor]:
+    """Many independent clips of different lengths in one call.  Each clip is a mapping with ``r_s`` (1, dim_w), ``wa``
+    (1, T_wa, dim_a), ``we`` (1, 1 or T_we, dim_e), optionally ``audio_num_frames`` (default T_wa) and either ``seed`` (its noise is
+    :func:`clip_noise`) or ``noise`` (n_win, L, dim_w).  Solver, guidance scales, precision and static / dynamic emotion are shared.
+    Clip i's result is what :func:`perform_ode_sampling_loop` gives for it alone with that noise.  Returns one (1, T_i, dim_w) tensor
+    per clip, in input order, on ``device`` (default: the model's ``target_device``).  ``progress(w, makespan)`` is called after
+    each window of the schedule is enqueued."""
+    # every check runs before the first device call (the weights are packed only once the clips are known to be valid)
+    if not isinstance(clips, (list, tuple)):
+        raise TypeError(f"clips must be a list of mappings, got {type(clips).__name__}")
+    if not clips:
+        raise ValueError("clips is empty")
+    d = _model_dims(fmt_model, fmt_model.state_dict())
+    L = d.frames_per_clip
+    build_schedule(nfe, method)                        # unknown solver -> ValueError
+    if int(nfe) < 1:
+        raise ValueError(f"nfe must be >= 1 (got {nfe})")
+    mode = resolve_mode(mode)
+    T, n_win, dyn = [], [], []
+    for i, c in enumerate(clips):
+        if not isinstance(c, Mapping):
+            raise TypeError(f"clip {i} must be a mapping (r_s, wa, we, seed or noise), got {type(c).__name__}")
+        r_s, wa, we = c.get("r_s"), c.get("wa"), c.get("we")
+        if not all(torch.is_tensor(t) for t in (r_s, wa, we)):
+            raise TypeError(f"clip {i}: r_s, wa and we must be torch.Tensors")
+        if wa.dim() != 3 or we.dim() != 3 or wa.shape[0] != 1 or we.shape[0] != 1 or r_s.shape[0] != 1:
+            raise ValueError(f"clip {i}: batch dimension must be 1 (r_s {tuple(r_s.shape)}, wa {tuple(wa.shape)}, we {tuple(we.shape)}); "
+                             "a batch of equal-length clips is one clip per entry here")
+        if wa.shape[2] != d.dim_a or wa.shape[1] < 1:
+            raise ValueError(f"clip {i}: wa shape {tuple(wa.shape)}: expected (1, T, {d.dim_a})")
+        if we.shape[2] != d.dim_e or we.shape[1] < 1:
+            raise ValueError(f"clip {i}: we shape {tuple(we.shape)}: expected (1, 1 or T, {d.dim_e})")
+        if r_s.numel() != d.dim_w:
+            raise ValueError(f"clip {i}: r_s shape {tuple(r_s.shape)}: expected (1, {d.dim_w})")
+        t = int(c.get("audio_num_frames", wa.shape[1]))
+        if t < 1:
+            raise ValueError(f"clip {i}: audio_num_frames must be >= 1 (got {t})")
+        nw = -(-t // L)
+        dynamic = we.shape[1] > 1
+        # the reference's F.pad(replicate) needs at least one real frame in every window (nodes_adv.py:614-616)
+        if (nw - 1) * L >= wa.shape[1]:
+            raise ValueError(f"clip {i}: wa has {wa.shape[1]} frames, but window {nw - 1} of its {t} frames starts at frame {(nw - 1) * L}")
+        if dynamic and (nw - 1) * L >= we.shape[1]:
+            raise ValueError(f"clip {i}: dynamic we has {we.shape[1]} frames, but window {nw - 1} starts at frame {(nw - 1) * L}")
+        has_seed, has_noise = c.get("seed") is not None, c.get("noise") is not None
+        if has_seed == has_noise:
+            raise ValueError(f"clip {i}: give exactly one of 'seed' and 'noise'")
+        if has_noise:
+            nz = c["noise"]
+            if not torch.is_tensor(nz):
+                raise TypeError(f"clip {i}: noise must be a torch.Tensor")
+            if tuple(nz.shape) not in ((nw, L, d.dim_w), (nw, 1, L, d.dim_w)):
+                raise ValueError(f"clip {i}: noise shape {tuple(nz.shape)} != {(nw, L, d.dim_w)}")
+        T.append(t)
+        n_win.append(nw)
+        dyn.append(dynamic)
+    if any(dyn) != all(dyn):
+        raise ValueError("clips mix static (1-frame) and dynamic (per-frame) emotion we; one call shares one of the two")
+
+    if device is None:
+        device = getattr(fmt_model, "target_device", None) or "cuda"
+    be = backend_for(fmt_model, device, d)
+    sched = clip_schedule(n_win)
+    be.configure(sched.slots, n_branches_for(a_cfg_scale, r_cfg_scale, e_cfg_scale, include_r_cfg), dyn[0], nfe, method, mode)
+    dev = be.device
+    noise = [_as_f32(c["noise"], dev) if c.get("noise") is not None else clip_noise(c["seed"], d, nw, dev)
+             for c, nw in zip(clips, n_win)]
+    return be.sample_clips([_as_f32(c["r_s"], dev) for c in clips], [_as_f32(c["wa"], dev) for c in clips],
+                           [_as_f32(c["we"], dev) for c in clips], T, noise, a_cfg_scale, r_cfg_scale, e_cfg_scale, progress)
 
 
 def float_sample(fmt_model, opt, r_s, wa, we, a_cfg_scale=1.0, r_cfg_scale=1.0, e_cfg_scale=1.0, seed=None,

@@ -123,6 +123,23 @@ typedef struct FmtClip {
   void* progress_user;
 } FmtClip;
 
+/* Many independent clips in one call (fmt_sample_clips): clip i is what fmt_sample_clip gives for it alone (batch 1) with its noise.
+ * Every pointer is a DEVICE pointer; the arrays themselves are host arrays of n_clips entries. */
+typedef struct FmtClipSet {
+  int32_t n_clips;
+  const float* const* r_s;          /* [i]: (1, dim_w)                                                                     */
+  const float* const* wa;           /* [i]: (1, T_wa[i], dim_a)                                                            */
+  const float* const* we;           /* [i]: (1, T_we[i], dim_e); T_we[i] == 1 for every clip or > 1 for every clip (plan.we_dynamic) */
+  const float* const* noise;        /* [i]: (n_win_i, L, dim_w), n_win_i = ceil(audio_num_frames[i] / L): x0 of each of its windows */
+  float* const* r_d;                /* [i]: out (1, audio_num_frames[i], dim_w); only these frames are written                  */
+  const int32_t* T_wa;
+  const int32_t* T_we;
+  const int32_t* audio_num_frames;
+  float a_cfg_scale, r_cfg_scale, e_cfg_scale;   /* shared by every clip                                                      */
+  fmt_progress_fn progress;         /* optional: called on the host after each window of the schedule is enqueued (index, makespan) */
+  void* progress_user;
+} FmtClipSet;
+
 /* One evaluation of forward_with_cfv (FMT.py:342-401) on explicit window inputs - tests and ncu. */
 typedef struct FmtEval {
   const float* x;         /* (B, L, dim_w)                     */
@@ -153,6 +170,20 @@ FMT_API int64_t fmt_workspace_bytes(const FmtHandle* h);
 
 /* Whole clip: all windows, chained on the device through prev_x / prev_wa / prev_we. */
 FMT_API int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* clip, void* stream);
+
+/* Host-only (no device work): the slot schedule of fmt_sample_clips.  n_windows[i] >= 1 is the window count of clip i.  Clips are
+ * taken in order of window count, descending (ties in input order); each goes to the slot that is free first (ties: lowest slot)
+ * and starts there at its own window 0 in the window that slot becomes free.  n_slots = 0 picks the smallest slot count <= 256
+ * whose schedule finishes in max(n_windows) windows (256 if none does); n_slots > 0 schedules on exactly that many slots.
+ * Fills slot_out[i] / start_out[i] (may be NULL) and *makespan_out (may be NULL, the number of windows the call runs) and
+ * returns the slot count, < 0 on bad arguments. */
+FMT_API int32_t fmt_clip_schedule(int32_t n_clips, const int32_t* n_windows, int32_t n_slots, int32_t* slot_out, int32_t* start_out,
+                                  int32_t* makespan_out);
+
+/* Many clips of different lengths in one call, on plan.batch slots refilled as clips finish (device pointers only).  plan.batch
+ * must equal fmt_clip_schedule(n_slots = 0)'s slot count for these clips' window counts; each clip must pass fmt_sample_clip's
+ * checks with batch 1.  The window graph of the plan is replayed once per window of the schedule (its makespan). */
+FMT_API int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* set, void* stream);
 
 /* Single CFG-combined model evaluation (device pointers). */
 FMT_API int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream);
