@@ -57,6 +57,11 @@ class FmtClipSet(C.Structure):
                 ("progress", PROGRESS_FN), ("progress_user", C.c_void_p)]
 
 
+class FmtClipGuidance(C.Structure):
+    _fields_ = [("a_cfg_scale", C.POINTER(C.c_float)), ("r_cfg_scale", C.POINTER(C.c_float)), ("e_cfg_scale", C.POINTER(C.c_float)),
+                ("n_branches", C.POINTER(C.c_int32))]
+
+
 class FmtEval(C.Structure):
     _fields_ = [("x", C.c_void_p), ("prev_x", C.c_void_p), ("wa", C.c_void_p), ("prev_wa", C.c_void_p), ("we", C.c_void_p),
                 ("prev_we", C.c_void_p), ("r_s", C.c_void_p), ("v_out", C.c_void_p), ("eval_index", C.c_int32),
@@ -72,6 +77,7 @@ _SIGNATURES = {
     "fmt_workspace_bytes": (C.c_int64, [C.c_void_p]),
     "fmt_sample_clip": (C.c_int32, [C.c_void_p, C.POINTER(FmtClip), C.c_void_p]),
     "fmt_sample_clips": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.c_void_p]),
+    "fmt_sample_clips_guided": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.POINTER(FmtClipGuidance), C.c_void_p]),
     "fmt_clip_schedule": (C.c_int32, [C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32)]),
     "fmt_velocity": (C.c_int32, [C.c_void_p, C.POINTER(FmtEval), C.c_void_p]),

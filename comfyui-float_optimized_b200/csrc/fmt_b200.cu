@@ -1424,18 +1424,23 @@ int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
 }
 
 // Many clips on plan.batch slots: window w of the call runs, in slot k, whichever clip the schedule put there (at that clip's own
-// window), through the same captured window graph; only cond_gather / init_window / finalize_window read the per-slot records.
-int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) {
-  REQUIRE(h && cs, "fmt_sample_clips: null argument");
+// window), through the same captured window graph.  cond_gather / init_window / finalize_window read the per-slot tensors and
+// lengths, the CFG combines (cfg_combine_kernel and the COMB stages of the persistent kernels) the per-slot guidance.
+int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, void* stream) {
+  REQUIRE(h && cs && g, "fmt_sample_clips_guided: null argument");
   REQUIRE(h->configured, "fmt_sample_clips: call fmt_configure first");
   const int n = cs->n_clips;
   REQUIRE(n >= 1, "fmt_sample_clips: no clips");
   REQUIRE(cs->r_s && cs->wa && cs->we && cs->noise && cs->r_d && cs->T_wa && cs->T_we && cs->audio_num_frames, "fmt_sample_clips: null array");
+  REQUIRE(g->a_cfg_scale && g->r_cfg_scale && g->e_cfg_scale && g->n_branches, "fmt_sample_clips_guided: null guidance array");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_OK(cudaSetDevice(h->device));
   const ModelShape& s = h->shape;
   std::vector<int32_t> n_win(n), slot(n), start(n);
   for (int i = 0; i < n; ++i) {   // fmt_sample_clip's checks, per clip
+    const int nb = g->n_branches[i];
+    REQUIRE((nb == 1 || nb == 3 || nb == 4) && nb <= s.nb,
+            "fmt_sample_clips_guided: clip %d: n_branches=%d must be 1, 3 or 4 and fit the plan's %d branches", i, nb, s.nb);
     REQUIRE(cs->r_s[i] && cs->wa[i] && cs->we[i] && cs->noise[i] && cs->r_d[i], "fmt_sample_clips: clip %d: null tensor pointer", i);
     const int T = cs->audio_num_frames[i], T_wa = cs->T_wa[i], T_we = cs->T_we[i];
     REQUIRE(T >= 1 && T_wa >= 1 && T_we >= 1, "fmt_sample_clips: clip %d is empty", i);
@@ -1467,6 +1472,7 @@ int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) {
     SlotArgs& z = rec[r];
     z.r_s = zero; z.wa = zero; z.we = zero; z.x0 = zero; z.r_d = nullptr;
     z.T_wa = 1; z.T_we = 1; z.T_out = 0; z.win_start = 0; z.first_window = 1;
+    z.a_scale = z.r_scale = z.e_scale = 1.f; z.n_branches = s.nb;
   }
   for (int i = 0; i < n; ++i) {
     for (int w = 0; w < n_win[i]; ++w) {
@@ -1475,6 +1481,7 @@ int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) {
       z.x0 = cs->noise[i] + static_cast<size_t>(w) * s.L * s.W;
       z.T_wa = cs->T_wa[i]; z.T_we = cs->T_we[i]; z.T_out = cs->audio_num_frames[i];
       z.win_start = w * s.L; z.first_window = (w == 0);
+      z.a_scale = g->a_cfg_scale[i]; z.r_scale = g->r_cfg_scale[i]; z.e_scale = g->e_cfg_scale[i]; z.n_branches = g->n_branches[i];
     }
   }
   FMT_OK(dev_alloc(h, h->slot_buf, n_rec * sizeof(SlotArgs)));
@@ -1485,13 +1492,22 @@ int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) {
   for (int w = 0; w < makespan; ++w) {
     WindowArgs a{};
     a.slots = base + static_cast<size_t>(w) * S;
-    a.a_scale = cs->a_cfg_scale; a.r_scale = cs->r_cfg_scale; a.e_scale = cs->e_cfg_scale;
     FMT_OK(set_wargs(h, a, st));
     CUDA_OK(cudaGraphLaunch(h->graph_exec, st));
     h->launches += h->capture_launches;
     if (cs->progress) cs->progress(w, makespan, cs->progress_user);
   }
   return 0;
+}
+
+// The set's shared scales and the plan's branch count for every clip
+int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) {
+  REQUIRE(h && cs, "fmt_sample_clips: null argument");
+  const int n = std::max(cs->n_clips, 0);
+  std::vector<float> a(n, cs->a_cfg_scale), r(n, cs->r_cfg_scale), e(n, cs->e_cfg_scale);
+  std::vector<int32_t> nb(n, h->shape.nb);
+  const FmtClipGuidance g{a.data(), r.data(), e.data(), nb.data()};
+  return fmt_sample_clips_guided(h, cs, &g, stream);
 }
 
 }  // extern "C"

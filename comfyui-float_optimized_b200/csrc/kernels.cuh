@@ -20,7 +20,14 @@ struct SlotArgs {
   int T_wa, T_we, T_out;
   int win_start;           // first frame of this window in the clip
   int first_window;        // 1: the clip starts in this window: zero context, whatever the slot ran before
+  float a_scale, r_scale, e_scale;   // the clip's guidance
+  int n_branches;          // 1, 3 or 4 (<= the plan's): the CFG branches the clip combines (slot_branch0)
 };
+
+// First plan branch of a clip that combines nb of the plan's s_nb CFG branches.  Branches 1..3 of a 4-branch plan are
+// [uncond | all | audio-only] with the null masks of a 3-branch plan (branch_nulls), so a 3-branch clip skips the truly-uncond
+// branch; a 1-branch clip reads the `all` branch alone, the single conditional forward of FMT.py:400-401.
+__host__ __device__ __forceinline__ int slot_branch0(int s_nb, int nb) { return nb == 1 ? (s_nb == 1 ? 0 : s_nb - 2) : s_nb - nb; }
 
 // Per-window arguments, written to device memory by set_window_args so that the captured graph never changes.
 struct WindowArgs {
@@ -469,6 +476,18 @@ __device__ __forceinline__ float cfg_combine(const float* __restrict__ V, size_t
   return tu + r * (u - tu) + a * (ao - u) + e * (c - ao);
 }
 
+// The same selection for the persistent kernels' COMB, which hold the plan's branches in vb[0..3]: with per-slot records, the
+// scales and branch count of the clip in slot b, and vb shifted so that vb[0] is its first branch (constant register indices).
+__device__ __forceinline__ void slot_guidance(const SlotArgs* slots, int s_nb, int b, float (&vb)[4], int& nb, float& a, float& r, float& e) {
+  if (slots == nullptr) return;
+  const SlotArgs& sl = slots[b];
+  nb = __ldg(&sl.n_branches);
+  a = __ldg(&sl.a_scale); r = __ldg(&sl.r_scale); e = __ldg(&sl.e_scale);
+  const int br0 = slot_branch0(s_nb, nb);
+  if (br0 >= 1) { vb[0] = vb[1]; vb[1] = vb[2]; vb[2] = vb[3]; }
+  if (br0 >= 2) { vb[0] = vb[1]; vb[1] = vb[2]; }
+}
+
 // Every producer of an ODE state also writes the x-embedder operand rows of that state (replicated over the CFG
 // branches, FMT.py:363): ax[(br, b, P + f), :] = bf16(y[b, f, :]).  Context rows are written once per window.
 template <typename AT>
@@ -501,7 +520,15 @@ __global__ void cfg_combine_kernel(const WindowArgs* __restrict__ wargs, ModelSh
   const int j = static_cast<int>(i % s.W);
   const int f = static_cast<int>((i / s.W) % s.N), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.N));
   if (mode != 0 && f < s.P) return;
-  const float v = cfg_combine(V, i, per_branch, s.nb, a.a_scale, a.r_scale, a.e_scale);
+  // per slot (fmt_sample_clips): the clip's own scales and branches; the combine expression below is the same either way
+  int nb = s.nb, br0 = 0;
+  float as = a.a_scale, rs = a.r_scale, es = a.e_scale;
+  if (a.slots != nullptr) {
+    const SlotArgs& sl = a.slots[b];
+    nb = sl.n_branches; br0 = slot_branch0(s.nb, nb);
+    as = sl.a_scale; rs = sl.r_scale; es = sl.e_scale;
+  }
+  const float v = cfg_combine(V, i + br0 * per_branch, per_branch, nb, as, rs, es);
   if (mode == 0) dst[i] = v;
   else {
     const size_t o = (static_cast<size_t>(b) * s.L + (f - s.P)) * s.W + j;

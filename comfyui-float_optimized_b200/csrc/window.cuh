@@ -869,7 +869,9 @@ __device__ __forceinline__ void win_comb_stage(const WinParams& p, const WinCtx&
       if (br < s.nb) vb[br] = __ldcg(p.Vacc + br * per_branch + i);
     const float bd = __ldg(p.b_dec + j);
     const float dt = __ldg(p.ddt + step);
-    const float a_s = __ldg(&p.wargs->a_scale), r_s = __ldg(&p.wargs->r_scale), e_s = __ldg(&p.wargs->e_scale);
+    float a_s = __ldg(&p.wargs->a_scale), r_s = __ldg(&p.wargs->r_scale), e_s = __ldg(&p.wargs->e_scale);
+    const SlotArgs* const slots = p.wargs->slots;
+    int nb = s.nb;
     const float y0 = cur ? __ldcg(p.x_state + o) : 0.f;
     float kprev[4] = {0.f, 0.f, 0.f, 0.f};
     if (G > 1 && cur) {
@@ -882,9 +884,10 @@ __device__ __forceinline__ void win_comb_stage(const WinParams& p, const WinCtx&
     for (int br = 0; br < 4; ++br)
       if (br < s.nb) { vb[br] += bd; p.Vacc[br * per_branch + i] = 0.f; }
     if (!cur) continue;
+    slot_guidance(slots, s.nb, b, vb, nb, a_s, r_s, e_s);
     float v;
-    if (s.nb == 1) v = vb[0];
-    else if (s.nb == 3) v = vb[0] + a_s * (vb[2] - vb[0]) + e_s * (vb[1] - vb[2]);
+    if (nb == 1) v = vb[0];
+    else if (nb == 3) v = vb[0] + a_s * (vb[2] - vb[0]) + e_s * (vb[1] - vb[2]);
     else v = vb[0] + r_s * (vb[1] - vb[0]) + a_s * (vb[3] - vb[1]) + e_s * (vb[2] - vb[3]);
     float y;
     if (G == 1) {

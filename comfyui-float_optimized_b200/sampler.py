@@ -10,6 +10,7 @@ RNG (one ``torch.randn`` per window, exactly like the reference) and streams.  T
 import ctypes as C
 import functools
 import math
+import numbers
 import os
 import weakref
 from dataclasses import dataclass
@@ -271,17 +272,30 @@ class FmtBackend:
         return out
 
     def sample_clips(self, r_s, wa, we, audio_num_frames, noise, a_cfg_scale, r_cfg_scale, e_cfg_scale,
-                     progress: Optional[Callable[[int, int], None]] = None, out: Optional[Sequence[torch.Tensor]] = None) -> List[torch.Tensor]:
+                     progress: Optional[Callable[[int, int], None]] = None, out: Optional[Sequence[torch.Tensor]] = None,
+                     n_branches: Optional[Sequence[int]] = None) -> List[torch.Tensor]:
         """Many clips of different lengths in one call on the plan's batch of slots (:func:`clip_schedule`).  Per clip i: r_s[i]
         (1, dim_w), wa[i] (1, T_wa, dim_a), we[i] (1, 1 or T_we, dim_e), noise[i] (n_win_i, L, dim_w) or (n_win_i, 1, L, dim_w), all on
         ``self.device`` (fp32, contiguous).  Returns one (1, audio_num_frames[i], dim_w) tensor per clip (``out[i]`` if given: any
-        contiguous fp32 tensor of that many elements); asynchronous."""
+        contiguous fp32 tensor of that many elements); asynchronous.
+
+        Each of the three scales is one float for every clip or a sequence of one float per clip.  ``n_branches[i]`` (1, 3 or 4, at
+        most the plan's; default: the plan's for every clip) is the branch count of clip i's guidance, :func:`n_branches_for`."""
         d = self.dims
         if self._plan_key is None:
             raise FmtError("sample_clips: configure() has not been called")
         n = len(wa)
         if n < 1 or not all(len(x) == n for x in (r_s, we, audio_num_frames, noise)) or (out is not None and len(out) != n):
             raise ValueError("sample_clips: r_s, wa, we, audio_num_frames, noise (and out) need one entry per clip")
+        scales = []
+        for name, v in (("a_cfg_scale", a_cfg_scale), ("r_cfg_scale", r_cfg_scale), ("e_cfg_scale", e_cfg_scale)):
+            v = [float(x) for x in v] if isinstance(v, Sequence) else [float(v)] * n
+            if len(v) != n:
+                raise ValueError(f"sample_clips: {name} needs one float, or one per clip ({n}), got {len(v)}")
+            scales.append(v)
+        nbr = [self._plan_key[1]] * n if n_branches is None else [int(x) for x in n_branches]
+        if len(nbr) != n:
+            raise ValueError(f"sample_clips: n_branches needs one entry per clip ({n}), got {len(nbr)}")
         L = d.frames_per_clip
         dynamic = self._plan_key[2]
         outs = []
@@ -317,12 +331,15 @@ class FmtBackend:
         def ints(vals):
             return (C.c_int32 * n)(*[int(v) for v in vals])
 
+        def floats(vals):
+            return (C.c_float * n)(*vals)
+
         cb = _cabi.PROGRESS_FN(lambda w, m, _u: progress(w, m)) if progress is not None else _cabi.PROGRESS_FN(0)
         cs = _cabi.FmtClipSet(n, ptrs(r_s), ptrs(wa), ptrs(we), ptrs(noise), ptrs(outs), ints(t.shape[1] for t in wa),
-                              ints(t.shape[1] for t in we), ints(audio_num_frames), float(a_cfg_scale), float(r_cfg_scale),
-                              float(e_cfg_scale), cb, None)
+                              ints(t.shape[1] for t in we), ints(audio_num_frames), 1.0, 1.0, 1.0, cb, None)
+        g = _cabi.FmtClipGuidance(floats(scales[0]), floats(scales[1]), floats(scales[2]), ints(nbr))
         with torch.cuda.device(self.device):
-            _cabi.check(self.lib.fmt_sample_clips(self._handle, C.byref(cs), self._stream()), "fmt_sample_clips")
+            _cabi.check(self.lib.fmt_sample_clips_guided(self._handle, C.byref(cs), C.byref(g), self._stream()), "fmt_sample_clips_guided")
         return outs
 
     def velocity(self, eval_index: int, x, wa, r_s, we, prev_x, prev_wa, prev_we, a_cfg_scale, r_cfg_scale, e_cfg_scale) -> torch.Tensor:
@@ -485,10 +502,12 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
                  device=None, progress: Optional[Callable[[int, int], None]] = None) -> List[torch.Tensor]:
     """Many independent clips of different lengths in one call.  Each clip is a mapping with ``r_s`` (1, dim_w), ``wa``
     (1, T_wa, dim_a), ``we`` (1, 1 or T_we, dim_e), optionally ``audio_num_frames`` (default T_wa) and either ``seed`` (its noise is
-    :func:`clip_noise`) or ``noise`` (n_win, L, dim_w).  Solver, guidance scales, precision and static / dynamic emotion are shared.
-    Clip i's result is what :func:`perform_ode_sampling_loop` gives for it alone with that noise.  Returns one (1, T_i, dim_w) tensor
-    per clip, in input order, on ``device`` (default: the model's ``target_device``).  ``progress(w, makespan)`` is called after
-    each window of the schedule is enqueued."""
+    :func:`clip_noise`) or ``noise`` (n_win, L, dim_w).  A clip may also hold ``a_cfg_scale``, ``r_cfg_scale``, ``e_cfg_scale``
+    and ``include_r_cfg``: each overrides the keyword of the same name for that clip.  Solver, precision and static / dynamic
+    emotion are shared.  The plan runs as many CFG branches as the clip that needs the most (:func:`n_branches_for`); a clip
+    that needs fewer combines only its own branches.  Clip i's result is what :func:`perform_ode_sampling_loop` gives for it
+    alone with its settings and noise.  Returns one (1, T_i, dim_w) tensor per clip, in input order, on ``device`` (default: the
+    model's ``target_device``).  ``progress(w, makespan)`` is called after each window of the schedule is enqueued."""
     # every check runs before the first device call (the weights are packed only once the clips are known to be valid)
     if not isinstance(clips, (list, tuple)):
         raise TypeError(f"clips must be a list of mappings, got {type(clips).__name__}")
@@ -500,7 +519,7 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
     if int(nfe) < 1:
         raise ValueError(f"nfe must be >= 1 (got {nfe})")
     mode = resolve_mode(mode)
-    T, n_win, dyn = [], [], []
+    T, n_win, dyn, guidance = [], [], [], []      # guidance: (a, r, e, n_branches) of every clip
     for i, c in enumerate(clips):
         if not isinstance(c, Mapping):
             raise TypeError(f"clip {i} must be a mapping (r_s, wa, we, seed or noise), got {type(c).__name__}")
@@ -535,6 +554,17 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
                 raise TypeError(f"clip {i}: noise must be a torch.Tensor")
             if tuple(nz.shape) not in ((nw, L, d.dim_w), (nw, 1, L, d.dim_w)):
                 raise ValueError(f"clip {i}: noise shape {tuple(nz.shape)} != {(nw, L, d.dim_w)}")
+        for k in ("a_cfg_scale", "r_cfg_scale", "e_cfg_scale"):
+            if k in c:
+                v = c[k]
+                if not isinstance(v, numbers.Real) or isinstance(v, bool):
+                    raise TypeError(f"clip {i}: {k} must be a number, got {type(v).__name__}")
+                if not math.isfinite(v):
+                    raise ValueError(f"clip {i}: {k} must be finite (got {v})")
+        if "include_r_cfg" in c and not isinstance(c["include_r_cfg"], bool):
+            raise TypeError(f"clip {i}: include_r_cfg must be a bool, got {type(c['include_r_cfg']).__name__}")
+        g = tuple(c.get(k, dflt) for k, dflt in (("a_cfg_scale", a_cfg_scale), ("r_cfg_scale", r_cfg_scale), ("e_cfg_scale", e_cfg_scale)))
+        guidance.append(g + (n_branches_for(*g, c.get("include_r_cfg", include_r_cfg)),))
         T.append(t)
         n_win.append(nw)
         dyn.append(dynamic)
@@ -545,12 +575,13 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
         device = getattr(fmt_model, "target_device", None) or "cuda"
     be = backend_for(fmt_model, device, d)
     sched = clip_schedule(n_win)
-    be.configure(sched.slots, n_branches_for(a_cfg_scale, r_cfg_scale, e_cfg_scale, include_r_cfg), dyn[0], nfe, method, mode)
+    a, r, e, nb = zip(*guidance)
+    be.configure(sched.slots, max(nb), dyn[0], nfe, method, mode)
     dev = be.device
     noise = [_as_f32(c["noise"], dev) if c.get("noise") is not None else clip_noise(c["seed"], d, nw, dev)
              for c, nw in zip(clips, n_win)]
     return be.sample_clips([_as_f32(c["r_s"], dev) for c in clips], [_as_f32(c["wa"], dev) for c in clips],
-                           [_as_f32(c["we"], dev) for c in clips], T, noise, a_cfg_scale, r_cfg_scale, e_cfg_scale, progress)
+                           [_as_f32(c["we"], dev) for c in clips], T, noise, a, r, e, progress, n_branches=nb)
 
 
 def float_sample(fmt_model, opt, r_s, wa, we, a_cfg_scale=1.0, r_cfg_scale=1.0, e_cfg_scale=1.0, seed=None,

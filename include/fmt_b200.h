@@ -140,6 +140,17 @@ typedef struct FmtClipSet {
   void* progress_user;
 } FmtClipSet;
 
+/* Guidance of every clip of a FmtClipSet (fmt_sample_clips_guided): host arrays of n_clips entries.  n_branches[i] is the
+ * reference's rule for clip i's scales and include_r_cfg (FMT.py:346,380,400): 1 when every scale is 1, else 3, or 4 with the
+ * r guidance term.  A clip with fewer branches than the plan combines only its own: a 3-branch clip in a 4-branch plan the
+ * branches [uncond | all | audio-only], a 1-branch clip the `all` branch alone. */
+typedef struct FmtClipGuidance {
+  const float* a_cfg_scale;
+  const float* r_cfg_scale;
+  const float* e_cfg_scale;
+  const int32_t* n_branches;        /* 1, 3 or 4, <= plan.n_branches; a 1-branch plan takes 1-branch clips only */
+} FmtClipGuidance;
+
 /* One evaluation of forward_with_cfv (FMT.py:342-401) on explicit window inputs - tests and ncu. */
 typedef struct FmtEval {
   const float* x;         /* (B, L, dim_w)                     */
@@ -182,8 +193,14 @@ FMT_API int32_t fmt_clip_schedule(int32_t n_clips, const int32_t* n_windows, int
 
 /* Many clips of different lengths in one call, on plan.batch slots refilled as clips finish (device pointers only).  plan.batch
  * must equal fmt_clip_schedule(n_slots = 0)'s slot count for these clips' window counts; each clip must pass fmt_sample_clip's
- * checks with batch 1.  The window graph of the plan is replayed once per window of the schedule (its makespan). */
+ * checks with batch 1.  The window graph of the plan is replayed once per window of the schedule (its makespan).
+ * Every clip uses the set's scales and plan.n_branches: fmt_sample_clips_guided with that guidance. */
 FMT_API int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* set, void* stream);
+
+/* fmt_sample_clips with each clip's own guidance; the set's a/r/e_cfg_scale are not read.  Clip i's result depends only on its
+ * own inputs and guidance and on the plan.  Returns -1 if an n_branches[i] is not 1, 3 or 4 or exceeds plan.n_branches, or if a
+ * 1-branch plan gets a clip with more than one branch. */
+FMT_API int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* set, const FmtClipGuidance* guidance, void* stream);
 
 /* Single CFG-combined model evaluation (device pointers). */
 FMT_API int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream);
