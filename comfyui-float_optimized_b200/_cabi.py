@@ -68,6 +68,15 @@ class FmtEval(C.Structure):
                 ("a_cfg_scale", C.c_float), ("r_cfg_scale", C.c_float), ("e_cfg_scale", C.c_float)]
 
 
+FMT_EPI_STORE, FMT_EPI_GELU, FMT_EPI_POS, FMT_EPI_GATE_RES = 0, 1, 2, 3
+
+
+class FmtDebugGemm(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("mode", "kind", "M", "N", "K", "block_n", "ksplit", "ldo", "out_f32", "frames")] + \
+               [(n, C.c_void_p) for n in ("A", "W", "bias", "out", "pos", "gate", "urow")] + \
+               [("ldg", C.c_int64), ("gate_off", C.c_int64)]
+
+
 _SIGNATURES = {
     "fmt_abi_version": (C.c_int32, []),
     "fmt_last_error": (C.c_char_p, []),
@@ -97,6 +106,11 @@ _SIGNATURES = {
     "fmt_debug_gemm_bench_bf16x3": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                                 C.c_void_p]),
     "fmt_debug_gemm_fp32": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "fmt_debug_gemm_epilogue": (C.c_int32, [C.POINTER(FmtDebugGemm), C.c_void_p]),
+    "fmt_debug_lnmod": (C.c_int32, [C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
+                                    C.c_void_p]),
+    "fmt_debug_band_attention": (C.c_int32, [C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
+                                             C.c_void_p]),
 }
 
 _lib = None

@@ -226,6 +226,9 @@ static int launch_tc(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ld
 template <int BN, bool SPLIT>
 static int launch_tc2(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ldw, const EpiParams& ep, int K, cudaStream_t st, int ksplit = 1) {
   using C = Tc2Cfg<BN, SPLIT>;
+  // every K slice must hold a K block: an empty slice issues no MMA, and its epilogue would add a stale accumulator into x
+  REQUIRE(ksplit == 1 || (ksplit > 1 && ep.kind == EPI_GATE_RES && K >= 64 * ksplit), "gemm: %d K slices need x += gate * (.) and K >= %d (K=%d)",
+          ksplit, 64 * ksplit, K);
   const auto kern = gemm_tc2_kernel<BN, typename std::conditional<SPLIT, float, bf16>::type, SPLIT>;
   static bool attr_set[64] = {};
   if (!attr_set[h->device & 63]) {
@@ -235,12 +238,12 @@ static int launch_tc2(FmtHandle* h, const bf16* A, int lda, const bf16* W, int l
   CUtensorMap ta, tb;
   FMT_OK(make_tmap(h, &ta, A, ep.M, K * C::HALVES, lda * C::HALVES, C::BMH));
   FMT_OK(make_tmap(h, &tb, W, ep.N, K * C::HALVES, ldw * C::HALVES, BN / 2));
-  const int tiles = ((ep.M + C::BM - 1) / C::BM) * ((ep.N + BN - 1) / BN) * ((ksplit > 1 && ep.kind == EPI_GATE_RES) ? ksplit : 1);
+  const int tiles = ((ep.M + C::BM - 1) / C::BM) * ((ep.N + BN - 1) / BN) * ksplit;
   const int max_pairs = h->num_sms / 2;
   const int pairs = tiles < max_pairs ? tiles : max_pairs;
   EpiParams ep2 = ep;
   ep2.raster_gm = h->raster_gm;
-  ep2.ksplit = (ksplit > 1 && ep.kind == EPI_GATE_RES) ? ksplit : 1;
+  ep2.ksplit = ksplit;
   // the kernel carries __cluster_dims__(2,1,1); launch() only adds the PDL attribute
   return launch(h, kern, dim3(2 * pairs), dim3(C::THREADS), C::SMEM_BYTES, st, 1, ta, tb, ep2, K);
 }
@@ -252,14 +255,17 @@ static int pick_bn(const FmtHandle* h, int M, int N) {
   return 64;
 }
 
-// SPLIT: the bf16x3 GEMM on pair operands (FMT_MODE_BF16X3): K % 64 == 0, never K-sliced (its results stay bitwise reproducible)
+// SPLIT: the bf16x3 GEMM on pair operands (FMT_MODE_BF16X3): K % 64 == 0, never K-sliced by the sampler (its results stay bitwise
+// reproducible).  force_ksplit: K slices of a forced CTA-pair kernel (unit tests); the sampler picks them itself.
 template <bool SPLIT = false>
-static int gemm_bf16(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ldw, const EpiParams& ep, int K, cudaStream_t st, int force_bn = 0) {
+static int gemm_bf16(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ldw, const EpiParams& ep, int K, cudaStream_t st, int force_bn = 0,
+                     int force_ksplit = 1) {
   REQUIRE(ep.N % 32 == 0 && K % 8 == 0 && lda % 8 == 0 && ldw % 8 == 0, "gemm_bf16: N %% 32, K/lda/ldw %% 8 required (N=%d K=%d)", ep.N, K);
   REQUIRE(!SPLIT || (K % 64 == 0 && lda % 64 == 0 && ldw % 64 == 0), "gemm_bf16x3: K, lda, ldw %% 64 required (K=%d)", K);
+  REQUIRE(force_ksplit == 1 || force_bn == 512 || force_bn == 1024, "gemm_bf16: K slices need the CTA-pair kernel (block_n 512 or 1024)");
   // CTA-pair kernel (force_bn 512 / 1024 = pair tiles 256x256 / 256x128): the default once there are enough 256-row tiles
-  if (force_bn == 512) return launch_tc2<256, SPLIT>(h, A, lda, W, ldw, ep, K, st);
-  if (force_bn == 1024) return launch_tc2<128, SPLIT>(h, A, lda, W, ldw, ep, K, st);
+  if (force_bn == 512) return launch_tc2<256, SPLIT>(h, A, lda, W, ldw, ep, K, st, force_ksplit);
+  if (force_bn == 1024) return launch_tc2<128, SPLIT>(h, A, lda, W, ldw, ep, K, st, force_ksplit);
   if (force_bn == 0 && h->use_pair && ep.M >= 512 && ep.N % 256 == 0 && K % 64 == 0) {
     // Wave model calibrated on B200 (tools/gemm_bench.py): time ~ waves x per-wave cost.  A pair tile (256x256 on two SMs)
     // and a single-CTA 128x256 tile cost the same per wave at 32 clips, but at >= 128 clips the pair kernel is 20 % cheaper
@@ -349,53 +355,66 @@ static int enqueue_tables(FmtHandle* h, int e0, int n, cudaStream_t st) {
   return 0;
 }
 
+// LayerNorm + modulate of `rows` rows of X into out (the GEMM operand of the next Linear); table rows are urow[r] (NULL = r) * ldt
+template <typename T>
+static int lnmod(FmtHandle* h, const float* X, int rows, int H, const typename ModeOps<T>::Tab* table, const int* urow, long long ldt,
+                 long long shift_off, long long scale_off, T* out, cudaStream_t st) {
+  using TT = typename ModeOps<T>::Tab;
+  const int warps = 4;
+  const dim3 grid((rows + warps - 1) / warps), block(warps * 32);
+  switch (H % 128 == 0 ? H / 128 : 0) {
+    case 1: return launch(h, lnmod_kernel<T, TT, 1>, grid, block, 0, st, 1, X, rows, H, table, urow, ldt, shift_off, scale_off, out);
+    case 2: return launch(h, lnmod_kernel<T, TT, 2>, grid, block, 0, st, 1, X, rows, H, table, urow, ldt, shift_off, scale_off, out);
+    case 4: return launch(h, lnmod_kernel<T, TT, 4>, grid, block, 0, st, 1, X, rows, H, table, urow, ldt, shift_off, scale_off, out);
+    case 8: return launch(h, lnmod_kernel<T, TT, 8>, grid, block, 0, st, 1, X, rows, H, table, urow, ldt, shift_off, scale_off, out);
+  }
+  return set_err(-1, "dim_h %d unsupported by the LayerNorm kernel (128, 256, 512, 1024)", H);
+}
+
 template <typename T>
 static int launch_lnmod(FmtHandle* h, const typename ModeOps<T>::Tab* table_e, long long shift_off, long long scale_off, cudaStream_t st) {
-  using TT = typename ModeOps<T>::Tab;
-  const ModelShape& s = h->shape;
-  const int warps = 4;
-  const dim3 grid((h->R + warps - 1) / warps), block(warps * 32);
-  const float* X = static_cast<const float*>(h->X.p);
-  T* out = static_cast<T*>(h->A1.p);
   const int* urow = h->dedup ? static_cast<const int*>(h->urow_buf.p) : nullptr;
-  const long long ldt = h->NT;
-  switch (s.H / 128) {
-    case 1: return launch(h, lnmod_kernel<T, TT, 1>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
-    case 2: return launch(h, lnmod_kernel<T, TT, 2>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
-    case 4: return launch(h, lnmod_kernel<T, TT, 4>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
-    case 8: return launch(h, lnmod_kernel<T, TT, 8>, grid, block, 0, st, 1, X, h->R, s.H, table_e, urow, ldt, shift_off, scale_off, out);
+  return lnmod<T>(h, static_cast<const float*>(h->X.p), h->R, h->shape.H, table_e, urow, h->NT, shift_off, scale_off, static_cast<T*>(h->A1.p), st);
+}
+
+// Band attention of n_seq sequences of N rows.  variant 0 picks the kernel, 1 forces the warp-per-row kernel, 2 the tile kernel.
+enum { ATTN_AUTO = 0, ATTN_WARP = 1, ATTN_TILE = 2 };
+template <typename T>
+static int band_attention(FmtHandle* h, const typename ModeOps<T>::Tab* qkv, int n_seq, int N, int heads, int hd, int win, T* out, int variant,
+                          cudaStream_t st) {
+  using Q = typename ModeOps<T>::Tab;
+  const float scale = 1.0f / sqrtf(static_cast<float>(hd));
+  // many sequences: one CTA per (sequence, head) with K / V staged in shared memory (every qkv byte read once)
+  const size_t tile_smem = static_cast<size_t>(2) * N * hd * sizeof(bf16);   // K, V of one (sequence, head)
+  const bool tile_ok = sizeof(T) == 2 && tile_smem <= 48 * 1024 && (hd == 64 || hd == 128);
+  if (variant == ATTN_AUTO) variant = tile_ok && n_seq * heads >= 2 * h->num_sms ? ATTN_TILE : ATTN_WARP;
+  if (variant == ATTN_TILE) {
+    REQUIRE(tile_ok, "band attention: the tile kernel needs bf16, head_dim 64 or 128 and K / V within 48 KB (N=%d hd=%d)", N, hd);
+    if constexpr (sizeof(T) == 2) {
+      const bf16* q16 = reinterpret_cast<const bf16*>(qkv);
+      bf16* o16 = reinterpret_cast<bf16*>(out);
+      const dim3 tg(n_seq * heads), tb(ATTN_TILE_THREADS);
+      if (hd == 64) return launch(h, band_attention_tile_kernel<64>, tg, tb, tile_smem, st, 1, q16, N, heads, win, scale, o16);
+      return launch(h, band_attention_tile_kernel<128>, tg, tb, tile_smem, st, 1, q16, N, heads, win, scale, o16);
+    }
   }
-  return set_err(-1, "dim_h %d unsupported by the LayerNorm kernel (128, 256, 512, 1024)", s.H);
+  REQUIRE(variant == ATTN_WARP, "band attention: unknown variant %d", variant);
+  const int total_warps = n_seq * heads * N, warps = 4;
+  const dim3 grid((total_warps + warps - 1) / warps), block(warps * 32);
+  switch (hd) {
+    case 32: return launch(h, band_attention_kernel<Q, 1, T>, grid, block, 0, st, 1, qkv, n_seq, N, heads, win, scale, out);
+    case 64: return launch(h, band_attention_kernel<Q, 2, T>, grid, block, 0, st, 1, qkv, n_seq, N, heads, win, scale, out);
+    case 128: return launch(h, band_attention_kernel<Q, 4, T>, grid, block, 0, st, 1, qkv, n_seq, N, heads, win, scale, out);
+  }
+  return set_err(-1, "head_dim %d unsupported (32, 64, 128)", hd);
 }
 
 template <typename T>
 static int launch_attn(FmtHandle* h, cudaStream_t st) {
   const ModelShape& s = h->shape;
-  const int heads = h->d.num_heads, hd = s.H / heads;
-  const int n_seq = s.nb * s.B, total_warps = n_seq * heads * s.N, warps = 4;
-  const float scale = 1.0f / sqrtf(static_cast<float>(hd));
-  const dim3 grid((total_warps + warps - 1) / warps), block(warps * 32);
-  using Q = typename ModeOps<T>::Tab;
-  const Q* qkv = static_cast<const Q*>(h->QKV.p);
-  T* out = static_cast<T*>(h->A2.p);
-  const int win = h->d.attention_window;
-  if constexpr (sizeof(T) == 2) {
-    // many sequences: one CTA per (sequence, head) with K / V staged in shared memory (every qkv byte read once)
-    const size_t tile_smem = static_cast<size_t>(2) * s.N * hd * sizeof(bf16);   // K, V of one (sequence, head)
-    if (n_seq * heads >= 2 * h->num_sms && tile_smem <= 48 * 1024 && (hd == 64 || hd == 128)) {
-      const bf16* q16 = reinterpret_cast<const bf16*>(qkv);
-      bf16* o16 = reinterpret_cast<bf16*>(out);
-      const dim3 tg(n_seq * heads), tb(ATTN_TILE_THREADS);
-      if (hd == 64) return launch(h, band_attention_tile_kernel<64>, tg, tb, tile_smem, st, 1, q16, s.N, heads, win, scale, o16);
-      return launch(h, band_attention_tile_kernel<128>, tg, tb, tile_smem, st, 1, q16, s.N, heads, win, scale, o16);
-    }
-  }
-  switch (hd) {
-    case 32: return launch(h, band_attention_kernel<Q, 1, T>, grid, block, 0, st, 1, qkv, n_seq, s.N, heads, win, scale, out);
-    case 64: return launch(h, band_attention_kernel<Q, 2, T>, grid, block, 0, st, 1, qkv, n_seq, s.N, heads, win, scale, out);
-    case 128: return launch(h, band_attention_kernel<Q, 4, T>, grid, block, 0, st, 1, qkv, n_seq, s.N, heads, win, scale, out);
-  }
-  return set_err(-1, "head_dim %d unsupported (32, 64, 128)", hd);
+  const int heads = h->d.num_heads;
+  return band_attention<T>(h, static_cast<const typename ModeOps<T>::Tab*>(h->QKV.p), s.nb * s.B, s.N, heads, s.H / heads, h->d.attention_window,
+                           static_cast<T*>(h->A2.p), ATTN_AUTO, st);
 }
 
 // One model evaluation: V[R, W] = FMT.forward over the nb-way batched CFG branches (FMT.py:277-340).  The x-embedder
@@ -1715,6 +1734,89 @@ int32_t fmt_debug_gemm_fp32(const float* A, const float* W, const float* bias, f
   FmtHandle h;
   EpiParams ep = epi(EPI_STORE, M, N, bias, out, N, 1);
   return gemm_f32(&h, A, K, W, K, ep, K, static_cast<cudaStream_t>(stream));
+}
+
+static_assert(FMT_EPI_STORE == int{EPI_STORE} && FMT_EPI_GELU == int{EPI_GELU} && FMT_EPI_POS == int{EPI_POS} && FMT_EPI_GATE_RES == int{EPI_GATE_RES},
+              "FMT_EPI_* are the kernels' EpiKind");
+
+int32_t fmt_debug_gemm_epilogue(const FmtDebugGemm* g, void* stream) {
+  REQUIRE(g && g->A && g->W && g->out, "fmt_debug_gemm_epilogue: null argument");
+  REQUIRE(g->M > 0 && g->N > 0 && g->K > 0 && g->ldo >= g->N, "fmt_debug_gemm_epilogue: bad shape M=%d N=%d K=%d ldo=%d", g->M, g->N, g->K, g->ldo);
+  REQUIRE(g->kind >= FMT_EPI_STORE && g->kind <= FMT_EPI_GATE_RES, "fmt_debug_gemm_epilogue: unknown kind %d", g->kind);
+  REQUIRE(g->kind != FMT_EPI_POS || (g->pos && g->frames > 0), "fmt_debug_gemm_epilogue: POS needs pos and frames");
+  REQUIRE(g->kind != FMT_EPI_GATE_RES || (g->gate && g->out_f32), "fmt_debug_gemm_epilogue: GATE_RES needs a gate table and fp32 out");
+  REQUIRE(g->mode == FMT_MODE_BF16 || g->mode == FMT_MODE_FP32_VALIDATE || g->mode == FMT_MODE_BF16X3, "fmt_debug_gemm_epilogue: unknown mode %d", g->mode);
+  REQUIRE(g->mode != FMT_MODE_FP32_VALIDATE || (g->block_n == 0 && g->ksplit == 1), "fmt_debug_gemm_epilogue: the fp32 SIMT GEMM has one tile shape");
+  REQUIRE(g->mode != FMT_MODE_BF16X3 || g->out_f32 || g->ldo % 64 == 0, "fmt_debug_gemm_epilogue: a pair output needs ldo %% 64 == 0");
+  FmtHandle h;
+  FMT_OK(debug_handle(h));
+  h.use_pdl = false;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  EpiParams ep = epi(g->kind, g->M, g->N, g->bias, g->out, g->ldo, g->out_f32);
+  ep.pos = g->pos; ep.frames = g->frames;
+  ep.gate = g->gate; ep.urow = g->urow; ep.ldg = g->ldg; ep.gate_off = g->gate_off;
+  const int M = g->M, N = g->N, K = g->K;
+  if (g->mode == FMT_MODE_FP32_VALIDATE) return gemm_f32(&h, g->A, K, g->W, K, ep, K, st);
+  // the operands as the sampler holds them: bf16, or bf16x3 pairs (4 bytes per element either way is enough room)
+  const size_t na = static_cast<size_t>(M) * K, nw = static_cast<size_t>(N) * K;
+  void *a = nullptr, *w = nullptr;
+  CUDA_OK(cudaMallocAsync(&a, na * sizeof(bf16x3_t), st));
+  CUDA_OK(cudaMallocAsync(&w, nw * sizeof(bf16x3_t), st));
+  int rc = 0;
+  if (g->mode == FMT_MODE_BF16) {
+    if (K % 8 != 0) rc = set_err(-1, "fmt_debug_gemm_epilogue: K %% 8 required (K=%d)", K);
+    if (rc == 0) {
+      f32_to_bf16_kernel<<<static_cast<unsigned>(std::min<size_t>((na / 8 + 255) / 256, 2368)), 256, 0, st>>>(g->A, static_cast<bf16*>(a), na / 8);
+      f32_to_bf16_kernel<<<static_cast<unsigned>(std::min<size_t>((nw / 8 + 255) / 256, 2368)), 256, 0, st>>>(g->W, static_cast<bf16*>(w), nw / 8);
+      rc = cudaGetLastError() == cudaSuccess ? 0 : set_err(-2, "fmt_debug_gemm_epilogue: operand conversion failed");
+    }
+    if (rc == 0) rc = gemm_bf16(&h, static_cast<const bf16*>(a), K, static_cast<const bf16*>(w), K, ep, K, st, g->block_n, g->ksplit);
+  } else {
+    if (K % 64 != 0) rc = set_err(-1, "fmt_debug_gemm_epilogue: bf16x3 mode needs K %% 64 == 0 (K=%d)", K);
+    if (rc == 0) {
+      f32_to_split_kernel<<<static_cast<unsigned>(std::min<size_t>((na / 4 + 255) / 256, 2368)), 256, 0, st>>>(g->A, static_cast<bf16x3_t*>(a), na / 4);
+      f32_to_split_kernel<<<static_cast<unsigned>(std::min<size_t>((nw / 4 + 255) / 256, 2368)), 256, 0, st>>>(g->W, static_cast<bf16x3_t*>(w), nw / 4);
+      rc = cudaGetLastError() == cudaSuccess ? 0 : set_err(-2, "fmt_debug_gemm_epilogue: operand split failed");
+    }
+    if (rc == 0) rc = gemm_bf16<true>(&h, static_cast<const bf16*>(a), K, static_cast<const bf16*>(w), K, ep, K, st, g->block_n, g->ksplit);
+  }
+  (void)cudaFreeAsync(a, st);
+  (void)cudaFreeAsync(w, st);
+  return rc;
+}
+
+int32_t fmt_debug_lnmod(int32_t mode, const float* X, int32_t rows, int32_t H, const void* table, const int32_t* urow, int64_t ldt,
+                        int64_t shift_off, int64_t scale_off, void* out, void* stream) {
+  REQUIRE(X && table && out && rows > 0, "fmt_debug_lnmod: null argument or no rows");
+  FmtHandle h;
+  FMT_OK(debug_handle(h));
+  h.use_pdl = false;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  switch (mode) {
+    case FMT_MODE_BF16: return lnmod<bf16>(&h, X, rows, H, static_cast<const bf16*>(table), urow, ldt, shift_off, scale_off, static_cast<bf16*>(out), st);
+    case FMT_MODE_FP32_VALIDATE: return lnmod<float>(&h, X, rows, H, static_cast<const float*>(table), urow, ldt, shift_off, scale_off, static_cast<float*>(out), st);
+    case FMT_MODE_BF16X3:
+      return lnmod<bf16x3_t>(&h, X, rows, H, static_cast<const float*>(table), urow, ldt, shift_off, scale_off, static_cast<bf16x3_t*>(out), st);
+  }
+  return set_err(-1, "fmt_debug_lnmod: unknown mode %d", mode);
+}
+
+int32_t fmt_debug_band_attention(int32_t mode, const void* qkv, int32_t n_seq, int32_t N, int32_t heads, int32_t hd, int32_t window, void* out,
+                                 int32_t variant, void* stream) {
+  REQUIRE(qkv && out && n_seq > 0 && N > 0 && heads > 0 && window >= 0, "fmt_debug_band_attention: null argument or bad shape");
+  REQUIRE(variant == ATTN_AUTO || variant == ATTN_WARP || variant == ATTN_TILE, "fmt_debug_band_attention: unknown variant %d", variant);
+  FmtHandle h;
+  FMT_OK(debug_handle(h));
+  h.use_pdl = false;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  switch (mode) {
+    case FMT_MODE_BF16: return band_attention<bf16>(&h, static_cast<const bf16*>(qkv), n_seq, N, heads, hd, window, static_cast<bf16*>(out), variant, st);
+    case FMT_MODE_FP32_VALIDATE:
+      return band_attention<float>(&h, static_cast<const float*>(qkv), n_seq, N, heads, hd, window, static_cast<float*>(out), variant, st);
+    case FMT_MODE_BF16X3:
+      return band_attention<bf16x3_t>(&h, static_cast<const float*>(qkv), n_seq, N, heads, hd, window, static_cast<bf16x3_t*>(out), variant, st);
+  }
+  return set_err(-1, "fmt_debug_band_attention: unknown mode %d", mode);
 }
 
 }  // extern "C"

@@ -256,6 +256,48 @@ FMT_API int32_t fmt_debug_gemm_bench_bf16x3(const void* A, const void* W, const 
 FMT_API int32_t fmt_debug_gemm_fp32(const float* A, const float* W, const float* bias, float* out, int32_t M, int32_t N,
                                     int32_t K, void* stream);
 
+/* Fused GEMM epilogues of the FMT step (FMT.py:171-176), applied to acc = A . W^T + bias:
+ *   STORE     out = acc
+ *   GELU      out = GELU_tanh(acc)
+ *   POS       out = acc + pos[(m % frames) * N + n]
+ *   GATE_RES  out[m, n] += gate[urow[m] * ldg + gate_off + n] * acc   (out fp32; urow NULL = identity)  */
+enum { FMT_EPI_STORE = 0, FMT_EPI_GELU = 1, FMT_EPI_POS = 2, FMT_EPI_GATE_RES = 3 };
+
+/* One GEMM of fmt_debug_gemm_epilogue.  Every pointer is a DEVICE pointer. */
+typedef struct FmtDebugGemm {
+  int32_t mode;           /* FMT_MODE_*: bf16 tcgen05, fp32 SIMT or bf16x3 tcgen05 GEMM                                  */
+  int32_t kind;           /* FMT_EPI_*                                                                                    */
+  int32_t M, N, K;
+  int32_t block_n;        /* 0 = the sampler's choice; 64 / 128 / 256 single-CTA kernel, 512 / 1024 CTA-pair kernel (not fp32) */
+  int32_t ksplit;         /* K slices of the CTA-pair kernel (1 = none; > 1: GATE_RES only, K >= 64 * ksplit)              */
+  int32_t ldo;            /* row stride of out in elements (>= N)                                                         */
+  int32_t out_f32;        /* 1: out is fp32; 0: the mode's activation type (bf16 bits, bf16x3 pairs or fp32).  GATE_RES: 1 */
+  int32_t frames;         /* POS: rows of pos                                                                             */
+  const float* A;         /* (M, K) fp32, rounded to bf16 (bf16) or split into pairs (bf16x3) on the device               */
+  const float* W;         /* (N, K) fp32, likewise                                                                        */
+  const float* bias;      /* (N) or NULL                                                                                  */
+  void* out;              /* (M, ldo); bf16x3 pairs: ldo % 64 == 0 and 256-byte aligned (gemm.cuh)                        */
+  const float* pos;       /* POS: (frames, N)                                                                             */
+  const void* gate;       /* GATE_RES: the AdaLN table in the mode's table type (bf16 bits in bf16 mode, else fp32)       */
+  const int32_t* urow;    /* GATE_RES: table row of every output row, or NULL                                            */
+  int64_t ldg;            /* GATE_RES: table row stride in elements                                                      */
+  int64_t gate_off;       /* GATE_RES: column of the gate's first element                                                */
+} FmtDebugGemm;
+
+/* One GEMM with a fused epilogue, dispatched exactly as the sampler dispatches its GEMMs in `mode`. */
+FMT_API int32_t fmt_debug_gemm_epilogue(const FmtDebugGemm* g, void* stream);
+/* LayerNorm (eps 1e-6, no affine) + modulate of the sampler: out[r] = LN(X[r]) * (1 + table[t + scale_off]) + table[t + shift_off]
+ * with t = (urow ? urow[r] : r) * ldt.  X (rows, H) fp32, H in {128, 256, 512, 1024}; table in the mode's table type; out (rows, H)
+ * in the mode's activation type. */
+FMT_API int32_t fmt_debug_lnmod(int32_t mode, const float* X, int32_t rows, int32_t H, const void* table, const int32_t* urow,
+                                int64_t ldt, int64_t shift_off, int64_t scale_off, void* out, void* stream);
+/* Band attention of the sampler (FMT.py:15-19,69-88): qkv (n_seq, N, 3 * heads * hd) in the mode's table type, columns [q | k | v]
+ * head-major; out (n_seq, N, heads * hd) in the mode's activation type.  hd in {32, 64, 128}.  variant 0 = the sampler's choice,
+ * 1 = one warp per query row, 2 = one CTA per (sequence, head) with K / V in shared memory (bf16 mode, hd 64 or 128, K and V of a
+ * head within 48 KB); returns -1 for a variant that cannot run these arguments. */
+FMT_API int32_t fmt_debug_band_attention(int32_t mode, const void* qkv, int32_t n_seq, int32_t N, int32_t heads, int32_t hd,
+                                         int32_t window, void* out, int32_t variant, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -22,7 +22,7 @@ def _stream():
 
 @pytest.mark.parametrize("block_n", [64, 128, 256])
 @pytest.mark.parametrize("M,N,K", [(180, 3072, 1024), (128, 256, 64), (100, 64, 64), (333, 1024, 4096), (1620, 512, 1088),
-                                    (5760, 1024, 1024)])
+                                    (5760, 1024, 1024), (333, 1024, 1040)])    # K = 1040: a last K block of 16 columns (fmt_proj_create allows in_dim % 16)
 def test_tcgen05_gemm_matches_torch(lib, M, N, K, block_n):
     L, cabi = lib
     g = torch.Generator(device="cuda").manual_seed(M * 7 + N * 3 + K)
