@@ -62,6 +62,11 @@ class FmtClipGuidance(C.Structure):
                 ("n_branches", C.POINTER(C.c_int32))]
 
 
+class FmtWindowSet(C.Structure):
+    _fields_ = [("n_streams", C.c_int32)] + [(n, C.POINTER(C.c_void_p)) for n in ("r_s", "wa", "we", "x0", "ctx", "r_d")] + \
+               [(n, C.POINTER(C.c_int32)) for n in ("T_wa", "T_we", "n_out", "first_window")]
+
+
 class FmtEval(C.Structure):
     _fields_ = [("x", C.c_void_p), ("prev_x", C.c_void_p), ("wa", C.c_void_p), ("prev_wa", C.c_void_p), ("we", C.c_void_p),
                 ("prev_we", C.c_void_p), ("r_s", C.c_void_p), ("v_out", C.c_void_p), ("eval_index", C.c_int32),
@@ -87,6 +92,7 @@ _SIGNATURES = {
     "fmt_sample_clip": (C.c_int32, [C.c_void_p, C.POINTER(FmtClip), C.c_void_p]),
     "fmt_sample_clips": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.c_void_p]),
     "fmt_sample_clips_guided": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.POINTER(FmtClipGuidance), C.c_void_p]),
+    "fmt_sample_windows": (C.c_int32, [C.c_void_p, C.POINTER(FmtWindowSet), C.POINTER(FmtClipGuidance), C.c_void_p]),
     "fmt_clip_schedule": (C.c_int32, [C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32)]),
     "fmt_velocity": (C.c_int32, [C.c_void_p, C.POINTER(FmtEval), C.c_void_p]),

@@ -1391,6 +1391,41 @@ static int set_wargs(FmtHandle* h, const WindowArgs& a, cudaStream_t st) {
   return 0;
 }
 
+// Slot records of one call (fmt_sample_clips, fmt_sample_windows) go up in ONE copy from a pinned staging buffer that the handle
+// owns; slot_ev marks the end of the previous call's copy, so the staging buffer is refilled only once that copy has read it.
+// stage_slot_records returns the staging buffer with n_rec idle records: zero inputs ((L, W) noise, and r_s / wa / we rows no wider
+// than that), no output, no context, scales of 1 and the plan's branch count.
+static int stage_slot_records(FmtHandle* h, size_t n_rec, cudaStream_t st, SlotArgs** out) {
+  const ModelShape& s = h->shape;
+  const size_t n_zero = std::max<size_t>(static_cast<size_t>(s.L) * s.W, static_cast<size_t>(std::max(s.A, s.E)));
+  FMT_OK(dev_alloc(h, h->slot_zero, n_zero * sizeof(float)));
+  CUDA_OK(cudaMemsetAsync(h->slot_zero.p, 0, n_zero * sizeof(float), st));
+  const float* zero = static_cast<const float*>(h->slot_zero.p);
+  if (h->slot_ev) CUDA_OK(cudaEventSynchronize(h->slot_ev));
+  if (h->slot_host_n < n_rec) {
+    if (h->slot_host) { CUDA_OK(cudaFreeHost(h->slot_host)); h->slot_host = nullptr; h->slot_host_n = 0; }
+    CUDA_OK(cudaHostAlloc(reinterpret_cast<void**>(&h->slot_host), n_rec * sizeof(SlotArgs), cudaHostAllocDefault));
+    h->slot_host_n = n_rec;
+  }
+  SlotArgs* rec = h->slot_host;
+  for (size_t r = 0; r < n_rec; ++r) {
+    SlotArgs& z = rec[r];
+    z.r_s = zero; z.wa = zero; z.we = zero; z.x0 = zero; z.r_d = nullptr; z.ctx = nullptr;
+    z.T_wa = 1; z.T_we = 1; z.T_out = 0; z.win_start = 0; z.out_start = 0; z.first_window = 1;
+    z.a_scale = z.r_scale = z.e_scale = 1.f; z.n_branches = s.nb;
+  }
+  *out = rec;
+  return 0;
+}
+
+static int upload_slot_records(FmtHandle* h, size_t n_rec, cudaStream_t st) {
+  FMT_OK(dev_alloc(h, h->slot_buf, n_rec * sizeof(SlotArgs)));
+  CUDA_OK(cudaMemcpyAsync(h->slot_buf.p, h->slot_host, n_rec * sizeof(SlotArgs), cudaMemcpyHostToDevice, st));
+  if (!h->slot_ev) CUDA_OK(cudaEventCreateWithFlags(&h->slot_ev, cudaEventDisableTiming));
+  CUDA_OK(cudaEventRecord(h->slot_ev, st));
+  return 0;
+}
+
 int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
   REQUIRE(h && c, "fmt_sample_clip: null argument");
   REQUIRE(h->configured, "fmt_sample_clip: call fmt_configure first");
@@ -1474,39 +1509,20 @@ int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* cs, const FmtCli
   const int S = clip_schedule(n, n_win.data(), 0, slot.data(), start.data(), &makespan);
   REQUIRE(s.B == S, "fmt_sample_clips: the plan has batch %d, but these %d clips are scheduled on %d slots (fmt_clip_schedule)", s.B, n, S);
 
-  // idle slots read zeros: (L, W) noise, and r_s / wa / we rows no wider than that
-  const size_t n_zero = std::max<size_t>(static_cast<size_t>(s.L) * s.W, static_cast<size_t>(std::max(s.A, s.E)));
-  FMT_OK(dev_alloc(h, h->slot_zero, n_zero * sizeof(float)));
-  CUDA_OK(cudaMemsetAsync(h->slot_zero.p, 0, n_zero * sizeof(float), st));
-  const float* zero = static_cast<const float*>(h->slot_zero.p);
+  SlotArgs* rec = nullptr;
   const size_t n_rec = static_cast<size_t>(makespan) * S;
-  if (h->slot_ev) CUDA_OK(cudaEventSynchronize(h->slot_ev));   // the previous call's upload has read the staging buffer
-  if (h->slot_host_n < n_rec) {
-    if (h->slot_host) { CUDA_OK(cudaFreeHost(h->slot_host)); h->slot_host = nullptr; h->slot_host_n = 0; }
-    CUDA_OK(cudaHostAlloc(reinterpret_cast<void**>(&h->slot_host), n_rec * sizeof(SlotArgs), cudaHostAllocDefault));
-    h->slot_host_n = n_rec;
-  }
-  SlotArgs* rec = h->slot_host;
-  for (size_t r = 0; r < n_rec; ++r) {
-    SlotArgs& z = rec[r];
-    z.r_s = zero; z.wa = zero; z.we = zero; z.x0 = zero; z.r_d = nullptr;
-    z.T_wa = 1; z.T_we = 1; z.T_out = 0; z.win_start = 0; z.first_window = 1;
-    z.a_scale = z.r_scale = z.e_scale = 1.f; z.n_branches = s.nb;
-  }
+  FMT_OK(stage_slot_records(h, n_rec, st, &rec));
   for (int i = 0; i < n; ++i) {
     for (int w = 0; w < n_win[i]; ++w) {
       SlotArgs& z = rec[static_cast<size_t>(start[i] + w) * S + slot[i]];
       z.r_s = cs->r_s[i]; z.wa = cs->wa[i]; z.we = cs->we[i]; z.r_d = cs->r_d[i];
       z.x0 = cs->noise[i] + static_cast<size_t>(w) * s.L * s.W;
       z.T_wa = cs->T_wa[i]; z.T_we = cs->T_we[i]; z.T_out = cs->audio_num_frames[i];
-      z.win_start = w * s.L; z.first_window = (w == 0);
+      z.win_start = z.out_start = w * s.L; z.first_window = (w == 0);
       z.a_scale = g->a_cfg_scale[i]; z.r_scale = g->r_cfg_scale[i]; z.e_scale = g->e_cfg_scale[i]; z.n_branches = g->n_branches[i];
     }
   }
-  FMT_OK(dev_alloc(h, h->slot_buf, n_rec * sizeof(SlotArgs)));
-  CUDA_OK(cudaMemcpyAsync(h->slot_buf.p, rec, n_rec * sizeof(SlotArgs), cudaMemcpyHostToDevice, st));
-  if (!h->slot_ev) CUDA_OK(cudaEventCreateWithFlags(&h->slot_ev, cudaEventDisableTiming));
-  CUDA_OK(cudaEventRecord(h->slot_ev, st));
+  FMT_OK(upload_slot_records(h, n_rec, st));
   const SlotArgs* base = static_cast<const SlotArgs*>(h->slot_buf.p);
   for (int w = 0; w < makespan; ++w) {
     WindowArgs a{};
@@ -1527,6 +1543,55 @@ int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) {
   std::vector<int32_t> nb(n, h->shape.nb);
   const FmtClipGuidance g{a.data(), r.data(), e.data(), nb.data()};
   return fmt_sample_clips_guided(h, cs, &g, stream);
+}
+
+// One window of each of n streams, stream i in slot i, through the plan's captured window graph; slots n.. are idle.  A stream's
+// context lives in its own ctx buffer, not in the handle, so a stream may run in any slot and the plan may be replaced between calls.
+// Its wa / we start at the window's first context frame (P frames before its first current frame), or at its first current frame in
+// a first window; its output is the window alone.
+int32_t fmt_sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, void* stream) {
+  REQUIRE(h && ws && g, "fmt_sample_windows: null argument");
+  REQUIRE(h->configured, "fmt_sample_windows: call fmt_configure first");
+  const ModelShape& s = h->shape;
+  const int n = ws->n_streams;
+  REQUIRE(n >= 1 && n <= s.B, "fmt_sample_windows: %d streams, the plan has %d slots", n, s.B);
+  REQUIRE(ws->r_s && ws->wa && ws->we && ws->x0 && ws->ctx && ws->r_d && ws->T_wa && ws->T_we && ws->n_out && ws->first_window,
+          "fmt_sample_windows: null array");
+  REQUIRE(g->a_cfg_scale && g->r_cfg_scale && g->e_cfg_scale && g->n_branches, "fmt_sample_windows: null guidance array");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CUDA_OK(cudaSetDevice(h->device));
+  for (int i = 0; i < n; ++i) {
+    const int nb = g->n_branches[i];
+    REQUIRE((nb == 1 || nb == 3 || nb == 4) && nb <= s.nb,
+            "fmt_sample_windows: stream %d: n_branches=%d must be 1, 3 or 4 and fit the plan's %d branches", i, nb, s.nb);
+    REQUIRE(ws->r_s[i] && ws->wa[i] && ws->we[i] && ws->x0[i] && ws->ctx[i] && ws->r_d[i], "fmt_sample_windows: stream %d: null tensor pointer", i);
+    const int first = ws->first_window[i], T_wa = ws->T_wa[i], T_we = ws->T_we[i], n_out = ws->n_out[i];
+    REQUIRE(first == 0 || first == 1, "fmt_sample_windows: stream %d: first_window=%d must be 0 or 1", i, first);
+    REQUIRE(n_out >= 1 && n_out <= s.L, "fmt_sample_windows: stream %d: n_out=%d outside [1, %d]", i, n_out, s.L);
+    REQUIRE(s.we_dynamic ? T_we >= 1 : T_we == 1, "fmt_sample_windows: stream %d: T_we=%d does not match plan.we_dynamic=%d", i, T_we, s.we_dynamic);
+    // the window's first current frame must be a real frame (the reference's F.pad(replicate) fails otherwise)
+    const int cur = first ? 0 : s.P;
+    REQUIRE(cur < T_wa, "fmt_sample_windows: stream %d: wa has %d frames but the window's first current frame is frame %d", i, T_wa, cur);
+    REQUIRE(!s.we_dynamic || cur < T_we, "fmt_sample_windows: stream %d: dynamic we has %d frames but the window's first current frame is frame %d",
+            i, T_we, cur);
+  }
+  SlotArgs* rec = nullptr;
+  FMT_OK(stage_slot_records(h, s.B, st, &rec));
+  for (int i = 0; i < n; ++i) {
+    SlotArgs& z = rec[i];
+    z.r_s = ws->r_s[i]; z.wa = ws->wa[i]; z.we = ws->we[i]; z.x0 = ws->x0[i]; z.r_d = ws->r_d[i]; z.ctx = ws->ctx[i];
+    z.T_wa = ws->T_wa[i]; z.T_we = ws->T_we[i]; z.T_out = ws->n_out[i];
+    z.first_window = ws->first_window[i];
+    z.win_start = z.first_window ? 0 : s.P; z.out_start = 0;
+    z.a_scale = g->a_cfg_scale[i]; z.r_scale = g->r_cfg_scale[i]; z.e_scale = g->e_cfg_scale[i]; z.n_branches = g->n_branches[i];
+  }
+  FMT_OK(upload_slot_records(h, s.B, st));
+  WindowArgs a{};
+  a.slots = static_cast<const SlotArgs*>(h->slot_buf.p);
+  FMT_OK(set_wargs(h, a, st));
+  CUDA_OK(cudaGraphLaunch(h->graph_exec, st));
+  h->launches += h->capture_launches;
+  return 0;
 }
 
 }  // extern "C"

@@ -9,7 +9,8 @@
 
 namespace fmt {
 
-// What one batch slot computes in one window of fmt_sample_clips: a window of its own clip (tensors of that clip alone, batch 1).
+// What one batch slot computes in one window of fmt_sample_clips or fmt_sample_windows: a window of its own clip (tensors of that
+// clip alone, batch 1).
 // An idle slot points at zeros, has r_d == nullptr and first_window == 1: it is computed and its output is dropped.
 struct SlotArgs {
   const float* r_s;        // (W)
@@ -18,10 +19,13 @@ struct SlotArgs {
   const float* x0;         // (L, W) noise of this window of the clip
   float* r_d;              // (T_out, W), or nullptr for an idle slot
   int T_wa, T_we, T_out;
-  int win_start;           // first frame of this window in the clip
+  int win_start;           // frame of wa / we that is this window's first current frame
   int first_window;        // 1: the clip starts in this window: zero context, whatever the slot ran before
   float a_scale, r_scale, e_scale;   // the clip's guidance
   int n_branches;          // 1, 3 or 4 (<= the plan's): the CFG branches the clip combines (slot_branch0)
+  int out_start;           // frame of r_d that is this window's first current frame
+  float* ctx;              // (P, W) the clip's motion context, read unless first_window and overwritten with this window's
+                           // last P frames (fmt_sample_windows); nullptr: the context stays in the handle's per-slot state
 };
 
 // First plan branch of a clip that combines nb of the plan's s_nb CFG branches.  Branches 1..3 of a 4-branch plan are
@@ -560,7 +564,7 @@ __global__ void rk_combine_kernel(ModelShape s, const float* __restrict__ y0, fl
   store_ax<AT>(s, ax, b, s.P + f, j, y);
 }
 
-// Window prologue: x_state <- x0, context rows <- prev_x (zero in the first window, nodes_adv.py:591), ax <- [prev_x | x0]
+// Window prologue: x_state <- x0, context rows <- prev_x or a stream's ctx (zero in the first window, nodes_adv.py:591), ax <- [prev_x | x0]
 template <typename AT>
 __global__ void init_window_kernel(const WindowArgs* __restrict__ wargs, ModelShape s, float* __restrict__ x_state,
                                    float* __restrict__ prev_x_state, AT* __restrict__ ax) {
@@ -570,14 +574,16 @@ __global__ void init_window_kernel(const WindowArgs* __restrict__ wargs, ModelSh
   const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<size_t>(s.B) * s.N * s.W) return;
   const int j = static_cast<int>(i % s.W), f = static_cast<int>((i / s.W) % s.N), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.N));
-  // per slot (fmt_sample_clips): the slot's own noise (L, W) and context reset
+  // per slot (fmt_sample_clips / fmt_sample_windows): the slot's own noise (L, W), context reset and, for a stream, its own context
   const float* x0 = a.x0;
+  const float* ctx = nullptr;
   int cb = b, first_window = a.first_window;
-  if (a.slots != nullptr) { x0 = a.slots[b].x0; first_window = a.slots[b].first_window; cb = 0; }
+  if (a.slots != nullptr) { x0 = a.slots[b].x0; first_window = a.slots[b].first_window; ctx = a.slots[b].ctx; cb = 0; }
   float v;
   if (f < s.P) {
     const size_t o = (static_cast<size_t>(b) * s.P + f) * s.W + j;
     if (first_window) { v = 0.f; prev_x_state[o] = 0.f; }
+    else if (ctx != nullptr) v = ctx[static_cast<size_t>(f) * s.W + j];
     else v = prev_x_state[o];
   } else {
     const size_t o = (static_cast<size_t>(b) * s.L + (f - s.P)) * s.W + j;
@@ -586,7 +592,7 @@ __global__ void init_window_kernel(const WindowArgs* __restrict__ wargs, ModelSh
   }
   store_ax<AT>(s, ax, b, f, j, v);
 }
-// Window epilogue: r_d[:, window] <- x_state, prev_x <- last P frames (nodes_adv.py:659-668,690-692)
+// Window epilogue: r_d[:, window] <- x_state, prev_x (and a stream's ctx) <- last P frames (nodes_adv.py:659-668,690-692)
 __global__ void finalize_window_kernel(const WindowArgs* __restrict__ wargs, ModelShape s, const float* __restrict__ x_state,
                                        float* __restrict__ prev_x_state) {
   pdl_launch_dependents();
@@ -596,13 +602,19 @@ __global__ void finalize_window_kernel(const WindowArgs* __restrict__ wargs, Mod
   if (i >= static_cast<size_t>(s.B) * s.L * s.W) return;
   const int j = static_cast<int>(i % s.W), f = static_cast<int>((i / s.W) % s.L), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.L));
   const float v = x_state[i];
-  // per slot (fmt_sample_clips): frames below the slot's own clip length, into that clip's output; idle slots write nothing
+  // per slot (fmt_sample_clips / fmt_sample_windows): frames below the slot's own clip length, into that clip's output; idle slots
+  // write nothing
   float* r_d = a.r_d;
-  int cb = b, T_out = a.T_out, win_start = a.win_start;
-  if (a.slots != nullptr) { const SlotArgs& sl = a.slots[b]; r_d = sl.r_d; T_out = sl.T_out; win_start = sl.win_start; cb = 0; }
-  const int g = win_start + f;
+  float* ctx = nullptr;
+  int cb = b, T_out = a.T_out, out_start = a.win_start;
+  if (a.slots != nullptr) { const SlotArgs& sl = a.slots[b]; r_d = sl.r_d; T_out = sl.T_out; out_start = sl.out_start; ctx = sl.ctx; cb = 0; }
+  const int g = out_start + f;
   if (r_d != nullptr && g < T_out) r_d[(static_cast<size_t>(cb) * T_out + g) * s.W + j] = v;
-  if (f >= s.L - s.P) prev_x_state[(static_cast<size_t>(b) * s.P + (f - (s.L - s.P))) * s.W + j] = v;
+  if (f >= s.L - s.P) {
+    const int c = f - (s.L - s.P);
+    prev_x_state[(static_cast<size_t>(b) * s.P + c) * s.W + j] = v;
+    if (ctx != nullptr) ctx[static_cast<size_t>(c) * s.W + j] = v;
+  }
 }
 
 // fp32 -> bf16 weight packing (with optional K padding)

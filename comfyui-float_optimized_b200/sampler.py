@@ -342,6 +342,41 @@ class FmtBackend:
             _cabi.check(self.lib.fmt_sample_clips_guided(self._handle, C.byref(cs), C.byref(g), self._stream()), "fmt_sample_clips_guided")
         return outs
 
+    def sample_windows(self, r_s, wa, we, x0, ctx, out, first_window, a_cfg_scale, r_cfg_scale, e_cfg_scale, n_branches) -> None:
+        """One window of each of n <= plan batch streams (``fmt_sample_windows``), stream i in slot i.  Per stream i: r_s[i]
+        (1, dim_w); wa[i] (T_wa, dim_a) and, dynamic, we[i] (T_we, dim_e) from the window's first context frame (frame 0 in a first
+        window), static we[i] (1, 1, dim_e); x0[i] (L, dim_w); ctx[i] (P, dim_w), read unless ``first_window[i]`` and overwritten
+        with the window's last P frames; out[i] receives the window's first ``out[i].shape[-2]`` frames.  Scales and n_branches are
+        one entry per stream.  All tensors on ``self.device`` (fp32, contiguous); asynchronous."""
+        d = self.dims
+        if self._plan_key is None:
+            raise FmtError("sample_windows: configure() has not been called")
+        n = len(wa)
+        groups = (r_s, we, x0, ctx, out, first_window, a_cfg_scale, r_cfg_scale, e_cfg_scale, n_branches)
+        if not 1 <= n <= self._plan_key[0] or not all(len(x) == n for x in groups):
+            raise ValueError(f"sample_windows: 1 to {self._plan_key[0]} streams, with one entry per stream in every argument")
+        for i in range(n):
+            for name, t in (("r_s", r_s[i]), ("wa", wa[i]), ("we", we[i]), ("x0", x0[i]), ("ctx", ctx[i]), ("out", out[i])):
+                if not torch.is_tensor(t) or t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device:
+                    raise ValueError(f"stream {i}: {name} must be a contiguous float32 tensor on {self.device}")
+            if x0[i].numel() != d.frames_per_clip * d.dim_w or ctx[i].numel() != d.num_prev_frames * d.dim_w or r_s[i].numel() != d.dim_w:
+                raise ValueError(f"stream {i}: r_s, x0 or ctx does not hold (dim_w), (L, dim_w) or (P, dim_w) elements")
+            if wa[i].numel() % d.dim_a or we[i].numel() % d.dim_e or out[i].numel() % d.dim_w:
+                raise ValueError(f"stream {i}: wa, we or out is not a whole number of frames")
+
+        def ptrs(ts):
+            return (C.c_void_p * n)(*[t.data_ptr() for t in ts])
+
+        def ints(vals):
+            return (C.c_int32 * n)(*[int(v) for v in vals])
+
+        ws = _cabi.FmtWindowSet(n, ptrs(r_s), ptrs(wa), ptrs(we), ptrs(x0), ptrs(ctx), ptrs(out), ints(t.numel() // d.dim_a for t in wa),
+                                ints(t.numel() // d.dim_e for t in we), ints(t.numel() // d.dim_w for t in out), ints(first_window))
+        g = _cabi.FmtClipGuidance(*[(C.c_float * n)(*[float(x) for x in v]) for v in (a_cfg_scale, r_cfg_scale, e_cfg_scale)],
+                                  ints(n_branches))
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.fmt_sample_windows(self._handle, C.byref(ws), C.byref(g), self._stream()), "fmt_sample_windows")
+
     def velocity(self, eval_index: int, x, wa, r_s, we, prev_x, prev_wa, prev_we, a_cfg_scale, r_cfg_scale, e_cfg_scale) -> torch.Tensor:
         """One ``forward_with_cfv`` (FMT.py:342-401) at plan time ``t_eval[eval_index]``; returns (B, P+L, dim_w)."""
         d = self.dims
@@ -497,6 +532,21 @@ def clip_noise(seed: int, dims: Dims, n_windows: int, device) -> torch.Tensor:
     return draw_window_noise(1, dims, n_windows, device, torch.Generator(torch.device(device)).manual_seed(int(seed)))
 
 
+def _own_guidance(who: str, c: Mapping, a_cfg_scale, r_cfg_scale, e_cfg_scale, include_r_cfg) -> tuple:
+    """(a, r, e, n_branches) of one clip or stream: each of its own guidance keys overrides the call's keyword of that name."""
+    for k in ("a_cfg_scale", "r_cfg_scale", "e_cfg_scale"):
+        if k in c:
+            v = c[k]
+            if not isinstance(v, numbers.Real) or isinstance(v, bool):
+                raise TypeError(f"{who}: {k} must be a number, got {type(v).__name__}")
+            if not math.isfinite(v):
+                raise ValueError(f"{who}: {k} must be finite (got {v})")
+    if "include_r_cfg" in c and not isinstance(c["include_r_cfg"], bool):
+        raise TypeError(f"{who}: include_r_cfg must be a bool, got {type(c['include_r_cfg']).__name__}")
+    g = tuple(c.get(k, dflt) for k, dflt in (("a_cfg_scale", a_cfg_scale), ("r_cfg_scale", r_cfg_scale), ("e_cfg_scale", e_cfg_scale)))
+    return g + (n_branches_for(*g, c.get("include_r_cfg", include_r_cfg)),)
+
+
 def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str = "euler", a_cfg_scale: float = 2.0,
                  r_cfg_scale: float = 1.0, e_cfg_scale: float = 1.0, include_r_cfg: bool = False, mode: Optional[str] = None,
                  device=None, progress: Optional[Callable[[int, int], None]] = None) -> List[torch.Tensor]:
@@ -554,17 +604,7 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
                 raise TypeError(f"clip {i}: noise must be a torch.Tensor")
             if tuple(nz.shape) not in ((nw, L, d.dim_w), (nw, 1, L, d.dim_w)):
                 raise ValueError(f"clip {i}: noise shape {tuple(nz.shape)} != {(nw, L, d.dim_w)}")
-        for k in ("a_cfg_scale", "r_cfg_scale", "e_cfg_scale"):
-            if k in c:
-                v = c[k]
-                if not isinstance(v, numbers.Real) or isinstance(v, bool):
-                    raise TypeError(f"clip {i}: {k} must be a number, got {type(v).__name__}")
-                if not math.isfinite(v):
-                    raise ValueError(f"clip {i}: {k} must be finite (got {v})")
-        if "include_r_cfg" in c and not isinstance(c["include_r_cfg"], bool):
-            raise TypeError(f"clip {i}: include_r_cfg must be a bool, got {type(c['include_r_cfg']).__name__}")
-        g = tuple(c.get(k, dflt) for k, dflt in (("a_cfg_scale", a_cfg_scale), ("r_cfg_scale", r_cfg_scale), ("e_cfg_scale", e_cfg_scale)))
-        guidance.append(g + (n_branches_for(*g, c.get("include_r_cfg", include_r_cfg)),))
+        guidance.append(_own_guidance(f"clip {i}", c, a_cfg_scale, r_cfg_scale, e_cfg_scale, include_r_cfg))
         T.append(t)
         n_win.append(nw)
         dyn.append(dynamic)
@@ -582,6 +622,218 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
              for c, nw in zip(clips, n_win)]
     return be.sample_clips([_as_f32(c["r_s"], dev) for c in clips], [_as_f32(c["wa"], dev) for c in clips],
                            [_as_f32(c["we"], dev) for c in clips], T, noise, a, r, e, progress, n_branches=nb)
+
+
+# ----------------------------------------------------------------------------------------------------
+# streams: clips fed audio in pieces, one window per step on a fixed set of batch slots
+# ----------------------------------------------------------------------------------------------------
+_GUIDANCE_KEYS = ("a_cfg_scale", "r_cfg_scale", "e_cfg_scale", "include_r_cfg")
+
+
+class Stream:
+    """One clip of a :class:`StreamSampler`, opened by :meth:`StreamSampler.open`.  ``fed`` frames have arrived, ``windows_run``
+    windows have been sampled; ``finished`` once :meth:`StreamSampler.finish` was called, ``done`` once its last window ran."""
+
+    def __init__(self, index, L, r_s, we, ctx, wa, we_buf, gen, noise, guidance):
+        self.index = index                  # open order: breaks ties between windows that became ready at the same tick
+        self.L = L
+        self.r_s, self.we, self.ctx = r_s, we, ctx
+        self.wa, self.we_buf = wa, we_buf   # frames [base, fed): from the next window's first context frame on
+        self.base = 0
+        self.fed = 0
+        self.windows_run = 0
+        self.finished = False
+        self.ready_at = None                # sampler clock when the next window became ready; None while it is not
+        self.gen, self.noise, self.guidance = gen, noise, guidance
+
+    @property
+    def done(self) -> bool:
+        return self.finished and self.windows_run * self.L >= self.fed
+
+    @property
+    def buffered_frames(self) -> int:
+        """Frames of wa this stream holds on the device."""
+        return self.wa.untyped_storage().nbytes() // (self.wa.element_size() * self.wa.shape[1]) if self.wa is not None else 0
+
+
+class StreamSampler:
+    """Clips whose audio arrives in pieces, sampled one window at a time on ``slots`` shared batch slots.
+
+    :meth:`open` starts a stream, :meth:`feed` appends its audio latents, :meth:`finish` ends its audio and :meth:`step` runs one
+    window for each of up to ``slots`` streams whose next window is ready: its L frames have arrived, or the stream is finished and
+    the window holds its last frames.  The window that has been ready longest goes first (a feed, finish or step that makes
+    several windows ready makes them ready at once); ties go in open order.  A stream's frames
+    are what :func:`sample_clips` gives for the whole clip (same noise, same guidance, same plan), however the audio was cut.
+
+    The plan (slot count, nfe, solver, precision, static or dynamic emotion, and the branch count of the keyword guidance) is fixed
+    at construction, so steps replay one captured window graph.  A stream may override the four guidance keywords in :meth:`open`
+    as a clip of :func:`sample_clips` does, within the plan's branch count.  A stream holds on the device its reference latent,
+    its last P motion frames and the audio frames from its next window's first context frame on, however long it runs."""
+
+    def __init__(self, fmt_model, *, slots: int, nfe: int, method: str = "euler", mode: Optional[str] = None, a_cfg_scale: float = 2.0,
+                 r_cfg_scale: float = 1.0, e_cfg_scale: float = 1.0, include_r_cfg: bool = False, we_dynamic: bool = False, device=None):
+        if isinstance(slots, bool) or not isinstance(slots, numbers.Integral) or not 1 <= slots <= 256:
+            raise ValueError(f"slots must be an int in [1, 256] (got {slots!r})")
+        build_schedule(nfe, method)                        # unknown solver -> ValueError
+        if int(nfe) < 1:
+            raise ValueError(f"nfe must be >= 1 (got {nfe})")
+        if not isinstance(we_dynamic, bool):
+            raise TypeError(f"we_dynamic must be a bool, got {type(we_dynamic).__name__}")
+        self._mode = resolve_mode(mode)
+        self._keywords = (a_cfg_scale, r_cfg_scale, e_cfg_scale, include_r_cfg)
+        # CFG branches of the plan: those of the keyword guidance
+        self.n_branches = _own_guidance("StreamSampler", dict(zip(_GUIDANCE_KEYS, self._keywords)), *self._keywords)[3]
+        self.dims = _model_dims(fmt_model, fmt_model.state_dict())
+        if device is None:
+            device = getattr(fmt_model, "target_device", None) or "cuda"
+        self.slots, self.nfe, self.method, self.we_dynamic = int(slots), int(nfe), method, we_dynamic
+        self._be = backend_for(fmt_model, device, self.dims)
+        self.device = self._be.device
+        self._configure()
+        self._streams: List[Stream] = []
+        self._opened = 0
+        self._clock = 0                                    # ticks once per feed(), finish() and step()
+
+    def _configure(self):
+        self._be.configure(self.slots, self.n_branches, self.we_dynamic, self.nfe, self.method, self._mode)
+
+    def _check_tensor(self, who, name, t, shape):
+        if not torch.is_tensor(t):
+            raise TypeError(f"{who}: {name} must be a torch.Tensor")
+        if not t.is_floating_point():
+            raise TypeError(f"{who}: {name} must be a floating-point tensor (got {t.dtype})")
+        if t.dim() != len(shape) or any(want is not None and got != want for got, want in zip(t.shape, shape)):
+            raise ValueError(f"{who}: {name} shape {tuple(t.shape)} != {tuple('T' if x is None else x for x in shape)}")
+
+    def _own(self, stream) -> Stream:
+        if not isinstance(stream, Stream) or stream not in self._streams:
+            raise ValueError("not an open stream of this sampler")
+        return stream
+
+    def open(self, r_s, we=None, seed: Optional[int] = None, noise: Optional[torch.Tensor] = None, **guidance) -> Stream:
+        """A new stream with reference latent ``r_s`` (1, dim_w) and, for static emotion, ``we`` (1, 1, dim_e) (dynamic emotion
+        arrives with :meth:`feed`).  Its noise is :func:`clip_noise` of ``seed``, drawn one window at a time, or ``noise``
+        (n_win, L, dim_w) for a clip of exactly n_win windows.  ``guidance`` may hold ``a_cfg_scale``, ``r_cfg_scale``,
+        ``e_cfg_scale`` and ``include_r_cfg``, each overriding the sampler's keyword for this stream."""
+        d, L = self.dims, self.dims.frames_per_clip
+        unknown = sorted(set(guidance) - set(_GUIDANCE_KEYS))
+        if unknown:
+            raise TypeError(f"open: unexpected keyword(s) {unknown}")
+        self._check_tensor("open", "r_s", r_s, (1, d.dim_w))
+        if self.we_dynamic:
+            if we is not None:
+                raise ValueError("open: this sampler has dynamic emotion: we arrives with feed(), one frame per audio frame")
+        else:
+            if we is None:
+                raise ValueError("open: this sampler has static emotion: give we (1, 1, dim_e) here")
+            self._check_tensor("open", "we", we, (1, 1, d.dim_e))
+        if (seed is None) == (noise is None):
+            raise ValueError("open: give exactly one of 'seed' and 'noise'")
+        if noise is not None:
+            self._check_tensor("open", "noise", noise, (None, L, d.dim_w) if torch.is_tensor(noise) and noise.dim() == 3 else (None, 1, L, d.dim_w))
+            if noise.shape[0] < 1:
+                raise ValueError("open: noise holds no window")
+        g = _own_guidance("open", guidance, *self._keywords)
+        if g[3] > self.n_branches:
+            raise ValueError(f"open: this stream's guidance needs {g[3]} CFG branches, the sampler's plan runs {self.n_branches} "
+                             "(construct it with the guidance of the stream that needs the most)")
+        dev = self.device
+        gen = torch.Generator(dev).manual_seed(int(seed)) if seed is not None else None
+        st = Stream(self._opened, L, _as_f32(r_s, dev).clone(), None if we is None else _as_f32(we, dev).clone(),
+                    torch.zeros(d.num_prev_frames, d.dim_w, device=dev), torch.empty(0, d.dim_a, device=dev),
+                    torch.empty(0, d.dim_e, device=dev) if self.we_dynamic else None, gen,
+                    None if noise is None else noise.reshape(noise.shape[0], L, d.dim_w), g)
+        self._opened += 1
+        self._streams.append(st)
+        return st
+
+    def feed(self, stream: Stream, wa, we=None) -> None:
+        """Appends audio latents ``wa`` (1, t, dim_a), t >= 1, and with dynamic emotion as many ``we`` frames (1, t, dim_e)."""
+        st, d = self._own(stream), self.dims
+        if st.finished:
+            raise ValueError("feed: the stream is finished")
+        self._check_tensor("feed", "wa", wa, (1, None, d.dim_a))
+        t = wa.shape[1]
+        if t < 1:
+            raise ValueError("feed: wa holds no frame")
+        if self.we_dynamic:
+            if we is None:
+                raise ValueError("feed: this sampler has dynamic emotion: give we (1, t, dim_e) with every wa")
+            self._check_tensor("feed", "we", we, (1, t, d.dim_e))
+        elif we is not None:
+            raise ValueError("feed: this sampler has static emotion, given to open(); feed takes wa only")
+        if st.noise is not None and -(-(st.fed + t) // d.frames_per_clip) > st.noise.shape[0]:
+            raise ValueError(f"feed: {st.fed + t} frames need more windows than the stream's {st.noise.shape[0]} windows of noise")
+        st.wa = torch.cat([st.wa, wa[0].to(device=self.device, dtype=torch.float32)])
+        if self.we_dynamic:
+            st.we_buf = torch.cat([st.we_buf, we[0].to(device=self.device, dtype=torch.float32)])
+        st.fed += t
+        self._clock += 1
+        self._refresh(st)
+
+    def finish(self, stream: Stream) -> None:
+        """No more audio comes for this stream: its clip has as many frames as were fed."""
+        st, L = self._own(stream), self.dims.frames_per_clip
+        if st.finished:
+            raise ValueError("finish: the stream is already finished")
+        if st.fed < 1:
+            raise ValueError("finish: no audio was fed to the stream")
+        if st.noise is not None and st.noise.shape[0] != -(-st.fed // L):
+            raise ValueError(f"finish: {st.fed} frames are {-(-st.fed // L)} windows, but the stream's noise holds {st.noise.shape[0]}")
+        st.finished = True
+        self._clock += 1
+        self._refresh(st)
+
+    def close(self, stream: Stream) -> None:
+        """Forgets the stream and frees its buffers, whether or not all its windows ran."""
+        st = self._own(stream)
+        self._streams.remove(st)
+        st.wa = st.we_buf = st.ctx = st.r_s = st.we = st.gen = st.noise = None
+        st.ready_at = None
+
+    def _ready(self, st: Stream) -> bool:
+        L, w = self.dims.frames_per_clip, st.windows_run
+        return st.fed >= (w + 1) * L or (st.finished and w * L < st.fed)
+
+    def _refresh(self, st: Stream):
+        if st.ready_at is None and self._ready(st):
+            st.ready_at = self._clock
+
+    def ready(self) -> List[Stream]:
+        """The streams the next :meth:`step` runs, in slot order."""
+        waiting = [st for st in self._streams if st.ready_at is not None]
+        return sorted(waiting, key=lambda st: (st.ready_at, st.index))[:self.slots]
+
+    def step(self) -> Dict[Stream, torch.Tensor]:
+        """One window of each of up to ``slots`` ready streams; returns their new frames, (1, n, dim_w) each, on the device.
+        Asynchronous, like :func:`sample_clips`.  Returns {} when no stream is ready."""
+        run = self.ready()
+        if not run:
+            return {}
+        d, dev = self.dims, self.device
+        L, P = d.frames_per_clip, d.num_prev_frames
+        self._configure()                                  # no-op unless the backend ran another plan in between
+        x0, outs = [], []
+        for st in run:
+            w = st.windows_run
+            x0.append(torch.randn(1, L, d.dim_w, device=dev, generator=st.gen) if st.gen is not None
+                      else st.noise[w].to(device=dev, dtype=torch.float32).contiguous())
+            outs.append(torch.empty(1, min(L, st.fed - w * L), d.dim_w, device=dev))
+        self._be.sample_windows([st.r_s for st in run], [st.wa for st in run],
+                                [st.we_buf if self.we_dynamic else st.we for st in run], x0, [st.ctx for st in run], outs,
+                                [int(st.windows_run == 0) for st in run], *zip(*[st.guidance for st in run]))
+        self._clock += 1
+        for st in run:
+            st.windows_run += 1
+            st.ready_at = None
+            # keep frames from the next window's first context frame on (copied, so the dropped frames are freed)
+            keep = st.windows_run * L - P - st.base
+            st.wa = st.wa[keep:].clone()
+            if self.we_dynamic:
+                st.we_buf = st.we_buf[keep:].clone()
+            st.base += keep
+            self._refresh(st)
+        return dict(zip(run, outs))
 
 
 def float_sample(fmt_model, opt, r_s, wa, we, a_cfg_scale=1.0, r_cfg_scale=1.0, e_cfg_scale=1.0, seed=None,

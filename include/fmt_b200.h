@@ -151,6 +151,25 @@ typedef struct FmtClipGuidance {
   const int32_t* n_branches;        /* 1, 3 or 4, <= plan.n_branches; a 1-branch plan takes 1-branch clips only */
 } FmtClipGuidance;
 
+/* One window of each of n_streams streams (fmt_sample_windows): a stream is a clip whose audio arrives in pieces, run one window per
+ * call.  Every pointer is a DEVICE pointer; the arrays themselves are host arrays of n_streams entries.  Window w of a stream reads
+ * wa / we frames [w*L - P, (w+1)*L) and writes its frames [w*L, w*L + n_out); the buffers below start at its first context frame. */
+typedef struct FmtWindowSet {
+  int32_t n_streams;                /* 1 <= n_streams <= plan.batch; stream i runs in slot i, slots n_streams.. are idle            */
+  const float* const* r_s;          /* [i]: (1, dim_w)                                                                           */
+  const float* const* wa;           /* [i]: (T_wa[i], dim_a) from frame w*L - P (frame 0 in a first window); frames beyond T_wa[i]
+                                       are the last frame repeated, as in a clip's last window                                  */
+  const float* const* we;           /* [i]: static (1, dim_e), or dynamic (T_we[i], dim_e) from the same frame as wa                */
+  const float* const* x0;           /* [i]: (L, dim_w) noise of this window                                                      */
+  float* const* ctx;                /* [i]: (P, dim_w) in / out: the last P frames of the stream's previous window (not read in a
+                                       first window); receives this window's last P frames                                       */
+  float* const* r_d;                /* [i]: out (n_out[i], dim_w): the window's first n_out[i] frames                             */
+  const int32_t* T_wa;              /* frames of wa[i]; the window's first current frame (P, or 0 in a first window) must be one  */
+  const int32_t* T_we;              /* 1 (static) or the frames of we[i] (dynamic), likewise                                     */
+  const int32_t* n_out;             /* 1 <= n_out[i] <= L                                                                        */
+  const int32_t* first_window;      /* 1: the stream's window 0: zero context                                                   */
+} FmtWindowSet;
+
 /* One evaluation of forward_with_cfv (FMT.py:342-401) on explicit window inputs - tests and ncu. */
 typedef struct FmtEval {
   const float* x;         /* (B, L, dim_w)                     */
@@ -201,6 +220,11 @@ FMT_API int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* set, void* stre
  * own inputs and guidance and on the plan.  Returns -1 if an n_branches[i] is not 1, 3 or 4 or exceeds plan.n_branches, or if a
  * 1-branch plan gets a clip with more than one branch. */
 FMT_API int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* set, const FmtClipGuidance* guidance, void* stream);
+
+/* One window of each stream of the set, with each stream's own guidance (n_streams entries; as in fmt_sample_clips_guided), through
+ * the plan's captured window graph.  A stream's window computes what the same window of fmt_sample_clips computes for the whole
+ * clip.  Returns -1 on bad arguments. */
+FMT_API int32_t fmt_sample_windows(FmtHandle* h, const FmtWindowSet* set, const FmtClipGuidance* guidance, void* stream);
 
 /* Single CFG-combined model evaluation (device pointers). */
 FMT_API int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream);
