@@ -67,6 +67,11 @@ class FmtWindowSet(C.Structure):
                [(n, C.POINTER(C.c_int32)) for n in ("T_wa", "T_we", "n_out", "first_window")]
 
 
+class FmtClipOde(C.Structure):
+    _fields_ = [("n_steps", C.POINTER(C.c_int32)), ("n_stages", C.POINTER(C.c_int32))] + \
+               [(n, C.POINTER(C.POINTER(C.c_float))) for n in ("t_eval", "dt", "rk_a", "rk_b")]
+
+
 class FmtEval(C.Structure):
     _fields_ = [("x", C.c_void_p), ("prev_x", C.c_void_p), ("wa", C.c_void_p), ("prev_wa", C.c_void_p), ("we", C.c_void_p),
                 ("prev_we", C.c_void_p), ("r_s", C.c_void_p), ("v_out", C.c_void_p), ("eval_index", C.c_int32),
@@ -93,14 +98,18 @@ _SIGNATURES = {
     "fmt_sample_clips": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.c_void_p]),
     "fmt_sample_clips_guided": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.POINTER(FmtClipGuidance), C.c_void_p]),
     "fmt_sample_windows": (C.c_int32, [C.c_void_p, C.POINTER(FmtWindowSet), C.POINTER(FmtClipGuidance), C.c_void_p]),
+    "fmt_sample_clips_ode": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.POINTER(FmtClipGuidance), C.POINTER(FmtClipOde), C.c_void_p]),
+    "fmt_sample_windows_ode": (C.c_int32, [C.c_void_p, C.POINTER(FmtWindowSet), C.POINTER(FmtClipGuidance), C.POINTER(FmtClipOde), C.c_void_p]),
     "fmt_clip_schedule": (C.c_int32, [C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32)]),
     "fmt_velocity": (C.c_int32, [C.c_void_p, C.POINTER(FmtEval), C.c_void_p]),
     "fmt_launch_count": (C.c_int64, [C.c_void_p, C.c_int32]),
     "fmt_graph_kernel_nodes": (C.c_int32, [C.c_void_p]),
+    "fmt_ode_graph_kernel_nodes": (C.c_int32, [C.c_void_p]),
     "fmt_window_kernel_status": (C.c_int32, [C.c_void_p]),
     "fmt_debug_window_trace": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int64]),
     "fmt_debug_condition_rows": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "fmt_debug_condition_rows_ode": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "fmt_proj_create": (C.c_int32, [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int32, C.c_int32,
                                     C.POINTER(C.c_void_p)]),
     "fmt_proj_destroy": (C.c_int32, [C.c_void_p]),

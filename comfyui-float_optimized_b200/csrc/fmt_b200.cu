@@ -94,11 +94,23 @@ struct FmtHandle {
   int use_dedup = 1;
   DevBuf st_rs, st_wa, st_we, st_noise, st_rd;   // staging for host-located clips
   // fmt_sample_clips: the slot records of every window of a call ([window][slot]), uploaded with one copy from a pinned staging
-  // buffer; slot_ev marks the end of that copy, so the next call waits for it before it refills the staging buffer
+  // buffer; slot_ev marks the end of that copy, so the next call waits for it before it refills the staging buffer.  A window's
+  // records are slot_stride bytes: B SlotArgs, followed by B SlotOde in calls of the per-slot window graph.
   DevBuf slot_buf, slot_zero;                    // slot_zero: the inputs of an idle slot
-  SlotArgs* slot_host = nullptr;
-  size_t slot_host_n = 0;
+  unsigned char* slot_host = nullptr;
+  size_t slot_host_bytes = 0, slot_stride = 0;
   cudaEvent_t slot_ev = nullptr;
+  // per-slot ODE schedules (fmt_sample_clips_ode, fmt_sample_windows_ode): a second window graph of the plan, captured on first use.
+  // It shares the plan's workspace and AdaLN table buffer; its condition rows never span two slots (sU rows, sU - U more than the
+  // plan's in 4-branch plans), its kbuf holds FMT_MAX_STAGES stages.
+  std::map<std::vector<float>, DevBuf> ode_cache;   // t-embeddings and step sizes of every schedule seen, keyed by its contents
+  DevBuf s_cond, s_cemb, s_urow, s_uidx, s_kbuf;
+  int sU = 0, s_chunk = 0;
+  bool s_dedup = false;
+  cudaGraphExec_t ode_exec = nullptr;
+  int ode_nodes = 0;
+  long long ode_launches = 0;
+  bool last_ode = false;                         // the last sampling call ran the per-slot graph
   bool use_splitk = false;                       // 2-way K slicing of gate+residual GEMMs with a ragged last wave (FMT_SPLITK=1; measured 3 % slower at 32 clips)
   int raster_gm = 8;                             // FMT_RASTER_GM
   bool use_pair = true;                          // CTA-pair (cta_group::2) GEMM for M >= 512 (FMT_PAIR=0 disables)
@@ -332,25 +344,51 @@ static EpiParams epi(int kind, int M, int N, const float* bias, void* out, int l
 }
 
 // ------------------------------------------------------------------------------------------------ the FMT step
+// The distinct condition rows a window graph works on: the plan's (fmt_configure), or the per-slot graph's, which never shares a row
+// between two slots.  urow / uidx: table row of every token row / token row of every table row (nullptr: the identity).
+struct CondRows {
+  int U;
+  const int* urow;
+  const int* uidx;
+  void* cond;
+  void* cemb;
+  int chunk;                                     // evaluations whose tables the table buffer holds at once
+  bool per_slot;                                 // t-embeddings of each slot's own schedule (silu_cond_sched_kernel)
+};
+
+static CondRows plan_rows(const FmtHandle* h) {
+  return CondRows{h->U, h->dedup ? static_cast<const int*>(h->urow_buf.p) : nullptr, h->dedup ? static_cast<const int*>(h->uidx_buf.p) : nullptr,
+                  h->cond.p, h->cemb.p, h->table_chunk, false};
+}
+
+static CondRows ode_rows(const FmtHandle* h) {
+  return CondRows{h->sU, h->s_dedup ? static_cast<const int*>(h->s_urow.p) : nullptr, h->s_dedup ? static_cast<const int*>(h->s_uidx.p) : nullptr,
+                  h->s_cond.p, h->s_cemb.p, h->s_chunk, true};
+}
+
 template <typename T>
-static int enqueue_prepare(FmtHandle* h, cudaStream_t st) {
+static int enqueue_prepare(FmtHandle* h, const CondRows& r, cudaStream_t st) {
   const ModelShape& s = h->shape;
   const WindowArgs* wa = static_cast<const WindowArgs*>(h->wargs.p);
-  FMT_OK(launch(h, cond_gather_kernel<T>, dim3(h->U), dim3(128), 0, st, 1, wa, s, h->dedup ? static_cast<const int*>(h->uidx_buf.p) : nullptr,
-                static_cast<T*>(h->cond.p)));
-  EpiParams ep = epi(EPI_STORE, h->U, s.H, h->c_emb.b, h->cemb.p, s.H, 1);
-  FMT_OK(ModeOps<T>::gemm(h, h->cond.p, s.Kc, h->c_emb, ep, st));
+  FMT_OK(launch(h, cond_gather_kernel<T>, dim3(r.U), dim3(128), 0, st, 1, wa, s, r.uidx, static_cast<T*>(r.cond)));
+  EpiParams ep = epi(EPI_STORE, r.U, s.H, h->c_emb.b, r.cemb, s.H, 1);
+  FMT_OK(ModeOps<T>::gemm(h, r.cond, s.Kc, h->c_emb, ep, st));
   return 0;
 }
 
 // AdaLN tables for evaluations [e0, e0+n): table[(e-e0)*U + u, :] = Linear_ada(SiLU(c_emb[u] + t_emb[e]))
 template <typename T>
-static int enqueue_tables(FmtHandle* h, int e0, int n, cudaStream_t st) {
+static int enqueue_tables(FmtHandle* h, const CondRows& r, int e0, int n, cudaStream_t st) {
   const ModelShape& s = h->shape;
-  const size_t total = static_cast<size_t>(n) * h->U * s.H;
-  FMT_OK(launch(h, silu_cond_kernel<T>, dim3(static_cast<unsigned>((total / 4 + 255) / 256)), dim3(256), 0, st, 1,
-                static_cast<const float*>(h->cemb.p), static_cast<const float*>(h->temb.p), e0, h->U, s.H, static_cast<T*>(h->silu.p), total));
-  EpiParams ep = epi(EPI_STORE, n * h->U, h->NT, h->ada.b, h->table.p, h->NT, sizeof(typename ModeOps<T>::Tab) == 4);
+  const size_t total = static_cast<size_t>(n) * r.U * s.H;
+  const dim3 grid(static_cast<unsigned>((total / 4 + 255) / 256));
+  if (r.per_slot)
+    FMT_OK(launch(h, silu_cond_sched_kernel<T>, grid, dim3(256), 0, st, 1, static_cast<const WindowArgs*>(h->wargs.p), s,
+                  static_cast<const float*>(r.cemb), r.uidx, e0, r.U, static_cast<T*>(h->silu.p), total));
+  else
+    FMT_OK(launch(h, silu_cond_kernel<T>, grid, dim3(256), 0, st, 1, static_cast<const float*>(r.cemb), static_cast<const float*>(h->temb.p), e0,
+                  r.U, s.H, static_cast<T*>(h->silu.p), total));
+  EpiParams ep = epi(EPI_STORE, n * r.U, h->NT, h->ada.b, h->table.p, h->NT, sizeof(typename ModeOps<T>::Tab) == 4);
   FMT_OK(ModeOps<T>::gemm(h, h->silu.p, s.H, h->ada, ep, st));
   return 0;
 }
@@ -372,9 +410,9 @@ static int lnmod(FmtHandle* h, const float* X, int rows, int H, const typename M
 }
 
 template <typename T>
-static int launch_lnmod(FmtHandle* h, const typename ModeOps<T>::Tab* table_e, long long shift_off, long long scale_off, cudaStream_t st) {
-  const int* urow = h->dedup ? static_cast<const int*>(h->urow_buf.p) : nullptr;
-  return lnmod<T>(h, static_cast<const float*>(h->X.p), h->R, h->shape.H, table_e, urow, h->NT, shift_off, scale_off, static_cast<T*>(h->A1.p), st);
+static int launch_lnmod(FmtHandle* h, const CondRows& r, const typename ModeOps<T>::Tab* table_e, long long shift_off, long long scale_off,
+                        cudaStream_t st) {
+  return lnmod<T>(h, static_cast<const float*>(h->X.p), h->R, h->shape.H, table_e, r.urow, h->NT, shift_off, scale_off, static_cast<T*>(h->A1.p), st);
 }
 
 // Band attention of n_seq sequences of N rows.  variant 0 picks the kernel, 1 forces the warp-per-row kernel, 2 the tile kernel.
@@ -420,12 +458,12 @@ static int launch_attn(FmtHandle* h, cudaStream_t st) {
 // One model evaluation: V[R, W] = FMT.forward over the nb-way batched CFG branches (FMT.py:277-340).  The x-embedder
 // operand `ax` has already been written by the producer of the ODE state (init_window / cfg_combine / rk_combine / pack_x).
 template <typename T>
-static int enqueue_forward(FmtHandle* h, int table_slot, cudaStream_t st) {
+static int enqueue_forward(FmtHandle* h, const CondRows& r, int table_slot, cudaStream_t st) {
   const ModelShape& s = h->shape;
   const FmtDims& d = h->d;
   const int R = h->R, H = s.H;
   using TT = typename ModeOps<T>::Tab;
-  const TT* table_e = static_cast<const TT*>(h->table.p) + static_cast<size_t>(table_slot) * h->U * h->NT;
+  const TT* table_e = static_cast<const TT*>(h->table.p) + static_cast<size_t>(table_slot) * r.U * h->NT;
   const int qkv_f32 = sizeof(TT) == 4;
   {
     EpiParams ep = epi(EPI_POS, R, H, h->x_emb.b, h->X.p, H, 1);
@@ -434,24 +472,24 @@ static int enqueue_forward(FmtHandle* h, int table_slot, cudaStream_t st) {
   }
   for (int i = 0; i < d.depth; ++i) {
     const long long base = static_cast<long long>(i) * 6 * H;
-    FMT_OK(launch_lnmod<T>(h, table_e, base + 0, base + H, st));
+    FMT_OK(launch_lnmod<T>(h, r, table_e, base + 0, base + H, st));
     FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->qkv[i], epi(EPI_STORE, R, 3 * H, h->qkv[i].b, h->QKV.p, 3 * H, qkv_f32), st));
     FMT_OK(launch_attn<T>(h, st));
     {
       EpiParams ep = epi(EPI_GATE_RES, R, H, h->proj[i].b, h->X.p, H, 1);
-      ep.gate = table_e; ep.urow = h->dedup ? static_cast<const int*>(h->urow_buf.p) : nullptr; ep.ldg = h->NT; ep.gate_off = base + 2 * H;
+      ep.gate = table_e; ep.urow = r.urow; ep.ldg = h->NT; ep.gate_off = base + 2 * H;
       FMT_OK(ModeOps<T>::gemm(h, h->A2.p, H, h->proj[i], ep, st));
     }
-    FMT_OK(launch_lnmod<T>(h, table_e, base + 3 * H, base + 4 * H, st));
+    FMT_OK(launch_lnmod<T>(h, r, table_e, base + 3 * H, base + 4 * H, st));
     FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->fc1[i], epi(EPI_GELU, R, d.mlp_hidden, h->fc1[i].b, h->Hm.p, d.mlp_hidden, 0), st));
     {
       EpiParams ep = epi(EPI_GATE_RES, R, H, h->fc2[i].b, h->X.p, H, 1);
-      ep.gate = table_e; ep.urow = h->dedup ? static_cast<const int*>(h->urow_buf.p) : nullptr; ep.ldg = h->NT; ep.gate_off = base + 5 * H;
+      ep.gate = table_e; ep.urow = r.urow; ep.ldg = h->NT; ep.gate_off = base + 5 * H;
       FMT_OK(ModeOps<T>::gemm(h, h->Hm.p, d.mlp_hidden, h->fc2[i], ep, st));
     }
   }
   const long long dbase = static_cast<long long>(d.depth) * 6 * H;
-  FMT_OK(launch_lnmod<T>(h, table_e, dbase, dbase + H, st));
+  FMT_OK(launch_lnmod<T>(h, r, table_e, dbase, dbase + H, st));
   FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->dec, epi(EPI_STORE, R, s.W, h->dec.b, h->V.p, s.W, 1), st));
   return 0;
 }
@@ -841,13 +879,14 @@ static int enqueue_window(FmtHandle* h, cudaStream_t st) {
   const float* ddt = static_cast<const float*>(h->ddt.p);
   const int S = h->plan.n_steps, G = h->plan.n_stages;
   const dim3 gx(static_cast<unsigned>((nx + 255) / 256)), blk(256);
+  const CondRows r = plan_rows(h);
 
   FMT_OK(launch(h, init_window_kernel<T>, dim3(static_cast<unsigned>((nfull + 255) / 256)), blk, 0, st, 1, wa, s, x_state,
                 static_cast<float*>(h->prevx.p), ax));
-  if (S > 0) FMT_OK(enqueue_prepare<T>(h, st));
+  if (S > 0) FMT_OK(enqueue_prepare<T>(h, r, st));
   if (h->window_active && S > 0) {
     // small-R plan: every evaluation of the window runs inside ONE persistent kernel (flow.cuh; window.cuh with FMT_WINDOW=1/2)
-    FMT_OK(enqueue_tables<T>(h, 0, h->n_eval, st));
+    FMT_OK(enqueue_tables<T>(h, r, 0, h->n_eval, st));
     if (h->flow_active) FMT_OK(launch_flow(h, st));
     else FMT_OK(launch_window(h, st));
     FMT_OK(launch(h, finalize_window_kernel, gx, blk, 0, st, 1, wa, s, static_cast<const float*>(x_state), static_cast<float*>(h->prevx.p)));
@@ -858,14 +897,14 @@ static int enqueue_window(FmtHandle* h, cudaStream_t st) {
       const int e = step * G + g;
       if (e % h->table_chunk == 0) {
         const int n = (h->n_eval - e) < h->table_chunk ? (h->n_eval - e) : h->table_chunk;
-        FMT_OK(enqueue_tables<T>(h, e, n, st));
+        FMT_OK(enqueue_tables<T>(h, r, e, n, st));
       }
       if (g > 0) {   // y_g = y0 + dt * sum_j a[g][j] k_j  (also refreshes the x-embedder operand)
         const float* a = &h->rk_a[g * G];
         FMT_OK(launch(h, rk_combine_kernel<T>, gx, blk, 0, st, 1, s, static_cast<const float*>(x_state), y_stage, static_cast<const float*>(kbuf), nx, nx, g,
                       a[0], G > 1 ? a[1] : 0.f, G > 2 ? a[2] : 0.f, G > 3 ? a[3] : 0.f, ddt + step, ax));
       }
-      FMT_OK(enqueue_forward<T>(h, e % h->table_chunk, st));
+      FMT_OK(enqueue_forward<T>(h, r, e % h->table_chunk, st));
       if (G == 1) FMT_OK(launch_combine<T>(h, 2, x_state, ddt + step, st));           // fused CFG + Euler
       else FMT_OK(launch_combine<T>(h, 1, kbuf + static_cast<size_t>(g) * nx, nullptr, st));
     }
@@ -885,6 +924,70 @@ static int enqueue_window_mode(FmtHandle* h, cudaStream_t st) {
     case FMT_MODE_BF16X3: return enqueue_window<bf16x3_t>(h, st);
   }
   return enqueue_window<float>(h, st);
+}
+
+// The per-slot window graph: the plan's evaluation count, every slot on its own schedule (SlotOde), always one kernel per op.  Each
+// evaluation e is [the stage combine of the slots at a stage > 0 (e > 0)] -> forward -> [CFG combine + the ODE update of each slot
+// that is at an evaluation of its own].
+template <typename T>
+static int enqueue_window_ode(FmtHandle* h, cudaStream_t st) {
+  const ModelShape& s = h->shape;
+  const WindowArgs* wa = static_cast<const WindowArgs*>(h->wargs.p);
+  const size_t nx = static_cast<size_t>(s.B) * s.L * s.W, nfull = static_cast<size_t>(s.B) * s.N * s.W;
+  float* x_state = static_cast<float*>(h->xstate.p);
+  float* kbuf = static_cast<float*>(h->s_kbuf.p);
+  T* ax = static_cast<T*>(h->ax.p);
+  const dim3 gx(static_cast<unsigned>((nx + 255) / 256)), gfull(static_cast<unsigned>((nfull + 255) / 256)), blk(256);
+  const CondRows r = ode_rows(h);
+  const int ne = h->n_eval;
+
+  FMT_OK(launch(h, init_window_kernel<T>, gfull, blk, 0, st, 1, wa, s, x_state, static_cast<float*>(h->prevx.p), ax));
+  if (ne > 0) FMT_OK(enqueue_prepare<T>(h, r, st));
+  for (int e = 0; e < ne; ++e) {
+    if (e % r.chunk == 0) FMT_OK(enqueue_tables<T>(h, r, e, std::min(ne - e, r.chunk), st));
+    if (e > 0)
+      FMT_OK(launch(h, sched_stage_kernel<T>, gx, blk, 0, st, 1, wa, s, static_cast<const float*>(x_state), static_cast<float*>(h->ystage.p),
+                    static_cast<const float*>(kbuf), nx, e, ax));
+    FMT_OK(enqueue_forward<T>(h, r, e % r.chunk, st));
+    FMT_OK(launch(h, sched_combine_kernel<T>, gfull, blk, 0, st, 1, wa, s, static_cast<const float*>(h->V.p), e, x_state, kbuf, nx, ax));
+  }
+  FMT_OK(launch(h, finalize_window_kernel, gx, blk, 0, st, 1, wa, s, static_cast<const float*>(x_state), static_cast<float*>(h->prevx.p)));
+  return 0;
+}
+
+static int enqueue_window_ode_mode(FmtHandle* h, cudaStream_t st) {
+  switch (h->plan.mode) {
+    case FMT_MODE_BF16: return enqueue_window_ode<bf16>(h, st);
+    case FMT_MODE_BF16X3: return enqueue_window_ode<bf16x3_t>(h, st);
+  }
+  return enqueue_window_ode<float>(h, st);
+}
+
+// Captures one window of enqueue(h, .) as a CUDA graph; *launches: the kernels it holds (counted by launch())
+static int capture_window(FmtHandle* h, int (*enqueue)(FmtHandle*, cudaStream_t), cudaGraphExec_t* exec, int* nodes, long long* launches) {
+  cudaGraph_t graph = nullptr;
+  cudaStream_t cs;
+  CUDA_OK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+  // make sure the lazily-set function attributes exist before capture (attribute calls are not capturable work but are legal)
+  CUDA_OK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
+  const long long outer = h->capture_launches;
+  h->capturing = true; h->capture_launches = 0;
+  int rc = enqueue(h, cs);
+  h->capturing = false;
+  const long long counted = h->capture_launches;
+  h->capture_launches = outer;
+  cudaError_t ce = cudaStreamEndCapture(cs, &graph);
+  if (rc != 0) { if (graph) cudaGraphDestroy(graph); cudaStreamDestroy(cs); return rc; }
+  if (ce != cudaSuccess) { cudaStreamDestroy(cs); return set_err(-2, "graph capture failed: %s", cudaGetErrorString(ce)); }
+  size_t n_nodes = 0;
+  cudaGraphGetNodes(graph, nullptr, &n_nodes);
+  *nodes = static_cast<int>(n_nodes);
+  ce = cudaGraphInstantiate(exec, graph, 0);
+  cudaGraphDestroy(graph);
+  cudaStreamDestroy(cs);
+  if (ce != cudaSuccess) return set_err(-2, "cudaGraphInstantiate failed: %s", cudaGetErrorString(ce));
+  *launches = counted;
+  return 0;
 }
 
 // ------------------------------------------------------------------------------------------------ create / destroy
@@ -1074,12 +1177,14 @@ int32_t fmt_destroy(FmtHandle* h) {
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();
   if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
+  if (h->ode_exec) cudaGraphExecDestroy(h->ode_exec);
   for (void* p : h->owned) cudaFree(p);
+  for (auto& kv : h->ode_cache) cudaFree(kv.second.p);
   DevBuf* bufs[] = {&h->cond, &h->cemb, &h->temb, &h->tfreq, &h->th, &h->silu, &h->table, &h->xstate, &h->ystage, &h->kbuf, &h->prevx, &h->ax,
                     &h->X, &h->A1, &h->QKV, &h->A2, &h->Hm, &h->V, &h->ddt, &h->dteval, &h->wargs, &h->st_rs, &h->st_wa, &h->st_we, &h->st_noise, &h->st_rd,
                     &h->win_params, &h->win_tmaps, &h->win_acc, &h->win_bar, &h->win_trace, &h->win_act,
                     &h->flow_gemms, &h->flow_tmaps, &h->flow_acc, &h->flow_act, &h->flow_flags, &h->flow_trace, &h->urow_buf, &h->uidx_buf,
-                    &h->slot_buf, &h->slot_zero};
+                    &h->slot_buf, &h->slot_zero, &h->s_cond, &h->s_cemb, &h->s_urow, &h->s_uidx, &h->s_kbuf};
   for (DevBuf* b : bufs)
     if (b->p) cudaFree(b->p);
   if (h->win_err_host) cudaFreeHost(h->win_err_host);
@@ -1098,6 +1203,7 @@ int64_t fmt_launch_count(const FmtHandle* hc, int32_t reset) {
   return v;
 }
 int32_t fmt_graph_kernel_nodes(const FmtHandle* h) { return h ? h->graph_nodes : 0; }
+int32_t fmt_ode_graph_kernel_nodes(const FmtHandle* h) { return h ? h->ode_nodes : 0; }
 int64_t fmt_debug_window_trace(const FmtHandle* h, int64_t* out, int64_t max_elems) {
   if (h && h->flow_active && h->flow_trace.p) {   // dataflow kernel: [cta][engine][stage][chunk][4] SM-clock stamps
     const int64_t nf = static_cast<int64_t>(h->flow_trace.bytes / sizeof(long long));
@@ -1115,26 +1221,29 @@ int64_t fmt_debug_window_trace(const FmtHandle* h, int64_t* out, int64_t max_ele
 }
 int32_t fmt_window_kernel_status(const FmtHandle* h) {
   if (!h || !h->window_active) return -1;
-  return h->win_err_host ? *h->win_err_host : 0;
+  const int trapped = h->win_err_host ? *h->win_err_host : 0;
+  if (trapped != 0) return trapped;             // a tripped spin of an earlier window stays visible after per-slot calls
+  return h->last_ode ? -1 : 0;
 }
 
 // Which token rows (branch, clip, frame) see the same condition row [wr | wa | we]?  urow[row] = index of the row's distinct
 // condition row, uidx[u] = the first token row that sees distinct row u.  The key is exactly what cond_gather_kernel reads for a
 // row: the identity latent unless nulled (per clip), the audio latent (context frames read prev_wa, never nulled, FMT.py:366,388;
 // current frames read wa unless nulled), the emotion (nulled; static = per clip, covering the context frames too, FMT.py:325-326;
-// dynamic = per frame).
-static void distinct_condition_rows(const ModelShape& s, std::vector<int>& urow, std::vector<int>& uidx) {
+// dynamic = per frame).  per_slot: rows of different slots are never shared (the per-slot window graph, whose slots have their own
+// times): only the truly-uncond current frames of 4-branch plans, [0 | 0 | 0] in every slot, are affected.
+static void distinct_condition_rows(const ModelShape& s, std::vector<int>& urow, std::vector<int>& uidx, bool per_slot = false) {
   const int R = s.nb * s.B * s.N;
   urow.assign(R, 0);
   uidx.clear();
-  std::map<std::tuple<int, int, int, int, int, int, int>, int> seen;
+  std::map<std::tuple<int, int, int, int, int, int, int, int>, int> seen;
   for (int row = 0; row < R; ++row) {
     const int br = row / (s.B * s.N), b = (row / s.N) % s.B, f = row % s.N;
     const bool za = (s.null_a >> br) & 1, zr = (s.null_r >> br) & 1, ze = (s.null_e >> br) & 1, ctx = f < s.P;
     const int kr = zr ? -1 : b;
     const int ka = ctx ? 0 : (za ? 1 : 2), kab = (ctx || !za) ? b : -1, kaf = (ctx || !za) ? f : -1;
     const int ke = ze ? 0 : (s.we_dynamic ? 2 : 1), keb = ze ? -1 : b, kef = (!ze && s.we_dynamic) ? f : -1;
-    const auto key = std::make_tuple(kr, ka, kab, kaf, ke, keb, kef);
+    const auto key = std::make_tuple(kr, ka, kab, kaf, ke, keb, kef, per_slot ? b : -1);
     auto it = seen.find(key);
     if (it == seen.end()) { it = seen.emplace(key, static_cast<int>(uidx.size())).first; uidx.push_back(row); }
     urow[row] = it->second;
@@ -1149,12 +1258,17 @@ static void branch_nulls(ModelShape& s) {
 
 // Host-only view of the deduplication for tests (no device work): fills urow[n_branches * batch * n_frames], returns U.
 int32_t fmt_debug_condition_rows(int32_t n_branches, int32_t batch, int32_t n_frames, int32_t n_prev, int32_t we_dynamic, int32_t* urow_out) {
+  return fmt_debug_condition_rows_ode(n_branches, batch, n_frames, n_prev, we_dynamic, 0, urow_out);
+}
+
+int32_t fmt_debug_condition_rows_ode(int32_t n_branches, int32_t batch, int32_t n_frames, int32_t n_prev, int32_t we_dynamic, int32_t per_slot,
+                                     int32_t* urow_out) {
   if (n_branches < 1 || n_branches > 4 || batch < 1 || n_frames < 1 || n_prev < 0 || n_prev > n_frames) return -1;
   ModelShape s{};
   s.nb = n_branches; s.B = batch; s.N = n_frames; s.P = n_prev; s.we_dynamic = we_dynamic;
   branch_nulls(s);
   std::vector<int> urow, uidx;
-  distinct_condition_rows(s, urow, uidx);
+  distinct_condition_rows(s, urow, uidx, per_slot != 0);
   if (urow_out != nullptr) std::copy(urow.begin(), urow.end(), urow_out);
   return static_cast<int32_t>(uidx.size());
 }
@@ -1228,6 +1342,7 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
   REQUIRE(p->mode == FMT_MODE_BF16 || p->mode == FMT_MODE_FP32_VALIDATE || p->mode == FMT_MODE_BF16X3, "fmt_configure: unknown mode %d", p->mode);
   REQUIRE(p->n_steps >= 0 && p->n_stages >= 1 && p->n_stages <= FMT_MAX_STAGES, "fmt_configure: bad n_steps/n_stages");
   REQUIRE(p->rk_a && p->rk_b && (p->n_steps == 0 || (p->t_eval && p->dt)), "fmt_configure: null schedule arrays");
+  h->last_ode = false;
   if (same_plan(h, p)) return 0;
   if (p->mode == FMT_MODE_BF16X3) {
     FMT_OK(pack_split_all(h, st));
@@ -1238,6 +1353,7 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
   const int ne = p->n_steps * p->n_stages;
   h->configured = false;
   if (h->graph_exec) { CUDA_OK(cudaStreamSynchronize(st)); cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; h->graph_nodes = 0; }
+  if (h->ode_exec) { CUDA_OK(cudaStreamSynchronize(st)); cudaGraphExecDestroy(h->ode_exec); h->ode_exec = nullptr; h->ode_nodes = 0; }
   h->plan = *p;
   h->t_eval.assign(p->t_eval, p->t_eval + ne);
   h->dt.assign(p->dt, p->dt + p->n_steps);
@@ -1297,6 +1413,9 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
   if (chunk < 1) chunk = 1;
   if (chunk > static_cast<size_t>(ne > 0 ? ne : 1)) chunk = ne > 0 ? ne : 1;
   h->table_chunk = static_cast<int>(chunk);
+  // the per-slot window graph (fmt_sample_clips_ode) keeps the truly-uncond current frames of a 4-branch plan one row per slot: B - 1
+  // more condition rows, for which the table and SiLU buffers keep room, so that it always fits at least one evaluation
+  const size_t slot_rows = h->dedup && s.nb == 4 ? static_cast<size_t>(s.B) - 1 : 0;
 
   const size_t nx = static_cast<size_t>(s.B) * s.L * s.W;
   FMT_OK(dev_alloc(h, h->cond, U * s.Kc * ts));
@@ -1304,8 +1423,8 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
   FMT_OK(dev_alloc(h, h->temb, static_cast<size_t>(ne > 0 ? ne : 1) * H * 4));
   FMT_OK(dev_alloc(h, h->tfreq, static_cast<size_t>(ne > 0 ? ne : 1) * 256 * 4));
   FMT_OK(dev_alloc(h, h->th, static_cast<size_t>(ne > 0 ? ne : 1) * H * 4));
-  FMT_OK(dev_alloc(h, h->silu, chunk * U * H * ts));
-  FMT_OK(dev_alloc(h, h->table, chunk * per_eval));
+  FMT_OK(dev_alloc(h, h->silu, (chunk * U + slot_rows) * H * ts));
+  FMT_OK(dev_alloc(h, h->table, chunk * per_eval + slot_rows * h->NT * ts));
   FMT_OK(dev_alloc(h, h->xstate, nx * 4));
   FMT_OK(dev_alloc(h, h->ystage, nx * 4));
   FMT_OK(dev_alloc(h, h->kbuf, nx * 4 * p->n_stages));
@@ -1361,26 +1480,7 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
   if (h->window_active && !h->flow_active) FMT_OK(setup_window(h, st));
 
   // capture one window as a CUDA graph
-  {
-    cudaGraph_t graph = nullptr;
-    cudaStream_t cs;
-    CUDA_OK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-    // make sure the lazily-set function attributes exist before capture (attribute calls are not capturable work but are legal)
-    CUDA_OK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-    h->capturing = true; h->capture_launches = 0;
-    int rc = enqueue_window_mode(h, cs);
-    h->capturing = false;
-    cudaError_t ce = cudaStreamEndCapture(cs, &graph);
-    if (rc != 0) { if (graph) cudaGraphDestroy(graph); cudaStreamDestroy(cs); return rc; }
-    if (ce != cudaSuccess) { cudaStreamDestroy(cs); return set_err(-2, "graph capture failed: %s", cudaGetErrorString(ce)); }
-    size_t n_nodes = 0;
-    cudaGraphGetNodes(graph, nullptr, &n_nodes);
-    h->graph_nodes = static_cast<int>(n_nodes);
-    ce = cudaGraphInstantiate(&h->graph_exec, graph, 0);
-    cudaGraphDestroy(graph);
-    cudaStreamDestroy(cs);
-    if (ce != cudaSuccess) return set_err(-2, "cudaGraphInstantiate failed: %s", cudaGetErrorString(ce));
-  }
+  FMT_OK(capture_window(h, enqueue_window_mode, &h->graph_exec, &h->graph_nodes, &h->capture_launches));
   h->configured = true;
   return 0;
 }
@@ -1393,37 +1493,145 @@ static int set_wargs(FmtHandle* h, const WindowArgs& a, cudaStream_t st) {
 
 // Slot records of one call (fmt_sample_clips, fmt_sample_windows) go up in ONE copy from a pinned staging buffer that the handle
 // owns; slot_ev marks the end of the previous call's copy, so the staging buffer is refilled only once that copy has read it.
-// stage_slot_records returns the staging buffer with n_rec idle records: zero inputs ((L, W) noise, and r_s / wa / we rows no wider
-// than that), no output, no context, scales of 1 and the plan's branch count.
-static int stage_slot_records(FmtHandle* h, size_t n_rec, cudaStream_t st, SlotArgs** out) {
+// stage_slot_records fills the staging buffer with n_win windows of idle records: zero inputs ((L, W) noise, and r_s / wa / we rows
+// no wider than that), no output, no context, scales of 1 and the plan's branch count; with ode, B SlotOde follow the B SlotArgs of
+// each window, idle as well (no evaluation).
+static int stage_slot_records(FmtHandle* h, size_t n_win, bool ode, cudaStream_t st) {
   const ModelShape& s = h->shape;
   const size_t n_zero = std::max<size_t>(static_cast<size_t>(s.L) * s.W, static_cast<size_t>(std::max(s.A, s.E)));
   FMT_OK(dev_alloc(h, h->slot_zero, n_zero * sizeof(float)));
   CUDA_OK(cudaMemsetAsync(h->slot_zero.p, 0, n_zero * sizeof(float), st));
   const float* zero = static_cast<const float*>(h->slot_zero.p);
   if (h->slot_ev) CUDA_OK(cudaEventSynchronize(h->slot_ev));
-  if (h->slot_host_n < n_rec) {
-    if (h->slot_host) { CUDA_OK(cudaFreeHost(h->slot_host)); h->slot_host = nullptr; h->slot_host_n = 0; }
-    CUDA_OK(cudaHostAlloc(reinterpret_cast<void**>(&h->slot_host), n_rec * sizeof(SlotArgs), cudaHostAllocDefault));
-    h->slot_host_n = n_rec;
+  h->slot_stride = static_cast<size_t>(s.B) * (sizeof(SlotArgs) + (ode ? sizeof(SlotOde) : 0));
+  const size_t bytes = n_win * h->slot_stride;
+  if (h->slot_host_bytes < bytes) {
+    if (h->slot_host) { CUDA_OK(cudaFreeHost(h->slot_host)); h->slot_host = nullptr; h->slot_host_bytes = 0; }
+    CUDA_OK(cudaHostAlloc(reinterpret_cast<void**>(&h->slot_host), bytes, cudaHostAllocDefault));
+    h->slot_host_bytes = bytes;
   }
-  SlotArgs* rec = h->slot_host;
-  for (size_t r = 0; r < n_rec; ++r) {
-    SlotArgs& z = rec[r];
-    z.r_s = zero; z.wa = zero; z.we = zero; z.x0 = zero; z.r_d = nullptr; z.ctx = nullptr;
-    z.T_wa = 1; z.T_we = 1; z.T_out = 0; z.win_start = 0; z.out_start = 0; z.first_window = 1;
-    z.a_scale = z.r_scale = z.e_scale = 1.f; z.n_branches = s.nb;
+  for (size_t w = 0; w < n_win; ++w) {
+    SlotArgs* rec = reinterpret_cast<SlotArgs*>(h->slot_host + w * h->slot_stride);
+    for (int k = 0; k < s.B; ++k) {
+      SlotArgs& z = rec[k];
+      z.r_s = zero; z.wa = zero; z.we = zero; z.x0 = zero; z.r_d = nullptr; z.ctx = nullptr;
+      z.T_wa = 1; z.T_we = 1; z.T_out = 0; z.win_start = 0; z.out_start = 0; z.first_window = 1;
+      z.a_scale = z.r_scale = z.e_scale = 1.f; z.n_branches = s.nb;
+    }
+    if (!ode) continue;
+    SlotOde* od = reinterpret_cast<SlotOde*>(rec + s.B);
+    for (int k = 0; k < s.B; ++k) {
+      SlotOde& o = od[k];
+      o = SlotOde{};
+      o.temb = static_cast<const float*>(h->temb.p); o.dt = static_cast<const float*>(h->ddt.p); o.n_eval = 0; o.n_stages = 1;
+    }
   }
-  *out = rec;
   return 0;
 }
 
-static int upload_slot_records(FmtHandle* h, size_t n_rec, cudaStream_t st) {
-  FMT_OK(dev_alloc(h, h->slot_buf, n_rec * sizeof(SlotArgs)));
-  CUDA_OK(cudaMemcpyAsync(h->slot_buf.p, h->slot_host, n_rec * sizeof(SlotArgs), cudaMemcpyHostToDevice, st));
+// window w's SlotArgs / SlotOde in the staging buffer, and its SlotArgs on the device after upload_slot_records
+static SlotArgs* staged_args(FmtHandle* h, size_t w) { return reinterpret_cast<SlotArgs*>(h->slot_host + w * h->slot_stride); }
+static SlotOde* staged_ode(FmtHandle* h, size_t w) { return reinterpret_cast<SlotOde*>(staged_args(h, w) + h->shape.B); }
+static const SlotArgs* device_args(const FmtHandle* h, size_t w) {
+  return reinterpret_cast<const SlotArgs*>(static_cast<const unsigned char*>(h->slot_buf.p) + w * h->slot_stride);
+}
+
+static int upload_slot_records(FmtHandle* h, size_t n_win, cudaStream_t st) {
+  const size_t bytes = n_win * h->slot_stride;
+  FMT_OK(dev_alloc(h, h->slot_buf, bytes));
+  CUDA_OK(cudaMemcpyAsync(h->slot_buf.p, h->slot_host, bytes, cudaMemcpyHostToDevice, st));
   if (!h->slot_ev) CUDA_OK(cudaEventCreateWithFlags(&h->slot_ev, cudaEventDisableTiming));
   CUDA_OK(cudaEventRecord(h->slot_ev, st));
   return 0;
+}
+
+// ---- per-slot ODE schedules
+// Checks the schedule of every one of n clips / streams against the plan: at most the plan's evaluations, 1..FMT_MAX_STAGES stages.
+static int check_odes(const FmtHandle* h, const FmtClipOde* ode, int n, const char* who) {
+  REQUIRE(ode->n_steps && ode->n_stages && ode->t_eval && ode->dt && ode->rk_a && ode->rk_b, "%s: null ODE array", who);
+  for (int i = 0; i < n; ++i) {
+    const int S = ode->n_steps[i], G = ode->n_stages[i];
+    REQUIRE(G >= 1 && G <= FMT_MAX_STAGES && S >= 0, "%s: %d: n_steps=%d, n_stages=%d (1..%d)", who, i, S, G, FMT_MAX_STAGES);
+    REQUIRE(static_cast<long long>(S) * G <= h->n_eval, "%s: %d needs %lld evaluations per window, the plan runs %d", who, i,
+            static_cast<long long>(S) * G, h->n_eval);
+    REQUIRE(ode->rk_a[i] && ode->rk_b[i] && (S == 0 || (ode->t_eval[i] && ode->dt[i])), "%s: %d: null schedule array", who, i);
+  }
+  return 0;
+}
+
+// Slot record of schedule i, with its t-embeddings and step sizes on the device: the plan's own when the schedule is the plan's,
+// else computed once per distinct schedule (timestep_freq_kernel and the two small_linear_kernel launches of fmt_configure, so the
+// same t gives the same bits) and kept in the handle.  A schedule without evaluations points at the plan's.
+static int slot_ode(FmtHandle* h, const FmtClipOde* ode, int i, cudaStream_t st, SlotOde* out) {
+  const int S = ode->n_steps[i], G = ode->n_stages[i], ne = S * G, H = h->shape.H;
+  SlotOde o{};
+  o.n_eval = ne; o.n_stages = G;
+  for (int g = 0; g < G; ++g) {
+    for (int j = 0; j < G; ++j) o.rk_a[g * 4 + j] = ode->rk_a[i][g * G + j];
+    o.rk_b[g] = ode->rk_b[i][g];
+  }
+  o.temb = static_cast<const float*>(h->temb.p); o.dt = static_cast<const float*>(h->ddt.p);
+  const bool plan = S == h->plan.n_steps && G == h->plan.n_stages && (ne == 0 || (memcmp(ode->t_eval[i], h->t_eval.data(), ne * sizeof(float)) == 0 &&
+                    memcmp(ode->dt[i], h->dt.data(), S * sizeof(float)) == 0));
+  if (ne > 0 && !plan) {
+    std::vector<float> key(ode->t_eval[i], ode->t_eval[i] + ne);
+    key.insert(key.end(), ode->dt[i], ode->dt[i] + S);
+    key.push_back(static_cast<float>(S));
+    auto it = h->ode_cache.find(key);
+    if (it == h->ode_cache.end()) {
+      DevBuf buf;
+      FMT_OK(dev_alloc(h, buf, (static_cast<size_t>(ne) * H + S) * sizeof(float)));
+      it = h->ode_cache.emplace(key, buf).first;
+      float* temb = static_cast<float*>(buf.p);
+      // dteval / tfreq / th hold the plan's evaluations (>= ne) and are only read while t-embeddings are computed
+      CUDA_OK(cudaMemcpyAsync(h->dteval.p, ode->t_eval[i], ne * sizeof(float), cudaMemcpyHostToDevice, st));
+      CUDA_OK(cudaMemcpyAsync(temb + static_cast<size_t>(ne) * H, ode->dt[i], S * sizeof(float), cudaMemcpyHostToDevice, st));
+      timestep_freq_kernel<<<ne, 128, 0, st>>>(static_cast<const float*>(h->dteval.p), ne, static_cast<float*>(h->tfreq.p));
+      LAUNCH_CHECK(); count_launch(h);
+      const int w1 = ne * H;
+      small_linear_kernel<<<(w1 * 32 + 255) / 256, 256, 0, st>>>(static_cast<const float*>(h->tfreq.p), h->t0_w, h->t0_b, static_cast<float*>(h->th.p), ne, H, 256, 1);
+      LAUNCH_CHECK(); count_launch(h);
+      small_linear_kernel<<<(w1 * 32 + 255) / 256, 256, 0, st>>>(static_cast<const float*>(h->th.p), h->t2_w, h->t2_b, temb, ne, H, H, 0);
+      LAUNCH_CHECK(); count_launch(h);
+      CUDA_OK(cudaStreamSynchronize(st));   // the caller's host arrays may go away after the call
+    }
+    o.temb = static_cast<const float*>(it->second.p);
+    o.dt = o.temb + static_cast<size_t>(ne) * H;
+  }
+  *out = o;
+  return 0;
+}
+
+// The per-slot window graph of the current plan, captured on first use: its distinct condition rows (the plan's deduplication with
+// no row shared between slots), their buffers, and a kbuf of FMT_MAX_STAGES stages.  The AdaLN tables go to the plan's table buffer,
+// as many evaluations at a time as it holds.
+static int ensure_ode_graph(FmtHandle* h, cudaStream_t st) {
+  if (h->ode_exec) return 0;
+  const ModelShape& s = h->shape;
+  h->sU = h->R;
+  h->s_dedup = false;
+  if (h->use_dedup && s.nb > 1) {
+    std::vector<int> urow, uidx;
+    distinct_condition_rows(s, urow, uidx, true);
+    if (static_cast<int>(uidx.size()) < h->R) {
+      h->sU = static_cast<int>(uidx.size());
+      h->s_dedup = true;
+      FMT_OK(dev_alloc(h, h->s_urow, urow.size() * sizeof(int)));
+      FMT_OK(dev_alloc(h, h->s_uidx, uidx.size() * sizeof(int)));
+      CUDA_OK(cudaMemcpyAsync(h->s_urow.p, urow.data(), urow.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+      CUDA_OK(cudaMemcpyAsync(h->s_uidx.p, uidx.data(), uidx.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+      CUDA_OK(cudaStreamSynchronize(st));      // `urow` / `uidx` are stack objects
+    }
+  }
+  const size_t U = h->sU, ts = h->tsize, nx = static_cast<size_t>(s.B) * s.L * s.W;
+  const size_t by_table = h->table.bytes / (U * h->NT * ts), by_silu = h->silu.bytes / (U * s.H * ts);
+  const size_t chunk = h->n_eval == 0 ? 1 : std::min<size_t>(std::min(by_table, by_silu), h->n_eval);
+  REQUIRE(chunk >= 1, "per-slot schedules: the AdaLN table buffer holds no evaluation of %zu condition rows", U);   // fmt_configure keeps room
+  h->s_chunk = static_cast<int>(chunk);
+  FMT_OK(dev_alloc(h, h->s_cond, U * s.Kc * ts));
+  FMT_OK(dev_alloc(h, h->s_cemb, U * s.H * 4));
+  FMT_OK(dev_alloc(h, h->s_kbuf, nx * 4 * FMT_MAX_STAGES));
+  return capture_window(h, enqueue_window_ode_mode, &h->ode_exec, &h->ode_nodes, &h->ode_launches);
 }
 
 int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
@@ -1456,6 +1664,7 @@ int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
     r_s = static_cast<float*>(h->st_rs.p); wa = static_cast<float*>(h->st_wa.p); we = static_cast<float*>(h->st_we.p);
     noise = static_cast<float*>(h->st_noise.p); r_d = static_cast<float*>(h->st_rd.p);
   }
+  h->last_ode = false;
   for (int w = 0; w < n_win; ++w) {
     WindowArgs a{};
     a.r_s = r_s; a.wa = wa; a.we = we; a.r_d = r_d;
@@ -1477,10 +1686,13 @@ int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
   return 0;
 }
 
+}  // extern "C"
+
 // Many clips on plan.batch slots: window w of the call runs, in slot k, whichever clip the schedule put there (at that clip's own
 // window), through the same captured window graph.  cond_gather / init_window / finalize_window read the per-slot tensors and
 // lengths, the CFG combines (cfg_combine_kernel and the COMB stages of the persistent kernels) the per-slot guidance.
-int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, void* stream) {
+// ode != nullptr: each clip on its own schedule, through the per-slot window graph.
+static int sample_clips(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, const FmtClipOde* ode, void* stream) {
   REQUIRE(h && cs && g, "fmt_sample_clips_guided: null argument");
   REQUIRE(h->configured, "fmt_sample_clips: call fmt_configure first");
   const int n = cs->n_clips;
@@ -1505,16 +1717,19 @@ int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* cs, const FmtCli
     REQUIRE(!s.we_dynamic || (n_win[i] - 1) * s.L < T_we, "fmt_sample_clips: clip %d: dynamic we has %d frames but the last window starts at %d",
             i, T_we, (n_win[i] - 1) * s.L);
   }
+  if (ode) FMT_OK(check_odes(h, ode, n, "fmt_sample_clips_ode: clip"));
   int makespan = 0;
   const int S = clip_schedule(n, n_win.data(), 0, slot.data(), start.data(), &makespan);
   REQUIRE(s.B == S, "fmt_sample_clips: the plan has batch %d, but these %d clips are scheduled on %d slots (fmt_clip_schedule)", s.B, n, S);
 
-  SlotArgs* rec = nullptr;
-  const size_t n_rec = static_cast<size_t>(makespan) * S;
-  FMT_OK(stage_slot_records(h, n_rec, st, &rec));
+  std::vector<SlotOde> od(ode ? n : 0);
+  for (int i = 0; i < static_cast<int>(od.size()); ++i) FMT_OK(slot_ode(h, ode, i, st, &od[i]));
+  if (ode) FMT_OK(ensure_ode_graph(h, st));
+  FMT_OK(stage_slot_records(h, makespan, ode != nullptr, st));
   for (int i = 0; i < n; ++i) {
     for (int w = 0; w < n_win[i]; ++w) {
-      SlotArgs& z = rec[static_cast<size_t>(start[i] + w) * S + slot[i]];
+      if (ode) staged_ode(h, start[i] + w)[slot[i]] = od[i];
+      SlotArgs& z = staged_args(h, start[i] + w)[slot[i]];
       z.r_s = cs->r_s[i]; z.wa = cs->wa[i]; z.we = cs->we[i]; z.r_d = cs->r_d[i];
       z.x0 = cs->noise[i] + static_cast<size_t>(w) * s.L * s.W;
       z.T_wa = cs->T_wa[i]; z.T_we = cs->T_we[i]; z.T_out = cs->audio_num_frames[i];
@@ -1522,17 +1737,27 @@ int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* cs, const FmtCli
       z.a_scale = g->a_cfg_scale[i]; z.r_scale = g->r_cfg_scale[i]; z.e_scale = g->e_cfg_scale[i]; z.n_branches = g->n_branches[i];
     }
   }
-  FMT_OK(upload_slot_records(h, n_rec, st));
-  const SlotArgs* base = static_cast<const SlotArgs*>(h->slot_buf.p);
+  FMT_OK(upload_slot_records(h, makespan, st));
+  h->last_ode = ode != nullptr;
   for (int w = 0; w < makespan; ++w) {
     WindowArgs a{};
-    a.slots = base + static_cast<size_t>(w) * S;
+    a.slots = device_args(h, w);
     FMT_OK(set_wargs(h, a, st));
-    CUDA_OK(cudaGraphLaunch(h->graph_exec, st));
-    h->launches += h->capture_launches;
+    CUDA_OK(cudaGraphLaunch(ode ? h->ode_exec : h->graph_exec, st));
+    h->launches += ode ? h->ode_launches : h->capture_launches;
     if (cs->progress) cs->progress(w, makespan, cs->progress_user);
   }
   return 0;
+}
+
+extern "C" {
+
+int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, void* stream) {
+  return sample_clips(h, cs, g, nullptr, stream);
+}
+
+int32_t fmt_sample_clips_ode(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, const FmtClipOde* ode, void* stream) {
+  return sample_clips(h, cs, g, ode, stream);
 }
 
 // The set's shared scales and the plan's branch count for every clip
@@ -1545,11 +1770,14 @@ int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) {
   return fmt_sample_clips_guided(h, cs, &g, stream);
 }
 
-// One window of each of n streams, stream i in slot i, through the plan's captured window graph; slots n.. are idle.  A stream's
-// context lives in its own ctx buffer, not in the handle, so a stream may run in any slot and the plan may be replaced between calls.
-// Its wa / we start at the window's first context frame (P frames before its first current frame), or at its first current frame in
-// a first window; its output is the window alone.
-int32_t fmt_sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, void* stream) {
+}  // extern "C"
+
+// One window of each of n streams, stream i in slot i, through the plan's captured window graph (ode != nullptr: each stream on its
+// own schedule, through the per-slot window graph); slots n.. are idle.  A stream's context lives in its own ctx buffer, not in the
+// handle, so a stream may run in any slot and the plan may be replaced between calls.  Its wa / we start at the window's first
+// context frame (P frames before its first current frame), or at its first current frame in a first window; its output is the
+// window alone.
+static int sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, const FmtClipOde* ode, void* stream) {
   REQUIRE(h && ws && g, "fmt_sample_windows: null argument");
   REQUIRE(h->configured, "fmt_sample_windows: call fmt_configure first");
   const ModelShape& s = h->shape;
@@ -1575,35 +1803,52 @@ int32_t fmt_sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGu
     REQUIRE(!s.we_dynamic || cur < T_we, "fmt_sample_windows: stream %d: dynamic we has %d frames but the window's first current frame is frame %d",
             i, T_we, cur);
   }
-  SlotArgs* rec = nullptr;
-  FMT_OK(stage_slot_records(h, s.B, st, &rec));
+  if (ode) FMT_OK(check_odes(h, ode, n, "fmt_sample_windows_ode: stream"));
+  std::vector<SlotOde> od(ode ? n : 0);
+  for (int i = 0; i < static_cast<int>(od.size()); ++i) FMT_OK(slot_ode(h, ode, i, st, &od[i]));
+  if (ode) FMT_OK(ensure_ode_graph(h, st));
+  FMT_OK(stage_slot_records(h, 1, ode != nullptr, st));
   for (int i = 0; i < n; ++i) {
-    SlotArgs& z = rec[i];
+    if (ode) staged_ode(h, 0)[i] = od[i];
+    SlotArgs& z = staged_args(h, 0)[i];
     z.r_s = ws->r_s[i]; z.wa = ws->wa[i]; z.we = ws->we[i]; z.x0 = ws->x0[i]; z.r_d = ws->r_d[i]; z.ctx = ws->ctx[i];
     z.T_wa = ws->T_wa[i]; z.T_we = ws->T_we[i]; z.T_out = ws->n_out[i];
     z.first_window = ws->first_window[i];
     z.win_start = z.first_window ? 0 : s.P; z.out_start = 0;
     z.a_scale = g->a_cfg_scale[i]; z.r_scale = g->r_cfg_scale[i]; z.e_scale = g->e_cfg_scale[i]; z.n_branches = g->n_branches[i];
   }
-  FMT_OK(upload_slot_records(h, s.B, st));
+  FMT_OK(upload_slot_records(h, 1, st));
+  h->last_ode = ode != nullptr;
   WindowArgs a{};
-  a.slots = static_cast<const SlotArgs*>(h->slot_buf.p);
+  a.slots = device_args(h, 0);
   FMT_OK(set_wargs(h, a, st));
-  CUDA_OK(cudaGraphLaunch(h->graph_exec, st));
-  h->launches += h->capture_launches;
+  CUDA_OK(cudaGraphLaunch(ode ? h->ode_exec : h->graph_exec, st));
+  h->launches += ode ? h->ode_launches : h->capture_launches;
   return 0;
 }
+
+extern "C" {
+
+int32_t fmt_sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, void* stream) {
+  return sample_windows(h, ws, g, nullptr, stream);
+}
+
+int32_t fmt_sample_windows_ode(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, const FmtClipOde* ode, void* stream) {
+  return sample_windows(h, ws, g, ode, stream);
+}
+
 
 }  // extern "C"
 
 template <typename T>
 static int enqueue_velocity(FmtHandle* h, const FmtEval* ev, cudaStream_t st) {
   const ModelShape& s = h->shape;
-  FMT_OK(enqueue_prepare<T>(h, st));
-  FMT_OK(enqueue_tables<T>(h, ev->eval_index, 1, st));
+  const CondRows r = plan_rows(h);
+  FMT_OK(enqueue_prepare<T>(h, r, st));
+  FMT_OK(enqueue_tables<T>(h, r, ev->eval_index, 1, st));
   FMT_OK(launch(h, pack_x_kernel<T>, dim3(s.B * s.N), dim3(128), 0, st, 1, static_cast<const WindowArgs*>(h->wargs.p), s, ev->x,
                 static_cast<const float*>(h->prevx.p), static_cast<T*>(h->ax.p)));
-  FMT_OK(enqueue_forward<T>(h, 0, st));
+  FMT_OK(enqueue_forward<T>(h, r, 0, st));
   FMT_OK(launch_combine<T>(h, 0, ev->v_out, nullptr, st));
   return 0;
 }

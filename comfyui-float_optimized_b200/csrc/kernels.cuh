@@ -28,6 +28,19 @@ struct SlotArgs {
                            // last P frames (fmt_sample_windows); nullptr: the context stays in the handle's per-slot state
 };
 
+// The ODE schedule one slot runs in one window of fmt_sample_clips_ode / fmt_sample_windows_ode (the per-slot window graph).  In the
+// slot-record buffer, the B SlotArgs of a window are followed by the B SlotOde of that window.  Plan evaluation e is the slot's step
+// e / n_stages, stage e % n_stages while e < n_eval; from n_eval on the slot is idle: its x stays as it is.
+struct SlotOde {
+  const float* temb;       // (max(n_eval, 1), H) t-embedding of each of its evaluations (an idle slot: any valid row)
+  const float* dt;         // (n_steps) step sizes
+  int n_eval;              // n_steps * n_stages <= the plan's evaluation count
+  int n_stages;            // 1..4
+  float rk_a[16];          // a[g][j] at [g * 4 + j], zero-padded
+  float rk_b[4];
+};
+__device__ __forceinline__ const SlotOde* slot_odes(const SlotArgs* slots, int B) { return reinterpret_cast<const SlotOde*>(slots + B); }
+
 // First plan branch of a clip that combines nb of the plan's s_nb CFG branches.  Branches 1..3 of a 4-branch plan are
 // [uncond | all | audio-only] with the null masks of a 3-branch plan (branch_nulls), so a 3-branch clip skips the truly-uncond
 // branch; a 1-branch clip reads the `all` branch alone, the single conditional forward of FMT.py:400-401.
@@ -151,6 +164,13 @@ __global__ void small_linear_kernel(const float* __restrict__ in, const float* _
   }
 }
 
+// SiLU(c + t) of four elements: the AdaLN input of one condition row at one evaluation
+__device__ __forceinline__ void silu_add4(const float4& c, const float4& t, float (&v)[4]) {
+  v[0] = c.x + t.x; v[1] = c.y + t.y; v[2] = c.z + t.z; v[3] = c.w + t.w;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) v[k] = v[k] / (1.f + expf(-v[k]));
+}
+
 // silu_c[(e*U + u), h] = SiLU(c_emb[u, h] + t_emb[e0 + e, h])      (FMT.py:335 then adaLN_modulation[0], :163-166)
 template <typename AT>
 __global__ void silu_cond_kernel(const float* __restrict__ c_emb, const float* __restrict__ t_emb, int e0, int U, int H,
@@ -164,9 +184,8 @@ __global__ void silu_cond_kernel(const float* __restrict__ c_emb, const float* _
   const int u = static_cast<int>(row % U), e = static_cast<int>(row / U);
   const float4 c = *reinterpret_cast<const float4*>(c_emb + static_cast<size_t>(u) * H + h);
   const float4 t = *reinterpret_cast<const float4*>(t_emb + static_cast<size_t>(e0 + e) * H + h);
-  float v[4] = {c.x + t.x, c.y + t.y, c.z + t.z, c.w + t.w};
-#pragma unroll
-  for (int k = 0; k < 4; ++k) v[k] = v[k] / (1.f + expf(-v[k]));
+  float v[4];
+  silu_add4(c, t, v);
   VecIO<AT, 4>::store(out + i, v);
 }
 
@@ -509,6 +528,17 @@ __device__ __forceinline__ void store_ax(const ModelShape& s, AT* __restrict__ a
   }
 }
 
+// The ODE updates of torchdiffeq's fixed-grid solvers, shared by the plan's kernels and the per-slot schedule kernels so that both
+// round alike: Euler y0 + dt * v, and the Runge-Kutta stage / final combination y0 + dt * sum_j c[j] * k_j over the first n_k stages
+__device__ __forceinline__ float euler_update(const float* dt, float v, const float* y0) { return fmaf(*dt, v, *y0); }
+__device__ __forceinline__ float rk_update(const float (&c)[4], const float* k, size_t k_stride, size_t i, int n_k,
+                                           const float* dt, const float* y0) {
+  float acc = 0.f;
+  for (int j = 0; j < n_k; ++j)
+    if (c[j] != 0.f) acc = fmaf(c[j], k[j * k_stride + i], acc);
+  return fmaf(*dt, acc, y0[i]);
+}
+
 // mode 0: v_full[b, f, :] = combined, all N frames (fmt_velocity)
 // mode 1: k_out[b, f-P, :] = combined, current frames only (RK stage derivative)
 // mode 2: y[b, f-P, :] += dt * combined   (fused CFG + Euler update, torchdiffeq euler: y1 = y0 + dt*f(t0,y0))
@@ -538,7 +568,7 @@ __global__ void cfg_combine_kernel(const WindowArgs* __restrict__ wargs, ModelSh
     const size_t o = (static_cast<size_t>(b) * s.L + (f - s.P)) * s.W + j;
     if (mode == 1) dst[o] = v;
     else {
-      const float y = fmaf(*dt_ptr, v, dst[o]);
+      const float y = euler_update(dt_ptr, v, dst + o);
       dst[o] = y;
       store_ax<AT>(s, ax, b, f, j, y);
     }
@@ -555,10 +585,7 @@ __global__ void rk_combine_kernel(ModelShape s, const float* __restrict__ y0, fl
   const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float c[4] = {c0, c1, c2, c3};
-  float acc = 0.f;
-  for (int j = 0; j < n_k; ++j)
-    if (c[j] != 0.f) acc = fmaf(c[j], k[j * k_stride + i], acc);
-  const float y = fmaf(*dt_ptr, acc, y0[i]);
+  const float y = rk_update(c, k, k_stride, i, n_k, dt_ptr, y0);
   y_out[i] = y;
   const int j = static_cast<int>(i % s.W), f = static_cast<int>((i / s.W) % s.L), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.L));
   store_ax<AT>(s, ax, b, s.P + f, j, y);
@@ -615,6 +642,87 @@ __global__ void finalize_window_kernel(const WindowArgs* __restrict__ wargs, Mod
     prev_x_state[(static_cast<size_t>(b) * s.P + c) * s.W + j] = v;
     if (ctx != nullptr) ctx[static_cast<size_t>(c) * s.W + j] = v;
   }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Per-slot ODE schedules (the per-slot window graph): every slot reads its own SlotOde; the arithmetic is the plan kernels'
+// ---------------------------------------------------------------------------------------------------------------
+// silu_c[(e*U + u), h] = SiLU(c_emb[u, h] + t_emb[h]) with the t-embedding of evaluation e0 + e of the schedule of the slot that
+// condition row u belongs to.  uidx: the token row of every distinct row (nullptr: row u); no distinct row spans two slots here.
+template <typename AT>
+__global__ void silu_cond_sched_kernel(const WindowArgs* __restrict__ wargs, ModelShape s, const float* __restrict__ c_emb,
+                                       const int* __restrict__ uidx, int e0, int U, AT* __restrict__ out, size_t total) {
+  pdl_launch_dependents();
+  pdl_wait_prior_grid();
+  const int H = s.H;
+  size_t i = (static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x) * 4;
+  if (i >= total) return;
+  const int h = static_cast<int>(i % H);
+  const size_t row = i / H;
+  const int u = static_cast<int>(row % U), e = e0 + static_cast<int>(row / U);
+  const int tok = uidx != nullptr ? uidx[u] : u;
+  const SlotOde& o = slot_odes(wargs->slots, s.B)[(tok / s.N) % s.B];
+  const float* t_emb = o.temb + (e < o.n_eval ? static_cast<size_t>(e) * H : 0);
+  const float4 c = *reinterpret_cast<const float4*>(c_emb + static_cast<size_t>(u) * H + h);
+  const float4 t = *reinterpret_cast<const float4*>(t_emb + h);
+  float v[4];
+  silu_add4(c, t, v);
+  VecIO<AT, 4>::store(out + i, v);
+}
+
+// Before plan evaluation e: y_g = y0 + dt * sum_j a[g][j] k_j for every slot that is at a stage g > 0 of its own schedule (also
+// refreshes ax); a slot at stage 0 already holds x in ax
+template <typename AT>
+__global__ void sched_stage_kernel(const WindowArgs* __restrict__ wargs, ModelShape s, const float* __restrict__ x_state,
+                                   float* __restrict__ y_stage, const float* __restrict__ k, size_t n, int e, AT* __restrict__ ax) {
+  pdl_launch_dependents();
+  pdl_wait_prior_grid();
+  const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int j = static_cast<int>(i % s.W), f = static_cast<int>((i / s.W) % s.L), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.L));
+  const SlotOde& o = slot_odes(wargs->slots, s.B)[b];
+  const int G = o.n_stages, g = e % G;
+  if (e >= o.n_eval || g == 0) return;
+  const float c[4] = {o.rk_a[g * 4], o.rk_a[g * 4 + 1], o.rk_a[g * 4 + 2], o.rk_a[g * 4 + 3]};
+  const float y = rk_update(c, k, n, i, g, o.dt + e / G, x_state);
+  y_stage[i] = y;
+  store_ax<AT>(s, ax, b, s.P + f, j, y);
+}
+
+// After plan evaluation e: every slot that is at an evaluation of its own schedule combines its CFG branches (as
+// cfg_combine_kernel does) and takes its Euler step (one-stage solvers), or stores k_g and, after its last stage, takes
+// x += dt * sum_j b[j] k_j (as rk_combine_kernel does).  k holds up to four stages of n elements each.
+template <typename AT>
+__global__ void sched_combine_kernel(const WindowArgs* __restrict__ wargs, ModelShape s, const float* __restrict__ V, int e,
+                                     float* __restrict__ x_state, float* k, size_t n, AT* __restrict__ ax) {
+  pdl_launch_dependents();
+  pdl_wait_prior_grid();
+  const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const size_t per_branch = static_cast<size_t>(s.B) * s.N * s.W;
+  if (i >= per_branch) return;
+  const int j = static_cast<int>(i % s.W);
+  const int f = static_cast<int>((i / s.W) % s.N), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.N));
+  if (f < s.P) return;
+  const SlotArgs* slots = wargs->slots;
+  const SlotOde& o = slot_odes(slots, s.B)[b];
+  if (e >= o.n_eval) return;
+  const SlotArgs& sl = slots[b];
+  const int nb = sl.n_branches;
+  const float v = cfg_combine(V, i + slot_branch0(s.nb, nb) * per_branch, per_branch, nb, sl.a_scale, sl.r_scale, sl.e_scale);
+  const size_t oi = (static_cast<size_t>(b) * s.L + (f - s.P)) * s.W + j;
+  const int G = o.n_stages, g = e % G;
+  const float* dt = o.dt + e / G;
+  float y;
+  if (G == 1) {
+    y = euler_update(dt, v, x_state + oi);
+  } else {
+    k[g * n + oi] = v;
+    if (g < G - 1) return;
+    const float c[4] = {o.rk_b[0], o.rk_b[1], o.rk_b[2], o.rk_b[3]};
+    y = rk_update(c, k, n, oi, G, dt, x_state);
+  }
+  x_state[oi] = y;
+  store_ax<AT>(s, ax, b, f, j, y);
 }
 
 // fp32 -> bf16 weight packing (with optional K padding)

@@ -105,6 +105,20 @@ def _build_schedule(nfe: int, method: str):
     return dict(n_steps=max(0, int(nfe) - 1), n_stages=stages, t_eval=t_eval, dt=[float(x) for x in dt], a=a_flat, b=tab["b"])
 
 
+def n_evals(nfe: int, method: str) -> int:
+    """Model evaluations per window of a fixed-grid solver: (nfe - 1) steps of one evaluation per stage."""
+    return max(0, int(nfe) - 1) * len(SOLVERS[method]["c"])
+
+
+def plan_schedule(schedules: Sequence[tuple], nfe: int, method: str) -> tuple:
+    """The (nfe, method) a call of clips with these schedules configures its plan with: a clip's schedule that needs the most
+    evaluations per window (:func:`n_evals`); on a tie the call's own (nfe, method) if some clip runs it, else the first in input
+    order.  So a call whose clips all run one schedule runs the plan's window graph."""
+    most = max(n_evals(*sc) for sc in schedules)
+    tied = [sc for sc in schedules if n_evals(*sc) == most]
+    return (int(nfe), method) if (int(nfe), method) in tied else tied[0]
+
+
 PRECISION_MODES = ("bf16", "fp32", "bf16x3")
 
 
@@ -210,6 +224,26 @@ class FmtBackend:
     def graph_kernel_nodes(self) -> int:
         return int(self.lib.fmt_graph_kernel_nodes(self._handle))
 
+    def ode_graph_kernel_nodes(self) -> int:
+        """Kernels of the per-slot window graph that calls with per-clip schedules run (0 before the first on this plan)."""
+        return int(self.lib.fmt_ode_graph_kernel_nodes(self._handle))
+
+    @staticmethod
+    def _clip_ode(schedules, n: int):
+        """FmtClipOde of n (nfe, method) pairs, and the ctypes arrays it points into (keep them alive for the call)."""
+        if len(schedules) != n:
+            raise ValueError(f"schedules needs one (nfe, method) per clip ({n}), got {len(schedules)}")
+        sched = []
+        for nfe, method in schedules:
+            if isinstance(nfe, bool) or not isinstance(nfe, numbers.Integral) or nfe < 1:
+                raise ValueError(f"nfe must be an int >= 1 (got {nfe!r})")
+            sched.append(build_schedule(nfe, method))
+        arrays = [[_f32_array(sc[k]) for sc in sched] for k in ("t_eval", "dt", "a", "b")]
+        fptr = C.POINTER(C.c_float)
+        ode = _cabi.FmtClipOde((C.c_int32 * n)(*[sc["n_steps"] for sc in sched]), (C.c_int32 * n)(*[sc["n_stages"] for sc in sched]),
+                               *[(fptr * n)(*[C.cast(x, fptr) for x in arr]) for arr in arrays])
+        return ode, arrays
+
     # ------------------------------------------------------------------------------------------------
     def _check_clip(self, r_s, wa, we, audio_num_frames, noise, host: bool):
         """Every tensor the C call indexes by the plan's dimensions is checked here (the reference would raise a torch shape
@@ -273,14 +307,17 @@ class FmtBackend:
 
     def sample_clips(self, r_s, wa, we, audio_num_frames, noise, a_cfg_scale, r_cfg_scale, e_cfg_scale,
                      progress: Optional[Callable[[int, int], None]] = None, out: Optional[Sequence[torch.Tensor]] = None,
-                     n_branches: Optional[Sequence[int]] = None) -> List[torch.Tensor]:
+                     n_branches: Optional[Sequence[int]] = None, schedules: Optional[Sequence[tuple]] = None) -> List[torch.Tensor]:
         """Many clips of different lengths in one call on the plan's batch of slots (:func:`clip_schedule`).  Per clip i: r_s[i]
         (1, dim_w), wa[i] (1, T_wa, dim_a), we[i] (1, 1 or T_we, dim_e), noise[i] (n_win_i, L, dim_w) or (n_win_i, 1, L, dim_w), all on
         ``self.device`` (fp32, contiguous).  Returns one (1, audio_num_frames[i], dim_w) tensor per clip (``out[i]`` if given: any
         contiguous fp32 tensor of that many elements); asynchronous.
 
         Each of the three scales is one float for every clip or a sequence of one float per clip.  ``n_branches[i]`` (1, 3 or 4, at
-        most the plan's; default: the plan's for every clip) is the branch count of clip i's guidance, :func:`n_branches_for`."""
+        most the plan's; default: the plan's for every clip) is the branch count of clip i's guidance, :func:`n_branches_for`.
+        ``schedules[i]`` = (nfe, method), at most the plan's evaluations per window (:func:`n_evals`), puts clip i on its own ODE
+        schedule; given, the call runs the per-slot window graph (``fmt_sample_clips_ode``), one kernel per op, even where every
+        schedule is the plan's."""
         d = self.dims
         if self._plan_key is None:
             raise FmtError("sample_clips: configure() has not been called")
@@ -338,16 +375,23 @@ class FmtBackend:
         cs = _cabi.FmtClipSet(n, ptrs(r_s), ptrs(wa), ptrs(we), ptrs(noise), ptrs(outs), ints(t.shape[1] for t in wa),
                               ints(t.shape[1] for t in we), ints(audio_num_frames), 1.0, 1.0, 1.0, cb, None)
         g = _cabi.FmtClipGuidance(floats(scales[0]), floats(scales[1]), floats(scales[2]), ints(nbr))
+        if schedules is not None:
+            ode, _keep = self._clip_ode(schedules, n)
+            with torch.cuda.device(self.device):
+                _cabi.check(self.lib.fmt_sample_clips_ode(self._handle, C.byref(cs), C.byref(g), C.byref(ode), self._stream()), "fmt_sample_clips_ode")
+            return outs
         with torch.cuda.device(self.device):
             _cabi.check(self.lib.fmt_sample_clips_guided(self._handle, C.byref(cs), C.byref(g), self._stream()), "fmt_sample_clips_guided")
         return outs
 
-    def sample_windows(self, r_s, wa, we, x0, ctx, out, first_window, a_cfg_scale, r_cfg_scale, e_cfg_scale, n_branches) -> None:
+    def sample_windows(self, r_s, wa, we, x0, ctx, out, first_window, a_cfg_scale, r_cfg_scale, e_cfg_scale, n_branches,
+                       schedules: Optional[Sequence[tuple]] = None) -> None:
         """One window of each of n <= plan batch streams (``fmt_sample_windows``), stream i in slot i.  Per stream i: r_s[i]
         (1, dim_w); wa[i] (T_wa, dim_a) and, dynamic, we[i] (T_we, dim_e) from the window's first context frame (frame 0 in a first
         window), static we[i] (1, 1, dim_e); x0[i] (L, dim_w); ctx[i] (P, dim_w), read unless ``first_window[i]`` and overwritten
         with the window's last P frames; out[i] receives the window's first ``out[i].shape[-2]`` frames.  Scales and n_branches are
-        one entry per stream.  All tensors on ``self.device`` (fp32, contiguous); asynchronous."""
+        one entry per stream; ``schedules`` (one (nfe, method) per stream) as in :meth:`sample_clips`.  All tensors on ``self.device``
+        (fp32, contiguous); asynchronous."""
         d = self.dims
         if self._plan_key is None:
             raise FmtError("sample_windows: configure() has not been called")
@@ -374,6 +418,12 @@ class FmtBackend:
                                 ints(t.numel() // d.dim_e for t in we), ints(t.numel() // d.dim_w for t in out), ints(first_window))
         g = _cabi.FmtClipGuidance(*[(C.c_float * n)(*[float(x) for x in v]) for v in (a_cfg_scale, r_cfg_scale, e_cfg_scale)],
                                   ints(n_branches))
+        if schedules is not None:
+            ode, _keep = self._clip_ode(schedules, n)
+            with torch.cuda.device(self.device):
+                _cabi.check(self.lib.fmt_sample_windows_ode(self._handle, C.byref(ws), C.byref(g), C.byref(ode), self._stream()),
+                            "fmt_sample_windows_ode")
+            return
         with torch.cuda.device(self.device):
             _cabi.check(self.lib.fmt_sample_windows(self._handle, C.byref(ws), C.byref(g), self._stream()), "fmt_sample_windows")
 
@@ -547,16 +597,31 @@ def _own_guidance(who: str, c: Mapping, a_cfg_scale, r_cfg_scale, e_cfg_scale, i
     return g + (n_branches_for(*g, c.get("include_r_cfg", include_r_cfg)),)
 
 
+def _own_schedule(who: str, c: Mapping, nfe, method) -> tuple:
+    """(nfe, method) of one clip or stream: each of its own keys overrides the call's keyword of that name."""
+    if "nfe" in c:
+        v = c["nfe"]
+        if isinstance(v, bool) or not isinstance(v, numbers.Integral):
+            raise TypeError(f"{who}: nfe must be an int, got {type(v).__name__}")
+        if v < 1:
+            raise ValueError(f"{who}: nfe must be >= 1 (got {v})")
+    if "method" in c and (not isinstance(c["method"], str) or c["method"] not in SOLVERS):
+        raise ValueError(f"{who}: unknown fixed-step solver {c['method']!r} (supported: {sorted(SOLVERS)})")
+    return int(c.get("nfe", nfe)), c.get("method", method)
+
+
 def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str = "euler", a_cfg_scale: float = 2.0,
                  r_cfg_scale: float = 1.0, e_cfg_scale: float = 1.0, include_r_cfg: bool = False, mode: Optional[str] = None,
                  device=None, progress: Optional[Callable[[int, int], None]] = None) -> List[torch.Tensor]:
     """Many independent clips of different lengths in one call.  Each clip is a mapping with ``r_s`` (1, dim_w), ``wa``
     (1, T_wa, dim_a), ``we`` (1, 1 or T_we, dim_e), optionally ``audio_num_frames`` (default T_wa) and either ``seed`` (its noise is
-    :func:`clip_noise`) or ``noise`` (n_win, L, dim_w).  A clip may also hold ``a_cfg_scale``, ``r_cfg_scale``, ``e_cfg_scale``
-    and ``include_r_cfg``: each overrides the keyword of the same name for that clip.  Solver, precision and static / dynamic
-    emotion are shared.  The plan runs as many CFG branches as the clip that needs the most (:func:`n_branches_for`); a clip
-    that needs fewer combines only its own branches.  Clip i's result is what :func:`perform_ode_sampling_loop` gives for it
-    alone with its settings and noise.  Returns one (1, T_i, dim_w) tensor per clip, in input order, on ``device`` (default: the
+    :func:`clip_noise`) or ``noise`` (n_win, L, dim_w).  A clip may also hold ``a_cfg_scale``, ``r_cfg_scale``, ``e_cfg_scale``,
+    ``include_r_cfg``, ``nfe`` and ``method``: each overrides the keyword of the same name for that clip.  Precision and static /
+    dynamic emotion are shared.  The plan runs as many CFG branches as the clip that needs the most (:func:`n_branches_for`); a clip
+    that needs fewer combines only its own branches.  Likewise it runs the evaluations per window of the clip that needs the most
+    (:func:`n_evals`, :func:`plan_schedule`); a clip that needs fewer runs its own and then idles, and a call whose clips do not all
+    run the plan's schedule goes through the per-slot window graph (one kernel per op).  Clip i's result is what
+    :func:`perform_ode_sampling_loop` gives for it alone with its settings and noise.  Returns one (1, T_i, dim_w) tensor per clip, in input order, on ``device`` (default: the
     model's ``target_device``).  ``progress(w, makespan)`` is called after each window of the schedule is enqueued."""
     # every check runs before the first device call (the weights are packed only once the clips are known to be valid)
     if not isinstance(clips, (list, tuple)):
@@ -569,7 +634,7 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
     if int(nfe) < 1:
         raise ValueError(f"nfe must be >= 1 (got {nfe})")
     mode = resolve_mode(mode)
-    T, n_win, dyn, guidance = [], [], [], []      # guidance: (a, r, e, n_branches) of every clip
+    T, n_win, dyn, guidance, schedules = [], [], [], [], []      # guidance: (a, r, e, n_branches) of every clip
     for i, c in enumerate(clips):
         if not isinstance(c, Mapping):
             raise TypeError(f"clip {i} must be a mapping (r_s, wa, we, seed or noise), got {type(c).__name__}")
@@ -605,6 +670,7 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
             if tuple(nz.shape) not in ((nw, L, d.dim_w), (nw, 1, L, d.dim_w)):
                 raise ValueError(f"clip {i}: noise shape {tuple(nz.shape)} != {(nw, L, d.dim_w)}")
         guidance.append(_own_guidance(f"clip {i}", c, a_cfg_scale, r_cfg_scale, e_cfg_scale, include_r_cfg))
+        schedules.append(_own_schedule(f"clip {i}", c, nfe, method))
         T.append(t)
         n_win.append(nw)
         dyn.append(dynamic)
@@ -616,25 +682,29 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
     be = backend_for(fmt_model, device, d)
     sched = clip_schedule(n_win)
     a, r, e, nb = zip(*guidance)
-    be.configure(sched.slots, max(nb), dyn[0], nfe, method, mode)
+    plan = plan_schedule(schedules, nfe, method)
+    be.configure(sched.slots, max(nb), dyn[0], *plan, mode)
     dev = be.device
     noise = [_as_f32(c["noise"], dev) if c.get("noise") is not None else clip_noise(c["seed"], d, nw, dev)
              for c, nw in zip(clips, n_win)]
+    # the plan's schedule for every clip: the plan's window graph, as without per-clip schedules
+    own = {} if all(sc == plan for sc in schedules) else dict(schedules=schedules)
     return be.sample_clips([_as_f32(c["r_s"], dev) for c in clips], [_as_f32(c["wa"], dev) for c in clips],
-                           [_as_f32(c["we"], dev) for c in clips], T, noise, a, r, e, progress, n_branches=nb)
+                           [_as_f32(c["we"], dev) for c in clips], T, noise, a, r, e, progress, n_branches=nb, **own)
 
 
 # ----------------------------------------------------------------------------------------------------
 # streams: clips fed audio in pieces, one window per step on a fixed set of batch slots
 # ----------------------------------------------------------------------------------------------------
 _GUIDANCE_KEYS = ("a_cfg_scale", "r_cfg_scale", "e_cfg_scale", "include_r_cfg")
+_SCHEDULE_KEYS = ("nfe", "method")
 
 
 class Stream:
     """One clip of a :class:`StreamSampler`, opened by :meth:`StreamSampler.open`.  ``fed`` frames have arrived, ``windows_run``
     windows have been sampled; ``finished`` once :meth:`StreamSampler.finish` was called, ``done`` once its last window ran."""
 
-    def __init__(self, index, L, r_s, we, ctx, wa, we_buf, gen, noise, guidance):
+    def __init__(self, index, L, r_s, we, ctx, wa, we_buf, gen, noise, guidance, schedule):
         self.index = index                  # open order: breaks ties between windows that became ready at the same tick
         self.L = L
         self.r_s, self.we, self.ctx = r_s, we, ctx
@@ -645,6 +715,7 @@ class Stream:
         self.finished = False
         self.ready_at = None                # sampler clock when the next window became ready; None while it is not
         self.gen, self.noise, self.guidance = gen, noise, guidance
+        self.schedule = schedule            # (nfe, method)
 
     @property
     def done(self) -> bool:
@@ -667,7 +738,9 @@ class StreamSampler:
 
     The plan (slot count, nfe, solver, precision, static or dynamic emotion, and the branch count of the keyword guidance) is fixed
     at construction, so steps replay one captured window graph.  A stream may override the four guidance keywords in :meth:`open`
-    as a clip of :func:`sample_clips` does, within the plan's branch count.  A stream holds on the device its reference latent,
+    as a clip of :func:`sample_clips` does, within the plan's branch count, and ``nfe`` and ``method`` within the plan's
+    evaluations per window (:func:`n_evals` of the constructor's nfe and method); a step that runs a stream on a schedule other
+    than the plan's goes through the per-slot window graph (one kernel per op).  A stream holds on the device its reference latent,
     its last P motion frames and the audio frames from its next window's first context frame on, however long it runs."""
 
     def __init__(self, fmt_model, *, slots: int, nfe: int, method: str = "euler", mode: Optional[str] = None, a_cfg_scale: float = 2.0,
@@ -687,6 +760,7 @@ class StreamSampler:
         if device is None:
             device = getattr(fmt_model, "target_device", None) or "cuda"
         self.slots, self.nfe, self.method, self.we_dynamic = int(slots), int(nfe), method, we_dynamic
+        self.capacity = n_evals(nfe, method)               # evaluations per window a stream may need
         self._be = backend_for(fmt_model, device, self.dims)
         self.device = self._be.device
         self._configure()
@@ -714,9 +788,9 @@ class StreamSampler:
         """A new stream with reference latent ``r_s`` (1, dim_w) and, for static emotion, ``we`` (1, 1, dim_e) (dynamic emotion
         arrives with :meth:`feed`).  Its noise is :func:`clip_noise` of ``seed``, drawn one window at a time, or ``noise``
         (n_win, L, dim_w) for a clip of exactly n_win windows.  ``guidance`` may hold ``a_cfg_scale``, ``r_cfg_scale``,
-        ``e_cfg_scale`` and ``include_r_cfg``, each overriding the sampler's keyword for this stream."""
+        ``e_cfg_scale``, ``include_r_cfg``, ``nfe`` and ``method``, each overriding the sampler's keyword for this stream."""
         d, L = self.dims, self.dims.frames_per_clip
-        unknown = sorted(set(guidance) - set(_GUIDANCE_KEYS))
+        unknown = sorted(set(guidance) - set(_GUIDANCE_KEYS) - set(_SCHEDULE_KEYS))
         if unknown:
             raise TypeError(f"open: unexpected keyword(s) {unknown}")
         self._check_tensor("open", "r_s", r_s, (1, d.dim_w))
@@ -737,12 +811,16 @@ class StreamSampler:
         if g[3] > self.n_branches:
             raise ValueError(f"open: this stream's guidance needs {g[3]} CFG branches, the sampler's plan runs {self.n_branches} "
                              "(construct it with the guidance of the stream that needs the most)")
+        sc = _own_schedule("open", guidance, self.nfe, self.method)
+        if n_evals(*sc) > self.capacity:
+            raise ValueError(f"open: nfe={sc[0]} with {sc[1]} needs {n_evals(*sc)} evaluations per window, the sampler's plan runs "
+                             f"{self.capacity} (construct it with the nfe and method of the stream that needs the most)")
         dev = self.device
         gen = torch.Generator(dev).manual_seed(int(seed)) if seed is not None else None
         st = Stream(self._opened, L, _as_f32(r_s, dev).clone(), None if we is None else _as_f32(we, dev).clone(),
                     torch.zeros(d.num_prev_frames, d.dim_w, device=dev), torch.empty(0, d.dim_a, device=dev),
                     torch.empty(0, d.dim_e, device=dev) if self.we_dynamic else None, gen,
-                    None if noise is None else noise.reshape(noise.shape[0], L, d.dim_w), g)
+                    None if noise is None else noise.reshape(noise.shape[0], L, d.dim_w), g, sc)
         self._opened += 1
         self._streams.append(st)
         return st
@@ -819,9 +897,11 @@ class StreamSampler:
             x0.append(torch.randn(1, L, d.dim_w, device=dev, generator=st.gen) if st.gen is not None
                       else st.noise[w].to(device=dev, dtype=torch.float32).contiguous())
             outs.append(torch.empty(1, min(L, st.fed - w * L), d.dim_w, device=dev))
+        schedules = [st.schedule for st in run]
+        own = {} if all(sc == (self.nfe, self.method) for sc in schedules) else dict(schedules=schedules)
         self._be.sample_windows([st.r_s for st in run], [st.wa for st in run],
                                 [st.we_buf if self.we_dynamic else st.we for st in run], x0, [st.ctx for st in run], outs,
-                                [int(st.windows_run == 0) for st in run], *zip(*[st.guidance for st in run]))
+                                [int(st.windows_run == 0) for st in run], *zip(*[st.guidance for st in run]), **own)
         self._clock += 1
         for st in run:
             st.windows_run += 1

@@ -170,6 +170,19 @@ typedef struct FmtWindowSet {
   const int32_t* first_window;      /* 1: the stream's window 0: zero context                                                   */
 } FmtWindowSet;
 
+/* The ODE schedule of every clip of a FmtClipSet or stream of a FmtWindowSet (fmt_sample_clips_ode, fmt_sample_windows_ode): host
+ * arrays of n_clips / n_streams entries, each entry laid out as the FmtPlan fields of the same names (HOST arrays).  Clip i runs
+ * n_steps[i] * n_stages[i] evaluations per window, at most the plan's n_steps * n_stages, with 1..FMT_MAX_STAGES stages; its result
+ * is what a plan with its own schedule gives for it.  n_steps[i] = 0 (nfe 1) returns the noise. */
+typedef struct FmtClipOde {
+  const int32_t* n_steps;
+  const int32_t* n_stages;
+  const float* const* t_eval;       /* [i]: (n_steps[i] * n_stages[i]) times of its evaluations                                  */
+  const float* const* dt;           /* [i]: (n_steps[i])                                                                          */
+  const float* const* rk_a;         /* [i]: (n_stages[i] * n_stages[i])                                                           */
+  const float* const* rk_b;         /* [i]: (n_stages[i])                                                                         */
+} FmtClipOde;
+
 /* One evaluation of forward_with_cfv (FMT.py:342-401) on explicit window inputs - tests and ncu. */
 typedef struct FmtEval {
   const float* x;         /* (B, L, dim_w)                     */
@@ -226,6 +239,16 @@ FMT_API int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* set, con
  * clip.  Returns -1 on bad arguments. */
 FMT_API int32_t fmt_sample_windows(FmtHandle* h, const FmtWindowSet* set, const FmtClipGuidance* guidance, void* stream);
 
+/* fmt_sample_clips_guided / fmt_sample_windows with each clip / stream on its own ODE schedule (ode == NULL: exactly the call without
+ * it).  They run a second window graph of the plan, captured on first use: every evaluation of the plan, in which a slot whose clip
+ * needs fewer runs its own ones first and then stays idle (its x is kept, its rows are computed and dropped), with one kernel per op
+ * at any row count (plans of <= 256 token rows too, which the plan's graph runs in the persistent window kernel).  The t-embeddings
+ * of each distinct schedule are computed the first time it is seen and kept in the handle.  Return -1 if a clip needs more
+ * evaluations than the plan or more than FMT_MAX_STAGES stages, or on the checks of the calls without ode. */
+FMT_API int32_t fmt_sample_clips_ode(FmtHandle* h, const FmtClipSet* set, const FmtClipGuidance* guidance, const FmtClipOde* ode, void* stream);
+FMT_API int32_t fmt_sample_windows_ode(FmtHandle* h, const FmtWindowSet* set, const FmtClipGuidance* guidance, const FmtClipOde* ode,
+                                       void* stream);
+
 /* Single CFG-combined model evaluation (device pointers). */
 FMT_API int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream);
 
@@ -233,9 +256,12 @@ FMT_API int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream);
 FMT_API int64_t fmt_launch_count(const FmtHandle* h, int32_t reset);
 /* Number of kernel nodes in the captured window graph (0 before fmt_configure). */
 FMT_API int32_t fmt_graph_kernel_nodes(const FmtHandle* h);
+/* The same for the per-slot window graph of fmt_sample_clips_ode / fmt_sample_windows_ode (0 before its first call on this plan). */
+FMT_API int32_t fmt_ode_graph_kernel_nodes(const FmtHandle* h);
 
-/* Persistent window kernel (plans with <= 256 token rows, bf16): -1 = not in use for the current plan, 0 = in use and
- * healthy, > 0 = id of the bounded spin that tripped (the kernel traps instead of hanging the GPU). */
+/* Persistent window kernel (plans with <= 256 token rows, bf16): > 0 = id of the bounded spin that tripped (the kernel traps instead
+ * of hanging the GPU), whatever ran since; else -1 = not in use for the current plan, or the last sampling call ran the per-slot
+ * window graph (one kernel per op); 0 = in use and healthy. */
 FMT_API int32_t fmt_window_kernel_status(const FmtHandle* h);
 
 /* With FMT_WIN_TRACE=1 in the environment at fmt_configure: copies the per-CTA barrier stamps of the last window,
@@ -247,6 +273,10 @@ FMT_API int64_t fmt_debug_window_trace(const FmtHandle* h, int64_t* out, int64_t
  * arguments. */
 FMT_API int32_t fmt_debug_condition_rows(int32_t n_branches, int32_t batch, int32_t n_frames, int32_t n_prev, int32_t we_dynamic,
                                          int32_t* urow_out);
+/* The same with per_slot = 1 for the per-slot window graph, whose distinct rows never span two slots (batch - 1 more rows in 4-branch
+ * plans: the truly-unconditional current frames are one row per slot). */
+FMT_API int32_t fmt_debug_condition_rows_ode(int32_t n_branches, int32_t batch, int32_t n_frames, int32_t n_prev, int32_t we_dynamic,
+                                             int32_t per_slot, int32_t* urow_out);
 
 /* ---- audio projection in front of the sampler (SURVEY.md 8f rank 2) ----
  * Replaces the nn.Sequential(Linear(in_dim, dim_w), LayerNorm(dim_w), SiLU) that FloatApplyAudioProjection runs
