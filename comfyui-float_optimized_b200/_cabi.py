@@ -87,6 +87,18 @@ class FmtDebugGemm(C.Structure):
                [("ldg", C.c_int64), ("gate_off", C.c_int64)]
 
 
+FMT_STAGE_ROW, FMT_STAGE_ATTN, FMT_STAGE_GELU, FMT_STAGE_COMB = 0, 1, 2, 3
+
+
+class FmtDebugStage(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("kind", "grid", "chunk_rows", "n_branches", "batch", "n_frames", "n_prev", "H", "heads", "window",
+                                          "mlp_hidden", "W", "row_mode", "zero_qkv", "parity", "n_stages", "stage", "step")] + \
+               [(n, C.c_int64) for n in ("ldt", "gate_off", "shift_off", "scale_off")] + \
+               [(n, C.c_float) for n in ("a_scale", "r_scale", "e_scale")] + [("rk_a", C.c_float * 16), ("rk_b", C.c_float * 4)] + \
+               [(n, C.c_void_p) for n in ("X", "Pacc", "QKVacc", "Hacc", "Vacc", "A1", "A2", "Hm", "ax", "table", "urow", "bias", "pos",
+                                          "x_state", "kbuf", "ddt", "slot_branches", "slot_scales")]
+
+
 _SIGNATURES = {
     "fmt_abi_version": (C.c_int32, []),
     "fmt_last_error": (C.c_char_p, []),
@@ -126,6 +138,8 @@ _SIGNATURES = {
                                     C.c_void_p]),
     "fmt_debug_band_attention": (C.c_int32, [C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
                                              C.c_void_p]),
+    "fmt_debug_flow_stage": (C.c_int32, [C.POINTER(FmtDebugStage), C.c_void_p]),
+    "fmt_debug_window_stage": (C.c_int32, [C.POINTER(FmtDebugStage), C.c_void_p]),
 }
 
 _lib = None

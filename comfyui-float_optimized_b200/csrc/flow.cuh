@@ -818,6 +818,47 @@ __device__ __forceinline__ void flow_simt_engine(const FlowParams& p, const Flow
 }
 
 // ---------------------------------------------------------------------------------------------------------------- kernel
+// The chunks and this CTA's units of every (SIMT kind, chunk), built by the CTA's FLOW_THREADS threads.  Units are dealt for a grid of
+// at least n_chunks CTAs (the kernel runs one CTA per SM): with fewer, chunk c >= gridDim.x would get no CTA.
+template <int NV>
+__device__ __forceinline__ void flow_chunk_tables(const FlowParams& p, FlowChunk* chunks, FlowUnits* units, int nctas, int cta) {
+  for (int c = threadIdx.x; c < p.n_chunks; c += FLOW_THREADS) {
+    FlowChunk ck;
+    ck.seq = c / p.nsub; ck.sub = c - ck.seq * p.nsub;
+    ck.f0 = ck.sub * p.CH;
+    ck.vr = min(p.CH, p.s.N - ck.f0);
+    ck.rr0 = ck.seq * p.s.N + ck.f0;
+    ck.rp0 = c * p.CH;
+    ck.clip = ck.seq % p.s.B;
+    ck.pad = 0;
+    chunks[c] = ck;
+    for (int kind = 0; kind < 4; ++kind) {
+      int n_units;
+      const int row_wpr = NV >= 4 ? 4 : NV;                                  // as in flow_row_units
+      if (kind == FK_ROW) n_units = (ck.vr + 8 / row_wpr - 1) / (8 / row_wpr);
+      else if (kind == FK_ATTN) n_units = p.heads * max(1, (nctas / p.n_chunks) / p.heads);   // (head, group of row pairs), see flow_attn_units
+      else if (kind == FK_GELU) n_units = ck.vr * ((p.mlp_hidden / 4 + FLOW_SIMT - 1) / FLOW_SIMT);
+      else n_units = ck.seq < p.s.B ? (max(0, ck.f0 + ck.vr - max(ck.f0, p.s.P)) * p.s.W + FLOW_SIMT - 1) / FLOW_SIMT : 0;   // published on branch 0's chunks
+      // The row-wise stages of a chunk run on that chunk's own slice of the grid, so that the in-order SIMT engine of a CTA
+      // serves ONE dependency chain and never holds a ready chunk back behind a late one; the CFG combine (once per
+      // evaluation, needs every branch) is dealt over the whole grid.
+      FlowUnits un;
+      un.n_units = n_units; un.pad = 0;
+      if (kind == FK_COMB) {
+        const int rot = (c * 29) % nctas;
+        int u0 = cta - rot;
+        if (u0 < 0) u0 += nctas;
+        un.stride = nctas; un.n_part = min(n_units, nctas); un.u0 = u0 < n_units ? u0 : -1;
+      } else {
+        const int gs = max(1, nctas / p.n_chunks);
+        const int u0 = cta - c * gs;
+        un.stride = gs; un.n_part = min(n_units, gs); un.u0 = (u0 >= 0 && u0 < gs && u0 < n_units) ? u0 : -1;
+      }
+      units[kind * FLOW_MAX_CHUNKS + c] = un;
+    }
+  }
+}
+
 template <int NV /* dim_h / 128 */>
 __global__ void __launch_bounds__(FLOW_THREADS, 1) fmt_flow_kernel(const __grid_constant__ FlowParams p) {
   extern __shared__ uint8_t smem_raw[];
@@ -856,41 +897,7 @@ __global__ void __launch_bounds__(FLOW_THREADS, 1) fmt_flow_kernel(const __grid_
     it.pad0 = it.pad1 = it.pad2 = 0;
     items[g] = it;
   }
-  for (int c = threadIdx.x; c < p.n_chunks; c += FLOW_THREADS) {
-    FlowChunk ck;
-    ck.seq = c / p.nsub; ck.sub = c - ck.seq * p.nsub;
-    ck.f0 = ck.sub * p.CH;
-    ck.vr = min(p.CH, p.s.N - ck.f0);
-    ck.rr0 = ck.seq * p.s.N + ck.f0;
-    ck.rp0 = c * p.CH;
-    ck.clip = ck.seq % p.s.B;
-    ck.pad = 0;
-    chunks[c] = ck;
-    for (int kind = 0; kind < 4; ++kind) {
-      int n_units;
-      const int row_wpr = NV >= 4 ? 4 : NV;                                  // as in flow_row_units
-      if (kind == FK_ROW) n_units = (ck.vr + 8 / row_wpr - 1) / (8 / row_wpr);
-      else if (kind == FK_ATTN) n_units = p.heads * max(1, (nctas / p.n_chunks) / p.heads);   // (head, group of row pairs), see flow_attn_units
-      else if (kind == FK_GELU) n_units = ck.vr * ((p.mlp_hidden / 4 + FLOW_SIMT - 1) / FLOW_SIMT);
-      else n_units = ck.seq < p.s.B ? (max(0, ck.f0 + ck.vr - max(ck.f0, p.s.P)) * p.s.W + FLOW_SIMT - 1) / FLOW_SIMT : 0;   // published on branch 0's chunks
-      // The row-wise stages of a chunk run on that chunk's own slice of the grid, so that the in-order SIMT engine of a CTA
-      // serves ONE dependency chain and never holds a ready chunk back behind a late one; the CFG combine (once per
-      // evaluation, needs every branch) is dealt over the whole grid.
-      FlowUnits un;
-      un.n_units = n_units; un.pad = 0;
-      if (kind == FK_COMB) {
-        const int rot = (c * 29) % nctas;
-        int u0 = cta - rot;
-        if (u0 < 0) u0 += nctas;
-        un.stride = nctas; un.n_part = min(n_units, nctas); un.u0 = u0 < n_units ? u0 : -1;
-      } else {
-        const int gs = max(1, nctas / p.n_chunks);
-        const int u0 = cta - c * gs;
-        un.stride = gs; un.n_part = min(n_units, gs); un.u0 = (u0 >= 0 && u0 < gs && u0 < n_units) ? u0 : -1;
-      }
-      units[kind * FLOW_MAX_CHUNKS + c] = un;
-    }
-  }
+  flow_chunk_tables<NV>(p, chunks, units, nctas, cta);
   if (warp == 0 && lane == 0) {
     for (int i = 0; i < FLOW_MAX_NW; ++i) { mbar_init(&sm.w_full[i], 1); mbar_init(&sm.w_empty[i], 1); }
     for (int i = 0; i < FLOW_MAX_NA; ++i) { mbar_init(&sm.a_full[i], 1); mbar_init(&sm.a_empty[i], 1); }

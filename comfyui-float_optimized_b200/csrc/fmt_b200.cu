@@ -7,6 +7,7 @@
 #include "kernels.cuh"
 #include "window.cuh"
 #include "flow.cuh"
+#include "stages.cuh"
 
 #include <algorithm>
 #include <functional>
@@ -2127,6 +2128,161 @@ int32_t fmt_debug_band_attention(int32_t mode, const void* qkv, int32_t n_seq, i
       return band_attention<bf16x3_t>(&h, static_cast<const float*>(qkv), n_seq, N, heads, hd, window, static_cast<bf16x3_t*>(out), variant, st);
   }
   return set_err(-1, "fmt_debug_band_attention: unknown mode %d", mode);
+}
+
+// ---- row-wise stages of the persistent window kernels
+static_assert(FMT_STAGE_ROW == int{FK_ROW} && FMT_STAGE_ATTN == int{FK_ATTN} && FMT_STAGE_GELU == int{FK_GELU} && FMT_STAGE_COMB == int{FK_COMB},
+              "FMT_STAGE_* are the kernels' stage kinds");
+
+// Shape and pointer checks shared by both kernels (no device call: bad arguments are refused on any machine)
+static int check_stage(const FmtDebugStage* d, const char* fn) {
+  REQUIRE(d, "%s: null argument", fn);
+  REQUIRE(d->kind >= FMT_STAGE_ROW && d->kind <= FMT_STAGE_COMB, "%s: unknown stage kind %d", fn, d->kind);
+  REQUIRE(d->grid >= 0, "%s: grid %d", fn, d->grid);
+  REQUIRE(d->H == 128 || d->H == 256 || d->H == 512 || d->H == 1024, "%s: H = %d is not 128, 256, 512 or 1024", fn, d->H);
+  REQUIRE(d->n_branches == 1 || d->n_branches == 3 || d->n_branches == 4, "%s: %d CFG branches", fn, d->n_branches);
+  REQUIRE(d->batch >= 1 && d->n_frames >= 1 && d->n_prev >= 0 && d->n_prev < d->n_frames, "%s: bad sequence shape batch=%d frames=%d prev=%d", fn,
+          d->batch, d->n_frames, d->n_prev);
+  if (d->kind == FMT_STAGE_ROW) {
+    REQUIRE(d->X && d->Pacc && d->A1 && d->table && d->bias && (d->row_mode == 1 || d->pos), "%s: ROW needs X, Pacc, A1, table, bias (and pos in mode 0)", fn);
+    REQUIRE(d->row_mode == 0 || d->row_mode == 1, "%s: row mode %d", fn, d->row_mode);
+    REQUIRE(d->shift_off >= 0 && d->scale_off >= 0 && d->gate_off >= 0 && d->ldt % 4 == 0 && d->shift_off % 4 == 0 && d->scale_off % 4 == 0 &&
+                d->gate_off % 4 == 0 && d->shift_off + d->H <= d->ldt && d->scale_off + d->H <= d->ldt && d->gate_off + d->H <= d->ldt,
+            "%s: table columns outside a row of %lld", fn, static_cast<long long>(d->ldt));
+  } else if (d->kind == FMT_STAGE_ATTN) {
+    REQUIRE(d->QKVacc && d->A2 && d->bias, "%s: ATTN needs QKVacc, A2 and bias", fn);
+    const int hd = d->heads > 0 && d->H % d->heads == 0 ? d->H / d->heads : 0;
+    REQUIRE(hd == 32 || hd == 64 || hd == 128, "%s: head_dim %d (H = %d, %d heads) is not 32, 64 or 128", fn, hd, d->H, d->heads);
+    REQUIRE(d->window >= 0, "%s: window %d", fn, d->window);
+  } else if (d->kind == FMT_STAGE_GELU) {
+    REQUIRE(d->Hacc && d->Hm && d->bias, "%s: GELU needs Hacc, Hm and bias", fn);
+    REQUIRE(d->mlp_hidden > 0 && d->mlp_hidden % 64 == 0, "%s: mlp_hidden %d is not a multiple of 64", fn, d->mlp_hidden);
+  } else {
+    REQUIRE(d->Vacc && d->bias && d->x_state && d->ddt && d->ax && (d->n_stages == 1 || d->kbuf), "%s: COMB needs Vacc, bias, x_state, ddt, ax (and kbuf)", fn);
+    REQUIRE(d->W > 0 && d->n_stages >= 1 && d->n_stages <= 4 && d->stage >= 0 && d->stage < d->n_stages && d->step >= 0,
+            "%s: bad COMB arguments W=%d stages=%d stage=%d step=%d", fn, d->W, d->n_stages, d->stage, d->step);
+    REQUIRE(!d->slot_branches == !d->slot_scales, "%s: slot_branches and slot_scales go together", fn);
+    for (int b = 0; d->slot_branches && b < d->batch; ++b) {
+      const int nb = d->slot_branches[b];
+      REQUIRE((nb == 1 || nb == 3 || nb == 4) && nb <= d->n_branches, "%s: clip %d combines %d of %d branches", fn, b, nb, d->n_branches);
+    }
+  }
+  return 0;
+}
+
+static ModelShape stage_shape(const FmtDebugStage* d) {
+  ModelShape s{};
+  s.B = d->batch; s.nb = d->n_branches; s.N = d->n_frames; s.P = d->n_prev; s.L = d->n_frames - d->n_prev; s.W = d->W; s.H = d->H;
+  return s;
+}
+
+static StageArgs stage_args(const FmtDebugStage* d) {
+  StageArgs a{};
+  a.kind = d->kind; a.row_mode = d->row_mode; a.zero_qkv = d->zero_qkv; a.parity = d->parity;
+  a.gate_off = d->gate_off; a.shift_off = d->shift_off; a.scale_off = d->scale_off;
+  a.bias = d->bias; a.step = d->step; a.stage = d->stage;
+  return a;
+}
+
+// One device buffer: a copy of `head` (WinParams, whose `wargs` field is set here), then the WindowArgs of a COMB stage and its
+// per-clip SlotArgs; *wargs points at the WindowArgs
+static int stage_upload(const FmtDebugStage* d, WinParams* head, cudaStream_t st, void** buf, const WindowArgs** wargs) {
+  const size_t head_bytes = head ? sizeof(WinParams) : 0;
+  const size_t off = (head_bytes + 255) / 256 * 256;
+  std::vector<unsigned char> host(off + sizeof(WindowArgs) + static_cast<size_t>(d->batch) * sizeof(SlotArgs), 0);
+  CUDA_OK(cudaMallocAsync(buf, host.size(), st));
+  WindowArgs wa{};
+  wa.a_scale = d->a_scale; wa.r_scale = d->r_scale; wa.e_scale = d->e_scale;
+  if (d->kind == FMT_STAGE_COMB && d->slot_branches) {
+    SlotArgs* sl = reinterpret_cast<SlotArgs*>(host.data() + off + sizeof(WindowArgs));
+    for (int b = 0; b < d->batch; ++b) {
+      sl[b].n_branches = d->slot_branches[b];
+      sl[b].a_scale = d->slot_scales[3 * b]; sl[b].r_scale = d->slot_scales[3 * b + 1]; sl[b].e_scale = d->slot_scales[3 * b + 2];
+    }
+    wa.slots = reinterpret_cast<const SlotArgs*>(static_cast<unsigned char*>(*buf) + off + sizeof(WindowArgs));
+  }
+  memcpy(host.data() + off, &wa, sizeof(WindowArgs));
+  *wargs = reinterpret_cast<const WindowArgs*>(static_cast<unsigned char*>(*buf) + off);
+  if (head) {
+    head->wargs = *wargs;
+    memcpy(host.data(), head, head_bytes);
+  }
+  CUDA_OK(cudaMemcpyAsync(*buf, host.data(), host.size(), cudaMemcpyHostToDevice, st));
+  CUDA_OK(cudaStreamSynchronize(st));   // `host` is a stack object
+  return 0;
+}
+
+int32_t fmt_debug_flow_stage(const FmtDebugStage* d, void* stream) {
+  FMT_OK(check_stage(d, "fmt_debug_flow_stage"));
+  const int CH = d->chunk_rows;
+  REQUIRE(CH == 32 || CH == 64, "fmt_debug_flow_stage: chunk_rows %d is not 32 or 64", CH);
+  const int nsub = (d->n_frames + CH - 1) / CH, n_chunks = d->n_branches * d->batch * nsub;
+  REQUIRE(n_chunks <= FLOW_MAX_CHUNKS, "fmt_debug_flow_stage: %d chunks > %d", n_chunks, FLOW_MAX_CHUNKS);
+  REQUIRE(d->kind != FMT_STAGE_ATTN || d->window <= CH, "fmt_debug_flow_stage: window %d > %d rows per chunk", d->window, CH);
+  REQUIRE(d->grid == 0 || d->grid >= n_chunks, "fmt_debug_flow_stage: grid %d < %d chunks", d->grid, n_chunks);
+  FmtHandle h;
+  FMT_OK(debug_handle(h));
+  const int grid = d->grid > 0 ? d->grid : h.num_sms;
+  REQUIRE(grid >= n_chunks, "fmt_debug_flow_stage: %d SMs < %d chunks", grid, n_chunks);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  FlowParams fp{};
+  fp.s = stage_shape(d); fp.R = d->n_branches * d->batch * d->n_frames;
+  fp.heads = d->heads; fp.window = d->window; fp.mlp_hidden = d->mlp_hidden; fp.NT = static_cast<int>(d->ldt);
+  fp.n_steps = d->step + 1; fp.n_stages = d->n_stages;
+  fp.CH = CH; fp.nsub = nsub; fp.NPs = nsub * CH; fp.n_chunks = n_chunks; fp.RP = n_chunks * CH;
+  fp.X = d->X; fp.Pacc = d->Pacc; fp.QKVacc = d->QKVacc; fp.Hacc = d->Hacc; fp.Vacc = d->Vacc;
+  fp.A1 = static_cast<bf16*>(d->A1); fp.A2 = static_cast<bf16*>(d->A2); fp.Hm = static_cast<bf16*>(d->Hm); fp.ax = static_cast<bf16*>(d->ax);
+  fp.table = static_cast<const bf16*>(d->table); fp.urow = d->urow; fp.pos = d->pos; fp.b_dec = d->bias;
+  fp.x_state = d->x_state; fp.kbuf = d->kbuf; fp.ddt = d->ddt;
+  for (int i = 0; i < 16; ++i) fp.rk_a[i] = d->rk_a[i];
+  for (int i = 0; i < 4; ++i) fp.rk_b[i] = d->rk_b[i];
+  fp.spin_limit = h.flow_spin_limit;
+  void* buf = nullptr;
+  FMT_OK(stage_upload(d, nullptr, st, &buf, &fp.wargs));
+  const StageArgs a = stage_args(d);
+  switch (d->H / 128) {
+    case 1: fmt_flow_stage_kernel<1><<<grid, FLOW_THREADS, 0, st>>>(fp, a); break;
+    case 2: fmt_flow_stage_kernel<2><<<grid, FLOW_THREADS, 0, st>>>(fp, a); break;
+    case 4: fmt_flow_stage_kernel<4><<<grid, FLOW_THREADS, 0, st>>>(fp, a); break;
+    default: fmt_flow_stage_kernel<8><<<grid, FLOW_THREADS, 0, st>>>(fp, a); break;
+  }
+  const cudaError_t e = cudaGetLastError();
+  (void)cudaFreeAsync(buf, st);
+  return e == cudaSuccess ? 0 : set_err(-2, "fmt_debug_flow_stage: launch failed: %s", cudaGetErrorString(e));
+}
+
+int32_t fmt_debug_window_stage(const FmtDebugStage* d, void* stream) {
+  FMT_OK(check_stage(d, "fmt_debug_window_stage"));
+  const int R = d->n_branches * d->batch * d->n_frames;
+  REQUIRE(R <= 256, "fmt_debug_window_stage: %d token rows > 256", R);
+  REQUIRE(d->urow == nullptr, "fmt_debug_window_stage: the window kernel's table has one row per token row (urow must be NULL)");
+  FmtHandle h;
+  FMT_OK(debug_handle(h));
+  const int grid = d->grid > 0 ? d->grid : h.num_sms;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  WinParams wp{};
+  wp.s = stage_shape(d); wp.R = R; wp.Rp = (R + 63) / 64 * 64;
+  wp.heads = d->heads; wp.window = d->window; wp.mlp_hidden = d->mlp_hidden; wp.NT = static_cast<int>(d->ldt);
+  wp.n_steps = d->step + 1; wp.n_stages = d->n_stages;
+  wp.X = d->X; wp.Pacc = d->Pacc; wp.QKVacc = d->QKVacc; wp.Hacc = d->Hacc; wp.Vacc = d->Vacc;
+  wp.A1 = static_cast<bf16*>(d->A1); wp.A2 = static_cast<bf16*>(d->A2); wp.Hm = static_cast<bf16*>(d->Hm); wp.ax = static_cast<bf16*>(d->ax);
+  wp.table = static_cast<const bf16*>(d->table); wp.pos = d->pos; wp.b_dec = d->bias;
+  wp.x_state = d->x_state; wp.kbuf = d->kbuf; wp.ddt = d->ddt;
+  for (int i = 0; i < 16; ++i) wp.rk_a[i] = d->rk_a[i];
+  for (int i = 0; i < 4; ++i) wp.rk_b[i] = d->rk_b[i];
+  void* buf = nullptr;
+  FMT_OK(stage_upload(d, &wp, st, &buf, &wp.wargs));
+  const WinParams* dp = static_cast<const WinParams*>(buf);
+  const StageArgs a = stage_args(d);
+  switch (d->H / 128) {
+    case 1: fmt_window_stage_kernel<1><<<grid, WIN_THREADS, 0, st>>>(dp, a); break;
+    case 2: fmt_window_stage_kernel<2><<<grid, WIN_THREADS, 0, st>>>(dp, a); break;
+    case 4: fmt_window_stage_kernel<4><<<grid, WIN_THREADS, 0, st>>>(dp, a); break;
+    default: fmt_window_stage_kernel<8><<<grid, WIN_THREADS, 0, st>>>(dp, a); break;
+  }
+  const cudaError_t e = cudaGetLastError();
+  (void)cudaFreeAsync(buf, st);
+  return e == cudaSuccess ? 0 : set_err(-2, "fmt_debug_window_stage: launch failed: %s", cudaGetErrorString(e));
 }
 
 }  // extern "C"

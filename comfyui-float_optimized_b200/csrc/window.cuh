@@ -923,6 +923,22 @@ __device__ __forceinline__ void win_attn_dispatch(const WinParams& p, const WinC
 }
 
 // ---------------------------------------------------------------------------------------------------------------- kernel
+// This CTA's rows, rank and operand buffers in the SIMT stages (one thread writes them)
+template <bool GROUPED>
+__device__ __forceinline__ void win_ctx(const WinParams& p, WinCtx& cx) {
+  if (GROUPED) {
+    const int g = blockIdx.x / p.Cg;
+    const size_t t_a1 = static_cast<size_t>((p.s.H + 63) / 64) * p.RgP * 64, t_hm = static_cast<size_t>((p.mlp_hidden + 63) / 64) * p.RgP * 64;
+    cx.row0 = g * p.Rg; cx.nrows = p.Rg; cx.rank = blockIdx.x % p.Cg; cx.nranks = p.Cg;
+    cx.all_rank = blockIdx.x; cx.all_n = p.G * p.Cg; cx.RgP = p.RgP;
+    cx.A1 = p.A1 + g * t_a1; cx.A2 = p.A2 + g * t_a1; cx.Hm = p.Hm + g * t_hm;
+    cx.bar = p.bar_counter + 32 * (1 + g);
+  } else {
+    cx.row0 = 0; cx.nrows = p.R; cx.rank = blockIdx.x; cx.nranks = gridDim.x; cx.all_rank = blockIdx.x; cx.all_n = gridDim.x; cx.RgP = p.Rp;
+    cx.A1 = p.A1; cx.A2 = p.A2; cx.Hm = p.Hm; cx.bar = p.bar_counter;
+  }
+}
+
 template <int NV /* dim_h / 128 */, bool GROUPED /* false: split-K over the whole grid; true: one group of CTAs per <= 128 rows */>
 __global__ void __launch_bounds__(WIN_THREADS, 1) fmt_window_kernel(const WinParams* __restrict__ pp) {
   extern __shared__ uint8_t smem_raw[];
@@ -954,19 +970,7 @@ __global__ void __launch_bounds__(WIN_THREADS, 1) fmt_window_kernel(const WinPar
   __syncthreads();
   if (GROUPED && static_cast<int>(blockIdx.x) >= p.G * p.Cg) return;    // CTAs left over by 148 = G * Cg + rest have no work
 
-  if (threadIdx.x == 0) {
-    if (GROUPED) {
-      const int g = blockIdx.x / p.Cg;
-      const size_t t_a1 = static_cast<size_t>((p.s.H + 63) / 64) * p.RgP * 64, t_hm = static_cast<size_t>((p.mlp_hidden + 63) / 64) * p.RgP * 64;
-      cx.row0 = g * p.Rg; cx.nrows = p.Rg; cx.rank = blockIdx.x % p.Cg; cx.nranks = p.Cg;
-      cx.all_rank = blockIdx.x; cx.all_n = p.G * p.Cg; cx.RgP = p.RgP;
-      cx.A1 = p.A1 + g * t_a1; cx.A2 = p.A2 + g * t_a1; cx.Hm = p.Hm + g * t_hm;
-      cx.bar = p.bar_counter + 32 * (1 + g);
-    } else {
-      cx.row0 = 0; cx.nrows = p.R; cx.rank = blockIdx.x; cx.nranks = gridDim.x; cx.all_rank = blockIdx.x; cx.all_n = gridDim.x; cx.RgP = p.Rp;
-      cx.A1 = p.A1; cx.A2 = p.A2; cx.Hm = p.Hm; cx.bar = p.bar_counter;
-    }
-  }
+  if (threadIdx.x == 0) win_ctx<GROUPED>(p, cx);
   __syncthreads();
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;

@@ -352,6 +352,51 @@ FMT_API int32_t fmt_debug_lnmod(int32_t mode, const float* X, int32_t rows, int3
 FMT_API int32_t fmt_debug_band_attention(int32_t mode, const void* qkv, int32_t n_seq, int32_t N, int32_t heads, int32_t hd,
                                          int32_t window, void* out, int32_t variant, void* stream);
 
+/* Row-wise stages of the persistent window kernels (bf16 mode), run by the kernels' own stage functions:
+ *   ROW   mode 0: X = Pacc + bias + pos[frame];  mode 1: X += gate * (Pacc + bias);  then A1 = bf16(LN(X) (1 + scale) + shift), Pacc <- 0
+ *         (window kernel with zero_qkv: the QKV accumulator rows <- 0 as well)
+ *   ATTN  A2 = bf16(band attention of QKVacc + bias) (flow kernel: QKV buffer `parity`, the valid rows of the other buffer <- 0)
+ *   GELU  Hm = bf16(GELU_tanh(Hacc + bias)), Hacc <- 0
+ *   COMB  CFG combine of Vacc + bias (decoder bias), then Euler or stage `stage` of an explicit Runge-Kutta step `step`: kbuf[stage],
+ *         x_state at the last stage, ax = bf16(y) in every branch; Vacc <- 0
+ * Token rows: n_branches x batch sequences of n_frames, the first n_prev of them context frames.  Row layouts:
+ *   flow kernel    chunks of chunk_rows (32 / 64) rows that never straddle a sequence: RP = chunks x chunk_rows padded rows, NPs =
+ *                  chunk_rows x ceil(n_frames / chunk_rows) per sequence.  X, Pacc, Hacc (RP, .); QKVacc two buffers (RP, 3H);
+ *                  Vacc (n_branches, batch, NPs, W); A1 / A2 / Hm [chunk][K block][chunk_rows][64] with the 16-byte XOR swizzle.
+ *   window kernel  R = n_branches x batch x n_frames <= 256 rows, Rp = R rounded up to 64: X, Pacc, QKVacc, Hacc (R, .); Vacc
+ *                  (n_branches, batch, n_frames, W); A1 / A2 / Hm [K block][Rp][64] with the same swizzle.
+ * Every pointer is a DEVICE pointer except slot_branches / slot_scales. */
+enum { FMT_STAGE_ROW = 0, FMT_STAGE_ATTN = 1, FMT_STAGE_GELU = 2, FMT_STAGE_COMB = 3 };
+
+typedef struct FmtDebugStage {
+  int32_t kind;           /* FMT_STAGE_*                                                                                 */
+  int32_t grid;           /* CTAs, 0 = one per SM (flow kernel: at least one per chunk)                                 */
+  int32_t chunk_rows;     /* flow kernel: 32 or 64 (window kernel: ignored)                                             */
+  int32_t n_branches, batch, n_frames, n_prev;
+  int32_t H, heads, window, mlp_hidden, W;   /* H in {128, 256, 512, 1024}; ATTN: H / heads in {32, 64, 128}          */
+  int32_t row_mode, zero_qkv, parity;
+  int32_t n_stages, stage, step;             /* COMB: stages of the solver (1 = Euler), the stage and step it runs       */
+  int64_t ldt;            /* ROW: AdaLN table row stride (elements)                                                     */
+  int64_t gate_off, shift_off, scale_off;    /* ROW: table columns of gate (mode 1), shift and scale                    */
+  float a_scale, r_scale, e_scale;           /* COMB: guidance of every clip without slot_branches                      */
+  float rk_a[16], rk_b[4];                   /* COMB: a[g][j] at [g * n_stages + j], b[j]                               */
+  float *X, *Pacc, *QKVacc, *Hacc, *Vacc;
+  void *A1, *A2, *Hm, *ax;                   /* bf16                                                                     */
+  const void* table;      /* ROW: bf16 AdaLN table (rows, ldt)                                                          */
+  const int32_t* urow;    /* ROW, flow kernel: table row of every token row, or NULL                                    */
+  const float* bias;      /* ROW: (H); ATTN: (3H); GELU: (mlp_hidden); COMB: (W)                                        */
+  const float* pos;       /* ROW mode 0: (n_frames, H)                                                                   */
+  float *x_state, *kbuf;  /* COMB: (batch, n_frames - n_prev, W) and n_stages of those                                  */
+  const float* ddt;       /* COMB: step sizes, at least step + 1                                                         */
+  const int32_t* slot_branches;              /* COMB, HOST or NULL: per clip 1, 3 or 4 branches (<= n_branches)         */
+  const float* slot_scales;                  /* COMB, HOST (batch, 3): per clip a, r, e scales (with slot_branches)     */
+} FmtDebugStage;
+
+/* One stage kind of the dataflow window kernel (flow.cuh) over every chunk. */
+FMT_API int32_t fmt_debug_flow_stage(const FmtDebugStage* d, void* stream);
+/* One stage kind of the barrier-stepped window kernel (window.cuh, split-K schedule) over every row. */
+FMT_API int32_t fmt_debug_window_stage(const FmtDebugStage* d, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
