@@ -705,9 +705,9 @@ __device__ __forceinline__ void flow_comb_unit(const FlowParams& p, const FlowCh
   for (int br = 0; br < 4; ++br) vb[br] = __ldcg(va0 + (br < s.nb ? br : 0) * vstride);
   const float bd = __ldg(p.b_dec + j);
   const float dt = __ldg(p.ddt + step);
-  float a_s = __ldg(&p.wargs->a_scale), r_s = __ldg(&p.wargs->r_scale), e_s = __ldg(&p.wargs->e_scale);
   const SlotArgs* const slots = p.wargs->slots;
-  int nb = s.nb;
+  float a_s, r_s, e_s;
+  int nb;
   const float y0 = __ldcg(p.x_state + o);
   float kprev[4] = {0.f, 0.f, 0.f, 0.f};
   if (G > 1) {

@@ -94,7 +94,8 @@ struct FmtHandle {
   bool dedup = false;                            // U < R: the AdaLN tables hold one row per DISTINCT condition row (FMT_DEDUP=0 switches it off)
   int use_dedup = 1;
   DevBuf st_rs, st_wa, st_we, st_noise, st_rd;   // staging for host-located clips
-  // fmt_sample_clips: the slot records of every window of a call ([window][slot]), uploaded with one copy from a pinned staging
+  DevBuf ev_wa, ev_we;                           // fmt_velocity: [prev_wa | wa] and [prev_we | we] of every clip, (B, P + L, .)
+  // the slot records of every window of a sampling call ([window][slot]), uploaded with one copy from a pinned staging
   // buffer; slot_ev marks the end of that copy, so the next call waits for it before it refills the staging buffer.  A window's
   // records are slot_stride bytes: B SlotArgs, followed by B SlotOde in calls of the per-slot window graph.
   DevBuf slot_buf, slot_zero;                    // slot_zero: the inputs of an idle slot
@@ -457,7 +458,7 @@ static int launch_attn(FmtHandle* h, cudaStream_t st) {
 }
 
 // One model evaluation: V[R, W] = FMT.forward over the nb-way batched CFG branches (FMT.py:277-340).  The x-embedder
-// operand `ax` has already been written by the producer of the ODE state (init_window / cfg_combine / rk_combine / pack_x).
+// operand `ax` has already been written by the producer of the ODE state (init_window / cfg_combine / rk_combine).
 template <typename T>
 static int enqueue_forward(FmtHandle* h, const CondRows& r, int table_slot, cudaStream_t st) {
   const ModelShape& s = h->shape;
@@ -1182,7 +1183,7 @@ int32_t fmt_destroy(FmtHandle* h) {
   for (void* p : h->owned) cudaFree(p);
   for (auto& kv : h->ode_cache) cudaFree(kv.second.p);
   DevBuf* bufs[] = {&h->cond, &h->cemb, &h->temb, &h->tfreq, &h->th, &h->silu, &h->table, &h->xstate, &h->ystage, &h->kbuf, &h->prevx, &h->ax,
-                    &h->X, &h->A1, &h->QKV, &h->A2, &h->Hm, &h->V, &h->ddt, &h->dteval, &h->wargs, &h->st_rs, &h->st_wa, &h->st_we, &h->st_noise, &h->st_rd,
+                    &h->X, &h->A1, &h->QKV, &h->A2, &h->Hm, &h->V, &h->ddt, &h->dteval, &h->wargs, &h->st_rs, &h->st_wa, &h->st_we, &h->st_noise, &h->st_rd, &h->ev_wa, &h->ev_we,
                     &h->win_params, &h->win_tmaps, &h->win_acc, &h->win_bar, &h->win_trace, &h->win_act,
                     &h->flow_gemms, &h->flow_tmaps, &h->flow_acc, &h->flow_act, &h->flow_flags, &h->flow_trace, &h->urow_buf, &h->uidx_buf,
                     &h->slot_buf, &h->slot_zero, &h->s_cond, &h->s_cemb, &h->s_urow, &h->s_uidx, &h->s_kbuf};
@@ -1492,16 +1493,18 @@ static int set_wargs(FmtHandle* h, const WindowArgs& a, cudaStream_t st) {
   return 0;
 }
 
-// Slot records of one call (fmt_sample_clips, fmt_sample_windows) go up in ONE copy from a pinned staging buffer that the handle
+// Slot records of one call (every sampling entry point and fmt_velocity) go up in ONE copy from a pinned staging buffer that the handle
 // owns; slot_ev marks the end of the previous call's copy, so the staging buffer is refilled only once that copy has read it.
 // stage_slot_records fills the staging buffer with n_win windows of idle records: zero inputs ((L, W) noise, and r_s / wa / we rows
 // no wider than that), no output, no context, scales of 1 and the plan's branch count; with ode, B SlotOde follow the B SlotArgs of
 // each window, idle as well (no evaluation).
 static int stage_slot_records(FmtHandle* h, size_t n_win, bool ode, cudaStream_t st) {
   const ModelShape& s = h->shape;
-  const size_t n_zero = std::max<size_t>(static_cast<size_t>(s.L) * s.W, static_cast<size_t>(std::max(s.A, s.E)));
-  FMT_OK(dev_alloc(h, h->slot_zero, n_zero * sizeof(float)));
-  CUDA_OK(cudaMemsetAsync(h->slot_zero.p, 0, n_zero * sizeof(float), st));
+  if (!h->slot_zero.p) {   // its size depends on the model's dims alone, and no kernel writes it: zeroed once per handle
+    const size_t n_zero = std::max<size_t>(static_cast<size_t>(s.L) * s.W, static_cast<size_t>(std::max(s.A, s.E)));
+    FMT_OK(dev_alloc(h, h->slot_zero, n_zero * sizeof(float)));
+    CUDA_OK(cudaMemsetAsync(h->slot_zero.p, 0, n_zero * sizeof(float), st));
+  }
   const float* zero = static_cast<const float*>(h->slot_zero.p);
   if (h->slot_ev) CUDA_OK(cudaEventSynchronize(h->slot_ev));
   h->slot_stride = static_cast<size_t>(s.B) * (sizeof(SlotArgs) + (ode ? sizeof(SlotOde) : 0));
@@ -1635,51 +1638,105 @@ static int ensure_ode_graph(FmtHandle* h, cudaStream_t st) {
   return capture_window(h, enqueue_window_ode_mode, &h->ode_exec, &h->ode_nodes, &h->ode_launches);
 }
 
+// One clip as its slot records see it: tensors of that clip alone (batch 1), the noise of its window w at noise + w * noise_stride,
+// and its guidance
+struct ClipIn {
+  const float *r_s, *wa, *we, *noise;
+  float* r_d;
+  size_t noise_stride;
+  int T_wa, T_we, T;
+  float a_scale, r_scale, e_scale;
+  int n_branches;
+};
+
+// The rules every clip of fmt_sample_clip / fmt_sample_clips follows; `who` names it in the error.  *n_win: its window count.
+static int check_clip(const ModelShape& s, const ClipIn& c, const char* who, int32_t* n_win) {
+  const int nb = c.n_branches;
+  REQUIRE((nb == 1 || nb == 3 || nb == 4) && nb <= s.nb, "%s: n_branches=%d must be 1, 3 or 4 and fit the plan's %d branches", who, nb, s.nb);
+  REQUIRE(c.r_s && c.wa && c.we && c.noise && c.r_d, "%s: null tensor pointer", who);
+  REQUIRE(c.T >= 1 && c.T_wa >= 1 && c.T_we >= 1, "%s: empty clip", who);
+  REQUIRE(s.we_dynamic ? c.T_we > 1 : c.T_we == 1, "%s: T_we=%d does not match plan.we_dynamic=%d", who, c.T_we, s.we_dynamic);
+  const int n = (c.T + s.L - 1) / s.L;
+  // every window must see at least one real wa (and dynamic we) frame; the reference's F.pad(replicate) fails otherwise
+  REQUIRE((n - 1) * s.L < c.T_wa, "%s: wa has %d frames but window %d starts at frame %d", who, c.T_wa, n - 1, (n - 1) * s.L);
+  REQUIRE(!s.we_dynamic || (n - 1) * s.L < c.T_we, "%s: dynamic we has %d frames but the last window starts at %d", who, c.T_we, (n - 1) * s.L);
+  *n_win = n;
+  return 0;
+}
+
+// Stages the slot records of `makespan` windows in which clip i runs its window w in slot slot[i] of window start[i] + w, every
+// other slot idle; od: the clips' SlotOde for the per-slot window graph (empty: the plan's graph).
+static int stage_clips(FmtHandle* h, const std::vector<ClipIn>& c, const int32_t* slot, const int32_t* start, int makespan,
+                       const std::vector<SlotOde>& od, cudaStream_t st) {
+  const ModelShape& s = h->shape;
+  FMT_OK(stage_slot_records(h, makespan, !od.empty(), st));
+  for (size_t i = 0; i < c.size(); ++i) {
+    const int n_win = (c[i].T + s.L - 1) / s.L;
+    for (int w = 0; w < n_win; ++w) {
+      if (!od.empty()) staged_ode(h, start[i] + w)[slot[i]] = od[i];
+      SlotArgs& z = staged_args(h, start[i] + w)[slot[i]];
+      z.r_s = c[i].r_s; z.wa = c[i].wa; z.we = c[i].we; z.r_d = c[i].r_d;
+      z.x0 = c[i].noise + w * c[i].noise_stride;
+      z.T_wa = c[i].T_wa; z.T_we = c[i].T_we; z.T_out = c[i].T;
+      z.win_start = z.out_start = w * s.L; z.first_window = (w == 0);
+      z.a_scale = c[i].a_scale; z.r_scale = c[i].r_scale; z.e_scale = c[i].e_scale; z.n_branches = c[i].n_branches;
+    }
+  }
+  return 0;
+}
+
+// Uploads the staged records of n_win windows and replays a window graph once per window: the plan's, or with ode the per-slot one
+static int replay_windows(FmtHandle* h, int n_win, bool ode, fmt_progress_fn progress, void* progress_user, cudaStream_t st) {
+  FMT_OK(upload_slot_records(h, n_win, st));
+  h->last_ode = ode;
+  for (int w = 0; w < n_win; ++w) {
+    FMT_OK(set_wargs(h, WindowArgs{device_args(h, w)}, st));
+    CUDA_OK(cudaGraphLaunch(ode ? h->ode_exec : h->graph_exec, st));
+    h->launches += ode ? h->ode_launches : h->capture_launches;
+    if (progress) progress(w, n_win, progress_user);
+  }
+  return 0;
+}
+
 int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
   REQUIRE(h && c, "fmt_sample_clip: null argument");
   REQUIRE(h->configured, "fmt_sample_clip: call fmt_configure first");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_OK(cudaSetDevice(h->device));
   const ModelShape& s = h->shape;
-  REQUIRE(c->r_s && c->wa && c->we && c->r_d, "fmt_sample_clip: null tensor pointer");
-  REQUIRE(c->audio_num_frames >= 1 && c->T_wa >= 1 && c->T_we >= 1, "fmt_sample_clip: empty clip");
-  REQUIRE(s.we_dynamic ? c->T_we > 1 : c->T_we == 1, "fmt_sample_clip: T_we=%d does not match plan.we_dynamic=%d", c->T_we, s.we_dynamic);
-  const int T = c->audio_num_frames;
-  const int n_win = (T + s.L - 1) / s.L;
-  REQUIRE(c->noise != nullptr, "fmt_sample_clip: noise (x0 of every window) is required");
-  // every window must see at least one real wa (and dynamic we) frame; the reference's F.pad(replicate) fails otherwise
-  REQUIRE((n_win - 1) * s.L < c->T_wa, "fmt_sample_clip: wa has %d frames but window %d starts at frame %d", c->T_wa, n_win - 1, (n_win - 1) * s.L);
-  REQUIRE(!s.we_dynamic || (n_win - 1) * s.L < c->T_we, "fmt_sample_clip: dynamic we has %d frames but the last window starts at %d", c->T_we, (n_win - 1) * s.L);
-
-  const float *r_s = c->r_s, *wa = c->wa, *we = c->we, *noise = c->noise;
-  float* r_d = c->r_d;
-  const size_t n_rs = static_cast<size_t>(s.B) * s.W, n_wa = static_cast<size_t>(s.B) * c->T_wa * s.A, n_we = static_cast<size_t>(s.B) * c->T_we * s.E;
+  ClipIn in{c->r_s, c->wa, c->we, c->noise, c->r_d, 0, c->T_wa, c->T_we, c->audio_num_frames, c->a_cfg_scale, c->r_cfg_scale, c->e_cfg_scale, s.nb};
+  int32_t n_win = 0;
+  FMT_OK(check_clip(s, in, "fmt_sample_clip", &n_win));
+  const int T = in.T;
+  const size_t n_rs = static_cast<size_t>(s.B) * s.W, n_wa = static_cast<size_t>(s.B) * in.T_wa * s.A, n_we = static_cast<size_t>(s.B) * in.T_we * s.E;
   const size_t n_noise = static_cast<size_t>(n_win) * s.B * s.L * s.W, n_rd = static_cast<size_t>(s.B) * T * s.W;
   if (c->location == FMT_LOC_HOST) {
     FMT_OK(dev_alloc(h, h->st_rs, n_rs * 4)); FMT_OK(dev_alloc(h, h->st_wa, n_wa * 4)); FMT_OK(dev_alloc(h, h->st_we, n_we * 4));
     FMT_OK(dev_alloc(h, h->st_noise, n_noise * 4)); FMT_OK(dev_alloc(h, h->st_rd, n_rd * 4));
-    CUDA_OK(cudaMemcpyAsync(h->st_rs.p, r_s, n_rs * 4, cudaMemcpyHostToDevice, st));
-    CUDA_OK(cudaMemcpyAsync(h->st_wa.p, wa, n_wa * 4, cudaMemcpyHostToDevice, st));
-    CUDA_OK(cudaMemcpyAsync(h->st_we.p, we, n_we * 4, cudaMemcpyHostToDevice, st));
-    CUDA_OK(cudaMemcpyAsync(h->st_noise.p, noise, n_noise * 4, cudaMemcpyHostToDevice, st));
-    r_s = static_cast<float*>(h->st_rs.p); wa = static_cast<float*>(h->st_wa.p); we = static_cast<float*>(h->st_we.p);
-    noise = static_cast<float*>(h->st_noise.p); r_d = static_cast<float*>(h->st_rd.p);
+    CUDA_OK(cudaMemcpyAsync(h->st_rs.p, in.r_s, n_rs * 4, cudaMemcpyHostToDevice, st));
+    CUDA_OK(cudaMemcpyAsync(h->st_wa.p, in.wa, n_wa * 4, cudaMemcpyHostToDevice, st));
+    CUDA_OK(cudaMemcpyAsync(h->st_we.p, in.we, n_we * 4, cudaMemcpyHostToDevice, st));
+    CUDA_OK(cudaMemcpyAsync(h->st_noise.p, in.noise, n_noise * 4, cudaMemcpyHostToDevice, st));
+    in.r_s = static_cast<float*>(h->st_rs.p); in.wa = static_cast<float*>(h->st_wa.p); in.we = static_cast<float*>(h->st_we.p);
+    in.noise = static_cast<float*>(h->st_noise.p); in.r_d = static_cast<float*>(h->st_rd.p);
   }
-  h->last_ode = false;
-  for (int w = 0; w < n_win; ++w) {
-    WindowArgs a{};
-    a.r_s = r_s; a.wa = wa; a.we = we; a.r_d = r_d;
-    a.x0 = noise + static_cast<size_t>(w) * s.B * s.L * s.W;
-    a.T_wa = c->T_wa; a.T_we = c->T_we; a.T_out = T;
-    a.win_start = w * s.L; a.first_window = (w == 0); a.use_ext = 0;
-    a.a_scale = c->a_cfg_scale; a.r_scale = c->r_cfg_scale; a.e_scale = c->e_cfg_scale;
-    FMT_OK(set_wargs(h, a, st));
-    CUDA_OK(cudaGraphLaunch(h->graph_exec, st));
-    h->launches += h->capture_launches;
-    if (c->progress) c->progress(w, n_win, c->progress_user);
+  // batch row b is slot b of every window: its rows of the batched tensors, the noise of its window w at noise[w][b]
+  std::vector<ClipIn> rows(s.B, in);
+  std::vector<int32_t> slot(s.B), start(s.B, 0);
+  for (int b = 0; b < s.B; ++b) {
+    ClipIn& r = rows[b];
+    r.r_s += static_cast<size_t>(b) * s.W;
+    r.wa += static_cast<size_t>(b) * in.T_wa * s.A;
+    r.we += static_cast<size_t>(b) * in.T_we * s.E;
+    r.noise += static_cast<size_t>(b) * s.L * s.W;
+    r.noise_stride = static_cast<size_t>(s.B) * s.L * s.W;
+    r.r_d += static_cast<size_t>(b) * T * s.W;
+    slot[b] = b;
   }
+  FMT_OK(stage_clips(h, rows, slot.data(), start.data(), n_win, {}, st));
+  FMT_OK(replay_windows(h, n_win, false, c->progress, c->progress_user, st));
   if (c->location == FMT_LOC_HOST) {
-    CUDA_OK(cudaMemcpyAsync(c->r_d, r_d, n_rd * 4, cudaMemcpyDeviceToHost, st));
+    CUDA_OK(cudaMemcpyAsync(c->r_d, in.r_d, n_rd * 4, cudaMemcpyDeviceToHost, st));
     CUDA_OK(cudaStreamSynchronize(st));
     // the persistent kernels report a tripped bounded spin through a mapped status word (the launch fails as well)
     if (h->window_active && h->win_err_host && *h->win_err_host != 0) return set_err(-6, "window kernel reported status 0x%08x", *h->win_err_host);
@@ -1690,9 +1747,7 @@ int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
 }  // extern "C"
 
 // Many clips on plan.batch slots: window w of the call runs, in slot k, whichever clip the schedule put there (at that clip's own
-// window), through the same captured window graph.  cond_gather / init_window / finalize_window read the per-slot tensors and
-// lengths, the CFG combines (cfg_combine_kernel and the COMB stages of the persistent kernels) the per-slot guidance.
-// ode != nullptr: each clip on its own schedule, through the per-slot window graph.
+// window), through the same captured window graph (ode != nullptr: each clip on its own schedule, through the per-slot window graph).
 static int sample_clips(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, const FmtClipOde* ode, void* stream) {
   REQUIRE(h && cs && g, "fmt_sample_clips_guided: null argument");
   REQUIRE(h->configured, "fmt_sample_clips: call fmt_configure first");
@@ -1703,20 +1758,14 @@ static int sample_clips(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidanc
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_OK(cudaSetDevice(h->device));
   const ModelShape& s = h->shape;
+  std::vector<ClipIn> c(n);
   std::vector<int32_t> n_win(n), slot(n), start(n);
-  for (int i = 0; i < n; ++i) {   // fmt_sample_clip's checks, per clip
-    const int nb = g->n_branches[i];
-    REQUIRE((nb == 1 || nb == 3 || nb == 4) && nb <= s.nb,
-            "fmt_sample_clips_guided: clip %d: n_branches=%d must be 1, 3 or 4 and fit the plan's %d branches", i, nb, s.nb);
-    REQUIRE(cs->r_s[i] && cs->wa[i] && cs->we[i] && cs->noise[i] && cs->r_d[i], "fmt_sample_clips: clip %d: null tensor pointer", i);
-    const int T = cs->audio_num_frames[i], T_wa = cs->T_wa[i], T_we = cs->T_we[i];
-    REQUIRE(T >= 1 && T_wa >= 1 && T_we >= 1, "fmt_sample_clips: clip %d is empty", i);
-    REQUIRE(s.we_dynamic ? T_we > 1 : T_we == 1, "fmt_sample_clips: clip %d: T_we=%d does not match plan.we_dynamic=%d", i, T_we, s.we_dynamic);
-    n_win[i] = (T + s.L - 1) / s.L;
-    REQUIRE((n_win[i] - 1) * s.L < T_wa, "fmt_sample_clips: clip %d: wa has %d frames but window %d starts at frame %d", i, T_wa, n_win[i] - 1,
-            (n_win[i] - 1) * s.L);
-    REQUIRE(!s.we_dynamic || (n_win[i] - 1) * s.L < T_we, "fmt_sample_clips: clip %d: dynamic we has %d frames but the last window starts at %d",
-            i, T_we, (n_win[i] - 1) * s.L);
+  for (int i = 0; i < n; ++i) {
+    c[i] = ClipIn{cs->r_s[i], cs->wa[i], cs->we[i], cs->noise[i], cs->r_d[i], static_cast<size_t>(s.L) * s.W, cs->T_wa[i], cs->T_we[i],
+                  cs->audio_num_frames[i], g->a_cfg_scale[i], g->r_cfg_scale[i], g->e_cfg_scale[i], g->n_branches[i]};
+    char who[48];
+    snprintf(who, sizeof(who), "fmt_sample_clips: clip %d", i);
+    FMT_OK(check_clip(s, c[i], who, &n_win[i]));
   }
   if (ode) FMT_OK(check_odes(h, ode, n, "fmt_sample_clips_ode: clip"));
   int makespan = 0;
@@ -1726,29 +1775,8 @@ static int sample_clips(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidanc
   std::vector<SlotOde> od(ode ? n : 0);
   for (int i = 0; i < static_cast<int>(od.size()); ++i) FMT_OK(slot_ode(h, ode, i, st, &od[i]));
   if (ode) FMT_OK(ensure_ode_graph(h, st));
-  FMT_OK(stage_slot_records(h, makespan, ode != nullptr, st));
-  for (int i = 0; i < n; ++i) {
-    for (int w = 0; w < n_win[i]; ++w) {
-      if (ode) staged_ode(h, start[i] + w)[slot[i]] = od[i];
-      SlotArgs& z = staged_args(h, start[i] + w)[slot[i]];
-      z.r_s = cs->r_s[i]; z.wa = cs->wa[i]; z.we = cs->we[i]; z.r_d = cs->r_d[i];
-      z.x0 = cs->noise[i] + static_cast<size_t>(w) * s.L * s.W;
-      z.T_wa = cs->T_wa[i]; z.T_we = cs->T_we[i]; z.T_out = cs->audio_num_frames[i];
-      z.win_start = z.out_start = w * s.L; z.first_window = (w == 0);
-      z.a_scale = g->a_cfg_scale[i]; z.r_scale = g->r_cfg_scale[i]; z.e_scale = g->e_cfg_scale[i]; z.n_branches = g->n_branches[i];
-    }
-  }
-  FMT_OK(upload_slot_records(h, makespan, st));
-  h->last_ode = ode != nullptr;
-  for (int w = 0; w < makespan; ++w) {
-    WindowArgs a{};
-    a.slots = device_args(h, w);
-    FMT_OK(set_wargs(h, a, st));
-    CUDA_OK(cudaGraphLaunch(ode ? h->ode_exec : h->graph_exec, st));
-    h->launches += ode ? h->ode_launches : h->capture_launches;
-    if (cs->progress) cs->progress(w, makespan, cs->progress_user);
-  }
-  return 0;
+  FMT_OK(stage_clips(h, c, slot.data(), start.data(), makespan, od, st));
+  return replay_windows(h, makespan, ode != nullptr, cs->progress, cs->progress_user, st);
 }
 
 extern "C" {
@@ -1818,14 +1846,7 @@ static int sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGui
     z.win_start = z.first_window ? 0 : s.P; z.out_start = 0;
     z.a_scale = g->a_cfg_scale[i]; z.r_scale = g->r_cfg_scale[i]; z.e_scale = g->e_cfg_scale[i]; z.n_branches = g->n_branches[i];
   }
-  FMT_OK(upload_slot_records(h, 1, st));
-  h->last_ode = ode != nullptr;
-  WindowArgs a{};
-  a.slots = device_args(h, 0);
-  FMT_OK(set_wargs(h, a, st));
-  CUDA_OK(cudaGraphLaunch(ode ? h->ode_exec : h->graph_exec, st));
-  h->launches += ode ? h->ode_launches : h->capture_launches;
-  return 0;
+  return replay_windows(h, 1, ode != nullptr, nullptr, nullptr, st);
 }
 
 extern "C" {
@@ -1841,14 +1862,27 @@ int32_t fmt_sample_windows_ode(FmtHandle* h, const FmtWindowSet* ws, const FmtCl
 
 }  // extern "C"
 
+// dst (B, P + L, C) <- [prev (B, P, C) | cur (B, L, C)] of every clip (device pointers)
+static int join_context(FmtHandle* h, DevBuf& dst, const float* prev, const float* cur, int C, cudaStream_t st) {
+  const ModelShape& s = h->shape;
+  const size_t np = static_cast<size_t>(s.P) * C * 4, nl = static_cast<size_t>(s.L) * C * 4;
+  FMT_OK(dev_alloc(h, dst, s.B * (np + nl)));
+  char* d = static_cast<char*>(dst.p);
+  if (np > 0) CUDA_OK(cudaMemcpy2DAsync(d, np + nl, prev, np, np, s.B, cudaMemcpyDeviceToDevice, st));
+  CUDA_OK(cudaMemcpy2DAsync(d + np, np + nl, cur, nl, nl, s.B, cudaMemcpyDeviceToDevice, st));
+  return 0;
+}
+
 template <typename T>
 static int enqueue_velocity(FmtHandle* h, const FmtEval* ev, cudaStream_t st) {
   const ModelShape& s = h->shape;
   const CondRows r = plan_rows(h);
   FMT_OK(enqueue_prepare<T>(h, r, st));
   FMT_OK(enqueue_tables<T>(h, r, ev->eval_index, 1, st));
-  FMT_OK(launch(h, pack_x_kernel<T>, dim3(s.B * s.N), dim3(128), 0, st, 1, static_cast<const WindowArgs*>(h->wargs.p), s, ev->x,
-                static_cast<const float*>(h->prevx.p), static_cast<T*>(h->ax.p)));
+  const size_t nfull = static_cast<size_t>(s.B) * s.N * s.W;
+  FMT_OK(launch(h, init_window_kernel<T>, dim3(static_cast<unsigned>((nfull + 255) / 256)), dim3(256), 0, st, 1,
+                static_cast<const WindowArgs*>(h->wargs.p), s, static_cast<float*>(h->xstate.p), static_cast<float*>(h->prevx.p),
+                static_cast<T*>(h->ax.p)));
   FMT_OK(enqueue_forward<T>(h, r, 0, st));
   FMT_OK(launch_combine<T>(h, 0, ev->v_out, nullptr, st));
   return 0;
@@ -1865,12 +1899,24 @@ int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_OK(cudaSetDevice(h->device));
   const ModelShape& s = h->shape;
-  WindowArgs a{};
-  a.r_s = ev->r_s; a.wa = ev->wa; a.we = ev->we; a.x0 = ev->x; a.r_d = nullptr;
-  a.prev_x_ext = ev->prev_x; a.prev_wa_ext = ev->prev_wa; a.prev_we_ext = ev->prev_we;
-  a.T_wa = s.L; a.T_we = s.we_dynamic ? s.L : 1; a.T_out = s.L; a.win_start = 0; a.first_window = 0; a.use_ext = 1;
-  a.a_scale = ev->a_cfg_scale; a.r_scale = ev->r_cfg_scale; a.e_scale = ev->e_cfg_scale;
-  FMT_OK(set_wargs(h, a, st));
+  // clip b is slot b: x and its explicit context (init_window_kernel reads ctx, and fmt_velocity runs no finalize_window_kernel that
+  // would write it), and [prev | current] frames of its conditions, read from frame P on
+  const int NF = s.P + s.L;
+  FMT_OK(join_context(h, h->ev_wa, ev->prev_wa, ev->wa, s.A, st));
+  if (s.we_dynamic) FMT_OK(join_context(h, h->ev_we, ev->prev_we, ev->we, s.E, st));
+  FMT_OK(stage_slot_records(h, 1, false, st));
+  for (int b = 0; b < s.B; ++b) {
+    SlotArgs& z = staged_args(h, 0)[b];
+    z.r_s = ev->r_s + static_cast<size_t>(b) * s.W;
+    z.wa = static_cast<const float*>(h->ev_wa.p) + static_cast<size_t>(b) * NF * s.A;
+    z.we = s.we_dynamic ? static_cast<const float*>(h->ev_we.p) + static_cast<size_t>(b) * NF * s.E : ev->we + static_cast<size_t>(b) * s.E;
+    z.x0 = ev->x + static_cast<size_t>(b) * s.L * s.W;
+    z.ctx = const_cast<float*>(ev->prev_x) + static_cast<size_t>(b) * s.P * s.W;
+    z.T_wa = NF; z.T_we = s.we_dynamic ? NF : 1; z.win_start = s.P; z.first_window = 0;
+    z.a_scale = ev->a_cfg_scale; z.r_scale = ev->r_cfg_scale; z.e_scale = ev->e_cfg_scale;
+  }
+  FMT_OK(upload_slot_records(h, 1, st));
+  FMT_OK(set_wargs(h, WindowArgs{device_args(h, 0)}, st));
   switch (h->plan.mode) {
     case FMT_MODE_BF16: return enqueue_velocity<bf16>(h, ev, st);
     case FMT_MODE_BF16X3: return enqueue_velocity<bf16x3_t>(h, ev, st);
@@ -2184,23 +2230,22 @@ static StageArgs stage_args(const FmtDebugStage* d) {
   return a;
 }
 
-// One device buffer: a copy of `head` (WinParams, whose `wargs` field is set here), then the WindowArgs of a COMB stage and its
-// per-clip SlotArgs; *wargs points at the WindowArgs
+// One device buffer: a copy of `head` (WinParams, whose `wargs` field is set here), then the WindowArgs and the SlotArgs of every
+// clip, with its guidance (slot_branches / slot_scales, else n_branches and a/r/e_scale); *wargs points at the WindowArgs
 static int stage_upload(const FmtDebugStage* d, WinParams* head, cudaStream_t st, void** buf, const WindowArgs** wargs) {
   const size_t head_bytes = head ? sizeof(WinParams) : 0;
   const size_t off = (head_bytes + 255) / 256 * 256;
   std::vector<unsigned char> host(off + sizeof(WindowArgs) + static_cast<size_t>(d->batch) * sizeof(SlotArgs), 0);
   CUDA_OK(cudaMallocAsync(buf, host.size(), st));
-  WindowArgs wa{};
-  wa.a_scale = d->a_scale; wa.r_scale = d->r_scale; wa.e_scale = d->e_scale;
-  if (d->kind == FMT_STAGE_COMB && d->slot_branches) {
-    SlotArgs* sl = reinterpret_cast<SlotArgs*>(host.data() + off + sizeof(WindowArgs));
-    for (int b = 0; b < d->batch; ++b) {
-      sl[b].n_branches = d->slot_branches[b];
-      sl[b].a_scale = d->slot_scales[3 * b]; sl[b].r_scale = d->slot_scales[3 * b + 1]; sl[b].e_scale = d->slot_scales[3 * b + 2];
-    }
-    wa.slots = reinterpret_cast<const SlotArgs*>(static_cast<unsigned char*>(*buf) + off + sizeof(WindowArgs));
+  SlotArgs* sl = reinterpret_cast<SlotArgs*>(host.data() + off + sizeof(WindowArgs));
+  for (int b = 0; b < d->batch; ++b) {
+    const bool own = d->slot_branches != nullptr;
+    sl[b].n_branches = own ? d->slot_branches[b] : d->n_branches;
+    sl[b].a_scale = own ? d->slot_scales[3 * b] : d->a_scale;
+    sl[b].r_scale = own ? d->slot_scales[3 * b + 1] : d->r_scale;
+    sl[b].e_scale = own ? d->slot_scales[3 * b + 2] : d->e_scale;
   }
+  const WindowArgs wa{reinterpret_cast<const SlotArgs*>(static_cast<unsigned char*>(*buf) + off + sizeof(WindowArgs))};
   memcpy(host.data() + off, &wa, sizeof(WindowArgs));
   *wargs = reinterpret_cast<const WindowArgs*>(static_cast<unsigned char*>(*buf) + off);
   if (head) {

@@ -9,8 +9,9 @@
 
 namespace fmt {
 
-// What one batch slot computes in one window of fmt_sample_clips or fmt_sample_windows: a window of its own clip (tensors of that
-// clip alone, batch 1).
+// What one batch slot computes in one window: a window of its own clip (tensors of that clip alone, batch 1).  Every sampling entry
+// point describes its windows this way: fmt_sample_clip's batch row b is slot b, fmt_velocity's clip b reads its explicit context
+// through ctx and its [prev | current] conditions from win_start = P.
 // An idle slot points at zeros, has r_d == nullptr and first_window == 1: it is computed and its output is dropped.
 struct SlotArgs {
   const float* r_s;        // (W)
@@ -48,20 +49,7 @@ __host__ __device__ __forceinline__ int slot_branch0(int s_nb, int nb) { return 
 
 // Per-window arguments, written to device memory by set_window_args so that the captured graph never changes.
 struct WindowArgs {
-  const float* r_s;        // (B, W)
-  const float* wa;         // (B, T_wa, A)
-  const float* we;         // (B, T_we, E)
-  const float* x0;         // (B, L, W) noise of this window (or the explicit x of fmt_velocity)
-  float* r_d;              // (B, T_out, W)
-  const float* prev_x_ext; // explicit context (fmt_velocity) or nullptr = use the chained device state
-  const float* prev_wa_ext;
-  const float* prev_we_ext;
-  int T_wa, T_we, T_out;
-  int win_start;           // first frame of this window in the clip
-  int first_window;        // 1: context is all-zero (nodes_adv.py:591-593)
-  int use_ext;             // 1: prev_* come from the *_ext pointers
-  float a_scale, r_scale, e_scale;
-  const SlotArgs* slots;   // (B) per-slot clip arguments (fmt_sample_clips): replace r_s .. first_window above; nullptr elsewhere
+  const SlotArgs* slots;   // (B) this window's slot records
 };
 
 struct ModelShape {
@@ -89,7 +77,6 @@ template <typename AT>
 __global__ void cond_gather_kernel(const WindowArgs* __restrict__ wargs, ModelShape s, const int* __restrict__ uidx, AT* __restrict__ cond) {
   pdl_launch_dependents();
   pdl_wait_prior_grid();
-  const WindowArgs a = *wargs;
   const int rows = s.nb * s.B * s.N;
   // uidx != nullptr: block u builds the u-th DISTINCT condition row, the one token row uidx[u] sees (fmt_configure)
   const int row = uidx != nullptr ? uidx[blockIdx.x] : blockIdx.x;
@@ -97,40 +84,23 @@ __global__ void cond_gather_kernel(const WindowArgs* __restrict__ wargs, ModelSh
   const int br = row / (s.B * s.N), b = (row / s.N) % s.B, f = row % s.N;
   const bool za = (s.null_a >> br) & 1, zr = (s.null_r >> br) & 1, ze = (s.null_e >> br) & 1;
   const bool ctx = f < s.P;
-  // the clip this row belongs to: clip b of the batch, or the clip that slot b runs (fmt_sample_clips; its tensors have batch 1)
-  const float *r_s = a.r_s, *wa = a.wa, *we = a.we;
-  int cb = b, T_wa = a.T_wa, T_we = a.T_we, win_start = a.win_start, first_window = a.first_window;
-  if (a.slots != nullptr) {
-    const SlotArgs& sl = a.slots[b];
-    r_s = sl.r_s; wa = sl.wa; we = sl.we; cb = 0;
-    T_wa = sl.T_wa; T_we = sl.T_we; win_start = sl.win_start; first_window = sl.first_window;
-  }
+  const SlotArgs& sl = wargs->slots[b];   // the clip that slot b runs
   // frame of the clip this row looks at; replicate padding == clamp to the last available frame
-  const int g = win_start + f - s.P;
+  const int g = sl.win_start + f - s.P;
   AT* out = cond + static_cast<size_t>(blockIdx.x) * s.Kc;
   for (int j = threadIdx.x; j < s.Kc; j += blockDim.x) {
     float v = 0.f;
     if (j < s.W) {
-      v = zr ? 0.f : r_s[static_cast<size_t>(cb) * s.W + j];
+      v = zr ? 0.f : sl.r_s[j];
     } else if (j < s.W + s.A) {
       const int k = j - s.W;
-      if (ctx) {   // prev_wa is replicated un-nulled in every branch (FMT.py:366,388)
-        if (a.use_ext) v = a.prev_wa_ext[(static_cast<size_t>(b) * s.P + f) * s.A + k];
-        else if (!first_window) v = wa[(static_cast<size_t>(cb) * T_wa + min(g, T_wa - 1)) * s.A + k];
-      } else if (!za) {
-        v = wa[(static_cast<size_t>(cb) * T_wa + min(g, T_wa - 1)) * s.A + k];
-      }
+      // prev_wa is replicated un-nulled in every branch (FMT.py:366,388)
+      if (ctx ? !sl.first_window : !za) v = sl.wa[static_cast<size_t>(min(g, sl.T_wa - 1)) * s.A + k];
     } else if (j < s.W + s.A + s.E) {
       const int k = j - s.W - s.A;
       if (!ze) {
-        if (!s.we_dynamic) {
-          v = we[static_cast<size_t>(cb) * s.E + k];     // static emotion covers the context frames too (FMT.py:325-326)
-        } else if (ctx) {
-          if (a.use_ext) v = a.prev_we_ext[(static_cast<size_t>(b) * s.P + f) * s.E + k];
-          else if (!first_window) v = we[(static_cast<size_t>(cb) * T_we + min(g, T_we - 1)) * s.E + k];
-        } else {
-          v = we[(static_cast<size_t>(cb) * T_we + min(g, T_we - 1)) * s.E + k];
-        }
+        if (!s.we_dynamic) v = sl.we[k];     // static emotion covers the context frames too (FMT.py:325-326)
+        else if (!ctx || !sl.first_window) v = sl.we[static_cast<size_t>(min(g, sl.T_we - 1)) * s.E + k];
       }
     }
     store_act(out + j, v);
@@ -187,27 +157,6 @@ __global__ void silu_cond_kernel(const float* __restrict__ c_emb, const float* _
   float v[4];
   silu_add4(c, t, v);
   VecIO<AT, 4>::store(out + i, v);
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// x-embedder input: rows [prev_x | y] replicated over the CFG branches (FMT.py:312,363-365)
-// ---------------------------------------------------------------------------------------------------------------
-template <typename AT>
-__global__ void pack_x_kernel(const WindowArgs* __restrict__ wargs, ModelShape s, const float* __restrict__ y /* (B,L,W) */,
-                              const float* __restrict__ prev_x_state /* (B,P,W) */, AT* __restrict__ ax) {
-  pdl_launch_dependents();
-  pdl_wait_prior_grid();
-  const WindowArgs a = *wargs;
-  const int row = blockIdx.x;   // b*N + f
-  const int b = row / s.N, f = row % s.N;
-  const float* src;
-  if (f < s.P) src = a.use_ext ? a.prev_x_ext + (static_cast<size_t>(b) * s.P + f) * s.W : prev_x_state + (static_cast<size_t>(b) * s.P + f) * s.W;
-  else src = y + (static_cast<size_t>(b) * s.L + (f - s.P)) * s.W;
-  for (int j = threadIdx.x * 4; j < s.W; j += blockDim.x * 4) {
-    const float4 t = *reinterpret_cast<const float4*>(src + j);
-    float v[4] = {t.x, t.y, t.z, t.w};
-    for (int br = 0; br < s.nb; ++br) VecIO<AT, 4>::store(ax + (static_cast<size_t>(br) * s.B * s.N + row) * s.W + j, v);
-  }
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -499,10 +448,9 @@ __device__ __forceinline__ float cfg_combine(const float* __restrict__ V, size_t
   return tu + r * (u - tu) + a * (ao - u) + e * (c - ao);
 }
 
-// The same selection for the persistent kernels' COMB, which hold the plan's branches in vb[0..3]: with per-slot records, the
-// scales and branch count of the clip in slot b, and vb shifted so that vb[0] is its first branch (constant register indices).
+// The same selection for the persistent kernels' COMB, which hold the plan's branches in vb[0..3]: the scales and branch count of
+// the clip in slot b, and vb shifted so that vb[0] is its first branch (constant register indices).
 __device__ __forceinline__ void slot_guidance(const SlotArgs* slots, int s_nb, int b, float (&vb)[4], int& nb, float& a, float& r, float& e) {
-  if (slots == nullptr) return;
   const SlotArgs& sl = slots[b];
   nb = __ldg(&sl.n_branches);
   a = __ldg(&sl.a_scale); r = __ldg(&sl.r_scale); e = __ldg(&sl.e_scale);
@@ -547,22 +495,15 @@ __global__ void cfg_combine_kernel(const WindowArgs* __restrict__ wargs, ModelSh
                                    float* __restrict__ dst, const float* __restrict__ dt_ptr, AT* __restrict__ ax) {
   pdl_launch_dependents();
   pdl_wait_prior_grid();
-  const WindowArgs a = *wargs;
   const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   const size_t per_branch = static_cast<size_t>(s.B) * s.N * s.W;
   if (i >= per_branch) return;
   const int j = static_cast<int>(i % s.W);
   const int f = static_cast<int>((i / s.W) % s.N), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.N));
   if (mode != 0 && f < s.P) return;
-  // per slot (fmt_sample_clips): the clip's own scales and branches; the combine expression below is the same either way
-  int nb = s.nb, br0 = 0;
-  float as = a.a_scale, rs = a.r_scale, es = a.e_scale;
-  if (a.slots != nullptr) {
-    const SlotArgs& sl = a.slots[b];
-    nb = sl.n_branches; br0 = slot_branch0(s.nb, nb);
-    as = sl.a_scale; rs = sl.r_scale; es = sl.e_scale;
-  }
-  const float v = cfg_combine(V, i + br0 * per_branch, per_branch, nb, as, rs, es);
+  const SlotArgs& sl = wargs->slots[b];   // the clip's own scales and branches
+  const int nb = sl.n_branches;
+  const float v = cfg_combine(V, i + slot_branch0(s.nb, nb) * per_branch, per_branch, nb, sl.a_scale, sl.r_scale, sl.e_scale);
   if (mode == 0) dst[i] = v;
   else {
     const size_t o = (static_cast<size_t>(b) * s.L + (f - s.P)) * s.W + j;
@@ -591,56 +532,47 @@ __global__ void rk_combine_kernel(ModelShape s, const float* __restrict__ y0, fl
   store_ax<AT>(s, ax, b, s.P + f, j, y);
 }
 
-// Window prologue: x_state <- x0, context rows <- prev_x or a stream's ctx (zero in the first window, nodes_adv.py:591), ax <- [prev_x | x0]
+// Window prologue: x_state <- the slot's x0, context rows <- prev_x or the slot's own ctx (zero in the first window,
+// nodes_adv.py:591), ax <- [context | x0]
 template <typename AT>
 __global__ void init_window_kernel(const WindowArgs* __restrict__ wargs, ModelShape s, float* __restrict__ x_state,
                                    float* __restrict__ prev_x_state, AT* __restrict__ ax) {
   pdl_launch_dependents();
   pdl_wait_prior_grid();
-  const WindowArgs a = *wargs;
   const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<size_t>(s.B) * s.N * s.W) return;
   const int j = static_cast<int>(i % s.W), f = static_cast<int>((i / s.W) % s.N), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.N));
-  // per slot (fmt_sample_clips / fmt_sample_windows): the slot's own noise (L, W), context reset and, for a stream, its own context
-  const float* x0 = a.x0;
-  const float* ctx = nullptr;
-  int cb = b, first_window = a.first_window;
-  if (a.slots != nullptr) { x0 = a.slots[b].x0; first_window = a.slots[b].first_window; ctx = a.slots[b].ctx; cb = 0; }
+  const SlotArgs& sl = wargs->slots[b];
   float v;
   if (f < s.P) {
     const size_t o = (static_cast<size_t>(b) * s.P + f) * s.W + j;
-    if (first_window) { v = 0.f; prev_x_state[o] = 0.f; }
-    else if (ctx != nullptr) v = ctx[static_cast<size_t>(f) * s.W + j];
+    if (sl.first_window) { v = 0.f; prev_x_state[o] = 0.f; }
+    else if (sl.ctx != nullptr) v = sl.ctx[static_cast<size_t>(f) * s.W + j];
     else v = prev_x_state[o];
   } else {
     const size_t o = (static_cast<size_t>(b) * s.L + (f - s.P)) * s.W + j;
-    v = x0[(static_cast<size_t>(cb) * s.L + (f - s.P)) * s.W + j];
+    v = sl.x0[static_cast<size_t>(f - s.P) * s.W + j];
     x_state[o] = v;
   }
   store_ax<AT>(s, ax, b, f, j, v);
 }
-// Window epilogue: r_d[:, window] <- x_state, prev_x (and a stream's ctx) <- last P frames (nodes_adv.py:659-668,690-692)
+// Window epilogue: the slot's r_d[out_start + f] <- x_state for the frames below its T_out (an idle slot writes nothing), prev_x
+// (and the slot's ctx) <- last P frames (nodes_adv.py:659-668,690-692)
 __global__ void finalize_window_kernel(const WindowArgs* __restrict__ wargs, ModelShape s, const float* __restrict__ x_state,
                                        float* __restrict__ prev_x_state) {
   pdl_launch_dependents();
   pdl_wait_prior_grid();
-  const WindowArgs a = *wargs;
   const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<size_t>(s.B) * s.L * s.W) return;
   const int j = static_cast<int>(i % s.W), f = static_cast<int>((i / s.W) % s.L), b = static_cast<int>(i / (static_cast<size_t>(s.W) * s.L));
   const float v = x_state[i];
-  // per slot (fmt_sample_clips / fmt_sample_windows): frames below the slot's own clip length, into that clip's output; idle slots
-  // write nothing
-  float* r_d = a.r_d;
-  float* ctx = nullptr;
-  int cb = b, T_out = a.T_out, out_start = a.win_start;
-  if (a.slots != nullptr) { const SlotArgs& sl = a.slots[b]; r_d = sl.r_d; T_out = sl.T_out; out_start = sl.out_start; ctx = sl.ctx; cb = 0; }
-  const int g = out_start + f;
-  if (r_d != nullptr && g < T_out) r_d[(static_cast<size_t>(cb) * T_out + g) * s.W + j] = v;
+  const SlotArgs& sl = wargs->slots[b];
+  const int g = sl.out_start + f;
+  if (sl.r_d != nullptr && g < sl.T_out) sl.r_d[static_cast<size_t>(g) * s.W + j] = v;
   if (f >= s.L - s.P) {
     const int c = f - (s.L - s.P);
     prev_x_state[(static_cast<size_t>(b) * s.P + c) * s.W + j] = v;
-    if (ctx != nullptr) ctx[static_cast<size_t>(c) * s.W + j] = v;
+    if (sl.ctx != nullptr) sl.ctx[static_cast<size_t>(c) * s.W + j] = v;
   }
 }
 

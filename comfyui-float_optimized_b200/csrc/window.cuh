@@ -869,9 +869,9 @@ __device__ __forceinline__ void win_comb_stage(const WinParams& p, const WinCtx&
       if (br < s.nb) vb[br] = __ldcg(p.Vacc + br * per_branch + i);
     const float bd = __ldg(p.b_dec + j);
     const float dt = __ldg(p.ddt + step);
-    float a_s = __ldg(&p.wargs->a_scale), r_s = __ldg(&p.wargs->r_scale), e_s = __ldg(&p.wargs->e_scale);
     const SlotArgs* const slots = p.wargs->slots;
-    int nb = s.nb;
+    float a_s, r_s, e_s;
+    int nb;
     const float y0 = cur ? __ldcg(p.x_state + o) : 0.f;
     float kprev[4] = {0.f, 0.f, 0.f, 0.f};
     if (G > 1 && cur) {
