@@ -112,6 +112,10 @@ _SIGNATURES = {
     "fmt_sample_windows": (C.c_int32, [C.c_void_p, C.POINTER(FmtWindowSet), C.POINTER(FmtClipGuidance), C.c_void_p]),
     "fmt_sample_clips_ode": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.POINTER(FmtClipGuidance), C.POINTER(FmtClipOde), C.c_void_p]),
     "fmt_sample_windows_ode": (C.c_int32, [C.c_void_p, C.POINTER(FmtWindowSet), C.POINTER(FmtClipGuidance), C.POINTER(FmtClipOde), C.c_void_p]),
+    "fmt_sample_clip_set": (C.c_int32, [C.c_void_p, C.POINTER(FmtClipSet), C.POINTER(FmtClipGuidance), C.POINTER(FmtClipOde),
+                                        C.POINTER(C.c_int32), C.c_void_p]),
+    "fmt_sample_window_set": (C.c_int32, [C.c_void_p, C.POINTER(FmtWindowSet), C.POINTER(FmtClipGuidance), C.POINTER(FmtClipOde),
+                                          C.POINTER(C.c_int32), C.c_void_p]),
     "fmt_clip_schedule": (C.c_int32, [C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32)]),
     "fmt_velocity": (C.c_int32, [C.c_void_p, C.POINTER(FmtEval), C.c_void_p]),
@@ -122,6 +126,7 @@ _SIGNATURES = {
     "fmt_debug_window_trace": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int64]),
     "fmt_debug_condition_rows": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "fmt_debug_condition_rows_ode": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "fmt_debug_condition_rows_slots": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.c_void_p]),
     "fmt_proj_create": (C.c_int32, [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int32, C.c_int32,
                                     C.POINTER(C.c_void_p)]),
     "fmt_proj_destroy": (C.c_int32, [C.c_void_p]),

@@ -1231,10 +1231,14 @@ int32_t fmt_window_kernel_status(const FmtHandle* h) {
 // Which token rows (branch, clip, frame) see the same condition row [wr | wa | we]?  urow[row] = index of the row's distinct
 // condition row, uidx[u] = the first token row that sees distinct row u.  The key is exactly what cond_gather_kernel reads for a
 // row: the identity latent unless nulled (per clip), the audio latent (context frames read prev_wa, never nulled, FMT.py:366,388;
-// current frames read wa unless nulled), the emotion (nulled; static = per clip, covering the context frames too, FMT.py:325-326;
-// dynamic = per frame).  per_slot: rows of different slots are never shared (the per-slot window graph, whose slots have their own
-// times): only the truly-uncond current frames of 4-branch plans, [0 | 0 | 0] in every slot, are affected.
-static void distinct_condition_rows(const ModelShape& s, std::vector<int>& urow, std::vector<int>& uidx, bool per_slot = false) {
+// current frames read wa unless nulled), the emotion (nulled; else slot b's mode we_dyn[b]: static = per clip, covering the context
+// frames too, FMT.py:325-326; dynamic = per frame).  per_slot: rows of different slots are never shared (the per-slot window graph,
+// whose slots have their own times): only the truly-uncond current frames of 4-branch plans, [0 | 0 | 0] in every slot, are affected.
+// The map does not depend on we_dyn: in every branch that keeps the emotion (branch_nulls) the audio term is kept too or is a context
+// frame's prev_wa, and both are keyed by (clip, frame) already.  So one map serves every mix of static and dynamic slots, and a call
+// that mixes them replays the graphs of the plan (fmt_debug_condition_rows_slots shows the map for any mix).
+static void distinct_condition_rows(const ModelShape& s, const int32_t* we_dyn, std::vector<int>& urow, std::vector<int>& uidx,
+                                    bool per_slot = false) {
   const int R = s.nb * s.B * s.N;
   urow.assign(R, 0);
   uidx.clear();
@@ -1244,7 +1248,7 @@ static void distinct_condition_rows(const ModelShape& s, std::vector<int>& urow,
     const bool za = (s.null_a >> br) & 1, zr = (s.null_r >> br) & 1, ze = (s.null_e >> br) & 1, ctx = f < s.P;
     const int kr = zr ? -1 : b;
     const int ka = ctx ? 0 : (za ? 1 : 2), kab = (ctx || !za) ? b : -1, kaf = (ctx || !za) ? f : -1;
-    const int ke = ze ? 0 : (s.we_dynamic ? 2 : 1), keb = ze ? -1 : b, kef = (!ze && s.we_dynamic) ? f : -1;
+    const int ke = ze ? 0 : (we_dyn[b] ? 2 : 1), keb = ze ? -1 : b, kef = (!ze && we_dyn[b]) ? f : -1;
     const auto key = std::make_tuple(kr, ka, kab, kaf, ke, keb, kef, per_slot ? b : -1);
     auto it = seen.find(key);
     if (it == seen.end()) { it = seen.emplace(key, static_cast<int>(uidx.size())).first; uidx.push_back(row); }
@@ -1265,12 +1269,19 @@ int32_t fmt_debug_condition_rows(int32_t n_branches, int32_t batch, int32_t n_fr
 
 int32_t fmt_debug_condition_rows_ode(int32_t n_branches, int32_t batch, int32_t n_frames, int32_t n_prev, int32_t we_dynamic, int32_t per_slot,
                                      int32_t* urow_out) {
-  if (n_branches < 1 || n_branches > 4 || batch < 1 || n_frames < 1 || n_prev < 0 || n_prev > n_frames) return -1;
+  if (batch < 1) return -1;
+  const std::vector<int32_t> modes(batch, we_dynamic);
+  return fmt_debug_condition_rows_slots(n_branches, batch, n_frames, n_prev, modes.data(), per_slot, urow_out);
+}
+
+int32_t fmt_debug_condition_rows_slots(int32_t n_branches, int32_t batch, int32_t n_frames, int32_t n_prev, const int32_t* we_dynamic,
+                                       int32_t per_slot, int32_t* urow_out) {
+  if (n_branches < 1 || n_branches > 4 || batch < 1 || n_frames < 1 || n_prev < 0 || n_prev > n_frames || we_dynamic == nullptr) return -1;
   ModelShape s{};
-  s.nb = n_branches; s.B = batch; s.N = n_frames; s.P = n_prev; s.we_dynamic = we_dynamic;
+  s.nb = n_branches; s.B = batch; s.N = n_frames; s.P = n_prev;
   branch_nulls(s);
   std::vector<int> urow, uidx;
-  distinct_condition_rows(s, urow, uidx, per_slot != 0);
+  distinct_condition_rows(s, we_dynamic, urow, uidx, per_slot != 0);
   if (urow_out != nullptr) std::copy(urow.begin(), urow.end(), urow_out);
   return static_cast<int32_t>(uidx.size());
 }
@@ -1321,10 +1332,12 @@ int32_t fmt_clip_schedule(int32_t n_clips, const int32_t* n_windows, int32_t n_s
   return S;
 }
 
+// we_dynamic takes no part: no graph, table or buffer depends on it (each slot record carries its clip's emotion mode, and the
+// condition-row map is the same for every mode, distinct_condition_rows), so a plan that differs only in it is the same plan.
 static bool same_plan(const FmtHandle* h, const FmtPlan* p) {
   if (!h->configured) return false;
   const FmtPlan& q = h->plan;
-  if (q.batch != p->batch || q.n_branches != p->n_branches || q.we_dynamic != p->we_dynamic || q.mode != p->mode ||
+  if (q.batch != p->batch || q.n_branches != p->n_branches || q.mode != p->mode ||
       q.n_steps != p->n_steps || q.n_stages != p->n_stages)
     return false;
   const int ne = p->n_steps * p->n_stages;
@@ -1345,7 +1358,10 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
   REQUIRE(p->n_steps >= 0 && p->n_stages >= 1 && p->n_stages <= FMT_MAX_STAGES, "fmt_configure: bad n_steps/n_stages");
   REQUIRE(p->rk_a && p->rk_b && (p->n_steps == 0 || (p->t_eval && p->dt)), "fmt_configure: null schedule arrays");
   h->last_ode = false;
-  if (same_plan(h, p)) return 0;
+  if (same_plan(h, p)) {
+    h->plan.we_dynamic = p->we_dynamic;    // the mode fmt_sample_clip, fmt_velocity and the calls without per-clip modes give every clip
+    return 0;
+  }
   if (p->mode == FMT_MODE_BF16X3) {
     FMT_OK(pack_split_all(h, st));
     CUDA_OK(cudaStreamSynchronize(st));
@@ -1366,7 +1382,7 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
 
   ModelShape& s = h->shape;
   s.B = p->batch; s.nb = p->n_branches; s.N = h->N; s.P = d.num_prev_frames; s.L = d.frames_per_clip;
-  s.W = d.dim_w; s.A = d.dim_a; s.E = d.dim_e; s.H = d.dim_h; s.Kc = h->Kc; s.we_dynamic = p->we_dynamic;
+  s.W = d.dim_w; s.A = d.dim_a; s.E = d.dim_e; s.H = d.dim_h; s.Kc = h->Kc;
   branch_nulls(s);
   h->R = s.nb * s.B * s.N;
   h->U = h->R;
@@ -1381,7 +1397,8 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
     const bool old_window_plan = h->use_window != 0 && window_eligible(h, p) && !(h->use_window == 3 && flow_eligible(h, p));
     if (h->use_dedup && s.nb > 1 && !old_window_plan) {
       std::vector<int> urow, uidx;
-      distinct_condition_rows(s, urow, uidx);
+      const std::vector<int32_t> modes(s.B, p->we_dynamic);
+      distinct_condition_rows(s, modes.data(), urow, uidx);
       if (static_cast<int>(uidx.size()) < h->R) {
         h->U = static_cast<int>(uidx.size());
         h->dedup = true;
@@ -1496,7 +1513,7 @@ static int set_wargs(FmtHandle* h, const WindowArgs& a, cudaStream_t st) {
 // Slot records of one call (every sampling entry point and fmt_velocity) go up in ONE copy from a pinned staging buffer that the handle
 // owns; slot_ev marks the end of the previous call's copy, so the staging buffer is refilled only once that copy has read it.
 // stage_slot_records fills the staging buffer with n_win windows of idle records: zero inputs ((L, W) noise, and r_s / wa / we rows
-// no wider than that), no output, no context, scales of 1 and the plan's branch count; with ode, B SlotOde follow the B SlotArgs of
+// no wider than that), no output, no context, static emotion, scales of 1 and the plan's branch count; with ode, B SlotOde follow the B SlotArgs of
 // each window, idle as well (no evaluation).
 static int stage_slot_records(FmtHandle* h, size_t n_win, bool ode, cudaStream_t st) {
   const ModelShape& s = h->shape;
@@ -1520,7 +1537,7 @@ static int stage_slot_records(FmtHandle* h, size_t n_win, bool ode, cudaStream_t
       SlotArgs& z = rec[k];
       z.r_s = zero; z.wa = zero; z.we = zero; z.x0 = zero; z.r_d = nullptr; z.ctx = nullptr;
       z.T_wa = 1; z.T_we = 1; z.T_out = 0; z.win_start = 0; z.out_start = 0; z.first_window = 1;
-      z.a_scale = z.r_scale = z.e_scale = 1.f; z.n_branches = s.nb;
+      z.a_scale = z.r_scale = z.e_scale = 1.f; z.n_branches = s.nb; z.we_dynamic = 0;
     }
     if (!ode) continue;
     SlotOde* od = reinterpret_cast<SlotOde*>(rec + s.B);
@@ -1616,7 +1633,8 @@ static int ensure_ode_graph(FmtHandle* h, cudaStream_t st) {
   h->s_dedup = false;
   if (h->use_dedup && s.nb > 1) {
     std::vector<int> urow, uidx;
-    distinct_condition_rows(s, urow, uidx, true);
+    const std::vector<int32_t> modes(s.B, h->plan.we_dynamic);
+    distinct_condition_rows(s, modes.data(), urow, uidx, true);
     if (static_cast<int>(uidx.size()) < h->R) {
       h->sU = static_cast<int>(uidx.size());
       h->s_dedup = true;
@@ -1647,19 +1665,22 @@ struct ClipIn {
   int T_wa, T_we, T;
   float a_scale, r_scale, e_scale;
   int n_branches;
+  int we_dynamic;
 };
 
-// The rules every clip of fmt_sample_clip / fmt_sample_clips follows; `who` names it in the error.  *n_win: its window count.
+// The rules every clip of fmt_sample_clip / fmt_sample_clips follows, those of its own emotion mode among them; `who` names it in the
+// error.  *n_win: its window count.
 static int check_clip(const ModelShape& s, const ClipIn& c, const char* who, int32_t* n_win) {
   const int nb = c.n_branches;
   REQUIRE((nb == 1 || nb == 3 || nb == 4) && nb <= s.nb, "%s: n_branches=%d must be 1, 3 or 4 and fit the plan's %d branches", who, nb, s.nb);
   REQUIRE(c.r_s && c.wa && c.we && c.noise && c.r_d, "%s: null tensor pointer", who);
   REQUIRE(c.T >= 1 && c.T_wa >= 1 && c.T_we >= 1, "%s: empty clip", who);
-  REQUIRE(s.we_dynamic ? c.T_we > 1 : c.T_we == 1, "%s: T_we=%d does not match plan.we_dynamic=%d", who, c.T_we, s.we_dynamic);
+  REQUIRE(c.we_dynamic == 0 || c.we_dynamic == 1, "%s: we_dynamic=%d must be 0 or 1", who, c.we_dynamic);
+  REQUIRE(c.we_dynamic ? c.T_we > 1 : c.T_we == 1, "%s: T_we=%d does not match we_dynamic=%d", who, c.T_we, c.we_dynamic);
   const int n = (c.T + s.L - 1) / s.L;
   // every window must see at least one real wa (and dynamic we) frame; the reference's F.pad(replicate) fails otherwise
   REQUIRE((n - 1) * s.L < c.T_wa, "%s: wa has %d frames but window %d starts at frame %d", who, c.T_wa, n - 1, (n - 1) * s.L);
-  REQUIRE(!s.we_dynamic || (n - 1) * s.L < c.T_we, "%s: dynamic we has %d frames but the last window starts at %d", who, c.T_we, (n - 1) * s.L);
+  REQUIRE(!c.we_dynamic || (n - 1) * s.L < c.T_we, "%s: dynamic we has %d frames but the last window starts at %d", who, c.T_we, (n - 1) * s.L);
   *n_win = n;
   return 0;
 }
@@ -1680,6 +1701,7 @@ static int stage_clips(FmtHandle* h, const std::vector<ClipIn>& c, const int32_t
       z.T_wa = c[i].T_wa; z.T_we = c[i].T_we; z.T_out = c[i].T;
       z.win_start = z.out_start = w * s.L; z.first_window = (w == 0);
       z.a_scale = c[i].a_scale; z.r_scale = c[i].r_scale; z.e_scale = c[i].e_scale; z.n_branches = c[i].n_branches;
+      z.we_dynamic = c[i].we_dynamic;
     }
   }
   return 0;
@@ -1704,7 +1726,8 @@ int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_OK(cudaSetDevice(h->device));
   const ModelShape& s = h->shape;
-  ClipIn in{c->r_s, c->wa, c->we, c->noise, c->r_d, 0, c->T_wa, c->T_we, c->audio_num_frames, c->a_cfg_scale, c->r_cfg_scale, c->e_cfg_scale, s.nb};
+  ClipIn in{c->r_s, c->wa, c->we, c->noise, c->r_d, 0, c->T_wa, c->T_we, c->audio_num_frames, c->a_cfg_scale, c->r_cfg_scale, c->e_cfg_scale, s.nb,
+             h->plan.we_dynamic};
   int32_t n_win = 0;
   FMT_OK(check_clip(s, in, "fmt_sample_clip", &n_win));
   const int T = in.T;
@@ -1744,17 +1767,17 @@ int32_t fmt_sample_clip(FmtHandle* h, const FmtClip* c, void* stream) {
   return 0;
 }
 
-}  // extern "C"
-
 // Many clips on plan.batch slots: window w of the call runs, in slot k, whichever clip the schedule put there (at that clip's own
 // window), through the same captured window graph (ode != nullptr: each clip on its own schedule, through the per-slot window graph).
-static int sample_clips(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, const FmtClipOde* ode, void* stream) {
-  REQUIRE(h && cs && g, "fmt_sample_clips_guided: null argument");
+// g == nullptr: the set's scales and the plan's branch count for every clip; we_dyn == nullptr: plan.we_dynamic for every clip.
+int32_t fmt_sample_clip_set(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, const FmtClipOde* ode, const int32_t* we_dyn,
+                            void* stream) {
+  REQUIRE(h && cs, "fmt_sample_clips: null argument");
   REQUIRE(h->configured, "fmt_sample_clips: call fmt_configure first");
   const int n = cs->n_clips;
   REQUIRE(n >= 1, "fmt_sample_clips: no clips");
   REQUIRE(cs->r_s && cs->wa && cs->we && cs->noise && cs->r_d && cs->T_wa && cs->T_we && cs->audio_num_frames, "fmt_sample_clips: null array");
-  REQUIRE(g->a_cfg_scale && g->r_cfg_scale && g->e_cfg_scale && g->n_branches, "fmt_sample_clips_guided: null guidance array");
+  REQUIRE(!g || (g->a_cfg_scale && g->r_cfg_scale && g->e_cfg_scale && g->n_branches), "fmt_sample_clips_guided: null guidance array");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_OK(cudaSetDevice(h->device));
   const ModelShape& s = h->shape;
@@ -1762,7 +1785,8 @@ static int sample_clips(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidanc
   std::vector<int32_t> n_win(n), slot(n), start(n);
   for (int i = 0; i < n; ++i) {
     c[i] = ClipIn{cs->r_s[i], cs->wa[i], cs->we[i], cs->noise[i], cs->r_d[i], static_cast<size_t>(s.L) * s.W, cs->T_wa[i], cs->T_we[i],
-                  cs->audio_num_frames[i], g->a_cfg_scale[i], g->r_cfg_scale[i], g->e_cfg_scale[i], g->n_branches[i]};
+                  cs->audio_num_frames[i], g ? g->a_cfg_scale[i] : cs->a_cfg_scale, g ? g->r_cfg_scale[i] : cs->r_cfg_scale,
+                  g ? g->e_cfg_scale[i] : cs->e_cfg_scale, g ? g->n_branches[i] : s.nb, we_dyn ? we_dyn[i] : h->plan.we_dynamic};
     char who[48];
     snprintf(who, sizeof(who), "fmt_sample_clips: clip %d", i);
     FMT_OK(check_clip(s, c[i], who, &n_win[i]));
@@ -1779,34 +1803,25 @@ static int sample_clips(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidanc
   return replay_windows(h, makespan, ode != nullptr, cs->progress, cs->progress_user, st);
 }
 
-extern "C" {
+int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) { return fmt_sample_clip_set(h, cs, nullptr, nullptr, nullptr, stream); }
 
 int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, void* stream) {
-  return sample_clips(h, cs, g, nullptr, stream);
+  REQUIRE(g, "fmt_sample_clips_guided: null argument");
+  return fmt_sample_clip_set(h, cs, g, nullptr, nullptr, stream);
 }
 
 int32_t fmt_sample_clips_ode(FmtHandle* h, const FmtClipSet* cs, const FmtClipGuidance* g, const FmtClipOde* ode, void* stream) {
-  return sample_clips(h, cs, g, ode, stream);
+  REQUIRE(g, "fmt_sample_clips_guided: null argument");
+  return fmt_sample_clip_set(h, cs, g, ode, nullptr, stream);
 }
-
-// The set's shared scales and the plan's branch count for every clip
-int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* cs, void* stream) {
-  REQUIRE(h && cs, "fmt_sample_clips: null argument");
-  const int n = std::max(cs->n_clips, 0);
-  std::vector<float> a(n, cs->a_cfg_scale), r(n, cs->r_cfg_scale), e(n, cs->e_cfg_scale);
-  std::vector<int32_t> nb(n, h->shape.nb);
-  const FmtClipGuidance g{a.data(), r.data(), e.data(), nb.data()};
-  return fmt_sample_clips_guided(h, cs, &g, stream);
-}
-
-}  // extern "C"
 
 // One window of each of n streams, stream i in slot i, through the plan's captured window graph (ode != nullptr: each stream on its
 // own schedule, through the per-slot window graph); slots n.. are idle.  A stream's context lives in its own ctx buffer, not in the
 // handle, so a stream may run in any slot and the plan may be replaced between calls.  Its wa / we start at the window's first
 // context frame (P frames before its first current frame), or at its first current frame in a first window; its output is the
-// window alone.
-static int sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, const FmtClipOde* ode, void* stream) {
+// window alone.  we_dyn == nullptr: plan.we_dynamic for every stream.
+int32_t fmt_sample_window_set(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, const FmtClipOde* ode, const int32_t* we_dyn,
+                              void* stream) {
   REQUIRE(h && ws && g, "fmt_sample_windows: null argument");
   REQUIRE(h->configured, "fmt_sample_windows: call fmt_configure first");
   const ModelShape& s = h->shape;
@@ -1823,13 +1838,15 @@ static int sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGui
             "fmt_sample_windows: stream %d: n_branches=%d must be 1, 3 or 4 and fit the plan's %d branches", i, nb, s.nb);
     REQUIRE(ws->r_s[i] && ws->wa[i] && ws->we[i] && ws->x0[i] && ws->ctx[i] && ws->r_d[i], "fmt_sample_windows: stream %d: null tensor pointer", i);
     const int first = ws->first_window[i], T_wa = ws->T_wa[i], T_we = ws->T_we[i], n_out = ws->n_out[i];
+    const int dyn = we_dyn ? we_dyn[i] : h->plan.we_dynamic;
     REQUIRE(first == 0 || first == 1, "fmt_sample_windows: stream %d: first_window=%d must be 0 or 1", i, first);
     REQUIRE(n_out >= 1 && n_out <= s.L, "fmt_sample_windows: stream %d: n_out=%d outside [1, %d]", i, n_out, s.L);
-    REQUIRE(s.we_dynamic ? T_we >= 1 : T_we == 1, "fmt_sample_windows: stream %d: T_we=%d does not match plan.we_dynamic=%d", i, T_we, s.we_dynamic);
+    REQUIRE(dyn == 0 || dyn == 1, "fmt_sample_windows: stream %d: we_dynamic=%d must be 0 or 1", i, dyn);
+    REQUIRE(dyn ? T_we >= 1 : T_we == 1, "fmt_sample_windows: stream %d: T_we=%d does not match we_dynamic=%d", i, T_we, dyn);
     // the window's first current frame must be a real frame (the reference's F.pad(replicate) fails otherwise)
     const int cur = first ? 0 : s.P;
     REQUIRE(cur < T_wa, "fmt_sample_windows: stream %d: wa has %d frames but the window's first current frame is frame %d", i, T_wa, cur);
-    REQUIRE(!s.we_dynamic || cur < T_we, "fmt_sample_windows: stream %d: dynamic we has %d frames but the window's first current frame is frame %d",
+    REQUIRE(!dyn || cur < T_we, "fmt_sample_windows: stream %d: dynamic we has %d frames but the window's first current frame is frame %d",
             i, T_we, cur);
   }
   if (ode) FMT_OK(check_odes(h, ode, n, "fmt_sample_windows_ode: stream"));
@@ -1845,20 +1862,18 @@ static int sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGui
     z.first_window = ws->first_window[i];
     z.win_start = z.first_window ? 0 : s.P; z.out_start = 0;
     z.a_scale = g->a_cfg_scale[i]; z.r_scale = g->r_cfg_scale[i]; z.e_scale = g->e_cfg_scale[i]; z.n_branches = g->n_branches[i];
+    z.we_dynamic = we_dyn ? we_dyn[i] : h->plan.we_dynamic;
   }
   return replay_windows(h, 1, ode != nullptr, nullptr, nullptr, st);
 }
 
-extern "C" {
-
 int32_t fmt_sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, void* stream) {
-  return sample_windows(h, ws, g, nullptr, stream);
+  return fmt_sample_window_set(h, ws, g, nullptr, nullptr, stream);
 }
 
 int32_t fmt_sample_windows_ode(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, const FmtClipOde* ode, void* stream) {
-  return sample_windows(h, ws, g, ode, stream);
+  return fmt_sample_window_set(h, ws, g, ode, nullptr, stream);
 }
-
 
 }  // extern "C"
 
@@ -1895,7 +1910,7 @@ int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream) {
   REQUIRE(h->configured, "fmt_velocity: call fmt_configure first");
   REQUIRE(ev->eval_index >= 0 && ev->eval_index < h->n_eval, "fmt_velocity: eval_index %d out of range [0,%d)", ev->eval_index, h->n_eval);
   REQUIRE(ev->x && ev->prev_x && ev->wa && ev->prev_wa && ev->we && ev->r_s && ev->v_out, "fmt_velocity: null tensor pointer");
-  REQUIRE(!h->shape.we_dynamic || ev->prev_we, "fmt_velocity: dynamic we requires prev_we (FMT.py:306-307)");
+  REQUIRE(!h->plan.we_dynamic || ev->prev_we, "fmt_velocity: dynamic we requires prev_we (FMT.py:306-307)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CUDA_OK(cudaSetDevice(h->device));
   const ModelShape& s = h->shape;
@@ -1903,16 +1918,17 @@ int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream) {
   // would write it), and [prev | current] frames of its conditions, read from frame P on
   const int NF = s.P + s.L;
   FMT_OK(join_context(h, h->ev_wa, ev->prev_wa, ev->wa, s.A, st));
-  if (s.we_dynamic) FMT_OK(join_context(h, h->ev_we, ev->prev_we, ev->we, s.E, st));
+  const int dyn = h->plan.we_dynamic;
+  if (dyn) FMT_OK(join_context(h, h->ev_we, ev->prev_we, ev->we, s.E, st));
   FMT_OK(stage_slot_records(h, 1, false, st));
   for (int b = 0; b < s.B; ++b) {
     SlotArgs& z = staged_args(h, 0)[b];
     z.r_s = ev->r_s + static_cast<size_t>(b) * s.W;
     z.wa = static_cast<const float*>(h->ev_wa.p) + static_cast<size_t>(b) * NF * s.A;
-    z.we = s.we_dynamic ? static_cast<const float*>(h->ev_we.p) + static_cast<size_t>(b) * NF * s.E : ev->we + static_cast<size_t>(b) * s.E;
+    z.we = dyn ? static_cast<const float*>(h->ev_we.p) + static_cast<size_t>(b) * NF * s.E : ev->we + static_cast<size_t>(b) * s.E;
     z.x0 = ev->x + static_cast<size_t>(b) * s.L * s.W;
     z.ctx = const_cast<float*>(ev->prev_x) + static_cast<size_t>(b) * s.P * s.W;
-    z.T_wa = NF; z.T_we = s.we_dynamic ? NF : 1; z.win_start = s.P; z.first_window = 0;
+    z.T_wa = NF; z.T_we = dyn ? NF : 1; z.we_dynamic = dyn; z.win_start = s.P; z.first_window = 0;
     z.a_scale = ev->a_cfg_scale; z.r_scale = ev->r_cfg_scale; z.e_scale = ev->e_cfg_scale;
   }
   FMT_OK(upload_slot_records(h, 1, st));

@@ -12,7 +12,7 @@ namespace fmt {
 // What one batch slot computes in one window: a window of its own clip (tensors of that clip alone, batch 1).  Every sampling entry
 // point describes its windows this way: fmt_sample_clip's batch row b is slot b, fmt_velocity's clip b reads its explicit context
 // through ctx and its [prev | current] conditions from win_start = P.
-// An idle slot points at zeros, has r_d == nullptr and first_window == 1: it is computed and its output is dropped.
+// An idle slot points at zeros, has r_d == nullptr, first_window == 1 and static emotion: it is computed and its output is dropped.
 struct SlotArgs {
   const float* r_s;        // (W)
   const float* wa;         // (T_wa, A)
@@ -27,6 +27,7 @@ struct SlotArgs {
   int out_start;           // frame of r_d that is this window's first current frame
   float* ctx;              // (P, W) the clip's motion context, read unless first_window and overwritten with this window's
                            // last P frames (fmt_sample_windows); nullptr: the context stays in the handle's per-slot state
+  int we_dynamic;          // the clip's emotion: 0 static, we is (1, E) over every frame; 1 dynamic, we is (T_we, E) per frame
 };
 
 // The ODE schedule one slot runs in one window of fmt_sample_clips_ode / fmt_sample_windows_ode (the per-slot window graph).  In the
@@ -54,7 +55,6 @@ struct WindowArgs {
 
 struct ModelShape {
   int B, nb, N, P, L, W, A, E, H, Kc;   // Kc = padded c_embedder K (multiple of 64)
-  int we_dynamic;
   unsigned null_a, null_r, null_e;      // bit br set = that condition is zeroed in branch br (FMT.py:360-392)
 };
 
@@ -99,7 +99,7 @@ __global__ void cond_gather_kernel(const WindowArgs* __restrict__ wargs, ModelSh
     } else if (j < s.W + s.A + s.E) {
       const int k = j - s.W - s.A;
       if (!ze) {
-        if (!s.we_dynamic) v = sl.we[k];     // static emotion covers the context frames too (FMT.py:325-326)
+        if (!sl.we_dynamic) v = sl.we[k];    // static emotion covers the context frames too (FMT.py:325-326)
         else if (!ctx || !sl.first_window) v = sl.we[static_cast<size_t>(min(g, sl.T_we - 1)) * s.E + k];
       }
     }

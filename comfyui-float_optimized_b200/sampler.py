@@ -307,7 +307,8 @@ class FmtBackend:
 
     def sample_clips(self, r_s, wa, we, audio_num_frames, noise, a_cfg_scale, r_cfg_scale, e_cfg_scale,
                      progress: Optional[Callable[[int, int], None]] = None, out: Optional[Sequence[torch.Tensor]] = None,
-                     n_branches: Optional[Sequence[int]] = None, schedules: Optional[Sequence[tuple]] = None) -> List[torch.Tensor]:
+                     n_branches: Optional[Sequence[int]] = None, schedules: Optional[Sequence[tuple]] = None,
+                     we_dynamic: Optional[Sequence[bool]] = None) -> List[torch.Tensor]:
         """Many clips of different lengths in one call on the plan's batch of slots (:func:`clip_schedule`).  Per clip i: r_s[i]
         (1, dim_w), wa[i] (1, T_wa, dim_a), we[i] (1, 1 or T_we, dim_e), noise[i] (n_win_i, L, dim_w) or (n_win_i, 1, L, dim_w), all on
         ``self.device`` (fp32, contiguous).  Returns one (1, audio_num_frames[i], dim_w) tensor per clip (``out[i]`` if given: any
@@ -317,7 +318,8 @@ class FmtBackend:
         most the plan's; default: the plan's for every clip) is the branch count of clip i's guidance, :func:`n_branches_for`.
         ``schedules[i]`` = (nfe, method), at most the plan's evaluations per window (:func:`n_evals`), puts clip i on its own ODE
         schedule; given, the call runs the per-slot window graph (``fmt_sample_clips_ode``), one kernel per op, even where every
-        schedule is the plan's."""
+        schedule is the plan's.  ``we_dynamic[i]`` (default: the plan's for every clip) is clip i's emotion mode, which its ``we``
+        must have: static (1 frame) or dynamic (per frame); clips of both modes share the plan's window graphs."""
         d = self.dims
         if self._plan_key is None:
             raise FmtError("sample_clips: configure() has not been called")
@@ -333,8 +335,10 @@ class FmtBackend:
         nbr = [self._plan_key[1]] * n if n_branches is None else [int(x) for x in n_branches]
         if len(nbr) != n:
             raise ValueError(f"sample_clips: n_branches needs one entry per clip ({n}), got {len(nbr)}")
+        modes = [self._plan_key[2]] * n if we_dynamic is None else [bool(x) for x in we_dynamic]
+        if len(modes) != n:
+            raise ValueError(f"sample_clips: we_dynamic needs one entry per clip ({n}), got {len(modes)}")
         L = d.frames_per_clip
-        dynamic = self._plan_key[2]
         outs = []
         for i in range(n):
             for name, t in (("r_s", r_s[i]), ("wa", wa[i]), ("we", we[i]), ("noise", noise[i])):
@@ -350,8 +354,8 @@ class FmtBackend:
                 raise ValueError(f"clip {i}: wa shape {tuple(wa[i].shape)} != (1, T > {(n_win - 1) * L}, dim_a={d.dim_a})")
             if r_s[i].shape[0] != 1 or r_s[i].numel() != d.dim_w:
                 raise ValueError(f"clip {i}: r_s shape {tuple(r_s[i].shape)} != (1, dim_w={d.dim_w})")
-            if we[i].dim() != 3 or we[i].shape[0] != 1 or we[i].shape[2] != d.dim_e or dynamic != (we[i].shape[1] > 1):
-                raise ValueError(f"clip {i}: we shape {tuple(we[i].shape)} does not match (1, {'T' if dynamic else 1}, dim_e={d.dim_e})")
+            if we[i].dim() != 3 or we[i].shape[0] != 1 or we[i].shape[2] != d.dim_e or modes[i] != (we[i].shape[1] > 1):
+                raise ValueError(f"clip {i}: we shape {tuple(we[i].shape)} does not match (1, {'T' if modes[i] else 1}, dim_e={d.dim_e})")
             if tuple(noise[i].shape) not in ((n_win, L, d.dim_w), (n_win, 1, L, d.dim_w)):
                 raise ValueError(f"clip {i}: noise shape {tuple(noise[i].shape)} != {(n_win, L, d.dim_w)}")
             if out is None:
@@ -375,28 +379,27 @@ class FmtBackend:
         cs = _cabi.FmtClipSet(n, ptrs(r_s), ptrs(wa), ptrs(we), ptrs(noise), ptrs(outs), ints(t.shape[1] for t in wa),
                               ints(t.shape[1] for t in we), ints(audio_num_frames), 1.0, 1.0, 1.0, cb, None)
         g = _cabi.FmtClipGuidance(floats(scales[0]), floats(scales[1]), floats(scales[2]), ints(nbr))
-        if schedules is not None:
-            ode, _keep = self._clip_ode(schedules, n)
-            with torch.cuda.device(self.device):
-                _cabi.check(self.lib.fmt_sample_clips_ode(self._handle, C.byref(cs), C.byref(g), C.byref(ode), self._stream()), "fmt_sample_clips_ode")
-            return outs
+        ode, _keep = self._clip_ode(schedules, n) if schedules is not None else (None, None)
         with torch.cuda.device(self.device):
-            _cabi.check(self.lib.fmt_sample_clips_guided(self._handle, C.byref(cs), C.byref(g), self._stream()), "fmt_sample_clips_guided")
+            _cabi.check(self.lib.fmt_sample_clip_set(self._handle, C.byref(cs), C.byref(g), None if ode is None else C.byref(ode),
+                                                     None if we_dynamic is None else ints(modes), self._stream()), "fmt_sample_clip_set")
         return outs
 
     def sample_windows(self, r_s, wa, we, x0, ctx, out, first_window, a_cfg_scale, r_cfg_scale, e_cfg_scale, n_branches,
-                       schedules: Optional[Sequence[tuple]] = None) -> None:
+                       schedules: Optional[Sequence[tuple]] = None, we_dynamic: Optional[Sequence[bool]] = None) -> None:
         """One window of each of n <= plan batch streams (``fmt_sample_windows``), stream i in slot i.  Per stream i: r_s[i]
         (1, dim_w); wa[i] (T_wa, dim_a) and, dynamic, we[i] (T_we, dim_e) from the window's first context frame (frame 0 in a first
         window), static we[i] (1, 1, dim_e); x0[i] (L, dim_w); ctx[i] (P, dim_w), read unless ``first_window[i]`` and overwritten
         with the window's last P frames; out[i] receives the window's first ``out[i].shape[-2]`` frames.  Scales and n_branches are
-        one entry per stream; ``schedules`` (one (nfe, method) per stream) as in :meth:`sample_clips`.  All tensors on ``self.device``
-        (fp32, contiguous); asynchronous."""
+        one entry per stream; ``schedules`` (one (nfe, method) per stream) and ``we_dynamic`` (one emotion mode per stream, which
+        decides the layout of we[i]) as in :meth:`sample_clips`.  All tensors on ``self.device`` (fp32, contiguous); asynchronous."""
         d = self.dims
         if self._plan_key is None:
             raise FmtError("sample_windows: configure() has not been called")
         n = len(wa)
         groups = (r_s, we, x0, ctx, out, first_window, a_cfg_scale, r_cfg_scale, e_cfg_scale, n_branches)
+        if we_dynamic is not None:
+            groups += (we_dynamic,)
         if not 1 <= n <= self._plan_key[0] or not all(len(x) == n for x in groups):
             raise ValueError(f"sample_windows: 1 to {self._plan_key[0]} streams, with one entry per stream in every argument")
         for i in range(n):
@@ -418,14 +421,11 @@ class FmtBackend:
                                 ints(t.numel() // d.dim_e for t in we), ints(t.numel() // d.dim_w for t in out), ints(first_window))
         g = _cabi.FmtClipGuidance(*[(C.c_float * n)(*[float(x) for x in v]) for v in (a_cfg_scale, r_cfg_scale, e_cfg_scale)],
                                   ints(n_branches))
-        if schedules is not None:
-            ode, _keep = self._clip_ode(schedules, n)
-            with torch.cuda.device(self.device):
-                _cabi.check(self.lib.fmt_sample_windows_ode(self._handle, C.byref(ws), C.byref(g), C.byref(ode), self._stream()),
-                            "fmt_sample_windows_ode")
-            return
+        ode, _keep = self._clip_ode(schedules, n) if schedules is not None else (None, None)
         with torch.cuda.device(self.device):
-            _cabi.check(self.lib.fmt_sample_windows(self._handle, C.byref(ws), C.byref(g), self._stream()), "fmt_sample_windows")
+            _cabi.check(self.lib.fmt_sample_window_set(self._handle, C.byref(ws), C.byref(g), None if ode is None else C.byref(ode),
+                                                       None if we_dynamic is None else ints(we_dynamic), self._stream()),
+                        "fmt_sample_window_set")
 
     def velocity(self, eval_index: int, x, wa, r_s, we, prev_x, prev_wa, prev_we, a_cfg_scale, r_cfg_scale, e_cfg_scale) -> torch.Tensor:
         """One ``forward_with_cfv`` (FMT.py:342-401) at plan time ``t_eval[eval_index]``; returns (B, P+L, dim_w)."""
@@ -612,12 +612,14 @@ def _own_schedule(who: str, c: Mapping, nfe, method) -> tuple:
 
 def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str = "euler", a_cfg_scale: float = 2.0,
                  r_cfg_scale: float = 1.0, e_cfg_scale: float = 1.0, include_r_cfg: bool = False, mode: Optional[str] = None,
-                 device=None, progress: Optional[Callable[[int, int], None]] = None) -> List[torch.Tensor]:
+                 we_dynamic: Optional[bool] = None, device=None, progress: Optional[Callable[[int, int], None]] = None) -> List[torch.Tensor]:
     """Many independent clips of different lengths in one call.  Each clip is a mapping with ``r_s`` (1, dim_w), ``wa``
     (1, T_wa, dim_a), ``we`` (1, 1 or T_we, dim_e), optionally ``audio_num_frames`` (default T_wa) and either ``seed`` (its noise is
     :func:`clip_noise`) or ``noise`` (n_win, L, dim_w).  A clip may also hold ``a_cfg_scale``, ``r_cfg_scale``, ``e_cfg_scale``,
-    ``include_r_cfg``, ``nfe`` and ``method``: each overrides the keyword of the same name for that clip.  Precision and static /
-    dynamic emotion are shared.  The plan runs as many CFG branches as the clip that needs the most (:func:`n_branches_for`); a clip
+    ``include_r_cfg``, ``nfe``, ``method`` and ``we_dynamic``: each overrides the keyword of the same name for that clip.  A clip's
+    emotion mode (``we_dynamic``: static, ``we`` of 1 frame, or dynamic, one frame per audio frame) must match its ``we``; with the
+    keyword left at None, the clips that do not declare one take the mode of their ``we`` and must all have the same.  Clips of both
+    modes share the call's slots and window graphs.  Precision is shared.  The plan runs as many CFG branches as the clip that needs the most (:func:`n_branches_for`); a clip
     that needs fewer combines only its own branches.  Likewise it runs the evaluations per window of the clip that needs the most
     (:func:`n_evals`, :func:`plan_schedule`); a clip that needs fewer runs its own and then idles, and a call whose clips do not all
     run the plan's schedule goes through the per-slot window graph (one kernel per op).  Clip i's result is what
@@ -633,8 +635,11 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
     build_schedule(nfe, method)                        # unknown solver -> ValueError
     if int(nfe) < 1:
         raise ValueError(f"nfe must be >= 1 (got {nfe})")
+    if we_dynamic is not None and not isinstance(we_dynamic, bool):
+        raise TypeError(f"we_dynamic must be a bool or None, got {type(we_dynamic).__name__}")
     mode = resolve_mode(mode)
-    T, n_win, dyn, guidance, schedules = [], [], [], [], []      # guidance: (a, r, e, n_branches) of every clip
+    T, n_win, dyn, guidance, schedules = [], [], [], [], []
+    inferred = set()                                   # modes of the clips that take theirs from the shape of their we      # guidance: (a, r, e, n_branches) of every clip
     for i, c in enumerate(clips):
         if not isinstance(c, Mapping):
             raise TypeError(f"clip {i} must be a mapping (r_s, wa, we, seed or noise), got {type(c).__name__}")
@@ -654,7 +659,15 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
         if t < 1:
             raise ValueError(f"clip {i}: audio_num_frames must be >= 1 (got {t})")
         nw = -(-t // L)
-        dynamic = we.shape[1] > 1
+        dynamic = c.get("we_dynamic", we_dynamic)
+        if dynamic is None:
+            dynamic = we.shape[1] > 1
+            inferred.add(dynamic)
+        elif not isinstance(dynamic, bool):
+            raise TypeError(f"clip {i}: we_dynamic must be a bool, got {type(dynamic).__name__}")
+        elif dynamic != (we.shape[1] > 1):
+            raise ValueError(f"clip {i}: we_dynamic={dynamic}, but we has {we.shape[1]} frame(s) "
+                             f"({'more than one' if dynamic else 'one'} expected)")
         # the reference's F.pad(replicate) needs at least one real frame in every window (nodes_adv.py:614-616)
         if (nw - 1) * L >= wa.shape[1]:
             raise ValueError(f"clip {i}: wa has {wa.shape[1]} frames, but window {nw - 1} of its {t} frames starts at frame {(nw - 1) * L}")
@@ -674,8 +687,9 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
         T.append(t)
         n_win.append(nw)
         dyn.append(dynamic)
-    if any(dyn) != all(dyn):
-        raise ValueError("clips mix static (1-frame) and dynamic (per-frame) emotion we; one call shares one of the two")
+    if len(inferred) > 1:
+        raise ValueError("clips mix static (1-frame) and dynamic (per-frame) emotion we; give the clips of one mode we_dynamic "
+                         "(or the call the keyword) to sample both in one call")
 
     if device is None:
         device = getattr(fmt_model, "target_device", None) or "cuda"
@@ -689,6 +703,8 @@ def sample_clips(fmt_model, clips: Sequence[Mapping], *, nfe: int, method: str =
              for c, nw in zip(clips, n_win)]
     # the plan's schedule for every clip: the plan's window graph, as without per-clip schedules
     own = {} if all(sc == plan for sc in schedules) else dict(schedules=schedules)
+    if any(x != dyn[0] for x in dyn):                  # the plan's emotion mode is clip 0's; the others say theirs only when they differ
+        own["we_dynamic"] = dyn
     return be.sample_clips([_as_f32(c["r_s"], dev) for c in clips], [_as_f32(c["wa"], dev) for c in clips],
                            [_as_f32(c["we"], dev) for c in clips], T, noise, a, r, e, progress, n_branches=nb, **own)
 
@@ -704,9 +720,10 @@ class Stream:
     """One clip of a :class:`StreamSampler`, opened by :meth:`StreamSampler.open`.  ``fed`` frames have arrived, ``windows_run``
     windows have been sampled; ``finished`` once :meth:`StreamSampler.finish` was called, ``done`` once its last window ran."""
 
-    def __init__(self, index, L, r_s, we, ctx, wa, we_buf, gen, noise, guidance, schedule):
+    def __init__(self, index, L, r_s, we, ctx, wa, we_buf, gen, noise, guidance, schedule, we_dynamic):
         self.index = index                  # open order: breaks ties between windows that became ready at the same tick
         self.L = L
+        self.we_dynamic = we_dynamic        # True: we arrives with feed(), one frame per audio frame (we_buf); False: we, from open()
         self.r_s, self.we, self.ctx = r_s, we, ctx
         self.wa, self.we_buf = wa, we_buf   # frames [base, fed): from the next window's first context frame on
         self.base = 0
@@ -736,9 +753,9 @@ class StreamSampler:
     several windows ready makes them ready at once); ties go in open order.  A stream's frames
     are what :func:`sample_clips` gives for the whole clip (same noise, same guidance, same plan), however the audio was cut.
 
-    The plan (slot count, nfe, solver, precision, static or dynamic emotion, and the branch count of the keyword guidance) is fixed
-    at construction, so steps replay one captured window graph.  A stream may override the four guidance keywords in :meth:`open`
-    as a clip of :func:`sample_clips` does, within the plan's branch count, and ``nfe`` and ``method`` within the plan's
+    The plan (slot count, nfe, solver, precision, and the branch count of the keyword guidance) is fixed at construction, so steps
+    replay one captured window graph.  A stream may override the four guidance keywords in :meth:`open` as a clip of
+    :func:`sample_clips` does, within the plan's branch count, ``we_dynamic`` (static or dynamic emotion) freely, and ``nfe`` and ``method`` within the plan's
     evaluations per window (:func:`n_evals` of the constructor's nfe and method); a step that runs a stream on a schedule other
     than the plan's goes through the per-slot window graph (one kernel per op).  A stream holds on the device its reference latent,
     its last P motion frames and the audio frames from its next window's first context frame on, however long it runs."""
@@ -784,9 +801,10 @@ class StreamSampler:
             raise ValueError("not an open stream of this sampler")
         return stream
 
-    def open(self, r_s, we=None, seed: Optional[int] = None, noise: Optional[torch.Tensor] = None, **guidance) -> Stream:
+    def open(self, r_s, we=None, seed: Optional[int] = None, noise: Optional[torch.Tensor] = None, we_dynamic: Optional[bool] = None,
+             **guidance) -> Stream:
         """A new stream with reference latent ``r_s`` (1, dim_w) and, for static emotion, ``we`` (1, 1, dim_e) (dynamic emotion
-        arrives with :meth:`feed`).  Its noise is :func:`clip_noise` of ``seed``, drawn one window at a time, or ``noise``
+        arrives with :meth:`feed`).  ``we_dynamic`` (default: the sampler's) is the stream's emotion mode.  Its noise is :func:`clip_noise` of ``seed``, drawn one window at a time, or ``noise``
         (n_win, L, dim_w) for a clip of exactly n_win windows.  ``guidance`` may hold ``a_cfg_scale``, ``r_cfg_scale``,
         ``e_cfg_scale``, ``include_r_cfg``, ``nfe`` and ``method``, each overriding the sampler's keyword for this stream."""
         d, L = self.dims, self.dims.frames_per_clip
@@ -794,12 +812,16 @@ class StreamSampler:
         if unknown:
             raise TypeError(f"open: unexpected keyword(s) {unknown}")
         self._check_tensor("open", "r_s", r_s, (1, d.dim_w))
-        if self.we_dynamic:
+        if we_dynamic is None:
+            we_dynamic = self.we_dynamic
+        elif not isinstance(we_dynamic, bool):
+            raise TypeError(f"open: we_dynamic must be a bool, got {type(we_dynamic).__name__}")
+        if we_dynamic:
             if we is not None:
-                raise ValueError("open: this sampler has dynamic emotion: we arrives with feed(), one frame per audio frame")
+                raise ValueError("open: this stream has dynamic emotion: we arrives with feed(), one frame per audio frame")
         else:
             if we is None:
-                raise ValueError("open: this sampler has static emotion: give we (1, 1, dim_e) here")
+                raise ValueError("open: this stream has static emotion: give we (1, 1, dim_e) here")
             self._check_tensor("open", "we", we, (1, 1, d.dim_e))
         if (seed is None) == (noise is None):
             raise ValueError("open: give exactly one of 'seed' and 'noise'")
@@ -819,14 +841,15 @@ class StreamSampler:
         gen = torch.Generator(dev).manual_seed(int(seed)) if seed is not None else None
         st = Stream(self._opened, L, _as_f32(r_s, dev).clone(), None if we is None else _as_f32(we, dev).clone(),
                     torch.zeros(d.num_prev_frames, d.dim_w, device=dev), torch.empty(0, d.dim_a, device=dev),
-                    torch.empty(0, d.dim_e, device=dev) if self.we_dynamic else None, gen,
-                    None if noise is None else noise.reshape(noise.shape[0], L, d.dim_w), g, sc)
+                    torch.empty(0, d.dim_e, device=dev) if we_dynamic else None, gen,
+                    None if noise is None else noise.reshape(noise.shape[0], L, d.dim_w), g, sc, we_dynamic)
         self._opened += 1
         self._streams.append(st)
         return st
 
     def feed(self, stream: Stream, wa, we=None) -> None:
-        """Appends audio latents ``wa`` (1, t, dim_a), t >= 1, and with dynamic emotion as many ``we`` frames (1, t, dim_e)."""
+        """Appends audio latents ``wa`` (1, t, dim_a), t >= 1, and, to a stream with dynamic emotion, as many ``we`` frames
+        (1, t, dim_e)."""
         st, d = self._own(stream), self.dims
         if st.finished:
             raise ValueError("feed: the stream is finished")
@@ -834,16 +857,16 @@ class StreamSampler:
         t = wa.shape[1]
         if t < 1:
             raise ValueError("feed: wa holds no frame")
-        if self.we_dynamic:
+        if st.we_dynamic:
             if we is None:
-                raise ValueError("feed: this sampler has dynamic emotion: give we (1, t, dim_e) with every wa")
+                raise ValueError("feed: this stream has dynamic emotion: give we (1, t, dim_e) with every wa")
             self._check_tensor("feed", "we", we, (1, t, d.dim_e))
         elif we is not None:
-            raise ValueError("feed: this sampler has static emotion, given to open(); feed takes wa only")
+            raise ValueError("feed: this stream has static emotion, given to open(); feed takes wa only")
         if st.noise is not None and -(-(st.fed + t) // d.frames_per_clip) > st.noise.shape[0]:
             raise ValueError(f"feed: {st.fed + t} frames need more windows than the stream's {st.noise.shape[0]} windows of noise")
         st.wa = torch.cat([st.wa, wa[0].to(device=self.device, dtype=torch.float32)])
-        if self.we_dynamic:
+        if st.we_dynamic:
             st.we_buf = torch.cat([st.we_buf, we[0].to(device=self.device, dtype=torch.float32)])
         st.fed += t
         self._clock += 1
@@ -899,8 +922,10 @@ class StreamSampler:
             outs.append(torch.empty(1, min(L, st.fed - w * L), d.dim_w, device=dev))
         schedules = [st.schedule for st in run]
         own = {} if all(sc == (self.nfe, self.method) for sc in schedules) else dict(schedules=schedules)
+        if any(st.we_dynamic != self.we_dynamic for st in run):
+            own["we_dynamic"] = [st.we_dynamic for st in run]
         self._be.sample_windows([st.r_s for st in run], [st.wa for st in run],
-                                [st.we_buf if self.we_dynamic else st.we for st in run], x0, [st.ctx for st in run], outs,
+                                [st.we_buf if st.we_dynamic else st.we for st in run], x0, [st.ctx for st in run], outs,
                                 [int(st.windows_run == 0) for st in run], *zip(*[st.guidance for st in run]), **own)
         self._clock += 1
         for st in run:
@@ -909,7 +934,7 @@ class StreamSampler:
             # keep frames from the next window's first context frame on (copied, so the dropped frames are freed)
             keep = st.windows_run * L - P - st.base
             st.wa = st.wa[keep:].clone()
-            if self.we_dynamic:
+            if st.we_dynamic:
                 st.we_buf = st.we_buf[keep:].clone()
             st.base += keep
             self._refresh(st)

@@ -94,7 +94,9 @@ enum { FMT_MODE_BF16 = 0,       /* bf16 tcgen05/TMA GEMMs, fp32 accumulate / res
 typedef struct FmtPlan {
   int32_t batch;          /* clips B                                                                        */
   int32_t n_branches;     /* 1: all scales == 1 (FMT.py:400-401); 3: default CFG; 4: include_r_cfg (:380-399) */
-  int32_t we_dynamic;     /* 0: we is (B,1,E) broadcast over all P+L frames; 1: we is (B,T,E)                */
+  int32_t we_dynamic;     /* 0: we is (B,1,E) broadcast over all P+L frames; 1: we is (B,T,E).  The emotion mode of
+                             fmt_sample_clip, fmt_velocity and of the clip / window sets without per-clip modes; no
+                             graph depends on it, so a plan that differs only in it is not re-captured            */
   int32_t mode;           /* FMT_MODE_*                                                                      */
   int32_t n_steps;        /* ODE steps S = nfe-1 (torchdiffeq fixed grid: nfe points)                        */
   int32_t n_stages;       /* explicit RK stages per step (euler 1, midpoint 2, heun2 2, heun3 3, rk4 4)      */
@@ -129,7 +131,7 @@ typedef struct FmtClipSet {
   int32_t n_clips;
   const float* const* r_s;          /* [i]: (1, dim_w)                                                                     */
   const float* const* wa;           /* [i]: (1, T_wa[i], dim_a)                                                            */
-  const float* const* we;           /* [i]: (1, T_we[i], dim_e); T_we[i] == 1 for every clip or > 1 for every clip (plan.we_dynamic) */
+  const float* const* we;           /* [i]: (1, T_we[i], dim_e); T_we[i] == 1 (static) or > 1 (dynamic), per clip's emotion mode    */
   const float* const* noise;        /* [i]: (n_win_i, L, dim_w), n_win_i = ceil(audio_num_frames[i] / L): x0 of each of its windows */
   float* const* r_d;                /* [i]: out (1, audio_num_frames[i], dim_w); only these frames are written                  */
   const int32_t* T_wa;
@@ -159,7 +161,8 @@ typedef struct FmtWindowSet {
   const float* const* r_s;          /* [i]: (1, dim_w)                                                                           */
   const float* const* wa;           /* [i]: (T_wa[i], dim_a) from frame w*L - P (frame 0 in a first window); frames beyond T_wa[i]
                                        are the last frame repeated, as in a clip's last window                                  */
-  const float* const* we;           /* [i]: static (1, dim_e), or dynamic (T_we[i], dim_e) from the same frame as wa                */
+  const float* const* we;           /* [i]: static (1, dim_e), or dynamic (T_we[i], dim_e) from the same frame as wa (the stream's
+                                       emotion mode: plan.we_dynamic, or its entry of fmt_sample_window_set's we_dynamic)       */
   const float* const* x0;           /* [i]: (L, dim_w) noise of this window                                                      */
   float* const* ctx;                /* [i]: (P, dim_w) in / out: the last P frames of the stream's previous window (not read in a
                                        first window); receives this window's last P frames                                       */
@@ -249,6 +252,18 @@ FMT_API int32_t fmt_sample_clips_ode(FmtHandle* h, const FmtClipSet* set, const 
 FMT_API int32_t fmt_sample_windows_ode(FmtHandle* h, const FmtWindowSet* set, const FmtClipGuidance* guidance, const FmtClipOde* ode,
                                        void* stream);
 
+/* The general entries the five calls above are written with.  guidance == NULL (clip sets only): the set's a/r/e_cfg_scale and
+ * plan.n_branches for every clip; ode == NULL: the plan's schedule (the plan's window graph); we_dynamic == NULL: plan.we_dynamic for
+ * every clip / stream, else a HOST array of n_clips / n_streams entries, 0 (static emotion: T_we[i] == 1) or 1 (dynamic: T_we[i] > 1
+ * for a clip, with the coverage checks of its mode).  Clips of both modes share one call and the plan's window graphs: the condition
+ * rows they share do not depend on the mode (fmt_debug_condition_rows_slots).  Clip i's result is what a call whose every clip has
+ * clip i's mode gives for it on the same plan.  Returns -1 on a mode other than 0 / 1 or a T_we that does not match it, or on the
+ * checks of the calls above. */
+FMT_API int32_t fmt_sample_clip_set(FmtHandle* h, const FmtClipSet* set, const FmtClipGuidance* guidance, const FmtClipOde* ode,
+                                    const int32_t* we_dynamic, void* stream);
+FMT_API int32_t fmt_sample_window_set(FmtHandle* h, const FmtWindowSet* set, const FmtClipGuidance* guidance, const FmtClipOde* ode,
+                                      const int32_t* we_dynamic, void* stream);
+
 /* Single CFG-combined model evaluation (device pointers). */
 FMT_API int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream);
 
@@ -277,6 +292,10 @@ FMT_API int32_t fmt_debug_condition_rows(int32_t n_branches, int32_t batch, int3
  * plans: the truly-unconditional current frames are one row per slot). */
 FMT_API int32_t fmt_debug_condition_rows_ode(int32_t n_branches, int32_t batch, int32_t n_frames, int32_t n_prev, int32_t we_dynamic,
                                              int32_t per_slot, int32_t* urow_out);
+/* The same with slot b's emotion mode we_dynamic[b] (HOST, batch entries): the map the keys of every slot's own mode give.  The
+ * sampler uses the map of plan.we_dynamic for every mix; this entry shows that the map is the same. */
+FMT_API int32_t fmt_debug_condition_rows_slots(int32_t n_branches, int32_t batch, int32_t n_frames, int32_t n_prev,
+                                               const int32_t* we_dynamic, int32_t per_slot, int32_t* urow_out);
 
 /* ---- audio projection in front of the sampler (SURVEY.md 8f rank 2) ----
  * Replaces the nn.Sequential(Linear(in_dim, dim_w), LayerNorm(dim_w), SiLU) that FloatApplyAudioProjection runs
