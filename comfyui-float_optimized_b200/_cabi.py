@@ -116,6 +116,8 @@ _SIGNATURES = {
                                         C.POINTER(C.c_int32), C.c_void_p]),
     "fmt_sample_window_set": (C.c_int32, [C.c_void_p, C.POINTER(FmtWindowSet), C.POINTER(FmtClipGuidance), C.POINTER(FmtClipOde),
                                           C.POINTER(C.c_int32), C.c_void_p]),
+    "fmt_occupancy_slots": (C.c_int32, [C.c_int32, C.c_int32]),
+    "fmt_last_window_slots": (C.c_int32, [C.c_void_p]),
     "fmt_clip_schedule": (C.c_int32, [C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32)]),
     "fmt_velocity": (C.c_int32, [C.c_void_p, C.POINTER(FmtEval), C.c_void_p]),

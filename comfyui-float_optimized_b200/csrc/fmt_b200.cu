@@ -97,10 +97,12 @@ struct FmtHandle {
   DevBuf ev_wa, ev_we;                           // fmt_velocity: [prev_wa | wa] and [prev_we | we] of every clip, (B, P + L, .)
   // the slot records of every window of a sampling call ([window][slot]), uploaded with one copy from a pinned staging
   // buffer; slot_ev marks the end of that copy, so the next call waits for it before it refills the staging buffer.  A window's
-  // records are slot_stride bytes: B SlotArgs, followed by B SlotOde in calls of the per-slot window graph.
+  // records are slot_stride bytes: one SlotArgs per slot of the graph it replays, followed by as many SlotOde in calls of the per-slot
+// window graph.
   DevBuf slot_buf, slot_zero;                    // slot_zero: the inputs of an idle slot
   unsigned char* slot_host = nullptr;
   size_t slot_host_bytes = 0, slot_stride = 0;
+  int slot_recs = 0;                             // records per window of the staged call
   cudaEvent_t slot_ev = nullptr;
   // per-slot ODE schedules (fmt_sample_clips_ode, fmt_sample_windows_ode): a second window graph of the plan, captured on first use.
   // It shares the plan's workspace and AdaLN table buffer; its condition rows never span two slots (sU rows, sU - U more than the
@@ -146,6 +148,25 @@ struct FmtHandle {
   long long launches = 0;
   bool capturing = false;
   long long capture_launches = 0;
+  bool ksliced = false;                          // a graph captured since the flag was cleared cuts a GEMM into K slices
+
+  // occupancy buckets of a plan whose window graph runs one kernel per op (fmt_sample_window_set): a step with k ready streams
+  // replays graphs captured for fmt_occupancy_slots(batch, k) slots.  Bucket i (of 2^i slots, below batch) gets its condition-row
+  // map in fmt_configure and its graphs on first use; the plan's own graphs serve the bucket of batch slots.
+  struct Bucket {
+    int B = 0, U = 0;                            // slots, distinct condition rows of the plan's graph for them
+    size_t map_off = 0;                          // its urow (R ints) | uidx (U ints) in bucket_maps
+    cudaGraphExec_t exec = nullptr;
+    long long launches = 0;
+    int sU = 0;                                  // the per-slot window graph's: condition rows, map (built on first use), graph
+    DevBuf s_map;
+    cudaGraphExec_t ode_exec = nullptr;
+    long long ode_launches = 0;
+  };
+  std::vector<Bucket> buckets;
+  DevBuf bucket_maps;
+  bool plan_ksliced = false;                     // the plan's window graph cuts a GEMM into K slices: its buckets may too
+  int last_slots = 0;                            // slots of the last window graph replayed
 };
 
 static int dev_alloc(FmtHandle* h, DevBuf& b, size_t bytes) {
@@ -270,10 +291,11 @@ static int pick_bn(const FmtHandle* h, int M, int N) {
 }
 
 // SPLIT: the bf16x3 GEMM on pair operands (FMT_MODE_BF16X3): K % 64 == 0, never K-sliced by the sampler (its results stay bitwise
-// reproducible).  force_ksplit: K slices of a forced CTA-pair kernel (unit tests); the sampler picks them itself.
+// reproducible).  force_ksplit: K slices of a forced CTA-pair kernel (unit tests); the sampler picks them itself where ksplit allows it
+// (a window graph's GraphShape::ksplit).  Every other choice of kernel and tile gives the same bits (tests/test_gpu_gemm_variants.py).
 template <bool SPLIT = false>
 static int gemm_bf16(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ldw, const EpiParams& ep, int K, cudaStream_t st, int force_bn = 0,
-                     int force_ksplit = 1) {
+                     int force_ksplit = 1, bool ksplit = false) {
   REQUIRE(ep.N % 32 == 0 && K % 8 == 0 && lda % 8 == 0 && ldw % 8 == 0, "gemm_bf16: N %% 32, K/lda/ldw %% 8 required (N=%d K=%d)", ep.N, K);
   REQUIRE(!SPLIT || (K % 64 == 0 && lda % 64 == 0 && ldw % 64 == 0), "gemm_bf16x3: K, lda, ldw %% 64 required (K=%d)", K);
   REQUIRE(force_ksplit == 1 || force_bn == 512 || force_bn == 1024, "gemm_bf16: K slices need the CTA-pair kernel (block_n 512 or 1024)");
@@ -293,11 +315,14 @@ static int gemm_bf16(FmtHandle* h, const bf16* A, int lda, const bf16* W, int ld
     // bf16x3: the same model (its operand bytes and MMAs both grow ~2-3x on every tile shape); a single-CTA 128 x 256 tile would
     // keep only 2 of its 96 KB stages, so the pair tile or 128 x 128 it is
     if (SPLIT) return c_pair <= c_128 ? launch_tc2<256, true>(h, A, lda, W, ldw, ep, K, st) : launch_tc<128, true>(h, A, lda, W, ldw, ep, K, st);
-    if (ep.kind == EPI_GATE_RES && h->use_splitk && K >= 1024 && c_pair >= 2.0) {   // single-wave problems stay bitwise deterministic
+    if (ep.kind == EPI_GATE_RES && ksplit && K >= 1024 && c_pair >= 2.0) {   // single-wave problems stay bitwise deterministic
       // x += gate * (.) is additive, so a tile may be cut into 2 K slices whose partial sums meet in x (fp32 RED):
       // N = 1024 at 32 clips = 92 pair tiles on 74 pairs (2 waves) -> 184 half-K units (2.5 half-waves)
       const double c_split = 0.5 * waves(2 * mt256 * (ep.N / 256), pairs) + 0.08;
-      if (c_split < c_pair && c_split < c_256 && c_split < c_128) return launch_tc2<256, false>(h, A, lda, W, ldw, ep, K, st, 2);
+      if (c_split < c_pair && c_split < c_256 && c_split < c_128) {
+        if (h->capturing) h->ksliced = true;
+        return launch_tc2<256, false>(h, A, lda, W, ldw, ep, K, st, 2);
+      }
     }
     if (c_pair <= c_256 && c_pair <= c_128) return launch_tc2<256, false>(h, A, lda, W, ldw, ep, K, st);
     return c_128 < c_256 ? launch_tc<128, false>(h, A, lda, W, ldw, ep, K, st) : launch_tc<256, false>(h, A, lda, W, ldw, ep, K, st);
@@ -322,19 +347,19 @@ static int gemm_f32(FmtHandle* h, const float* A, int lda, const float* W, int l
 template <typename T> struct ModeOps;
 template <> struct ModeOps<bf16> {
   using Tab = bf16;
-  static int gemm(FmtHandle* h, const void* A, int lda, const Linear& L, const EpiParams& ep, cudaStream_t st) {
-    return gemm_bf16(h, static_cast<const bf16*>(A), lda, L.w16, L.K, ep, L.K, st);
+  static int gemm(FmtHandle* h, const void* A, int lda, const Linear& L, const EpiParams& ep, bool ksplit, cudaStream_t st) {
+    return gemm_bf16(h, static_cast<const bf16*>(A), lda, L.w16, L.K, ep, L.K, st, 0, 1, ksplit);
   }
 };
 template <> struct ModeOps<float> {
   using Tab = float;
-  static int gemm(FmtHandle* h, const void* A, int lda, const Linear& L, const EpiParams& ep, cudaStream_t st) {
+  static int gemm(FmtHandle* h, const void* A, int lda, const Linear& L, const EpiParams& ep, bool, cudaStream_t st) {
     return gemm_f32(h, static_cast<const float*>(A), lda, L.w32, L.K, ep, L.K, st);
   }
 };
 template <> struct ModeOps<bf16x3_t> {
   using Tab = float;                                   // only GEMM operands are pairs: tables and QKV stay fp32, as in the fp32 mode
-  static int gemm(FmtHandle* h, const void* A, int lda, const Linear& L, const EpiParams& ep, cudaStream_t st) {
+  static int gemm(FmtHandle* h, const void* A, int lda, const Linear& L, const EpiParams& ep, bool, cudaStream_t st) {
     return gemm_bf16<true>(h, static_cast<const bf16*>(A), lda, L.w3, L.K, ep, L.K, st);
   }
 };
@@ -368,20 +393,51 @@ static CondRows ode_rows(const FmtHandle* h) {
                   h->s_cond.p, h->s_cemb.p, h->s_chunk, true};
 }
 
+// Band attention of n_seq sequences of N rows.  variant 0 picks the kernel, 1 forces the warp-per-row kernel, 2 the tile kernel.
+enum { ATTN_AUTO = 0, ATTN_WARP = 1, ATTN_TILE = 2 };
+
+// What one captured window graph works on.  The plan's graphs run all plan.batch slots; an occupancy bucket's graphs
+// (fmt_sample_window_set) run the first B of them, on a prefix of every workspace buffer.  A bucket keeps whatever changes the bits of
+// a slot's rows: the band-attention kernel (the tile and the warp-per-row kernel reduce in different orders, and the plan's choice
+// depends on its sequence count) and K slicing (its partial sums meet in x in any order).  It picks its own GEMM tiles: every tile
+// shape and the CTA-pair kernel compute each output element the same way.
+struct GraphShape {
+  ModelShape s;                                  // s.B: the graph's slots
+  int R;                                         // token rows, s.nb * s.B * s.N
+  CondRows rows;                                 // condition rows of those slots (the plan's table_chunk, so the same node count)
+  int attn;                                      // ATTN_WARP or ATTN_TILE: the plan's
+  bool ksplit;                                   // gate + residual GEMMs may be cut into K slices
+};
+
+// the band-attention kernel ATTN_AUTO picks for n_seq sequences of the model in this activation type
+static int attn_variant(const FmtHandle* h, bool bf16_act, int n_seq) {
+  const int hd = h->d.dim_h / h->d.num_heads;
+  const bool tile_ok = bf16_act && static_cast<size_t>(2) * h->N * hd * sizeof(bf16) <= 48 * 1024 && (hd == 64 || hd == 128);
+  return tile_ok && n_seq * h->d.num_heads >= 2 * h->num_sms ? ATTN_TILE : ATTN_WARP;
+}
+
+// the plan's window graph (ode: its per-slot window graph)
+static GraphShape plan_graph(const FmtHandle* h, bool ode = false) {
+  return GraphShape{h->shape, h->R, ode ? ode_rows(h) : plan_rows(h), attn_variant(h, h->plan.mode == FMT_MODE_BF16, h->shape.nb * h->shape.B),
+                    h->use_splitk};
+}
+
 template <typename T>
-static int enqueue_prepare(FmtHandle* h, const CondRows& r, cudaStream_t st) {
-  const ModelShape& s = h->shape;
+static int enqueue_prepare(FmtHandle* h, const GraphShape& g, cudaStream_t st) {
+  const ModelShape& s = g.s;
+  const CondRows& r = g.rows;
   const WindowArgs* wa = static_cast<const WindowArgs*>(h->wargs.p);
   FMT_OK(launch(h, cond_gather_kernel<T>, dim3(r.U), dim3(128), 0, st, 1, wa, s, r.uidx, static_cast<T*>(r.cond)));
   EpiParams ep = epi(EPI_STORE, r.U, s.H, h->c_emb.b, r.cemb, s.H, 1);
-  FMT_OK(ModeOps<T>::gemm(h, r.cond, s.Kc, h->c_emb, ep, st));
+  FMT_OK(ModeOps<T>::gemm(h, r.cond, s.Kc, h->c_emb, ep, g.ksplit, st));
   return 0;
 }
 
 // AdaLN tables for evaluations [e0, e0+n): table[(e-e0)*U + u, :] = Linear_ada(SiLU(c_emb[u] + t_emb[e]))
 template <typename T>
-static int enqueue_tables(FmtHandle* h, const CondRows& r, int e0, int n, cudaStream_t st) {
-  const ModelShape& s = h->shape;
+static int enqueue_tables(FmtHandle* h, const GraphShape& g, int e0, int n, cudaStream_t st) {
+  const ModelShape& s = g.s;
+  const CondRows& r = g.rows;
   const size_t total = static_cast<size_t>(n) * r.U * s.H;
   const dim3 grid(static_cast<unsigned>((total / 4 + 255) / 256));
   if (r.per_slot)
@@ -391,7 +447,7 @@ static int enqueue_tables(FmtHandle* h, const CondRows& r, int e0, int n, cudaSt
     FMT_OK(launch(h, silu_cond_kernel<T>, grid, dim3(256), 0, st, 1, static_cast<const float*>(r.cemb), static_cast<const float*>(h->temb.p), e0,
                   r.U, s.H, static_cast<T*>(h->silu.p), total));
   EpiParams ep = epi(EPI_STORE, n * r.U, h->NT, h->ada.b, h->table.p, h->NT, sizeof(typename ModeOps<T>::Tab) == 4);
-  FMT_OK(ModeOps<T>::gemm(h, h->silu.p, s.H, h->ada, ep, st));
+  FMT_OK(ModeOps<T>::gemm(h, h->silu.p, s.H, h->ada, ep, g.ksplit, st));
   return 0;
 }
 
@@ -412,13 +468,11 @@ static int lnmod(FmtHandle* h, const float* X, int rows, int H, const typename M
 }
 
 template <typename T>
-static int launch_lnmod(FmtHandle* h, const CondRows& r, const typename ModeOps<T>::Tab* table_e, long long shift_off, long long scale_off,
+static int launch_lnmod(FmtHandle* h, const GraphShape& g, const typename ModeOps<T>::Tab* table_e, long long shift_off, long long scale_off,
                         cudaStream_t st) {
-  return lnmod<T>(h, static_cast<const float*>(h->X.p), h->R, h->shape.H, table_e, r.urow, h->NT, shift_off, scale_off, static_cast<T*>(h->A1.p), st);
+  return lnmod<T>(h, static_cast<const float*>(h->X.p), g.R, g.s.H, table_e, g.rows.urow, h->NT, shift_off, scale_off, static_cast<T*>(h->A1.p), st);
 }
 
-// Band attention of n_seq sequences of N rows.  variant 0 picks the kernel, 1 forces the warp-per-row kernel, 2 the tile kernel.
-enum { ATTN_AUTO = 0, ATTN_WARP = 1, ATTN_TILE = 2 };
 template <typename T>
 static int band_attention(FmtHandle* h, const typename ModeOps<T>::Tab* qkv, int n_seq, int N, int heads, int hd, int win, T* out, int variant,
                           cudaStream_t st) {
@@ -450,55 +504,56 @@ static int band_attention(FmtHandle* h, const typename ModeOps<T>::Tab* qkv, int
 }
 
 template <typename T>
-static int launch_attn(FmtHandle* h, cudaStream_t st) {
-  const ModelShape& s = h->shape;
+static int launch_attn(FmtHandle* h, const GraphShape& g, cudaStream_t st) {
+  const ModelShape& s = g.s;
   const int heads = h->d.num_heads;
   return band_attention<T>(h, static_cast<const typename ModeOps<T>::Tab*>(h->QKV.p), s.nb * s.B, s.N, heads, s.H / heads, h->d.attention_window,
-                           static_cast<T*>(h->A2.p), ATTN_AUTO, st);
+                           static_cast<T*>(h->A2.p), g.attn, st);
 }
 
 // One model evaluation: V[R, W] = FMT.forward over the nb-way batched CFG branches (FMT.py:277-340).  The x-embedder
 // operand `ax` has already been written by the producer of the ODE state (init_window / cfg_combine / rk_combine).
 template <typename T>
-static int enqueue_forward(FmtHandle* h, const CondRows& r, int table_slot, cudaStream_t st) {
-  const ModelShape& s = h->shape;
+static int enqueue_forward(FmtHandle* h, const GraphShape& g, int table_slot, cudaStream_t st) {
+  const ModelShape& s = g.s;
+  const CondRows& r = g.rows;
   const FmtDims& d = h->d;
-  const int R = h->R, H = s.H;
+  const int R = g.R, H = s.H;
+  const bool ks = g.ksplit;
   using TT = typename ModeOps<T>::Tab;
   const TT* table_e = static_cast<const TT*>(h->table.p) + static_cast<size_t>(table_slot) * r.U * h->NT;
   const int qkv_f32 = sizeof(TT) == 4;
   {
     EpiParams ep = epi(EPI_POS, R, H, h->x_emb.b, h->X.p, H, 1);
     ep.pos = h->pos; ep.frames = s.N;
-    FMT_OK(ModeOps<T>::gemm(h, h->ax.p, s.W, h->x_emb, ep, st));
+    FMT_OK(ModeOps<T>::gemm(h, h->ax.p, s.W, h->x_emb, ep, ks, st));
   }
   for (int i = 0; i < d.depth; ++i) {
     const long long base = static_cast<long long>(i) * 6 * H;
-    FMT_OK(launch_lnmod<T>(h, r, table_e, base + 0, base + H, st));
-    FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->qkv[i], epi(EPI_STORE, R, 3 * H, h->qkv[i].b, h->QKV.p, 3 * H, qkv_f32), st));
-    FMT_OK(launch_attn<T>(h, st));
+    FMT_OK(launch_lnmod<T>(h, g, table_e, base + 0, base + H, st));
+    FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->qkv[i], epi(EPI_STORE, R, 3 * H, h->qkv[i].b, h->QKV.p, 3 * H, qkv_f32), ks, st));
+    FMT_OK(launch_attn<T>(h, g, st));
     {
       EpiParams ep = epi(EPI_GATE_RES, R, H, h->proj[i].b, h->X.p, H, 1);
       ep.gate = table_e; ep.urow = r.urow; ep.ldg = h->NT; ep.gate_off = base + 2 * H;
-      FMT_OK(ModeOps<T>::gemm(h, h->A2.p, H, h->proj[i], ep, st));
+      FMT_OK(ModeOps<T>::gemm(h, h->A2.p, H, h->proj[i], ep, ks, st));
     }
-    FMT_OK(launch_lnmod<T>(h, r, table_e, base + 3 * H, base + 4 * H, st));
-    FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->fc1[i], epi(EPI_GELU, R, d.mlp_hidden, h->fc1[i].b, h->Hm.p, d.mlp_hidden, 0), st));
+    FMT_OK(launch_lnmod<T>(h, g, table_e, base + 3 * H, base + 4 * H, st));
+    FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->fc1[i], epi(EPI_GELU, R, d.mlp_hidden, h->fc1[i].b, h->Hm.p, d.mlp_hidden, 0), ks, st));
     {
       EpiParams ep = epi(EPI_GATE_RES, R, H, h->fc2[i].b, h->X.p, H, 1);
       ep.gate = table_e; ep.urow = r.urow; ep.ldg = h->NT; ep.gate_off = base + 5 * H;
-      FMT_OK(ModeOps<T>::gemm(h, h->Hm.p, d.mlp_hidden, h->fc2[i], ep, st));
+      FMT_OK(ModeOps<T>::gemm(h, h->Hm.p, d.mlp_hidden, h->fc2[i], ep, ks, st));
     }
   }
   const long long dbase = static_cast<long long>(d.depth) * 6 * H;
-  FMT_OK(launch_lnmod<T>(h, r, table_e, dbase, dbase + H, st));
-  FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->dec, epi(EPI_STORE, R, s.W, h->dec.b, h->V.p, s.W, 1), st));
+  FMT_OK(launch_lnmod<T>(h, g, table_e, dbase, dbase + H, st));
+  FMT_OK(ModeOps<T>::gemm(h, h->A1.p, H, h->dec, epi(EPI_STORE, R, s.W, h->dec.b, h->V.p, s.W, 1), ks, st));
   return 0;
 }
 
 template <typename T>
-static int launch_combine(FmtHandle* h, int mode, float* dst, const float* dt_ptr, cudaStream_t st) {
-  const ModelShape& s = h->shape;
+static int launch_combine(FmtHandle* h, const ModelShape& s, int mode, float* dst, const float* dt_ptr, cudaStream_t st) {
   const size_t n = static_cast<size_t>(s.B) * s.N * s.W;
   return launch(h, cfg_combine_kernel<T>, dim3(static_cast<unsigned>((n + 255) / 256)), dim3(256), 0, st, 1,
                 static_cast<const WindowArgs*>(h->wargs.p), s, static_cast<const float*>(h->V.p), mode, dst, dt_ptr, static_cast<T*>(h->ax.p));
@@ -870,8 +925,8 @@ static int launch_flow(FmtHandle* h, cudaStream_t st, bool probe_only = false) {
 
 // The whole window: prepare -> tables -> S steps x stages -> finalize.  This is what gets captured in the graph.
 template <typename T>
-static int enqueue_window(FmtHandle* h, cudaStream_t st) {
-  const ModelShape& s = h->shape;
+static int enqueue_window(FmtHandle* h, const GraphShape& gs, cudaStream_t st) {
+  const ModelShape& s = gs.s;
   const WindowArgs* wa = static_cast<const WindowArgs*>(h->wargs.p);
   const size_t nx = static_cast<size_t>(s.B) * s.L * s.W, nfull = static_cast<size_t>(s.B) * s.N * s.W;
   float* x_state = static_cast<float*>(h->xstate.p);
@@ -881,14 +936,14 @@ static int enqueue_window(FmtHandle* h, cudaStream_t st) {
   const float* ddt = static_cast<const float*>(h->ddt.p);
   const int S = h->plan.n_steps, G = h->plan.n_stages;
   const dim3 gx(static_cast<unsigned>((nx + 255) / 256)), blk(256);
-  const CondRows r = plan_rows(h);
+  const int chunk = gs.rows.chunk;
 
   FMT_OK(launch(h, init_window_kernel<T>, dim3(static_cast<unsigned>((nfull + 255) / 256)), blk, 0, st, 1, wa, s, x_state,
                 static_cast<float*>(h->prevx.p), ax));
-  if (S > 0) FMT_OK(enqueue_prepare<T>(h, r, st));
+  if (S > 0) FMT_OK(enqueue_prepare<T>(h, gs, st));
   if (h->window_active && S > 0) {
     // small-R plan: every evaluation of the window runs inside ONE persistent kernel (flow.cuh; window.cuh with FMT_WINDOW=1/2)
-    FMT_OK(enqueue_tables<T>(h, r, 0, h->n_eval, st));
+    FMT_OK(enqueue_tables<T>(h, gs, 0, h->n_eval, st));
     if (h->flow_active) FMT_OK(launch_flow(h, st));
     else FMT_OK(launch_window(h, st));
     FMT_OK(launch(h, finalize_window_kernel, gx, blk, 0, st, 1, wa, s, static_cast<const float*>(x_state), static_cast<float*>(h->prevx.p)));
@@ -897,18 +952,18 @@ static int enqueue_window(FmtHandle* h, cudaStream_t st) {
   for (int step = 0; step < S; ++step) {
     for (int g = 0; g < G; ++g) {
       const int e = step * G + g;
-      if (e % h->table_chunk == 0) {
-        const int n = (h->n_eval - e) < h->table_chunk ? (h->n_eval - e) : h->table_chunk;
-        FMT_OK(enqueue_tables<T>(h, r, e, n, st));
+      if (e % chunk == 0) {
+        const int n = (h->n_eval - e) < chunk ? (h->n_eval - e) : chunk;
+        FMT_OK(enqueue_tables<T>(h, gs, e, n, st));
       }
       if (g > 0) {   // y_g = y0 + dt * sum_j a[g][j] k_j  (also refreshes the x-embedder operand)
         const float* a = &h->rk_a[g * G];
         FMT_OK(launch(h, rk_combine_kernel<T>, gx, blk, 0, st, 1, s, static_cast<const float*>(x_state), y_stage, static_cast<const float*>(kbuf), nx, nx, g,
                       a[0], G > 1 ? a[1] : 0.f, G > 2 ? a[2] : 0.f, G > 3 ? a[3] : 0.f, ddt + step, ax));
       }
-      FMT_OK(enqueue_forward<T>(h, r, e % h->table_chunk, st));
-      if (G == 1) FMT_OK(launch_combine<T>(h, 2, x_state, ddt + step, st));           // fused CFG + Euler
-      else FMT_OK(launch_combine<T>(h, 1, kbuf + static_cast<size_t>(g) * nx, nullptr, st));
+      FMT_OK(enqueue_forward<T>(h, gs, e % chunk, st));
+      if (G == 1) FMT_OK(launch_combine<T>(h, s, 2, x_state, ddt + step, st));           // fused CFG + Euler
+      else FMT_OK(launch_combine<T>(h, s, 1, kbuf + static_cast<size_t>(g) * nx, nullptr, st));
     }
     if (G > 1) {
       const float* b = h->rk_b.data();
@@ -920,53 +975,64 @@ static int enqueue_window(FmtHandle* h, cudaStream_t st) {
   return 0;
 }
 
-static int enqueue_window_mode(FmtHandle* h, cudaStream_t st) {
+static int enqueue_window_mode(FmtHandle* h, const GraphShape& gs, cudaStream_t st) {
   switch (h->plan.mode) {
-    case FMT_MODE_BF16: return enqueue_window<bf16>(h, st);
-    case FMT_MODE_BF16X3: return enqueue_window<bf16x3_t>(h, st);
+    case FMT_MODE_BF16: return enqueue_window<bf16>(h, gs, st);
+    case FMT_MODE_BF16X3: return enqueue_window<bf16x3_t>(h, gs, st);
   }
-  return enqueue_window<float>(h, st);
+  return enqueue_window<float>(h, gs, st);
 }
 
 // The per-slot window graph: the plan's evaluation count, every slot on its own schedule (SlotOde), always one kernel per op.  Each
 // evaluation e is [the stage combine of the slots at a stage > 0 (e > 0)] -> forward -> [CFG combine + the ODE update of each slot
 // that is at an evaluation of its own].
 template <typename T>
-static int enqueue_window_ode(FmtHandle* h, cudaStream_t st) {
-  const ModelShape& s = h->shape;
+static int enqueue_window_ode(FmtHandle* h, const GraphShape& gs, cudaStream_t st) {
+  const ModelShape& s = gs.s;
   const WindowArgs* wa = static_cast<const WindowArgs*>(h->wargs.p);
   const size_t nx = static_cast<size_t>(s.B) * s.L * s.W, nfull = static_cast<size_t>(s.B) * s.N * s.W;
   float* x_state = static_cast<float*>(h->xstate.p);
   float* kbuf = static_cast<float*>(h->s_kbuf.p);
   T* ax = static_cast<T*>(h->ax.p);
   const dim3 gx(static_cast<unsigned>((nx + 255) / 256)), gfull(static_cast<unsigned>((nfull + 255) / 256)), blk(256);
-  const CondRows r = ode_rows(h);
+  const CondRows& r = gs.rows;
   const int ne = h->n_eval;
 
   FMT_OK(launch(h, init_window_kernel<T>, gfull, blk, 0, st, 1, wa, s, x_state, static_cast<float*>(h->prevx.p), ax));
-  if (ne > 0) FMT_OK(enqueue_prepare<T>(h, r, st));
+  if (ne > 0) FMT_OK(enqueue_prepare<T>(h, gs, st));
   for (int e = 0; e < ne; ++e) {
-    if (e % r.chunk == 0) FMT_OK(enqueue_tables<T>(h, r, e, std::min(ne - e, r.chunk), st));
+    if (e % r.chunk == 0) FMT_OK(enqueue_tables<T>(h, gs, e, std::min(ne - e, r.chunk), st));
     if (e > 0)
       FMT_OK(launch(h, sched_stage_kernel<T>, gx, blk, 0, st, 1, wa, s, static_cast<const float*>(x_state), static_cast<float*>(h->ystage.p),
                     static_cast<const float*>(kbuf), nx, e, ax));
-    FMT_OK(enqueue_forward<T>(h, r, e % r.chunk, st));
+    FMT_OK(enqueue_forward<T>(h, gs, e % r.chunk, st));
     FMT_OK(launch(h, sched_combine_kernel<T>, gfull, blk, 0, st, 1, wa, s, static_cast<const float*>(h->V.p), e, x_state, kbuf, nx, ax));
   }
   FMT_OK(launch(h, finalize_window_kernel, gx, blk, 0, st, 1, wa, s, static_cast<const float*>(x_state), static_cast<float*>(h->prevx.p)));
   return 0;
 }
 
-static int enqueue_window_ode_mode(FmtHandle* h, cudaStream_t st) {
+static int enqueue_window_ode_mode(FmtHandle* h, const GraphShape& gs, cudaStream_t st) {
   switch (h->plan.mode) {
-    case FMT_MODE_BF16: return enqueue_window_ode<bf16>(h, st);
-    case FMT_MODE_BF16X3: return enqueue_window_ode<bf16x3_t>(h, st);
+    case FMT_MODE_BF16: return enqueue_window_ode<bf16>(h, gs, st);
+    case FMT_MODE_BF16X3: return enqueue_window_ode<bf16x3_t>(h, gs, st);
   }
-  return enqueue_window_ode<float>(h, st);
+  return enqueue_window_ode<float>(h, gs, st);
 }
 
-// Captures one window of enqueue(h, .) as a CUDA graph; *launches: the kernels it holds (counted by launch())
-static int capture_window(FmtHandle* h, int (*enqueue)(FmtHandle*, cudaStream_t), cudaGraphExec_t* exec, int* nodes, long long* launches) {
+// Destroys the occupancy buckets' graphs and maps (the caller has synchronised the stream that replays them)
+static void drop_buckets(FmtHandle* h) {
+  for (FmtHandle::Bucket& b : h->buckets) {
+    if (b.exec) cudaGraphExecDestroy(b.exec);
+    if (b.ode_exec) cudaGraphExecDestroy(b.ode_exec);
+    if (b.s_map.p) { cudaFree(b.s_map.p); h->ws_bytes -= b.s_map.bytes; }
+  }
+  h->buckets.clear();
+}
+
+// Captures one window of enqueue(h, gs, .) as a CUDA graph; *launches: the kernels it holds (counted by launch())
+static int capture_window(FmtHandle* h, int (*enqueue)(FmtHandle*, const GraphShape&, cudaStream_t), const GraphShape& gs, cudaGraphExec_t* exec,
+                          int* nodes, long long* launches) {
   cudaGraph_t graph = nullptr;
   cudaStream_t cs;
   CUDA_OK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
@@ -974,7 +1040,7 @@ static int capture_window(FmtHandle* h, int (*enqueue)(FmtHandle*, cudaStream_t)
   CUDA_OK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
   const long long outer = h->capture_launches;
   h->capturing = true; h->capture_launches = 0;
-  int rc = enqueue(h, cs);
+  int rc = enqueue(h, gs, cs);
   h->capturing = false;
   const long long counted = h->capture_launches;
   h->capture_launches = outer;
@@ -1180,13 +1246,14 @@ int32_t fmt_destroy(FmtHandle* h) {
   cudaDeviceSynchronize();
   if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
   if (h->ode_exec) cudaGraphExecDestroy(h->ode_exec);
+  drop_buckets(h);
   for (void* p : h->owned) cudaFree(p);
   for (auto& kv : h->ode_cache) cudaFree(kv.second.p);
   DevBuf* bufs[] = {&h->cond, &h->cemb, &h->temb, &h->tfreq, &h->th, &h->silu, &h->table, &h->xstate, &h->ystage, &h->kbuf, &h->prevx, &h->ax,
                     &h->X, &h->A1, &h->QKV, &h->A2, &h->Hm, &h->V, &h->ddt, &h->dteval, &h->wargs, &h->st_rs, &h->st_wa, &h->st_we, &h->st_noise, &h->st_rd, &h->ev_wa, &h->ev_we,
                     &h->win_params, &h->win_tmaps, &h->win_acc, &h->win_bar, &h->win_trace, &h->win_act,
                     &h->flow_gemms, &h->flow_tmaps, &h->flow_acc, &h->flow_act, &h->flow_flags, &h->flow_trace, &h->urow_buf, &h->uidx_buf,
-                    &h->slot_buf, &h->slot_zero, &h->s_cond, &h->s_cemb, &h->s_urow, &h->s_uidx, &h->s_kbuf};
+                    &h->slot_buf, &h->slot_zero, &h->s_cond, &h->s_cemb, &h->s_urow, &h->s_uidx, &h->s_kbuf, &h->bucket_maps};
   for (DevBuf* b : bufs)
     if (b->p) cudaFree(b->p);
   if (h->win_err_host) cudaFreeHost(h->win_err_host);
@@ -1205,6 +1272,7 @@ int64_t fmt_launch_count(const FmtHandle* hc, int32_t reset) {
   return v;
 }
 int32_t fmt_graph_kernel_nodes(const FmtHandle* h) { return h ? h->graph_nodes : 0; }
+int32_t fmt_last_window_slots(const FmtHandle* h) { return h ? h->last_slots : 0; }
 int32_t fmt_ode_graph_kernel_nodes(const FmtHandle* h) { return h ? h->ode_nodes : 0; }
 int64_t fmt_debug_window_trace(const FmtHandle* h, int64_t* out, int64_t max_elems) {
   if (h && h->flow_active && h->flow_trace.p) {   // dataflow kernel: [cta][engine][stage][chunk][4] SM-clock stamps
@@ -1322,6 +1390,13 @@ static int clip_schedule(int n, const int32_t* n_win, int n_slots, int32_t* slot
   return S;
 }
 
+int32_t fmt_occupancy_slots(int32_t plan_slots, int32_t n_ready) {
+  if (plan_slots < 1 || plan_slots > kMaxSlots || n_ready < 1 || n_ready > plan_slots) return -1;
+  int b = 1;
+  while (b < n_ready) b *= 2;
+  return b < plan_slots ? b : plan_slots;
+}
+
 int32_t fmt_clip_schedule(int32_t n_clips, const int32_t* n_windows, int32_t n_slots, int32_t* slot_out, int32_t* start_out, int32_t* makespan_out) {
   if (n_clips < 1 || n_windows == nullptr || n_slots < 0 || n_slots > kMaxSlots) return -1;
   for (int i = 0; i < n_clips; ++i)
@@ -1334,6 +1409,37 @@ int32_t fmt_clip_schedule(int32_t n_clips, const int32_t* n_windows, int32_t n_s
 
 // we_dynamic takes no part: no graph, table or buffer depends on it (each slot record carries its clip's emotion mode, and the
 // condition-row map is the same for every mode, distinct_condition_rows), so a plan that differs only in it is the same plan.
+// The occupancy buckets of a plan that runs one kernel per op: 1, 2, 4, ... slots below plan.batch, with the condition-row map of
+// each (the plan's deduplication on its first B slots), uploaded here in one copy.  Their graphs are captured on first use.
+static int make_buckets(FmtHandle* h, cudaStream_t st) {
+  if (h->window_active) return 0;
+  const ModelShape& s = h->shape;
+  std::vector<int> maps;
+  for (int B = 1; B < s.B; B *= 2) {
+    FmtHandle::Bucket b;
+    b.B = B;
+    b.U = s.nb * B * s.N;
+    if (h->dedup) {
+      ModelShape sb = s;
+      sb.B = B;
+      std::vector<int> urow, uidx;
+      const std::vector<int32_t> modes(B, h->plan.we_dynamic);
+      distinct_condition_rows(sb, modes.data(), urow, uidx);
+      b.U = static_cast<int>(uidx.size());
+      b.map_off = maps.size();
+      maps.insert(maps.end(), urow.begin(), urow.end());
+      maps.insert(maps.end(), uidx.begin(), uidx.end());
+    }
+    h->buckets.push_back(b);
+  }
+  if (!maps.empty()) {
+    FMT_OK(dev_alloc(h, h->bucket_maps, maps.size() * sizeof(int)));
+    CUDA_OK(cudaMemcpyAsync(h->bucket_maps.p, maps.data(), maps.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    CUDA_OK(cudaStreamSynchronize(st));          // `maps` is a stack object
+  }
+  return 0;
+}
+
 static bool same_plan(const FmtHandle* h, const FmtPlan* p) {
   if (!h->configured) return false;
   const FmtPlan& q = h->plan;
@@ -1371,7 +1477,10 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
   const int ne = p->n_steps * p->n_stages;
   h->configured = false;
   if (h->graph_exec) { CUDA_OK(cudaStreamSynchronize(st)); cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; h->graph_nodes = 0; }
-  if (h->ode_exec) { CUDA_OK(cudaStreamSynchronize(st)); cudaGraphExecDestroy(h->ode_exec); h->ode_exec = nullptr; h->ode_nodes = 0; }
+  if (h->ode_exec) { CUDA_OK(cudaStreamSynchronize(st)); cudaGraphExecDestroy(h->ode_exec); h->ode_exec = nullptr; }
+  if (!h->buckets.empty()) { CUDA_OK(cudaStreamSynchronize(st)); drop_buckets(h); }
+  h->ode_nodes = 0;
+  h->s_chunk = 0;                                // the per-slot graph's condition rows are built again on first use
   h->plan = *p;
   h->t_eval.assign(p->t_eval, p->t_eval + ne);
   h->dt.assign(p->dt, p->dt + p->n_steps);
@@ -1499,7 +1608,10 @@ int32_t fmt_configure(FmtHandle* h, const FmtPlan* p, void* stream) {
   if (h->window_active && !h->flow_active) FMT_OK(setup_window(h, st));
 
   // capture one window as a CUDA graph
-  FMT_OK(capture_window(h, enqueue_window_mode, &h->graph_exec, &h->graph_nodes, &h->capture_launches));
+  h->ksliced = false;
+  FMT_OK(capture_window(h, enqueue_window_mode, plan_graph(h), &h->graph_exec, &h->graph_nodes, &h->capture_launches));
+  h->plan_ksliced = h->ksliced;
+  FMT_OK(make_buckets(h, st));
   h->configured = true;
   return 0;
 }
@@ -1512,10 +1624,10 @@ static int set_wargs(FmtHandle* h, const WindowArgs& a, cudaStream_t st) {
 
 // Slot records of one call (every sampling entry point and fmt_velocity) go up in ONE copy from a pinned staging buffer that the handle
 // owns; slot_ev marks the end of the previous call's copy, so the staging buffer is refilled only once that copy has read it.
-// stage_slot_records fills the staging buffer with n_win windows of idle records: zero inputs ((L, W) noise, and r_s / wa / we rows
-// no wider than that), no output, no context, static emotion, scales of 1 and the plan's branch count; with ode, B SlotOde follow the B SlotArgs of
-// each window, idle as well (no evaluation).
-static int stage_slot_records(FmtHandle* h, size_t n_win, bool ode, cudaStream_t st) {
+// stage_slot_records fills the staging buffer with n_win windows of `slots` idle records each (the slots of the window graph the call
+// replays): zero inputs ((L, W) noise, and r_s / wa / we rows no wider than that), no output, no context, static emotion, scales of 1
+// and the plan's branch count; with ode, `slots` SlotOde follow the SlotArgs of each window, idle as well (no evaluation).
+static int stage_slot_records(FmtHandle* h, size_t n_win, bool ode, int slots, cudaStream_t st) {
   const ModelShape& s = h->shape;
   if (!h->slot_zero.p) {   // its size depends on the model's dims alone, and no kernel writes it: zeroed once per handle
     const size_t n_zero = std::max<size_t>(static_cast<size_t>(s.L) * s.W, static_cast<size_t>(std::max(s.A, s.E)));
@@ -1524,7 +1636,8 @@ static int stage_slot_records(FmtHandle* h, size_t n_win, bool ode, cudaStream_t
   }
   const float* zero = static_cast<const float*>(h->slot_zero.p);
   if (h->slot_ev) CUDA_OK(cudaEventSynchronize(h->slot_ev));
-  h->slot_stride = static_cast<size_t>(s.B) * (sizeof(SlotArgs) + (ode ? sizeof(SlotOde) : 0));
+  h->slot_recs = slots;
+  h->slot_stride = static_cast<size_t>(slots) * (sizeof(SlotArgs) + (ode ? sizeof(SlotOde) : 0));
   const size_t bytes = n_win * h->slot_stride;
   if (h->slot_host_bytes < bytes) {
     if (h->slot_host) { CUDA_OK(cudaFreeHost(h->slot_host)); h->slot_host = nullptr; h->slot_host_bytes = 0; }
@@ -1533,15 +1646,15 @@ static int stage_slot_records(FmtHandle* h, size_t n_win, bool ode, cudaStream_t
   }
   for (size_t w = 0; w < n_win; ++w) {
     SlotArgs* rec = reinterpret_cast<SlotArgs*>(h->slot_host + w * h->slot_stride);
-    for (int k = 0; k < s.B; ++k) {
+    for (int k = 0; k < slots; ++k) {
       SlotArgs& z = rec[k];
       z.r_s = zero; z.wa = zero; z.we = zero; z.x0 = zero; z.r_d = nullptr; z.ctx = nullptr;
       z.T_wa = 1; z.T_we = 1; z.T_out = 0; z.win_start = 0; z.out_start = 0; z.first_window = 1;
       z.a_scale = z.r_scale = z.e_scale = 1.f; z.n_branches = s.nb; z.we_dynamic = 0;
     }
     if (!ode) continue;
-    SlotOde* od = reinterpret_cast<SlotOde*>(rec + s.B);
-    for (int k = 0; k < s.B; ++k) {
+    SlotOde* od = reinterpret_cast<SlotOde*>(rec + slots);
+    for (int k = 0; k < slots; ++k) {
       SlotOde& o = od[k];
       o = SlotOde{};
       o.temb = static_cast<const float*>(h->temb.p); o.dt = static_cast<const float*>(h->ddt.p); o.n_eval = 0; o.n_stages = 1;
@@ -1552,7 +1665,7 @@ static int stage_slot_records(FmtHandle* h, size_t n_win, bool ode, cudaStream_t
 
 // window w's SlotArgs / SlotOde in the staging buffer, and its SlotArgs on the device after upload_slot_records
 static SlotArgs* staged_args(FmtHandle* h, size_t w) { return reinterpret_cast<SlotArgs*>(h->slot_host + w * h->slot_stride); }
-static SlotOde* staged_ode(FmtHandle* h, size_t w) { return reinterpret_cast<SlotOde*>(staged_args(h, w) + h->shape.B); }
+static SlotOde* staged_ode(FmtHandle* h, size_t w) { return reinterpret_cast<SlotOde*>(staged_args(h, w) + h->slot_recs); }
 static const SlotArgs* device_args(const FmtHandle* h, size_t w) {
   return reinterpret_cast<const SlotArgs*>(static_cast<const unsigned char*>(h->slot_buf.p) + w * h->slot_stride);
 }
@@ -1626,8 +1739,8 @@ static int slot_ode(FmtHandle* h, const FmtClipOde* ode, int i, cudaStream_t st,
 // The per-slot window graph of the current plan, captured on first use: its distinct condition rows (the plan's deduplication with
 // no row shared between slots), their buffers, and a kbuf of FMT_MAX_STAGES stages.  The AdaLN tables go to the plan's table buffer,
 // as many evaluations at a time as it holds.
-static int ensure_ode_graph(FmtHandle* h, cudaStream_t st) {
-  if (h->ode_exec) return 0;
+static int ensure_ode_rows(FmtHandle* h, cudaStream_t st) {
+  if (h->s_chunk > 0) return 0;
   const ModelShape& s = h->shape;
   h->sU = h->R;
   h->s_dedup = false;
@@ -1653,7 +1766,64 @@ static int ensure_ode_graph(FmtHandle* h, cudaStream_t st) {
   FMT_OK(dev_alloc(h, h->s_cond, U * s.Kc * ts));
   FMT_OK(dev_alloc(h, h->s_cemb, U * s.H * 4));
   FMT_OK(dev_alloc(h, h->s_kbuf, nx * 4 * FMT_MAX_STAGES));
-  return capture_window(h, enqueue_window_ode_mode, &h->ode_exec, &h->ode_nodes, &h->ode_launches);
+  return 0;
+}
+
+static int ensure_ode_graph(FmtHandle* h, cudaStream_t st) {
+  if (h->ode_exec) return 0;
+  FMT_OK(ensure_ode_rows(h, st));
+  return capture_window(h, enqueue_window_ode_mode, plan_graph(h, true), &h->ode_exec, &h->ode_nodes, &h->ode_launches);
+}
+
+// ---- occupancy buckets
+// A bucket's graphs: the plan's GraphShape on its first B slots, with the bucket's condition-row map in the plan's buffers
+static GraphShape bucket_graph(const FmtHandle* h, const FmtHandle::Bucket& b, bool ode) {
+  GraphShape g = plan_graph(h, ode);
+  g.s.B = b.B;
+  g.R = g.s.nb * b.B * g.s.N;
+  g.ksplit = h->plan_ksliced;
+  CondRows& r = g.rows;
+  r.U = ode ? b.sU : b.U;
+  const int* map = ode ? (h->s_dedup ? static_cast<const int*>(b.s_map.p) : nullptr)
+                       : (h->dedup ? static_cast<const int*>(h->bucket_maps.p) + b.map_off : nullptr);
+  r.urow = map;
+  r.uidx = map ? map + g.R : nullptr;
+  return g;
+}
+
+// Bucket b's window graph (ode: its per-slot window graph), captured the first time a step needs it.  It holds the kernels of the
+// plan's graph of the same kind, one for one.
+static int ensure_bucket_graph(FmtHandle* h, FmtHandle::Bucket& b, bool ode, cudaStream_t st) {
+  if (ode ? b.ode_exec != nullptr : b.exec != nullptr) return 0;
+  if (ode) {
+    FMT_OK(ensure_ode_rows(h, st));
+    const ModelShape& s = h->shape;
+    b.sU = s.nb * b.B * s.N;
+    if (h->s_dedup) {   // the plan's per-slot graph shares no row between slots, so neither does the bucket's
+      ModelShape sb = s;
+      sb.B = b.B;
+      std::vector<int> urow, uidx;
+      const std::vector<int32_t> modes(b.B, h->plan.we_dynamic);
+      distinct_condition_rows(sb, modes.data(), urow, uidx, true);
+      b.sU = static_cast<int>(uidx.size());
+      urow.insert(urow.end(), uidx.begin(), uidx.end());
+      FMT_OK(dev_alloc(h, b.s_map, urow.size() * sizeof(int)));
+      CUDA_OK(cudaMemcpyAsync(b.s_map.p, urow.data(), urow.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+      CUDA_OK(cudaStreamSynchronize(st));      // `urow` is a stack object
+    }
+  }
+  cudaGraphExec_t exec = nullptr;
+  int nodes = 0;
+  long long launches = 0;
+  FMT_OK(capture_window(h, ode ? enqueue_window_ode_mode : enqueue_window_mode, bucket_graph(h, b, ode), &exec, &nodes, &launches));
+  if (ode && h->ode_nodes == 0) h->ode_nodes = nodes;   // every bucket's per-slot graph has the same kernels
+  if (nodes != (ode ? h->ode_nodes : h->graph_nodes)) {
+    cudaGraphExecDestroy(exec);
+    return set_err(-2, "occupancy bucket of %d slots: its graph has %d nodes, the plan's %d", b.B, nodes, ode ? h->ode_nodes : h->graph_nodes);
+  }
+  (ode ? b.ode_exec : b.exec) = exec;
+  (ode ? b.ode_launches : b.launches) = launches;
+  return 0;
 }
 
 // One clip as its slot records see it: tensors of that clip alone (batch 1), the noise of its window w at noise + w * noise_stride,
@@ -1690,7 +1860,7 @@ static int check_clip(const ModelShape& s, const ClipIn& c, const char* who, int
 static int stage_clips(FmtHandle* h, const std::vector<ClipIn>& c, const int32_t* slot, const int32_t* start, int makespan,
                        const std::vector<SlotOde>& od, cudaStream_t st) {
   const ModelShape& s = h->shape;
-  FMT_OK(stage_slot_records(h, makespan, !od.empty(), st));
+  FMT_OK(stage_slot_records(h, makespan, !od.empty(), s.B, st));
   for (size_t i = 0; i < c.size(); ++i) {
     const int n_win = (c[i].T + s.L - 1) / s.L;
     for (int w = 0; w < n_win; ++w) {
@@ -1708,13 +1878,18 @@ static int stage_clips(FmtHandle* h, const std::vector<ClipIn>& c, const int32_t
 }
 
 // Uploads the staged records of n_win windows and replays a window graph once per window: the plan's, or with ode the per-slot one
-static int replay_windows(FmtHandle* h, int n_win, bool ode, fmt_progress_fn progress, void* progress_user, cudaStream_t st) {
+// (bk: those of an occupancy bucket)
+static int replay_windows(FmtHandle* h, int n_win, bool ode, fmt_progress_fn progress, void* progress_user, cudaStream_t st,
+                          const FmtHandle::Bucket* bk = nullptr) {
+  cudaGraphExec_t exec = bk ? (ode ? bk->ode_exec : bk->exec) : (ode ? h->ode_exec : h->graph_exec);
+  const long long n_launch = bk ? (ode ? bk->ode_launches : bk->launches) : (ode ? h->ode_launches : h->capture_launches);
   FMT_OK(upload_slot_records(h, n_win, st));
   h->last_ode = ode;
+  h->last_slots = bk ? bk->B : h->shape.B;
   for (int w = 0; w < n_win; ++w) {
     FMT_OK(set_wargs(h, WindowArgs{device_args(h, w)}, st));
-    CUDA_OK(cudaGraphLaunch(ode ? h->ode_exec : h->graph_exec, st));
-    h->launches += ode ? h->ode_launches : h->capture_launches;
+    CUDA_OK(cudaGraphLaunch(exec, st));
+    h->launches += n_launch;
     if (progress) progress(w, n_win, progress_user);
   }
   return 0;
@@ -1815,8 +1990,9 @@ int32_t fmt_sample_clips_ode(FmtHandle* h, const FmtClipSet* cs, const FmtClipGu
   return fmt_sample_clip_set(h, cs, g, ode, nullptr, stream);
 }
 
-// One window of each of n streams, stream i in slot i, through the plan's captured window graph (ode != nullptr: each stream on its
-// own schedule, through the per-slot window graph); slots n.. are idle.  A stream's context lives in its own ctx buffer, not in the
+// One window of each of n streams, stream i in slot i, through the captured window graph of fmt_occupancy_slots(batch, n) slots (ode !=
+// nullptr: each stream on its own schedule, through the per-slot window graph of those slots); its slots n.. are idle.  A plan whose
+// window graph is a persistent kernel replays its one graph of batch slots.  A stream's context lives in its own ctx buffer, not in the
 // handle, so a stream may run in any slot and the plan may be replaced between calls.  Its wa / we start at the window's first
 // context frame (P frames before its first current frame), or at its first current frame in a first window; its output is the
 // window alone.  we_dyn == nullptr: plan.we_dynamic for every stream.
@@ -1852,8 +2028,16 @@ int32_t fmt_sample_window_set(FmtHandle* h, const FmtWindowSet* ws, const FmtCli
   if (ode) FMT_OK(check_odes(h, ode, n, "fmt_sample_windows_ode: stream"));
   std::vector<SlotOde> od(ode ? n : 0);
   for (int i = 0; i < static_cast<int>(od.size()); ++i) FMT_OK(slot_ode(h, ode, i, st, &od[i]));
-  if (ode) FMT_OK(ensure_ode_graph(h, st));
-  FMT_OK(stage_slot_records(h, 1, ode != nullptr, st));
+  // the graphs of the occupancy bucket of n streams; a plan whose window graph is a persistent kernel has no buckets
+  const int slots = h->buckets.empty() ? s.B : fmt_occupancy_slots(s.B, n);
+  FmtHandle::Bucket* bk = nullptr;
+  if (slots < s.B) {
+    bk = &h->buckets[__builtin_ctz(static_cast<unsigned>(slots))];   // bucket i holds 2^i slots
+    FMT_OK(ensure_bucket_graph(h, *bk, ode != nullptr, st));
+  } else if (ode) {
+    FMT_OK(ensure_ode_graph(h, st));
+  }
+  FMT_OK(stage_slot_records(h, 1, ode != nullptr, slots, st));
   for (int i = 0; i < n; ++i) {
     if (ode) staged_ode(h, 0)[i] = od[i];
     SlotArgs& z = staged_args(h, 0)[i];
@@ -1864,7 +2048,7 @@ int32_t fmt_sample_window_set(FmtHandle* h, const FmtWindowSet* ws, const FmtCli
     z.a_scale = g->a_cfg_scale[i]; z.r_scale = g->r_cfg_scale[i]; z.e_scale = g->e_cfg_scale[i]; z.n_branches = g->n_branches[i];
     z.we_dynamic = we_dyn ? we_dyn[i] : h->plan.we_dynamic;
   }
-  return replay_windows(h, 1, ode != nullptr, nullptr, nullptr, st);
+  return replay_windows(h, 1, ode != nullptr, nullptr, nullptr, st, bk);
 }
 
 int32_t fmt_sample_windows(FmtHandle* h, const FmtWindowSet* ws, const FmtClipGuidance* g, void* stream) {
@@ -1891,15 +2075,15 @@ static int join_context(FmtHandle* h, DevBuf& dst, const float* prev, const floa
 template <typename T>
 static int enqueue_velocity(FmtHandle* h, const FmtEval* ev, cudaStream_t st) {
   const ModelShape& s = h->shape;
-  const CondRows r = plan_rows(h);
-  FMT_OK(enqueue_prepare<T>(h, r, st));
-  FMT_OK(enqueue_tables<T>(h, r, ev->eval_index, 1, st));
+  const GraphShape g = plan_graph(h);
+  FMT_OK(enqueue_prepare<T>(h, g, st));
+  FMT_OK(enqueue_tables<T>(h, g, ev->eval_index, 1, st));
   const size_t nfull = static_cast<size_t>(s.B) * s.N * s.W;
   FMT_OK(launch(h, init_window_kernel<T>, dim3(static_cast<unsigned>((nfull + 255) / 256)), dim3(256), 0, st, 1,
                 static_cast<const WindowArgs*>(h->wargs.p), s, static_cast<float*>(h->xstate.p), static_cast<float*>(h->prevx.p),
                 static_cast<T*>(h->ax.p)));
-  FMT_OK(enqueue_forward<T>(h, r, 0, st));
-  FMT_OK(launch_combine<T>(h, 0, ev->v_out, nullptr, st));
+  FMT_OK(enqueue_forward<T>(h, g, 0, st));
+  FMT_OK(launch_combine<T>(h, s, 0, ev->v_out, nullptr, st));
   return 0;
 }
 
@@ -1920,7 +2104,7 @@ int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream) {
   FMT_OK(join_context(h, h->ev_wa, ev->prev_wa, ev->wa, s.A, st));
   const int dyn = h->plan.we_dynamic;
   if (dyn) FMT_OK(join_context(h, h->ev_we, ev->prev_we, ev->we, s.E, st));
-  FMT_OK(stage_slot_records(h, 1, false, st));
+  FMT_OK(stage_slot_records(h, 1, false, s.B, st));
   for (int b = 0; b < s.B; ++b) {
     SlotArgs& z = staged_args(h, 0)[b];
     z.r_s = ev->r_s + static_cast<size_t>(b) * s.W;

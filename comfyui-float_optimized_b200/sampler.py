@@ -228,6 +228,11 @@ class FmtBackend:
         """Kernels of the per-slot window graph that calls with per-clip schedules run (0 before the first on this plan)."""
         return int(self.lib.fmt_ode_graph_kernel_nodes(self._handle))
 
+    def last_window_slots(self) -> int:
+        """Slots of the window graph the last sampling call replayed: :func:`occupancy_slots` of the plan's slots and the streams of
+        the last :meth:`sample_windows`, or the plan's slots (0 before the first call)."""
+        return int(self.lib.fmt_last_window_slots(self._handle))
+
     @staticmethod
     def _clip_ode(schedules, n: int):
         """FmtClipOde of n (nfe, method) pairs, and the ctypes arrays it points into (keep them alive for the call)."""
@@ -576,6 +581,19 @@ def clip_schedule(n_windows: Sequence[int], n_slots: int = 0) -> ClipSchedule:
     return ClipSchedule(S, tuple(slot[:n]), tuple(start[:n]), makespan.value)
 
 
+def occupancy_slots(slots: int, n_ready: int) -> int:
+    """Slots of the window graph a :class:`StreamSampler` step with ``n_ready`` ready streams runs on a sampler of ``slots`` slots: the
+    smallest of 1, 2, 4, ... (the powers of two below ``slots``) and ``slots`` that is >= ``n_ready`` (``fmt_occupancy_slots``,
+    host-only).  Raises ValueError unless 1 <= n_ready <= slots <= 256."""
+    for name, v in (("slots", slots), ("n_ready", n_ready)):
+        if isinstance(v, bool) or not isinstance(v, numbers.Integral):
+            raise ValueError(f"{name} must be an int (got {v!r})")
+    k = _cabi.load_library().fmt_occupancy_slots(int(slots), int(n_ready))
+    if k < 0:
+        raise ValueError(f"occupancy_slots: need 1 <= n_ready <= slots <= 256 (got slots={slots}, n_ready={n_ready})")
+    return k
+
+
 def clip_noise(seed: int, dims: Dims, n_windows: int, device) -> torch.Tensor:
     """(n_windows, 1, L, dim_w): the x0 of every window of one clip drawn from its own seed - what the VA node draws for a batch of
     one clip with ``fix_noise_seed`` (a ``torch.Generator`` on the target device, nodes_vadv.py:673-689)."""
@@ -753,8 +771,11 @@ class StreamSampler:
     several windows ready makes them ready at once); ties go in open order.  A stream's frames
     are what :func:`sample_clips` gives for the whole clip (same noise, same guidance, same plan), however the audio was cut.
 
-    The plan (slot count, nfe, solver, precision, and the branch count of the keyword guidance) is fixed at construction, so steps
-    replay one captured window graph.  A stream may override the four guidance keywords in :meth:`open` as a clip of
+    The plan (slot count, nfe, solver, precision, and the branch count of the keyword guidance) is fixed at construction.  A step
+    with k ready streams runs them in slots 0..k-1 of a window graph captured for :func:`occupancy_slots` ``(slots, k)`` slots - the
+    smallest power of two >= k, or ``slots`` - the first time a step needs that graph, so it costs about what a sampler of that many
+    slots costs; its idle slots run on zeros.  A stream's frames are the same bits at every occupancy.  Plans whose window graph is
+    the persistent window kernel (at most 256 token rows) run their one graph of ``slots`` slots.  A stream may override the four guidance keywords in :meth:`open` as a clip of
     :func:`sample_clips` does, within the plan's branch count, ``we_dynamic`` (static or dynamic emotion) freely, and ``nfe`` and ``method`` within the plan's
     evaluations per window (:func:`n_evals` of the constructor's nfe and method); a step that runs a stream on a schedule other
     than the plan's goes through the per-slot window graph (one kernel per op).  A stream holds on the device its reference latent,

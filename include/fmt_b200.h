@@ -237,9 +237,11 @@ FMT_API int32_t fmt_sample_clips(FmtHandle* h, const FmtClipSet* set, void* stre
  * 1-branch plan gets a clip with more than one branch. */
 FMT_API int32_t fmt_sample_clips_guided(FmtHandle* h, const FmtClipSet* set, const FmtClipGuidance* guidance, void* stream);
 
-/* One window of each stream of the set, with each stream's own guidance (n_streams entries; as in fmt_sample_clips_guided), through
- * the plan's captured window graph.  A stream's window computes what the same window of fmt_sample_clips computes for the whole
- * clip.  Returns -1 on bad arguments. */
+/* One window of each stream of the set, with each stream's own guidance (n_streams entries; as in fmt_sample_clips_guided), stream i
+ * in slot i.  The call replays a window graph of fmt_occupancy_slots(plan.batch, n_streams) slots, captured the first time a call
+ * needs it (a plan whose window graph is the persistent window kernel replays its one graph of plan.batch slots).  A stream's window
+ * computes what the same window of fmt_sample_clips computes for the whole clip, bit for bit, whichever graph it runs in.  Returns -1
+ * on bad arguments. */
 FMT_API int32_t fmt_sample_windows(FmtHandle* h, const FmtWindowSet* set, const FmtClipGuidance* guidance, void* stream);
 
 /* fmt_sample_clips_guided / fmt_sample_windows with each clip / stream on its own ODE schedule (ode == NULL: exactly the call without
@@ -263,6 +265,13 @@ FMT_API int32_t fmt_sample_clip_set(FmtHandle* h, const FmtClipSet* set, const F
                                     const int32_t* we_dynamic, void* stream);
 FMT_API int32_t fmt_sample_window_set(FmtHandle* h, const FmtWindowSet* set, const FmtClipGuidance* guidance, const FmtClipOde* ode,
                                       const int32_t* we_dynamic, void* stream);
+
+/* Host-only (no device work): the slots of the window graph a call of fmt_sample_window_set with n_ready streams runs on a plan of
+ * plan_slots slots - the smallest of 1, 2, 4, ... (the powers of two below plan_slots) and plan_slots that is >= n_ready.  Returns
+ * < 0 unless 1 <= n_ready <= plan_slots <= 256. */
+FMT_API int32_t fmt_occupancy_slots(int32_t plan_slots, int32_t n_ready);
+/* Slots of the window graph the last sampling call replayed (0 before the first). */
+FMT_API int32_t fmt_last_window_slots(const FmtHandle* h);
 
 /* Single CFG-combined model evaluation (device pointers). */
 FMT_API int32_t fmt_velocity(FmtHandle* h, const FmtEval* ev, void* stream);
